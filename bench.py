@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native path tracer (contract: see the task statement / DESIGN.md).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--spp S] [--size W]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--spp S] [--size W] [--dump-outputs DIR]
 
 One "step" = one full render of the workload through the hot path:
   workload (N=1)  BASELINE.json configs[1]: Cornell box 1024x1024, 1024 spp, max depth 50
@@ -79,7 +79,42 @@ def parse():
     ap.add_argument("--ref-spp", type=int, default=1, help="samples per step of the CPU reference arm")
     ap.add_argument("--total-spp", type=int, default=4096, help="N>1: samples per pixel of the whole (fixed) job")
     ap.add_argument("--weak", action="store_true", help="N>1: weak scaling, --spp samples per rank")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the radiance sum of the last timed step to DIR/radiance_sum.npy (float32 [W*H, 4], "
+                         "NaN-poisoned channels as 0) and where they were to DIR/radiance_sum_nonfinite.npy; above %d "
+                         "MB in all a fixed, seeded sample of pixel rows" % (DUMP_LIMIT_BYTES >> 20))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+NPY_HEADER_BYTES = 4096  # upper bound of one .npy header (numpy writes 128 bytes for these shapes)
+
+
+def dump_outputs(out_dir, **arrays):
+    """Saves each array as out_dir/<name>.npy with finite values only: a non-finite entry (a NaN-poisoned pixel sum) is
+    stored as 0, as the reference's NormalizeFunctor de-NaNs it, and out_dir/<name>_nonfinite.npy holds 1 where that
+    happened (the mask does not tell NaN from inf).  The inputs of a run are fixed by its arguments (scene, camera, sample
+    range, seed offset 0), so two builds can be compared file for file.  When the files, headers included, would exceed
+    DUMP_LIMIT_BYTES in all, every file keeps the same sorted sample of rows drawn with a fixed seed: the same rows for
+    the same arguments."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    out = {}
+    for name, a in arrays.items():
+        bad = ~np.isfinite(a)
+        out[name] = np.where(bad, 0, a).astype(a.dtype)
+        out[name + "_nonfinite"] = bad.astype(a.dtype)
+    rows = {a.shape[0] for a in out.values()}.pop()  # every output has one row per pixel
+    payload = DUMP_LIMIT_BYTES - NPY_HEADER_BYTES * len(out)
+    total = sum(a.nbytes for a in out.values())
+    if total > payload:
+        keep = np.sort(np.random.default_rng(0).choice(rows, payload // (total // rows), replace=False))
+        out = {name: a[keep] for name, a in out.items()}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler(threading.Thread):
@@ -377,7 +412,9 @@ def main():
     segments_per_step = float(seg.item())
     paths_per_step = float(N) * total_spp
     value = paths_per_step * args.steps / (ms * 1e-3)
-    img_sum = color.cpu().numpy()
+    img_sum = color.cpu().numpy()  # the last timed step's radiance sum (every step clears the canvas first)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, radiance_sum=img_sum)
     # Per-launch durations for the roofline: the timed steps keep 4 sample batches in flight on 4 streams, so their
     # launches overlap and a launch's own duration cannot be read off them.  One extra render of a single batch with
     # B2PT_FLAG_NO_OVERLAP (outside the timed region, same stream, CUDA events around every launch) times the
@@ -493,4 +530,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from as it found it
     main()

@@ -1,5 +1,5 @@
-import time, sys
-sys.path.insert(0,'/root/repo')
+import os, time, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import raytracingtherestofyourlife_b200 as B
 t=time.time(); s=B.Scene.spheres(1000000); print("scene gen", time.time()-t)
 ctx=B.Context(0)
