@@ -194,8 +194,20 @@ int b2pt_primary_hits(b2pt_ctx* ctx, int32_t* primId, float* t);
  *             light at camera + 2 up,
  *   depth   = hit distance along the unit ray (VTK-m's canvas stores a projected depth; not restated),
  * and (0,0,0,0) / 0 / -1 where nothing is hit.  Host outputs W*H*4, W*H*4, W*H floats and W*H ids; any may be NULL.
- * Small scenes (kernel-parameter path) only; the Phong colour image of VTK-m's stock shader is out of scope. */
+ * Every scene: small scenes on the kernel-parameter path, larger ones (or B2PT_FLAG_FORCE_BVH) through the binary BVH
+ * the context holds, whichever builder made it; spheres are never hit.  Synchronises the stream.  The Phong colour
+ * image of VTK-m's stock shader is out of scope. */
 int b2pt_render_direct(b2pt_ctx* ctx, float* normals, float* albedo, float* depth, int32_t* primId);
+/* The same G-buffers for nViews views in one call: the camera loop of generateHemisphere / fibonacciHemisphere with
+ * -direct (main.cc:386-561).  views holds 10 floats per view as in b2pt_render_views (pos[3], lookAt[3], up[3],
+ * fovDeg); all views share W x H.  Outputs are [view][j*W+i]: normals and albedo nViews*W*H*4 floats, depth nViews*W*H
+ * floats, primId nViews*W*H ids; any may be NULL.  View v gets the bits b2pt_set_camera(view v) + b2pt_render_direct
+ * give.  A bad view fails with b2pt_set_camera's message and nothing is rendered; nViews == 0 does nothing.  Device
+ * memory is bounded: views run in chunks of whole views of at most 2^22 pixels (one view per chunk when a view is
+ * larger), each chunk one launch into library-owned staging buffers copied to its slice of the outputs.  The context's
+ * own camera and canvas are left untouched.  Synchronises the stream. */
+int b2pt_render_direct_views(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, float* normals,
+                             float* albedo, float* depth, int32_t* primId);
 /* Replaces pathtracing::Camera::CreateRays (pathtracing/Camera.cxx:880-960): one jittered primary ray
  * per pixel from the current per-pixel seeds; host outputs, any may be NULL. seedsInOut (W*H) is
  * read as the RNG state and updated (2 draws per pixel). */

@@ -87,6 +87,7 @@ SIGNATURES = {
     "b2pt_get_stage_profile": (_i32, [_vp, _i32, _vp, _vp, _vp]),
     "b2pt_primary_hits": (_i32, [_vp, _vp, _vp]),
     "b2pt_render_direct": (_i32, [_vp] * 5),
+    "b2pt_render_direct_views": (_i32, [_vp, _i32, _vp, _i32, _i32, _vp, _vp, _vp, _vp]),
     "b2pt_create_rays": (_i32, [_vp] * 9),
     "b2pt_intersect": (_i32, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _f, _f, _vp, _vp, _vp, _vp]),
     "b2pt_allreduce": (_i32, [C.POINTER(_vp), _i32]),
@@ -348,6 +349,16 @@ class Context:
         normals, albedo = np.zeros((n, 4), np.float32), np.zeros((n, 4), np.float32)
         depth, prim = np.zeros(n, np.float32), np.zeros(n, np.int32)
         _check(lib().b2pt_render_direct(self._h, _p(normals), _p(albedo), _p(depth), _p(prim)))
+        return normals, albedo, depth, prim
+
+    def render_direct_views(self, views, W, H):
+        """b2pt_render_direct_views: `views` is [nViews, 10] float32 (pos, lookAt, up, fovDeg); returns
+        (normals[V,H*W,4], albedo[V,H*W,4], depth[V,H*W], prim[V,H*W]), view v bit-identical to set_camera + render_direct."""
+        v = np.ascontiguousarray(views, np.float32).reshape(-1, 10)
+        nv, n = v.shape[0], W * H
+        normals, albedo = np.zeros((nv, n, 4), np.float32), np.zeros((nv, n, 4), np.float32)
+        depth, prim = np.zeros((nv, n), np.float32), np.zeros((nv, n), np.int32)
+        _check(lib().b2pt_render_direct_views(self._h, nv, _p(v), W, H, _p(normals), _p(albedo), _p(depth), _p(prim)))
         return normals, albedo, depth, prim
 
     def create_rays(self, seeds):

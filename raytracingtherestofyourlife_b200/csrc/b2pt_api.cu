@@ -146,6 +146,7 @@ struct b2pt_ctx
   DevBuf<int> dArrived;
   bool haveParents = false;
   DevBuf<int32_t> dSlots;
+  DevBuf<int32_t> dBinSlots; // B2PT_FLAG_WIDE_BVH: the slots in the binary tree's leaf order (direct rays walk that tree)
   DevBuf<float4> dLeafSph;
   DevBuf<B2Quad> dQuads;
   DevBuf<B2Sphere> dSph;
@@ -206,6 +207,11 @@ struct b2pt_ctx
   DevBuf<uint2> primMask;         // primary-ray specialisation: [views][tiles] candidate masks (k_primary_prep)
   DevBuf<B2PrimQuad> primQuads;   // ... and [views][B2PT_SMALL_MAX_QUADS] per-quad constants
   int64_t viewCount = 0, viewPixels = 0;
+  // -direct G-buffers (b2pt_render_direct*): per-view constants and the device staging of one chunk of views
+  DevBuf<b2pt::DirectView> dDirectViews;
+  DevBuf<float4> directNormals, directAlbedo;
+  DevBuf<float> directDepth;
+  DevBuf<int32_t> directPrim;
 
   // tail-mode depths chosen by the last render with the same scene / canvas / depth / batch shape (reused without
   // a new synchronisation; they are heuristics, any value is correct)
@@ -450,12 +456,14 @@ void b2pt_destroy(b2pt_ctx* ctx)
   for (cudaStream_t st : ctx->extra)
     if (st)
       cudaStreamSynchronize(st);
-  ctx->dNodes.release(), ctx->dWide.release(), ctx->dParent.release(), ctx->dArrived.release(), ctx->dSlots.release(), ctx->dLeafSph.release(), ctx->dQuads.release(), ctx->dSph.release(), ctx->dGates.release();
+  ctx->dNodes.release(), ctx->dWide.release(), ctx->dParent.release(), ctx->dArrived.release(), ctx->dSlots.release(), ctx->dBinSlots.release(), ctx->dLeafSph.release(), ctx->dQuads.release(), ctx->dSph.release(), ctx->dGates.release();
   ctx->colorOwn.release();
   for (auto& b : ctx->bufs)
     b.release_all();
   ctx->counters.release(), ctx->binTotals.release(), ctx->seeds.release(), ctx->nanCounter.release();
   ctx->dViews.release(), ctx->viewColor.release(), ctx->pnm.release(), ctx->primMask.release(), ctx->primQuads.release(); // (DevBuf's destructor would free them too)
+  ctx->dDirectViews.release(), ctx->directNormals.release(), ctx->directAlbedo.release(), ctx->directDepth.release(),
+    ctx->directPrim.release();
   if (ctx->evFork)
     cudaEventDestroy(ctx->evFork);
   for (int k = 0; k < b2pt_ctx::kMaxSets; ++k)
@@ -1096,6 +1104,8 @@ static int build_trace_structures(b2pt_ctx* ctx, uint32_t flags)
         const B2Sphere& sp = ctx->sph[(size_t)(~wr.slots[i])];
         leafSph[i] = make_float4(sp.c[0], sp.c[1], sp.c[2], sp.r);
       }
+    CU(ctx->dBinSlots.reserve(nSlots));
+    CU(cudaMemcpy(ctx->dBinSlots.p, ctx->dSlots.p, nSlots * sizeof(int32_t), cudaMemcpyDeviceToDevice));
     CU(ctx->dWide.reserve(wr.nodes.size() * 5));
     CU(cudaMemcpy(ctx->dWide.p, wr.nodes.data(), wr.nodes.size() * sizeof(B2WideNode), cudaMemcpyHostToDevice));
     CU(cudaMemcpy(ctx->dSlots.p, wr.slots.data(), nSlots * sizeof(int32_t), cudaMemcpyHostToDevice));
@@ -1264,6 +1274,15 @@ static int make_camera(const float pos[3], const float lookAt[3], const float up
   return B2PT_OK;
 }
 
+// The up vector as Camera::SetUp (Camera.cxx:803-811) stores it: normalised unless it is exactly (0,1,0).
+static void stored_up(const float up[3], float out[3])
+{
+  H3 upv = { up[0], up[1], up[2] };
+  if (!(upv.x == 0.f && upv.y == 1.f && upv.z == 0.f))
+    upv = hnormalize(upv);
+  hst(out, upv);
+}
+
 int b2pt_set_camera(b2pt_ctx* ctx, const float pos[3], const float lookAt[3], const float up[3], float fovDeg, int W,
                     int H)
 {
@@ -1275,10 +1294,7 @@ int b2pt_set_camera(b2pt_ctx* ctx, const float pos[3], const float lookAt[3], co
   const bool resized = (W != ctx->cam.W || H != ctx->cam.H);
   ctx->cam = c;
   ctx->haveCamera = true;
-  H3 upv = { up[0], up[1], up[2] };
-  if (!(upv.x == 0.f && upv.y == 1.f && upv.z == 0.f))
-    upv = hnormalize(upv); // Camera::SetUp (Camera.cxx:803-811)
-  hst(ctx->camUpN, upv);
+  stored_up(up, ctx->camUpN);
   for (int k = 0; k < 3; ++k)
     ctx->camLookAt[k] = lookAt[k];
   if (resized && !ctx->colorExt)
@@ -2140,41 +2156,88 @@ int b2pt_read_pnm16(b2pt_ctx* ctx, int spp, uint16_t* rgb)
 
 static int ensure_trace(b2pt_ctx* ctx);
 
+// G-buffers of nViews views of N pixels each (views: host array), written to the host arrays at [view][pixel].  Chunks
+// of whole views, at most kDirectChunkPixels pixels unless one view alone is larger, run one launch each into the
+// context's staging buffers, whose contents are then copied to the chunk's slice of the outputs.
+static constexpr int64_t kDirectChunkPixels = (int64_t)1 << 22;
+static int render_direct_chunks(b2pt_ctx* ctx, int nViews, const b2pt::DirectView* views, int64_t N, float* normals,
+                                float* albedo, float* depth, int32_t* primId)
+{
+  if (int rc = ensure_trace(ctx))
+    return rc;
+  B2BvhScene bvh = ctx->bvh;
+  if (bvh.wide)
+    bvh.primSlots = ctx->dBinSlots.p; // the binary tree's leaf order (the wide tree rewrote dSlots)
+  const int64_t perChunk = std::max<int64_t>(1, kDirectChunkPixels / N);
+  const size_t cap = (size_t)(std::min<int64_t>(perChunk, nViews) * N);
+  CU(ctx->dDirectViews.reserve((size_t)nViews));
+  CU(cudaMemcpyAsync(ctx->dDirectViews.p, views, sizeof(b2pt::DirectView) * (size_t)nViews, cudaMemcpyHostToDevice,
+                     ctx->stream));
+  if (normals)
+    CU(ctx->directNormals.reserve(cap));
+  if (albedo)
+    CU(ctx->directAlbedo.reserve(cap));
+  if (depth)
+    CU(ctx->directDepth.reserve(cap));
+  if (primId)
+    CU(ctx->directPrim.reserve(cap));
+  for (int64_t v0 = 0; v0 < nViews; v0 += perChunk)
+  {
+    const int nv = (int)std::min<int64_t>(perChunk, nViews - v0);
+    const size_t n = (size_t)(nv * N), off = (size_t)(v0 * N);
+    CU(b2pt::launch_direct_views(ctx->useBvh ? nullptr : &ctx->small, ctx->useBvh ? &bvh : nullptr,
+                                 ctx->dDirectViews.p + v0, nv, (int)N, normals ? ctx->directNormals.p : nullptr,
+                                 albedo ? ctx->directAlbedo.p : nullptr, depth ? ctx->directDepth.p : nullptr,
+                                 primId ? ctx->directPrim.p : nullptr, ctx->stream));
+    if (normals)
+      CU(cudaMemcpyAsync(normals + 4 * off, ctx->directNormals.p, n * sizeof(float4), cudaMemcpyDeviceToHost,
+                         ctx->stream));
+    if (albedo)
+      CU(cudaMemcpyAsync(albedo + 4 * off, ctx->directAlbedo.p, n * sizeof(float4), cudaMemcpyDeviceToHost,
+                         ctx->stream));
+    if (depth)
+      CU(cudaMemcpyAsync(depth + off, ctx->directDepth.p, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    if (primId)
+      CU(cudaMemcpyAsync(primId + off, ctx->directPrim.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  CU(cudaStreamSynchronize(ctx->stream));
+  return B2PT_OK;
+}
+
 int b2pt_render_direct(b2pt_ctx* ctx, float* normals, float* albedo, float* depth, int32_t* primId)
 {
   if (int rc = bind(ctx))
     return rc;
   if (!ctx->haveCamera)
     return fail(B2PT_ERR_STATE, "b2pt_render_direct before b2pt_set_camera");
-  if (int rc = ensure_trace(ctx))
+  b2pt::DirectView v;
+  v.cam = ctx->cam;
+  for (int c = 0; c < 3; ++c)
+    v.lookAt[c] = ctx->camLookAt[c], v.upN[c] = ctx->camUpN[c];
+  return render_direct_chunks(ctx, 1, &v, (int64_t)ctx->cam.W * ctx->cam.H, normals, albedo, depth, primId);
+}
+
+int b2pt_render_direct_views(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, float* normals,
+                             float* albedo, float* depth, int32_t* primId)
+{
+  if (int rc = bind(ctx))
     return rc;
-  if (ctx->useBvh)
-    return fail(B2PT_ERR_UNSUPPORTED, "b2pt_render_direct serves scenes on the kernel-parameter path (<= %d quads)",
-                B2PT_SMALL_MAX_QUADS);
-  const size_t N = (size_t)ctx->cam.W * ctx->cam.H;
-  DevBuf<float4> dN, dA;
-  DevBuf<float> dD;
-  DevBuf<int32_t> dP;
-  if (normals)
-    CU(dN.reserve(N));
-  if (albedo)
-    CU(dA.reserve(N));
-  if (depth)
-    CU(dD.reserve(N));
-  if (primId)
-    CU(dP.reserve(N));
-  CU(b2pt::launch_direct(ctx->cam, ctx->small, ctx->cam.pos, ctx->camLookAt, ctx->camUpN, dN.p, dA.p, dD.p, dP.p,
-                         ctx->stream));
-  if (normals)
-    CU(cudaMemcpyAsync(normals, dN.p, N * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
-  if (albedo)
-    CU(cudaMemcpyAsync(albedo, dA.p, N * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
-  if (depth)
-    CU(cudaMemcpyAsync(depth, dD.p, N * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-  if (primId)
-    CU(cudaMemcpyAsync(primId, dP.p, N * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaStreamSynchronize(ctx->stream));
-  return B2PT_OK;
+  if (nViews < 0 || (nViews > 0 && !views))
+    return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_direct_views: bad view list");
+  std::vector<b2pt::DirectView> dv((size_t)nViews);
+  for (int v = 0; v < nViews; ++v)
+  {
+    const float* p = views + 10 * (size_t)v;
+    b2pt::DirectView& d = dv[(size_t)v];
+    if (int rc = make_camera(p, p + 3, p + 6, p[9], W, H, d.cam))
+      return rc;
+    for (int c = 0; c < 3; ++c)
+      d.lookAt[c] = p[3 + c];
+    stored_up(p + 6, d.upN);
+  }
+  if (nViews == 0)
+    return B2PT_OK;
+  return render_direct_chunks(ctx, nViews, dv.data(), (int64_t)W * H, normals, albedo, depth, primId);
 }
 
 static int ensure_trace(b2pt_ctx* ctx)

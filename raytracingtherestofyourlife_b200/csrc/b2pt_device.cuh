@@ -808,7 +808,12 @@ __device__ __forceinline__ uint32_t bvh_pack(float leftBits, float countBits)
 {
   return ((uint32_t)__float_as_int(countBits) << 24) | (uint32_t)__float_as_int(leftBits);
 }
-__device__ __forceinline__ int closest_bvh(const B2BvhScene& S, f3 o, f3 d, float tmin, float tmax, float& tHit)
+// withSpheres = false skips the sphere entries of the leaves (the -direct G-buffers see quads only).
+// tiesToLowestIndex = true: an exact-t tie between quads of different leaves goes to the lower quad index, as in
+// closest_small and the oracle, instead of to the leaf visited first -- the hit no longer depends on the tree's shape
+// (quads only: use with withSpheres = false).
+__device__ __forceinline__ int closest_bvh(const B2BvhScene& S, f3 o, f3 d, float tmin, float tmax, float& tHit,
+                                           bool withSpheres = true, bool tiesToLowestIndex = false)
 {
   f3 inv = mk3(rcp_safe(d.x), rcp_safe(d.y), rcp_safe(d.z));
   f3 od = mk3(o.x * inv.x, o.y * inv.y, o.z * inv.z);
@@ -831,14 +836,17 @@ __device__ __forceinline__ int closest_bvh(const B2BvhScene& S, f3 o, f3 d, floa
         float t;
         if (enc >= 0)
         {
-          if (quad_accept(S.quads[enc], o, d, tmin, closest, t))
+          const bool accept = tiesToLowestIndex
+            ? quad_hit(S.quads[enc], o, d, t) && t > tmin && (t < closest || (t == closest && enc < best))
+            : quad_accept(S.quads[enc], o, d, tmin, closest, t);
+          if (accept)
           {
             closest = t;
             best = enc;
             found = true;
           }
         }
-        else
+        else if (withSpheres)
         {
           const float4 cr = __ldg(reinterpret_cast<const float4*>(S.sph + (~enc)));
           if (sphere_may_hit(mk3(cr.x, cr.y, cr.z), cr.w, o, d) &&

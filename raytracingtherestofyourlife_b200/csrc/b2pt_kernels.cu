@@ -1766,40 +1766,54 @@ __global__ void __launch_bounds__(256)
 // -direct G-buffers (main.cc:402-422: runNorms / runAlbedo + the depth buffer): one un-jittered ray per pixel
 // (Camera::PerspectiveRayGen), closest QUAD hit (MapperQuad.cxx:103-113 extracts quads only) beyond t = 0, the two
 // Shade rules.  Misses leave (0,0,0,0) / depth 0.  The Phong colour image of the stock VTK-m shader is out of scope.
-struct DirectView
+// Closest quad of a direct ray beyond t = 0; on both paths an exact-t tie goes to the lowest quad index (the oracle's
+// brute-force order), so the G-buffers do not depend on the trace structure or on the tree a builder made.
+__device__ __forceinline__ int closest_direct(const B2SmallScene& S, f3 o, f3 d, float& t)
 {
-  float pos[3], lookAt[3], upN[3];
-};
+  return closest_small(S, o, d, 0.f, FLT_MAX, t, /*withSpheres*/ false);
+}
+__device__ __forceinline__ int closest_direct(const B2BvhScene& S, f3 o, f3 d, float& t)
+{
+  return closest_bvh(S, o, d, 0.f, FLT_MAX, t, /*withSpheres*/ false, /*tiesToLowestIndex*/ true);
+}
+// One thread per (view, pixel) of a chunk of whole views: idx = view * nPixels + pixel, outputs [view][pixel].  The
+// chunk holds fewer than 2^32 pixels, so fastdiv's 32-bit numerator takes idx.
+template <class SceneT>
 __global__ void __launch_bounds__(256)
-  k_direct(const __grid_constant__ B2Camera cam, const __grid_constant__ B2SmallScene scene,
-           const __grid_constant__ DirectView view, float4* normals, float4* albedo, float* depth, int32_t* primOut)
+  k_direct_views(const __grid_constant__ SceneT scene, const DirectView* __restrict__ views, int64_t n,
+                 uint32_t nPixels, uint32_t divMagic, uint32_t divShift, float4* normals, float4* albedo, float* depth,
+                 int32_t* primOut)
 {
-  const int p = blockIdx.x * blockDim.x + threadIdx.x;
-  if (p >= cam.W * cam.H)
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n)
     return;
+  const uint32_t view = fastdiv((uint32_t)idx, divMagic, divShift);
+  const int p = (int)((uint32_t)idx - view * nPixels);
+  const DirectView& V = views[view];
+  const B2Camera cam = V.cam;
   const f3 o = ld3(cam.pos);
   const f3 d = raygen_corner(cam, p);
   float t;
-  const int code = closest_small(scene, o, d, 0.f, FLT_MAX, t, /*withSpheres*/ false);
+  const int code = closest_direct(scene, o, d, t);
   float4 nrm = make_float4(0.f, 0.f, 0.f, 0.f), alb = nrm;
   float dep = 0.f;
   int prim = -1;
   if (code != B2PT_MISS)
   {
     Hit hit;
-    fill_small(scene, code, o, d, t, hit);
-    direct_shade(hit.n, hit.p, ld3(view.pos), ld3(view.lookAt), ld3(view.upN), nrm, alb);
+    fill_hit(scene, code, o, d, t, hit);
+    direct_shade(hit.n, hit.p, o, ld3(V.lookAt), ld3(V.upN), nrm, alb);
     dep = t;
     prim = hit.prim;
   }
   if (normals)
-    normals[p] = nrm;
+    normals[idx] = nrm;
   if (albedo)
-    albedo[p] = alb;
+    albedo[idx] = alb;
   if (depth)
-    depth[p] = dep;
+    depth[idx] = dep;
   if (primOut)
-    primOut[p] = prim;
+    primOut[idx] = prim;
 }
 
 // pathtracing/Camera.cxx:894-953: fills + RayGen + origin broadcast, fused.
@@ -2132,15 +2146,24 @@ cudaError_t launch_primary_hits(const B2Camera& cam, const B2SmallScene* small, 
   return cudaGetLastError();
 }
 
-cudaError_t launch_direct(const B2Camera& cam, const B2SmallScene& S, const float pos[3], const float lookAt[3],
-                          const float upN[3], float4* normals, float4* albedo, float* depth, int32_t* primOut,
-                          cudaStream_t stream)
+cudaError_t launch_direct_views(const B2SmallScene* small, const B2BvhScene* bvh, const DirectView* views, int nViews,
+                                int nPixels, float4* normals, float4* albedo, float* depth, int32_t* primOut,
+                                cudaStream_t stream)
 {
-  DirectView v;
-  for (int c = 0; c < 3; ++c)
-    v.pos[c] = pos[c], v.lookAt[c] = lookAt[c], v.upN[c] = upN[c];
-  const int n = cam.W * cam.H;
-  k_direct<<<(n + 255) / 256, 256, 0, stream>>>(cam, S, v, normals, albedo, depth, primOut);
+  const int64_t n = (int64_t)nViews * nPixels;
+  if (n <= 0)
+    return cudaSuccess;
+  if (n > 0xffffffffLL)
+    return cudaErrorInvalidValue;
+  uint32_t magic, shift;
+  make_fastdiv((uint32_t)nPixels, magic, shift);
+  const unsigned grid = (unsigned)((n + 255) / 256);
+  if (bvh)
+    k_direct_views<B2BvhScene><<<grid, 256, 0, stream>>>(*bvh, views, n, (uint32_t)nPixels, magic, shift, normals,
+                                                         albedo, depth, primOut);
+  else
+    k_direct_views<B2SmallScene><<<grid, 256, 0, stream>>>(*small, views, n, (uint32_t)nPixels, magic, shift, normals,
+                                                           albedo, depth, primOut);
   return cudaGetLastError();
 }
 

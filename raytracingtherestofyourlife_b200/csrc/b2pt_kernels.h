@@ -83,10 +83,18 @@ cudaError_t launch_accumulate(float4* color, const float4* rad, int nPixels, int
                               unsigned long long* nanCounter, cudaStream_t stream);
 cudaError_t launch_primary_hits(const B2Camera& cam, const B2SmallScene* small, const B2BvhScene* bvh,
                                 uint32_t seedOffset, int32_t* primOut, float* tOut, cudaStream_t stream);
-// -direct G-buffers of a small scene (k_direct): normals / albedo W*H float4, depth W*H float, prim ids; any may be null.
-cudaError_t launch_direct(const B2Camera& cam, const B2SmallScene& S, const float pos[3], const float lookAt[3],
-                          const float upN[3], float4* normals, float4* albedo, float* depth, int32_t* primOut,
-                          cudaStream_t stream);
+// -direct G-buffers of nViews views (k_direct_views): per view the camera basis, its look-at point and its up vector
+// as Camera::SetUp stores it.  Outputs [view][pixel]: normals / albedo float4, depth float, prim ids; any may be null.
+// bvh != nullptr traverses its binary tree (nodes / primSlots in binary leaf order), else the small scene.
+// nViews * nPixels must stay below 2^32.
+struct DirectView
+{
+  B2Camera cam;
+  float lookAt[3], upN[3];
+};
+cudaError_t launch_direct_views(const B2SmallScene* small, const B2BvhScene* bvh, const DirectView* views, int nViews,
+                                int nPixels, float4* normals, float4* albedo, float* depth, int32_t* primOut,
+                                cudaStream_t stream);
 cudaError_t launch_create_rays(const B2Camera& cam, uint32_t* seeds, float* dx, float* dy, float* dz, float* ox,
                                float* oy, float* oz, long long* pixelIdx, cudaStream_t stream);
 cudaError_t launch_intersect(const B2SmallScene* small, const B2BvhScene* bvh, int64_t n, const float* ox,

@@ -309,6 +309,62 @@ void MapperPathTracer::RenderDirectBuffers(const vtkm::cont::DynamicCellSet& cel
                                         reinterpret_cast<float*>(albedo.GetStorage()), depth.GetStorage(), nullptr));
 }
 
+// b2pt_render_views / b2pt_render_direct_views view list: pos[3], lookAt[3], up[3], fovDeg per camera
+static std::vector<float> packViews(const std::vector<vtkm::rendering::Camera>& cameras)
+{
+  std::vector<float> views(cameras.size() * 10);
+  for (size_t v = 0; v < cameras.size(); ++v)
+  {
+    const auto pos = cameras[v].GetPosition(), at = cameras[v].GetLookAt(), up = cameras[v].GetViewUp();
+    float* p = &views[10 * v];
+    for (int k = 0; k < 3; ++k)
+      p[k] = pos[k], p[3 + k] = at[k], p[6 + k] = up[k];
+    p[9] = cameras[v].GetFieldOfView();
+  }
+  return views;
+}
+
+void MapperPathTracer::RenderDirectBuffersViews(const vtkm::cont::DynamicCellSet& cellset,
+                                                const vtkm::cont::CoordinateSystem& coords,
+                                                const std::vector<vtkm::rendering::Camera>& cameras,
+                                                std::vector<vtkm::cont::ArrayHandle<vtkm::Vec<vtkm::Float32, 4>>>& normals,
+                                                std::vector<vtkm::cont::ArrayHandle<vtkm::Vec<vtkm::Float32, 4>>>& albedo,
+                                                std::vector<vtkm::cont::ArrayHandle<vtkm::Float32>>& depth)
+{
+  if (Internals->Canvas == nullptr)
+    throw vtkm::cont::ErrorBadValue("MapperPathTracer: no canvas set");
+  auto* canvas = Internals->Canvas;
+  const vtkm::Id nx = canvas->GetWidth(), ny = canvas->GetHeight();
+  for (const auto& camera : cameras)
+    Internals->RayCamera.SetParameters(camera, *canvas); // validates every view like the reference (:372)
+  auto tup = extract(cellset);
+  auto SphereIds = std::get<0>(tup);
+  auto SphereRadii = std::get<1>(tup);
+  auto QuadIds = std::get<3>(tup);
+  vtkm::cont::ArrayHandle<vtkm::Int32> matIdArray, texIdArray;
+  matIdArray.Allocate(nx * ny);
+  texIdArray.Allocate(nx * ny);
+  buildBVH(coords, QuadIds, SphereIds, SphereRadii, matIdArray, texIdArray, MatIdx, TexIdx);
+  const std::vector<float> views = packViews(cameras);
+  const size_t n = static_cast<size_t>(nx * ny), V = cameras.size();
+  std::vector<float> nrm(V * n * 4), alb(V * n * 4), dep(V * n);
+  b2pt_ctx* ctx = b2pt_facade::Context(Devices.empty() ? -1 : Devices[0]);
+  b2pt_facade::Check(b2pt_render_direct_views(ctx, static_cast<int>(V), views.data(), static_cast<int>(nx),
+                                              static_cast<int>(ny), nrm.data(), alb.data(), dep.data(), nullptr));
+  normals.resize(V);
+  albedo.resize(V);
+  depth.resize(V);
+  for (size_t v = 0; v < V; ++v)
+  {
+    normals[v].Allocate(static_cast<vtkm::Id>(n));
+    albedo[v].Allocate(static_cast<vtkm::Id>(n));
+    depth[v].Allocate(static_cast<vtkm::Id>(n));
+    std::memcpy(static_cast<void*>(normals[v].GetStorage()), &nrm[v * n * 4], sizeof(float) * 4 * n);
+    std::memcpy(static_cast<void*>(albedo[v].GetStorage()), &alb[v * n * 4], sizeof(float) * 4 * n);
+    std::memcpy(depth[v].GetStorage(), &dep[v * n], sizeof(float) * n);
+  }
+}
+
 void MapperPathTracer::RenderViewsImpl(const vtkm::cont::DynamicCellSet& cellset,
                                        const vtkm::cont::CoordinateSystem& coords,
                                        const std::vector<vtkm::rendering::Camera>& cameras, unsigned int flags,
@@ -329,15 +385,7 @@ void MapperPathTracer::RenderViewsImpl(const vtkm::cont::DynamicCellSet& cellset
   texIdArray.Allocate(nx * ny);
   buildBVH(coords, QuadIds, SphereIds, SphereRadii, matIdArray, texIdArray, MatIdx, TexIdx);
 
-  std::vector<float> views(cameras.size() * 10);
-  for (size_t v = 0; v < cameras.size(); ++v)
-  {
-    const auto pos = cameras[v].GetPosition(), at = cameras[v].GetLookAt(), up = cameras[v].GetViewUp();
-    float* p = &views[10 * v];
-    for (int k = 0; k < 3; ++k)
-      p[k] = pos[k], p[3 + k] = at[k], p[6 + k] = up[k];
-    p[9] = cameras[v].GetFieldOfView();
-  }
+  std::vector<float> views = packViews(cameras);
   b2pt_ctx* ctx = b2pt_facade::Context();
   b2pt_facade::Check(b2pt_seed(ctx, 0)); // seeds[i] = i, MapperPathTracer.cxx:265-267
   b2pt_facade::Check(b2pt_render_views(ctx, static_cast<int>(cameras.size()), views.data(), static_cast<int>(nx),

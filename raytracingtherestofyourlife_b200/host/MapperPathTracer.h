@@ -118,6 +118,15 @@ public:
                            vtkm::cont::ArrayHandle<vtkm::Vec<vtkm::Float32, 4>>& normals,
                            vtkm::cont::ArrayHandle<vtkm::Vec<vtkm::Float32, 4>>& albedo,
                            vtkm::cont::ArrayHandle<vtkm::Float32>& depth);
+  // The same G-buffers for many cameras in one call: what main.cc's generateHemisphere / fibonacciHemisphere do with
+  // -direct by calling generate() per view point (main.cc:386-561).  Every camera is validated against the canvas set
+  // with SetCanvas; view v lands in normals[v] / albedo[v] / depth[v] with the bits RenderDirectBuffers gives for that
+  // camera (b2pt_render_direct_views, on the first device of SetDevices).
+  void RenderDirectBuffersViews(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
+                                const std::vector<vtkm::rendering::Camera>& cameras,
+                                std::vector<vtkm::cont::ArrayHandle<vtkm::Vec<vtkm::Float32, 4>>>& normals,
+                                std::vector<vtkm::cont::ArrayHandle<vtkm::Vec<vtkm::Float32, 4>>>& albedo,
+                                std::vector<vtkm::cont::ArrayHandle<vtkm::Float32>>& depth);
   double GetLastRenderMilliseconds() const { return LastRenderMs; }
   long long GetLastSegments() const { return LastSegments; }
 
