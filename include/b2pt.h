@@ -148,6 +148,22 @@ int b2pt_render_range(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxDe
  * are left untouched.  B2PT_FLAG_REFERENCE_STREAM is rejected (B2PT_ERR_BAD_VALUE). */
 int b2pt_render_views(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int spp, int maxDepth,
                       uint32_t flags, void* rgbaOut);
+/* b2pt_render_views at several sample counts from one render: renders checkpoints[K-1] samples of every view as
+ * b2pt_render_views does (same batching rule) and keeps the running sums at every checkpoint.  checkpoints holds
+ * K = nCheckpoints strictly increasing counts >= 1, 1 <= K <= 32.  Slice k of rgbaOut, [k][view][j*W+i], holds the
+ * bits b2pt_render_views(..., spp = checkpoints[k], flags) returns: float4 sums, normalised with checkpoints[k] under
+ * B2PT_FLAG_VIEWS_NORMALIZE, uint16_t[3] integers computed with checkpoints[k] under B2PT_FLAG_VIEWS_PNM16.
+ * moment2Out receives, whatever the flags, the float4 per-pixel sums of squared samples r*r (alpha lane 0, sample
+ * order) at every checkpoint, [k][view][j*W+i]: with the sums they give each checkpoint's sample variance.  Either
+ * output may be NULL; the call synchronises when one is not.  Afterwards b2pt_views_device_ptr holds the last
+ * checkpoint as b2pt_render_views(checkpoints[K-1]) leaves it, and stats.paths is W*H*checkpoints[K-1]*nViews.  The
+ * context's own camera and canvas are left untouched.  B2PT_ERR_BAD_VALUE, before anything runs: a bad checkpoint
+ * list, B2PT_FLAG_REFERENCE_STREAM, a bad view (b2pt_set_camera's message), or more than 2^30 float4 of device output
+ * ((K-1) snapshots, K sums of squares when moment2Out is not NULL, and the image, of nViews*W*H each).  nViews == 0
+ * does nothing.  The reference has no counterpart: it renders one sample count per sweep (main.cc:386-561). */
+int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
+                                  const int* checkpoints, int maxDepth, uint32_t flags, void* rgbaOut,
+                                  float* moment2Out);
 void* b2pt_views_device_ptr(b2pt_ctx* ctx);
 int b2pt_clear_color(b2pt_ctx* ctx);
 /* Host-side planning rule of the renders above, exposed for tests and capacity planning (no GPU needed): `units`

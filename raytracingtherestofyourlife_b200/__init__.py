@@ -71,6 +71,7 @@ SIGNATURES = {
     "b2pt_render": (_i32, [_vp, _i32, _i32, C.c_uint32]),
     "b2pt_render_range": (_i32, [_vp, _i32, _i32, _i32, C.c_uint32]),
     "b2pt_render_views": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _i32, C.c_uint32, _vp]),
+    "b2pt_render_views_checkpoints": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, _i32, C.c_uint32, _vp, _vp]),
     "b2pt_views_device_ptr": (_vp, [_vp]),
     "b2pt_plan_batches": (_i32, [_i64, _i64, _i64, _i32, _vp, _vp]),
     "b2pt_clear_color": (_i32, [_vp]),
@@ -280,6 +281,21 @@ class Context:
         assert out.dtype == dt and out.flags.c_contiguous and out.size == v.shape[0] * W * H * ch
         _check(lib().b2pt_render_views(self._h, v.shape[0], _p(v), W, H, spp, max_depth, flags, _p(out)))
         return out
+
+    def render_views_checkpoints(self, views, W, H, checkpoints, max_depth, flags=0, moments=False):
+        """b2pt_render_views_checkpoints: one render of checkpoints[-1] samples per view; returns the [K, nViews, H*W, 4]
+        images (uint16 [K, nViews, H*W, 3] under FLAG_VIEWS_PNM16), slice k bit-identical to
+        render_views(spp=checkpoints[k], flags), and with moments=True also the [K, nViews, H*W, 4] float32 sums of
+        squared samples at every checkpoint."""
+        v = np.ascontiguousarray(views, np.float32).reshape(-1, 10)
+        c = np.ascontiguousarray(checkpoints, np.int32).reshape(-1)
+        K = c.shape[0]
+        dt, ch = (np.uint16, 3) if flags & FLAG_VIEWS_PNM16 else (np.float32, 4)
+        out = np.empty((K, v.shape[0], W * H, ch), dt)
+        m2 = np.empty((K, v.shape[0], W * H, 4), np.float32) if moments else None
+        _check(lib().b2pt_render_views_checkpoints(self._h, v.shape[0], _p(v), W, H, K, _p(c), max_depth, flags,
+                                                   _p(out), _p(m2)))
+        return (out, m2) if moments else out
 
     def clear_color(self):
         _check(lib().b2pt_clear_color(self._h))

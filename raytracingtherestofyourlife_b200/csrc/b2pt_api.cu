@@ -204,6 +204,8 @@ struct b2pt_ctx
   DevBuf<B2Camera> dViews;
   DevBuf<float4> viewColor;
   DevBuf<uint16_t> pnm; // packed PNM integers (b2pt_read_pnm16, B2PT_FLAG_VIEWS_PNM16)
+  // b2pt_render_views_checkpoints: [K-1][nViews][W*H] prefix sums and [K][nViews][W*H] sums of squares
+  DevBuf<float4> ckptSnap, ckptMoment;
   DevBuf<uint2> primMask;         // primary-ray specialisation: [views][tiles] candidate masks (k_primary_prep)
   DevBuf<B2PrimQuad> primQuads;   // ... and [views][B2PT_SMALL_MAX_QUADS] per-quad constants
   int64_t viewCount = 0, viewPixels = 0;
@@ -462,6 +464,7 @@ void b2pt_destroy(b2pt_ctx* ctx)
     b.release_all();
   ctx->counters.release(), ctx->binTotals.release(), ctx->seeds.release(), ctx->nanCounter.release();
   ctx->dViews.release(), ctx->viewColor.release(), ctx->pnm.release(), ctx->primMask.release(), ctx->primQuads.release(); // (DevBuf's destructor would free them too)
+  ctx->ckptSnap.release(), ctx->ckptMoment.release();
   ctx->dDirectViews.release(), ctx->directNormals.release(), ctx->directAlbedo.release(), ctx->directDepth.release(),
     ctx->directPrim.release();
   if (ctx->evFork)
@@ -1435,8 +1438,11 @@ static void plan_batches(int64_t units, int64_t unitPaths, int64_t maxPathsPerBa
 // One render of the current scene.  nViews == 0: the context's camera, samples [sampleBegin, sampleBegin+sampleCount)
 // accumulated into the context's canvas.  nViews > 0 (b2pt_render_views): the same sample range for every camera of
 // ctx->dViews, accumulated into ctx->viewColor[view]; a batch holds whole views (viewsPerBatch x sampleCount sample
-// slots), so the caller guarantees W*H*sampleCount <= the batch target.
-static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxDepth, uint32_t flags, int64_t nViews)
+// slots), so the caller guarantees W*H*sampleCount <= the batch target.  ckpt (b2pt_render_views_checkpoints): the
+// batches accumulate through k_accumulate_checkpoints into these snapshot slices as well; entry0 is the first canvas
+// entry of the render (its view's slice offset when nViews == 0).
+static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxDepth, uint32_t flags, int64_t nViews,
+                       const b2pt::CheckpointArgs* ckpt = nullptr)
 {
   if (int rc = bind(ctx))
     return rc;
@@ -1762,7 +1768,16 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
     // (view batches write disjoint canvases: no order needed)
     if (overlap && batch > 0 && !viewMode)
       CU(cudaStreamWaitEvent(bs, ctx->evAcc[(set + nSets - 1) % nSets], 0));
-    if (viewMode)
+    if (ckpt)
+    {
+      b2pt::CheckpointArgs ck = *ckpt;
+      ck.sampleBase = A.sampleBase;
+      ck.entry0 += v0 * N;
+      CU(b2pt::launch_accumulate_checkpoints(viewMode ? ctx->viewColor.p + v0 * N : ctx->color(), bb.rad.p, (int)N,
+                                             viewMode ? sampleCount : (int)nb, viewMode ? (int)nv : 1,
+                                             ctx->nanCounter.p, ck, bs));
+    }
+    else if (viewMode)
       CU(b2pt::launch_accumulate(ctx->viewColor.p + v0 * N, bb.rad.p, (int)N, sampleCount, (int)nv,
                                  ctx->nanCounter.p, bs));
     else
@@ -1990,6 +2005,143 @@ int b2pt_render_views(b2pt_ctx* ctx, int nViews, const float* views, int W, int 
                        ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
   }
+  return B2PT_OK;
+}
+
+// b2pt_render_views at spp = checkpoints[K-1] through k_accumulate_checkpoints: sample s of a pixel is the same RNG
+// stream and is added in the same order at every spp, so the prefix sum after checkpoints[k] samples is the image
+// b2pt_render_views(spp = checkpoints[k]) returns, whatever the batching.
+int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
+                                  const int* checkpoints, int maxDepth, uint32_t flags, void* rgbaOut,
+                                  float* moment2Out)
+{
+  if (int rc = bind(ctx))
+    return rc;
+  if (nViews < 0 || (nViews > 0 && !views))
+    return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views_checkpoints: bad view list");
+  if (nCheckpoints < 1 || nCheckpoints > b2pt::kMaxCheckpoints || !checkpoints)
+    return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views_checkpoints: nCheckpoints must be in [1,%d] with a non-NULL list",
+                b2pt::kMaxCheckpoints);
+  for (int k = 0; k < nCheckpoints; ++k)
+    if (checkpoints[k] < 1 || (k > 0 && checkpoints[k] <= checkpoints[k - 1]))
+      return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views_checkpoints: checkpoints must be >= 1 and strictly increasing");
+  if (flags & B2PT_FLAG_REFERENCE_STREAM)
+    return fail(B2PT_ERR_BAD_VALUE, "REFERENCE_STREAM cannot be combined with a view-batched render");
+  std::vector<B2Camera> cams((size_t)nViews);
+  for (int v = 0; v < nViews; ++v)
+  {
+    const float* p = views + 10 * (size_t)v;
+    if (int rc = make_camera(p, p + 3, p + 6, p[9], W, H, cams[(size_t)v]))
+      return rc;
+  }
+  if (nViews == 0)
+  {
+    ctx->viewCount = 0;
+    return B2PT_OK;
+  }
+  const int K = nCheckpoints, spp = checkpoints[K - 1];
+  const int64_t N = (int64_t)W * H, NV = N * nViews;
+  const bool moments = moment2Out != nullptr;
+  const int64_t slices = (K - 1) + (moments ? K : 0) + 1; // snapshots, sums of squares, the last image
+  if (NV > ((int64_t)1 << 30) / slices)
+    return fail(B2PT_ERR_BAD_VALUE,
+                "b2pt_render_views_checkpoints: more than 2^30 float4 of device output (16 GiB); split the view list");
+  CU(ctx->viewColor.reserve((size_t)NV));
+  CU(ctx->dViews.reserve((size_t)nViews));
+  if (K > 1)
+    CU(ctx->ckptSnap.reserve((size_t)(NV * (K - 1))));
+  if (moments)
+    CU(ctx->ckptMoment.reserve((size_t)(NV * K)));
+  ctx->viewCount = nViews;
+  ctx->viewPixels = N;
+  b2pt::CheckpointArgs ck{};
+  ck.n = K;
+  std::copy(checkpoints, checkpoints + K, ck.count);
+  ck.snap = ctx->ckptSnap.p;
+  ck.moment = moments ? ctx->ckptMoment.p : nullptr;
+  ck.sliceStride = NV;
+  // the running sums start from zero: the image and the running sum of squares (slice K-1); every other slice is
+  // written exactly once
+  auto clear = [&]() -> cudaError_t {
+    cudaError_t e = cudaMemsetAsync(ctx->viewColor.p, 0, sizeof(float4) * (size_t)NV, ctx->stream);
+    if (e == cudaSuccess && moments)
+      e = cudaMemsetAsync(ctx->ckptMoment.p + NV * (K - 1), 0, sizeof(float4) * (size_t)NV, ctx->stream);
+    return e;
+  };
+  // the context's own camera gives the canvas shape to the launches; it is restored afterwards
+  const B2Camera savedCam = ctx->cam;
+  const bool savedHave = ctx->haveCamera;
+  float4* const savedExt = ctx->colorExt;
+  CU(clear());
+  ctx->cam = cams[0];
+  ctx->haveCamera = true;
+  int rc = B2PT_OK;
+  auto restore = [&]() {
+    ctx->cam = savedCam;
+    ctx->haveCamera = savedHave;
+    ctx->colorExt = savedExt;
+  };
+  // b2pt_render_views' batching rule for spp = checkpoints[K-1]
+  bool perView = !(N * spp <= std::min<int64_t>(batch_target_paths(ctx, true), 0xfffffff0LL));
+  if (!perView)
+  {
+    cudaError_t e = cudaMemcpyAsync(ctx->dViews.p, cams.data(), sizeof(B2Camera) * (size_t)nViews,
+                                    cudaMemcpyHostToDevice, ctx->stream);
+    if (e != cudaSuccess)
+    {
+      restore();
+      return fail(B2PT_ERR_CUDA, "cudaMemcpyAsync(views): %s", cudaGetErrorString(e));
+    }
+    rc = render_impl(ctx, 0, spp, maxDepth, flags, nViews, &ck);
+    perView = rc == B2PT_ERR_ALLOC;
+  }
+  if (perView)
+  { // one render per view into its slice of every output; sample batches carry the running sums in viewColor and
+    // moment slice K-1
+    rc = B2PT_OK;
+    if (clear() != cudaSuccess)
+      rc = fail(B2PT_ERR_CUDA, "clearing the view canvases failed");
+    int64_t paths = 0, launches = 0;
+    for (int v = 0; v < nViews && rc == B2PT_OK; ++v)
+    {
+      ctx->cam = cams[(size_t)v];
+      ctx->colorExt = ctx->viewColor.p + (size_t)v * N;
+      ck.entry0 = v * N;
+      rc = render_impl(ctx, 0, spp, maxDepth, flags, 0, &ck);
+      paths += ctx->stats.paths;
+      launches += ctx->stats.launches;
+    }
+    ctx->stats.paths = paths;
+    ctx->stats.launches = launches;
+  }
+  restore();
+  if (rc != B2PT_OK)
+    return rc;
+  // per checkpoint, the conversion b2pt_render_views applies to its image (the last one is viewColor itself)
+  for (int k = 0; k < K; ++k)
+  {
+    float4* const img = k + 1 < K ? ctx->ckptSnap.p + NV * k : ctx->viewColor.p;
+    if (flags & B2PT_FLAG_VIEWS_PNM16)
+    {
+      if (!rgbaOut)
+        break;
+      CU(ctx->pnm.reserve((size_t)NV * 3));
+      CU(b2pt::launch_pnm16(img, NV, checkpoints[k], ctx->pnm.p, ctx->stream));
+      CU(cudaMemcpyAsync(static_cast<uint16_t*>(rgbaOut) + (size_t)(NV * k) * 3, ctx->pnm.p,
+                         sizeof(uint16_t) * 3 * (size_t)NV, cudaMemcpyDeviceToHost, ctx->stream));
+      continue;
+    }
+    if ((flags & B2PT_FLAG_VIEWS_NORMALIZE) && (rgbaOut || k + 1 == K))
+      CU(b2pt::launch_normalize(img, NV, checkpoints[k], ctx->stream));
+    if (rgbaOut)
+      CU(cudaMemcpyAsync(static_cast<float4*>(rgbaOut) + NV * k, img, sizeof(float4) * (size_t)NV,
+                         cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  if (moments)
+    CU(cudaMemcpyAsync(moment2Out, ctx->ckptMoment.p, sizeof(float4) * (size_t)(NV * K), cudaMemcpyDeviceToHost,
+                       ctx->stream));
+  if (rgbaOut || moments)
+    CU(cudaStreamSynchronize(ctx->stream));
   return B2PT_OK;
 }
 

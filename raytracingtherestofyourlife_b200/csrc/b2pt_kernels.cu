@@ -13,6 +13,8 @@
 //   k_tail_loop<Scene>            every remaining bounce of a batch in one launch of one 8-CTA cluster.
 //   k_accumulate                  per pixel: sum the batch's samples in registers (sample order) and do a
 //                                 single read-modify-write of the canvas float4.
+//   k_accumulate_checkpoints      the same loop, also storing the running sum (and sum of squares) at chosen sample
+//                                 counts: the images of several sample counts from one render.
 //   k_primary_hits                parity hook: production raygen + trace, writes hit primitive id / t.
 //   k_create_rays, k_intersect, k_normalize, k_pnm16, k_fill_seeds, k_sum_peers: stage-level API kernels.
 //
@@ -1745,6 +1747,54 @@ __global__ void __launch_bounds__(256)
     atomicAdd(nanCounter, (unsigned long long)nan);
 }
 
+// k_accumulate's loop (same sums, same order, same NaN count) that also keeps the prefix sums at sample counts
+// ck.count[0..n-2]: when sample sampleBase + b is the count[k]-th of the pixel, the running sum goes to snapshot
+// slice k.  The last checkpoint is `color` itself.  With ck.moment, the running sum of squares r*r (alpha lane 0)
+// lives in moment slice n-1 across sample batches and is snapshotted at the same counts.
+__global__ void __launch_bounds__(256)
+  k_accumulate_checkpoints(float4* __restrict__ color, const float4* __restrict__ rad, int nPixels, int samplesPerView,
+                           int nViews, unsigned long long* nanCounter, const __grid_constant__ CheckpointArgs ck)
+{
+  const int64_t P = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (P >= (int64_t)nPixels * nViews)
+    return;
+  const int64_t view = P / nPixels;
+  const float4* r0 = rad + view * samplesPerView * (int64_t)nPixels + (P - view * nPixels);
+  const int64_t e = ck.entry0 + P; // entry of every slice
+  float4 c = color[P];
+  float4 m = ck.moment ? ck.moment[(ck.n - 1) * ck.sliceStride + e] : make_float4(0.f, 0.f, 0.f, 0.f);
+  int k = 0; // next checkpoint this batch can reach
+  while (k < ck.n - 1 && ck.count[k] <= ck.sampleBase)
+    ++k;
+  int nan = 0;
+  for (int b = 0; b < samplesPerView; ++b)
+  {
+    const float4 r = r0[(size_t)b * nPixels];
+    nan += (r.x != r.x || r.y != r.y || r.z != r.z) ? 1 : 0;
+    c.x += r.x;
+    c.y += r.y;
+    c.z += r.z;
+    if (ck.moment)
+    {
+      m.x += r.x * r.x;
+      m.y += r.y * r.y;
+      m.z += r.z * r.z;
+    }
+    if (k < ck.n - 1 && ck.sampleBase + b + 1 == ck.count[k])
+    {
+      ck.snap[k * ck.sliceStride + e] = c;
+      if (ck.moment)
+        ck.moment[k * ck.sliceStride + e] = m;
+      ++k;
+    }
+  }
+  color[P] = c;
+  if (ck.moment)
+    ck.moment[(ck.n - 1) * ck.sliceStride + e] = m;
+  if (nan)
+    atomicAdd(nanCounter, (unsigned long long)nan);
+}
+
 template <class SceneT>
 __global__ void __launch_bounds__(256)
   k_primary_hits(const __grid_constant__ B2Camera cam, const __grid_constant__ SceneT scene, uint32_t seedOffset,
@@ -2126,6 +2176,15 @@ cudaError_t launch_accumulate(float4* color, const float4* rad, int nPixels, int
   const int64_t n = (int64_t)nPixels * nViews;
   k_accumulate<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(color, rad, nPixels, samplesPerView, nViews,
                                                                 nanCounter);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_accumulate_checkpoints(float4* color, const float4* rad, int nPixels, int samplesPerView, int nViews,
+                                          unsigned long long* nanCounter, const CheckpointArgs& ck, cudaStream_t stream)
+{
+  const int64_t n = (int64_t)nPixels * nViews;
+  k_accumulate_checkpoints<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(color, rad, nPixels, samplesPerView,
+                                                                            nViews, nanCounter, ck);
   return cudaGetLastError();
 }
 

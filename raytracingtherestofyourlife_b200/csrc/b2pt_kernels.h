@@ -81,6 +81,22 @@ inline void make_fastdiv(uint32_t d, uint32_t& magic, uint32_t& shift)
 }
 cudaError_t launch_accumulate(float4* color, const float4* rad, int nPixels, int samplesPerView, int nViews,
                               unsigned long long* nanCounter, cudaStream_t stream);
+// launch_accumulate that also stores the running sums at sample counts count[0..n-2] (k_accumulate_checkpoints).
+// Slices are sliceStride float4 apart; entry0 + P is canvas entry P's index in every slice.  snap: n-1 slices, written
+// once each; moment (nullptr: none): n slices of sums of squares, slice n-1 the running one (cleared before the first
+// batch).  sampleBase: global sample index of the batch's first slot.
+constexpr int kMaxCheckpoints = 32;
+struct CheckpointArgs
+{
+  int n;
+  int sampleBase;
+  int count[kMaxCheckpoints]; // strictly increasing
+  float4* snap;
+  float4* moment;
+  int64_t sliceStride, entry0;
+};
+cudaError_t launch_accumulate_checkpoints(float4* color, const float4* rad, int nPixels, int samplesPerView, int nViews,
+                                          unsigned long long* nanCounter, const CheckpointArgs& ck, cudaStream_t stream);
 cudaError_t launch_primary_hits(const B2Camera& cam, const B2SmallScene* small, const B2BvhScene* bvh,
                                 uint32_t seedOffset, int32_t* primOut, float* tOut, cudaStream_t stream);
 // -direct G-buffers of nViews views (k_direct_views): per view the camera basis, its look-at point and its up vector

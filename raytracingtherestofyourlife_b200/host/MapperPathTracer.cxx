@@ -368,7 +368,7 @@ void MapperPathTracer::RenderDirectBuffersViews(const vtkm::cont::DynamicCellSet
 void MapperPathTracer::RenderViewsImpl(const vtkm::cont::DynamicCellSet& cellset,
                                        const vtkm::cont::CoordinateSystem& coords,
                                        const std::vector<vtkm::rendering::Camera>& cameras, unsigned int flags,
-                                       void* out)
+                                       void* out, const std::vector<int>* checkpoints)
 {
   if (Internals->Canvas == nullptr)
     throw vtkm::cont::ErrorBadValue("MapperPathTracer: no canvas set");
@@ -388,8 +388,13 @@ void MapperPathTracer::RenderViewsImpl(const vtkm::cont::DynamicCellSet& cellset
   std::vector<float> views = packViews(cameras);
   b2pt_ctx* ctx = b2pt_facade::Context();
   b2pt_facade::Check(b2pt_seed(ctx, 0)); // seeds[i] = i, MapperPathTracer.cxx:265-267
-  b2pt_facade::Check(b2pt_render_views(ctx, static_cast<int>(cameras.size()), views.data(), static_cast<int>(nx),
-                                       static_cast<int>(ny), samplecount, depthcount, RenderFlags | flags, out));
+  if (checkpoints)
+    b2pt_facade::Check(b2pt_render_views_checkpoints(
+      ctx, static_cast<int>(cameras.size()), views.data(), static_cast<int>(nx), static_cast<int>(ny),
+      static_cast<int>(checkpoints->size()), checkpoints->data(), depthcount, RenderFlags | flags, out, nullptr));
+  else
+    b2pt_facade::Check(b2pt_render_views(ctx, static_cast<int>(cameras.size()), views.data(), static_cast<int>(nx),
+                                         static_cast<int>(ny), samplecount, depthcount, RenderFlags | flags, out));
   b2pt_stats st;
   b2pt_facade::Check(b2pt_get_stats(ctx, &st));
   LastRenderMs = st.renderMs;
@@ -425,6 +430,24 @@ void MapperPathTracer::RenderCellsViewsPnm(const vtkm::cont::DynamicCellSet& cel
   const size_t n = static_cast<size_t>(Internals->Canvas->GetWidth()) * Internals->Canvas->GetHeight();
   pnm.assign(cameras.size() * n * 3, 0);
   RenderViewsImpl(cellset, coords, cameras, B2PT_FLAG_VIEWS_PNM16, pnm.data());
+}
+
+void MapperPathTracer::RenderCellsViewsCheckpointsPnm(const vtkm::cont::DynamicCellSet& cellset,
+                                                      const vtkm::cont::CoordinateSystem& coords,
+                                                      const std::vector<vtkm::rendering::Camera>& cameras,
+                                                      const std::vector<int>& checkpoints,
+                                                      std::vector<unsigned short>& pnm)
+{
+  if (Internals->Canvas == nullptr)
+    throw vtkm::cont::ErrorBadValue("MapperPathTracer: no canvas set");
+  if (checkpoints.empty() || checkpoints.back() != samplecount)
+    throw vtkm::cont::ErrorBadValue("MapperPathTracer: the checkpoint list must end with the sample count");
+  for (size_t k = 0; k < checkpoints.size(); ++k)
+    if (checkpoints[k] < 1 || (k > 0 && checkpoints[k] <= checkpoints[k - 1]))
+      throw vtkm::cont::ErrorBadValue("MapperPathTracer: checkpoints must be >= 1 and strictly increasing");
+  const size_t n = static_cast<size_t>(Internals->Canvas->GetWidth()) * Internals->Canvas->GetHeight();
+  pnm.assign(checkpoints.size() * cameras.size() * n * 3, 0);
+  RenderViewsImpl(cellset, coords, cameras, B2PT_FLAG_VIEWS_PNM16, pnm.data(), &checkpoints);
 }
 
 void MapperPathTracer::SetCompositeBackground(bool on) { Internals->CompositeBackground = on; }

@@ -109,6 +109,13 @@ public:
   // Packed on the GPU, 6 bytes per pixel cross PCIe instead of 16.
   void RenderCellsViewsPnm(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
                            const std::vector<vtkm::rendering::Camera>& cameras, std::vector<unsigned short>& pnm);
+  // Same for several sample counts from one render of samplecount samples per view: checkpoints is strictly increasing
+  // and ends with samplecount (else ErrorBadValue); pnm[((k * V + v) * W*H + i) * 3 + c] holds the integers
+  // RenderCellsViewsPnm gives with samplecount = checkpoints[k] (b2pt_render_views_checkpoints).
+  void RenderCellsViewsCheckpointsPnm(const vtkm::cont::DynamicCellSet& cellset,
+                                      const vtkm::cont::CoordinateSystem& coords,
+                                      const std::vector<vtkm::rendering::Camera>& cameras,
+                                      const std::vector<int>& checkpoints, std::vector<unsigned short>& pnm);
   // The -direct G-buffers of main.cc:402-422 (what MapperQuadNormals / MapperQuadAlbedo leave in the canvas colour
   // buffer, raytracing/RayTracerNormals.cxx / RayTracerAlbedo.cxx, and a depth image) for the canvas set with
   // SetCanvas: one un-jittered ray per pixel, closest quad hit, the reference's two Shade rules (b2pt_render_direct).
@@ -143,7 +150,8 @@ private:
   struct InternalsType;
   std::shared_ptr<InternalsType> Internals;
   void RenderViewsImpl(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
-                       const std::vector<vtkm::rendering::Camera>& cameras, unsigned int flags, void* out);
+                       const std::vector<vtkm::rendering::Camera>& cameras, unsigned int flags, void* out,
+                       const std::vector<int>* checkpoints = nullptr);
   void RenderCellsImpl(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
                        const vtkm::cont::Field& scalarField, const vtkm::rendering::Camera& camera);
   void UploadScene(const vtkm::cont::CoordinateSystem& coord, vtkm::cont::ArrayHandle<vtkm::Vec<vtkm::Id, 5>>& QuadIds,

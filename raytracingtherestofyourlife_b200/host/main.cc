@@ -16,6 +16,11 @@
 // normals-<phi>-<theta>.pnm, albedo-<phi>-<theta>.pnm and depth-<phi>-<theta>.pnm (phi and theta formatted as in the
 // path-traced names; the Fibonacci sweep uses phi = 0, theta = i).  All views of a sweep are rendered in one call.
 // The reference's own file names for the swept G-buffers are not restated here: this rule is the driver's.
+// -checkpoints c1,c2,... (with -hemisphere or -fibonacci, path-traced) also keeps the images at the lower sample counts
+// c1 < c2 < ... < samplecount of the same render: <out>-s<c>-<phi>-<theta>.pnm for every listed c, each the file a
+// sweep with -samplecount c writes, next to the usual <out>-<phi>-<theta>.pnm of samplecount samples (a denoiser
+// dataset's noisy inputs and target from one sweep).  A malformed or non-increasing list, an entry >= samplecount,
+// -direct, or no sweep is an error (exit 1).
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
@@ -46,6 +51,9 @@ struct Options
   bool fibonacci = false;
   int viewCount = 10000, viewSeed = 0; // main.cc:612 / :468
   int phiCount = 15, thetaCount = 15;  // main.cc:59-60
+  bool checkpointsGiven = false;
+  std::string checkpointsArg;
+  std::vector<int> checkpoints; // -checkpoints, parsed and checked by checkCheckpoints
 };
 
 Options parse(int argc, char** argv)
@@ -83,8 +91,41 @@ Options parse(int argc, char** argv)
       next(o.viewCount);
     else if (!std::strcmp(argv[i], "-viewseed"))
       next(o.viewSeed);
+    else if (!std::strcmp(argv[i], "-checkpoints"))
+    {
+      o.checkpointsGiven = true;
+      if (i + 1 < argc)
+        o.checkpointsArg = argv[++i];
+    }
   }
   return o;
+}
+
+// Parses -checkpoints into o.checkpoints; returns an error message, empty when the list is usable.
+std::string checkCheckpoints(Options& o)
+{
+  if (!o.checkpointsGiven)
+    return "";
+  if (o.direct)
+    return "-checkpoints cannot be combined with -direct";
+  if (!o.hemi && !o.fibonacci)
+    return "-checkpoints needs -hemisphere or -fibonacci";
+  const std::string malformed =
+    "-checkpoints takes strictly increasing positive integers separated by commas, got '" + o.checkpointsArg + "'";
+  std::stringstream list(o.checkpointsArg + ","); // every item, the last one too, ends with a comma
+  std::string item;
+  while (std::getline(list, item, ','))
+  {
+    if (item.empty() || item.size() > 9 || item.find_first_not_of("0123456789") != std::string::npos)
+      return malformed;
+    const int c = std::atoi(item.c_str());
+    if (c < 1 || (!o.checkpoints.empty() && c <= o.checkpoints.back()))
+      return malformed;
+    o.checkpoints.push_back(c);
+  }
+  if (o.checkpoints.back() >= o.samples)
+    return "-checkpoints entries must be below -samplecount (" + std::to_string(o.samples) + ")";
+  return "";
 }
 
 // NormalizeFunctor (main.cc:253-287): sqrt(de_nan(sum) / samplecount), alpha through the same sqrt
@@ -253,15 +294,24 @@ int renderViews(CornellBox& cb, const Options& o, const std::vector<vtkm::render
   vtkm::rendering::MapperPathTracer mapper(o.samples, o.depth, cb.matIdx, cb.texIdx, cb.matType, cb.texType, cb.tex);
   mapper.SetCanvas(&canvas);
   std::vector<unsigned short> pnm;
-  mapper.RenderCellsViewsPnm(cb.ds.GetCellSet(), cb.coord, cameras, pnm);
+  std::vector<int> counts = o.checkpoints; // -checkpoints: one render, its images at every count up to samplecount
+  counts.push_back(o.samples);
+  if (counts.size() > 1)
+    mapper.RenderCellsViewsCheckpointsPnm(cb.ds.GetCellSet(), cb.coord, cameras, counts, pnm);
+  else
+    mapper.RenderCellsViewsPnm(cb.ds.GetCellSet(), cb.coord, cameras, pnm);
   if (o.stats)
     std::cout << " GPU render ms = " << mapper.GetLastRenderMilliseconds() << " for " << cameras.size() << " views"
               << "  path samples/s = " << double(o.x) * o.y * o.samples * double(cameras.size()) /
         (mapper.GetLastRenderMilliseconds() * 1e-3)
               << "  segments = " << mapper.GetLastSegments() << std::endl;
-  for (size_t v = 0; v < cameras.size(); ++v)
-    savePnm16(viewName(o.out, angles[v].first, angles[v].second), o.x, o.y,
-              &pnm[v * static_cast<size_t>(o.x) * o.y * 3]);
+  const size_t n3 = static_cast<size_t>(o.x) * o.y * 3, V = cameras.size();
+  for (size_t k = 0; k < counts.size(); ++k)
+  { // slice k of pnm: counts[k] samples; the last is the ordinary image
+    const std::string stem = k + 1 < counts.size() ? o.out + "-s" + std::to_string(counts[k]) : o.out;
+    for (size_t v = 0; v < V; ++v)
+      savePnm16(viewName(stem, angles[v].first, angles[v].second), o.x, o.y, &pnm[(k * V + v) * n3]);
+  }
   return static_cast<int>(cameras.size());
 }
 
@@ -336,7 +386,13 @@ int fibonacciHemisphere(CornellBox& cb, const Options& o)
 
 int main(int argc, char* argv[])
 {
-  const Options o = parse(argc, argv);
+  Options o = parse(argc, argv);
+  const std::string bad = checkCheckpoints(o);
+  if (!bad.empty())
+  {
+    std::cerr << "error: " << bad << std::endl;
+    return 1;
+  }
   const auto t0 = std::chrono::steady_clock::now();
   try
   {
