@@ -164,6 +164,28 @@ int b2pt_render_views(b2pt_ctx* ctx, int nViews, const float* views, int W, int 
 int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
                                   const int* checkpoints, int maxDepth, uint32_t flags, void* rgbaOut,
                                   float* moment2Out);
+/* Denoiser guide buffers of a view sweep: per pixel, the first-hit albedo, normal and depth of the SAME path samples
+ * b2pt_render_views_checkpoints averages, summed over the first checkpoints[k] samples.  For view v, pixel
+ * p = j*W+i (j = 0 bottom row) and sample s, the primary ray is the renderer's: rng = p + seedOffset + s*0x9E3779B9
+ * (b2pt_seed), the jittered raygen of the path tracer, origin at the camera, closest hit in (0.001, FLT_MAX) through
+ * the trace structure a render with `flags` uses (quads and spheres).  Per sample, on a hit:
+ *   albedo = lambertian (matType 0): the primitive's texture colour; dielectric (2): (1,1,1), the attenuation of the
+ *            specular bounce; emitter (1): its colour clamped per channel to [0,1];
+ *   hit = 1;  normal = the shading normal (quads: geometric normal flipped to oppose the ray; spheres: (p-c)/r);
+ *   depth = t (the ray is unit length: a distance);
+ * and all zero on a miss.  albedoOut = (sum albedo.rgb, sum hit) and normalDepthOut = (sum normal.xyz, sum depth),
+ * float32 sums over s = 0 .. c-1 in sample order from +0.0, c = checkpoints[k]; layout [k][view][j*W+i] float4,
+ * K*nViews*W*H*4 floats each; either may be NULL.  Means are sum / c; the mean depth of the hitting samples is
+ * sum depth / sum hit.  views holds 10 floats per view as in b2pt_render_views.  flags may hold only the build flags
+ * FORCE_BVH, NO_DEDUP, NO_AA, GPU_LBVH, WIDE_BVH, and (re)builds the trace structures as a render would.
+ * B2PT_ERR_BAD_VALUE, before anything runs: a bad view list or view (b2pt_set_camera's message), a checkpoint list of
+ * other than 1..32 strictly increasing counts >= 1, checkpoints[K-1] > 2^24 (the hit count must stay an exact float),
+ * another flag, or K*W*H > 2^30.  nViews == 0 does nothing; no scene gives B2PT_ERR_STATE.  Views run in chunks of
+ * whole views through library-owned staging of at most max(2^23, K*W*H) float4 per requested output.  The context's
+ * camera, canvas, b2pt_views_device_ptr image and statistics are left untouched.  Synchronises the stream.  The
+ * reference has no counterpart. */
+int b2pt_render_views_features(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
+                               const int* checkpoints, uint32_t flags, float* albedoOut, float* normalDepthOut);
 void* b2pt_views_device_ptr(b2pt_ctx* ctx);
 int b2pt_clear_color(b2pt_ctx* ctx);
 /* Host-side planning rule of the renders above, exposed for tests and capacity planning (no GPU needed): `units`

@@ -72,6 +72,7 @@ SIGNATURES = {
     "b2pt_render_range": (_i32, [_vp, _i32, _i32, _i32, C.c_uint32]),
     "b2pt_render_views": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _i32, C.c_uint32, _vp]),
     "b2pt_render_views_checkpoints": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, _i32, C.c_uint32, _vp, _vp]),
+    "b2pt_render_views_features": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, C.c_uint32, _vp, _vp]),
     "b2pt_views_device_ptr": (_vp, [_vp]),
     "b2pt_plan_batches": (_i32, [_i64, _i64, _i64, _i32, _vp, _vp]),
     "b2pt_clear_color": (_i32, [_vp]),
@@ -296,6 +297,19 @@ class Context:
         _check(lib().b2pt_render_views_checkpoints(self._h, v.shape[0], _p(v), W, H, K, _p(c), max_depth, flags,
                                                    _p(out), _p(m2)))
         return (out, m2) if moments else out
+
+    def render_views_features(self, views, W, H, checkpoints, flags=0):
+        """b2pt_render_views_features: denoiser guides of the path samples render_views_checkpoints averages; returns
+        (albedo, normal_depth), each float32 [K, nViews, H*W, 4]: sums over the first checkpoints[k] samples of
+        (albedo rgb, hit) and (normal xyz, depth)."""
+        v = np.ascontiguousarray(views, np.float32).reshape(-1, 10)
+        c = np.ascontiguousarray(checkpoints, np.int32).reshape(-1)
+        K = c.shape[0]
+        albedo = np.empty((K, v.shape[0], W * H, 4), np.float32)
+        normal_depth = np.empty((K, v.shape[0], W * H, 4), np.float32)
+        _check(lib().b2pt_render_views_features(self._h, v.shape[0], _p(v), W, H, K, _p(c), flags, _p(albedo),
+                                                _p(normal_depth)))
+        return albedo, normal_depth
 
     def clear_color(self):
         _check(lib().b2pt_clear_color(self._h))

@@ -206,6 +206,8 @@ struct b2pt_ctx
   DevBuf<uint16_t> pnm; // packed PNM integers (b2pt_read_pnm16, B2PT_FLAG_VIEWS_PNM16)
   // b2pt_render_views_checkpoints: [K-1][nViews][W*H] prefix sums and [K][nViews][W*H] sums of squares
   DevBuf<float4> ckptSnap, ckptMoment;
+  // b2pt_render_views_features: [K][chunk views][W*H] staging of one chunk's sums
+  DevBuf<float4> featAlbedo, featNormalDepth;
   DevBuf<uint2> primMask;         // primary-ray specialisation: [views][tiles] candidate masks (k_primary_prep)
   DevBuf<B2PrimQuad> primQuads;   // ... and [views][B2PT_SMALL_MAX_QUADS] per-quad constants
   int64_t viewCount = 0, viewPixels = 0;
@@ -464,7 +466,7 @@ void b2pt_destroy(b2pt_ctx* ctx)
     b.release_all();
   ctx->counters.release(), ctx->binTotals.release(), ctx->seeds.release(), ctx->nanCounter.release();
   ctx->dViews.release(), ctx->viewColor.release(), ctx->pnm.release(), ctx->primMask.release(), ctx->primQuads.release(); // (DevBuf's destructor would free them too)
-  ctx->ckptSnap.release(), ctx->ckptMoment.release();
+  ctx->ckptSnap.release(), ctx->ckptMoment.release(), ctx->featAlbedo.release(), ctx->featNormalDepth.release();
   ctx->dDirectViews.release(), ctx->directNormals.release(), ctx->directAlbedo.release(), ctx->directDepth.release(),
     ctx->directPrim.release();
   if (ctx->evFork)
@@ -639,10 +641,14 @@ int b2pt_set_scene(b2pt_ctx* ctx, const float* pts, int64_t nPts, const int64_t*
   return B2PT_OK;
 }
 
+// The flags that choose and shape the trace structures (every other flag only affects a render).
+static constexpr uint32_t kBuildFlags =
+  B2PT_FLAG_FORCE_BVH | B2PT_FLAG_NO_DEDUP | B2PT_FLAG_NO_AA | B2PT_FLAG_GPU_LBVH | B2PT_FLAG_WIDE_BVH;
+
 static int build_trace_structures(b2pt_ctx* ctx, uint32_t flags)
 {
   ctx->haveParents = false;
-  ctx->builtFlags = flags & (B2PT_FLAG_FORCE_BVH | B2PT_FLAG_NO_DEDUP | B2PT_FLAG_NO_AA | B2PT_FLAG_GPU_LBVH | B2PT_FLAG_WIDE_BVH);
+  ctx->builtFlags = flags & kBuildFlags;
   // Drop bit-identical duplicate quads: a later copy computes the same t and loses the strict t<tmax
   // comparison (Surface.h:178-179), so removing it cannot change any result.
   std::vector<int32_t> keptQuads;
@@ -1435,6 +1441,20 @@ static void plan_batches(int64_t units, int64_t unitPaths, int64_t maxPathsPerBa
   nBatches = (units + per - 1) / per;
 }
 
+// MapperPathTracer::RenderCellsImpl builds its acceleration structures on every call (:275-276); here
+// they are rebuilt only when the scene or the build-affecting flags changed.
+static int ensure_built_for(b2pt_ctx* ctx, uint32_t flags)
+{
+  const uint32_t buildFlags = flags & kBuildFlags;
+  if (!ctx->haveBvh || ctx->builtFlags != buildFlags)
+  {
+    if (int rc = build_trace_structures(ctx, buildFlags))
+      return rc;
+    ctx->haveBvh = true;
+  }
+  return B2PT_OK;
+}
+
 // One render of the current scene.  nViews == 0: the context's camera, samples [sampleBegin, sampleBegin+sampleCount)
 // accumulated into the context's canvas.  nViews > 0 (b2pt_render_views): the same sample range for every camera of
 // ctx->dViews, accumulated into ctx->viewColor[view]; a batch holds whole views (viewsPerBatch x sampleCount sample
@@ -1459,15 +1479,8 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
     return fail(B2PT_ERR_BAD_VALUE, "KILL_ZERO_THROUGHPUT cannot be combined with REFERENCE_STREAM");
   if (refStream && sampleBegin != 0)
     return fail(B2PT_ERR_BAD_VALUE, "REFERENCE_STREAM renders samples from 0 (one persistent stream per pixel)");
-  // MapperPathTracer::RenderCellsImpl builds its acceleration structures on every call (:275-276); here
-  // they are rebuilt only when the scene or the build-affecting flags changed.
-  const uint32_t buildFlags = flags & (B2PT_FLAG_FORCE_BVH | B2PT_FLAG_NO_DEDUP | B2PT_FLAG_NO_AA | B2PT_FLAG_GPU_LBVH | B2PT_FLAG_WIDE_BVH);
-  if (!ctx->haveBvh || ctx->builtFlags != buildFlags)
-  {
-    if (int rc = build_trace_structures(ctx, buildFlags))
-      return rc;
-    ctx->haveBvh = true;
-  }
+  if (int rc = ensure_built_for(ctx, flags))
+    return rc;
   const bool viewMode = nViews > 0;
   if (!viewMode)
     if (int rc = ensure_color(ctx))
@@ -2142,6 +2155,83 @@ int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views,
                        ctx->stream));
   if (rgbaOut || moments)
     CU(cudaStreamSynchronize(ctx->stream));
+  return B2PT_OK;
+}
+
+// Denoiser guides of a view sweep (k_view_features).  Sample s of a pixel is traced from the stream the render gives it
+// (pixel + seedOffset + s * B2PT_GOLDEN), through the trace structure a render with these flags would use, so the
+// features average the rays the radiance image averages.  Views run in chunks of whole views, each chunk one launch
+// into the context's staging buffers (at most max(kFeatureChunkFloat4, K*W*H) float4 per output) and K copies per
+// output into the caller's arrays.  The context's camera, canvas, view images and statistics are not touched.
+static constexpr int64_t kFeatureChunkFloat4 = (int64_t)1 << 23;
+int b2pt_render_views_features(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
+                               const int* checkpoints, uint32_t flags, float* albedoOut, float* normalDepthOut)
+{
+  if (int rc = bind(ctx))
+    return rc;
+  if (nViews < 0 || (nViews > 0 && !views))
+    return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views_features: bad view list");
+  if (nCheckpoints < 1 || nCheckpoints > b2pt::kMaxCheckpoints || !checkpoints)
+    return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views_features: nCheckpoints must be in [1,%d] with a non-NULL list",
+                b2pt::kMaxCheckpoints);
+  for (int k = 0; k < nCheckpoints; ++k)
+    if (checkpoints[k] < 1 || (k > 0 && checkpoints[k] <= checkpoints[k - 1]))
+      return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views_features: checkpoints must be >= 1 and strictly increasing");
+  if (checkpoints[nCheckpoints - 1] > (1 << 24))
+    return fail(B2PT_ERR_BAD_VALUE,
+                "b2pt_render_views_features: more than 2^24 samples (the hit count must stay an exact float)");
+  if (flags & ~kBuildFlags)
+    return fail(B2PT_ERR_BAD_VALUE,
+                "b2pt_render_views_features: flags may only hold FORCE_BVH, NO_DEDUP, NO_AA, GPU_LBVH and WIDE_BVH");
+  std::vector<B2Camera> cams((size_t)nViews);
+  for (int v = 0; v < nViews; ++v)
+  {
+    const float* p = views + 10 * (size_t)v;
+    if (int rc = make_camera(p, p + 3, p + 6, p[9], W, H, cams[(size_t)v]))
+      return rc;
+  }
+  if (nViews == 0)
+    return B2PT_OK;
+  const int K = nCheckpoints;
+  const int64_t N = (int64_t)W * H, KN = N * K;
+  if (KN > ((int64_t)1 << 30))
+    return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views_features: one view's %d slices exceed 2^30 float4", K);
+  if (!ctx->haveScene)
+    return fail(B2PT_ERR_STATE, "b2pt_render_views_features before b2pt_set_scene");
+  if (int rc = ensure_built_for(ctx, flags))
+    return rc;
+  b2pt::FeatureCheckpoints ck{};
+  ck.n = K;
+  std::copy(checkpoints, checkpoints + K, ck.count);
+  const int64_t perChunk = std::max<int64_t>(1, kFeatureChunkFloat4 / KN);
+  const size_t cap = (size_t)(std::min<int64_t>(perChunk, nViews) * KN);
+  CU(ctx->dViews.reserve((size_t)nViews));
+  CU(cudaMemcpyAsync(ctx->dViews.p, cams.data(), sizeof(B2Camera) * (size_t)nViews, cudaMemcpyHostToDevice,
+                     ctx->stream));
+  if (albedoOut)
+    CU(ctx->featAlbedo.reserve(cap));
+  if (normalDepthOut)
+    CU(ctx->featNormalDepth.reserve(cap));
+  for (int64_t v0 = 0; v0 < nViews; v0 += perChunk)
+  {
+    const int nv = (int)std::min<int64_t>(perChunk, nViews - v0);
+    const int64_t n = nv * N; // one slice of the chunk
+    CU(b2pt::launch_view_features(ctx->useBvh ? nullptr : &ctx->small, ctx->useBvh ? &ctx->bvh : nullptr,
+                                  ctx->dViews.p + v0, nv, (int)N, ctx->seedOffset, ck,
+                                  albedoOut ? ctx->featAlbedo.p : nullptr,
+                                  normalDepthOut ? ctx->featNormalDepth.p : nullptr, ctx->stream));
+    for (int k = 0; k < K; ++k)
+    {
+      const size_t dst = 4 * (size_t)((k * (int64_t)nViews + v0) * N);
+      if (albedoOut)
+        CU(cudaMemcpyAsync(albedoOut + dst, ctx->featAlbedo.p + k * n, sizeof(float4) * (size_t)n,
+                           cudaMemcpyDeviceToHost, ctx->stream));
+      if (normalDepthOut)
+        CU(cudaMemcpyAsync(normalDepthOut + dst, ctx->featNormalDepth.p + k * n, sizeof(float4) * (size_t)n,
+                           cudaMemcpyDeviceToHost, ctx->stream));
+    }
+  }
+  CU(cudaStreamSynchronize(ctx->stream));
   return B2PT_OK;
 }
 

@@ -16,6 +16,8 @@
 //   k_accumulate_checkpoints      the same loop, also storing the running sum (and sum of squares) at chosen sample
 //                                 counts: the images of several sample counts from one render.
 //   k_primary_hits                parity hook: production raygen + trace, writes hit primitive id / t.
+//   k_view_features<Scene>        per (view, pixel): albedo, normal and depth of the primary hits of its path samples,
+//                                 summed in sample order and stored at chosen sample counts (denoiser guides).
 //   k_create_rays, k_intersect, k_normalize, k_pnm16, k_fill_seeds, k_sum_peers: stage-level API kernels.
 //
 // Work distribution: queue and bins are statically partitioned into one region per persistent warp
@@ -1866,6 +1868,60 @@ __global__ void __launch_bounds__(256)
     primOut[idx] = prim;
 }
 
+// Denoiser guides of a chunk of whole views: one thread per (view, pixel), idx = view * nPixels + pixel as in
+// k_direct_views.  Sample s is the render's path sample s: its stream, raygen and closest hit (trace) are k_trace's, so
+// the features describe the same rays the radiance image averages.  Per sample: albedo = the reflectance the path's
+// first bounce applies (lambertian: the texture colour; dielectric: 1, shade_specular's attenuation; emitter: its
+// colour clamped to [0,1]), a hit flag, the shading normal and t; all zero on a miss.  The sums run in registers in
+// sample order (plain adds under -fmad=false) and slice k receives them after count[k] samples.
+template <class SceneT>
+__global__ void __launch_bounds__(256)
+  k_view_features(const __grid_constant__ SceneT scene, const B2Camera* __restrict__ cams, int64_t n,
+                  uint32_t nPixels, uint32_t divMagic, uint32_t divShift, uint32_t seedOffset,
+                  const __grid_constant__ FeatureCheckpoints ck, float4* albedoOut, float4* normalDepthOut)
+{
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n)
+    return;
+  const uint32_t view = fastdiv((uint32_t)idx, divMagic, divShift);
+  const int p = (int)((uint32_t)idx - view * nPixels);
+  const B2Camera cam = cams[view];
+  const f3 o = ld3(cam.pos);
+  float4 alb = make_float4(0.f, 0.f, 0.f, 0.f), nd = alb;
+  const int last = ck.count[ck.n - 1];
+  int k = 0, next = ck.count[0];
+  for (int s = 0; s < last; ++s)
+  {
+    uint32_t rng = (uint32_t)p + seedOffset + (uint32_t)s * B2PT_GOLDEN;
+    const f3 d = raygen(cam, p, rng);
+    Hit hit;
+    f3 a = mk3(0.f, 0.f, 0.f), nrm = a;
+    float h = 0.f, t = 0.f;
+    if (trace(scene, o, d, 0.001f, FLT_MAX, hit))
+    {
+      a = hit.kind == 2 ? mk3(1.f, 1.f, 1.f)
+        : hit.kind == 1 ? mk3(fminf(fmaxf(hit.alb.x, 0.f), 1.f), fminf(fmaxf(hit.alb.y, 0.f), 1.f),
+                              fminf(fmaxf(hit.alb.z, 0.f), 1.f))
+                        : hit.alb;
+      nrm = hit.n;
+      h = 1.f;
+      t = hit.t;
+    }
+    alb.x += a.x, alb.y += a.y, alb.z += a.z, alb.w += h;
+    nd.x += nrm.x, nd.y += nrm.y, nd.z += nrm.z, nd.w += t;
+    if (s + 1 == next)
+    {
+      const int64_t e = (int64_t)k * n + idx;
+      if (albedoOut)
+        albedoOut[e] = alb;
+      if (normalDepthOut)
+        normalDepthOut[e] = nd;
+      ++k;
+      next = k < ck.n ? ck.count[k] : 0;
+    }
+  }
+}
+
 // pathtracing/Camera.cxx:894-953: fills + RayGen + origin broadcast, fused.
 __global__ void __launch_bounds__(256)
   k_create_rays(const __grid_constant__ B2Camera cam, uint32_t* seeds, float* dx, float* dy, float* dz, float* ox,
@@ -2223,6 +2279,34 @@ cudaError_t launch_direct_views(const B2SmallScene* small, const B2BvhScene* bvh
   else
     k_direct_views<B2SmallScene><<<grid, 256, 0, stream>>>(*small, views, n, (uint32_t)nPixels, magic, shift, normals,
                                                            albedo, depth, primOut);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_view_features(const B2SmallScene* small, const B2BvhScene* bvh, const B2Camera* cams, int nViews,
+                                 int nPixels, uint32_t seedOffset, const FeatureCheckpoints& ck, float4* albedo,
+                                 float4* normalDepth, cudaStream_t stream)
+{
+  const int64_t n = (int64_t)nViews * nPixels;
+  if (n <= 0)
+    return cudaSuccess;
+  if (n > 0xffffffffLL || ck.n < 1 || ck.n > kMaxCheckpoints)
+    return cudaErrorInvalidValue;
+  uint32_t magic, shift;
+  make_fastdiv((uint32_t)nPixels, magic, shift);
+  const unsigned grid = (unsigned)((n + 255) / 256);
+  if (bvh && bvh->wide)
+  {
+    B2WideScene ws;
+    static_cast<B2BvhScene&>(ws) = *bvh;
+    k_view_features<B2WideScene><<<grid, 256, 0, stream>>>(ws, cams, n, (uint32_t)nPixels, magic, shift, seedOffset,
+                                                           ck, albedo, normalDepth);
+  }
+  else if (bvh)
+    k_view_features<B2BvhScene><<<grid, 256, 0, stream>>>(*bvh, cams, n, (uint32_t)nPixels, magic, shift, seedOffset,
+                                                          ck, albedo, normalDepth);
+  else
+    k_view_features<B2SmallScene><<<grid, 256, 0, stream>>>(*small, cams, n, (uint32_t)nPixels, magic, shift,
+                                                            seedOffset, ck, albedo, normalDepth);
   return cudaGetLastError();
 }
 

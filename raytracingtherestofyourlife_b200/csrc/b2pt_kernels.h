@@ -111,6 +111,19 @@ struct DirectView
 cudaError_t launch_direct_views(const B2SmallScene* small, const B2BvhScene* bvh, const DirectView* views, int nViews,
                                 int nPixels, float4* normals, float4* albedo, float* depth, int32_t* primOut,
                                 cudaStream_t stream);
+// First-hit features of nViews views over their path samples (k_view_features): per (view, pixel) the primary rays of
+// samples s = 0 .. count[n-1]-1 (the render's streams: rng = pixel + seedOffset + s * B2PT_GOLDEN), summed in sample
+// order; at s + 1 == count[k] the sums go to slice k, outputs [k][view][pixel] with slices nViews * nPixels apart.
+// albedo: (albedo rgb, hit); normalDepth: (normal xyz, t); either may be null.  The trace structure is the one the
+// renders use (bvh->wide: the 8-wide tree).  nViews * nPixels must stay below 2^32.
+struct FeatureCheckpoints
+{
+  int n;
+  int count[kMaxCheckpoints]; // strictly increasing
+};
+cudaError_t launch_view_features(const B2SmallScene* small, const B2BvhScene* bvh, const B2Camera* cams, int nViews,
+                                 int nPixels, uint32_t seedOffset, const FeatureCheckpoints& ck, float4* albedo,
+                                 float4* normalDepth, cudaStream_t stream);
 cudaError_t launch_create_rays(const B2Camera& cam, uint32_t* seeds, float* dx, float* dy, float* dz, float* ox,
                                float* oy, float* oz, long long* pixelIdx, cudaStream_t stream);
 cudaError_t launch_intersect(const B2SmallScene* small, const B2BvhScene* bvh, int64_t n, const float* ox,

@@ -450,6 +450,45 @@ void MapperPathTracer::RenderCellsViewsCheckpointsPnm(const vtkm::cont::DynamicC
   RenderViewsImpl(cellset, coords, cameras, B2PT_FLAG_VIEWS_PNM16, pnm.data(), &checkpoints);
 }
 
+void MapperPathTracer::RenderCellsViewsFeatures(const vtkm::cont::DynamicCellSet& cellset,
+                                                const vtkm::cont::CoordinateSystem& coords,
+                                                const std::vector<vtkm::rendering::Camera>& cameras,
+                                                const std::vector<int>& checkpoints, std::vector<float>& albedo,
+                                                std::vector<float>& normalDepth)
+{
+  if (Internals->Canvas == nullptr)
+    throw vtkm::cont::ErrorBadValue("MapperPathTracer: no canvas set");
+  if (checkpoints.empty() || checkpoints.back() != samplecount)
+    throw vtkm::cont::ErrorBadValue("MapperPathTracer: the checkpoint list must end with the sample count");
+  for (size_t k = 0; k < checkpoints.size(); ++k)
+    if (checkpoints[k] < 1 || (k > 0 && checkpoints[k] <= checkpoints[k - 1]))
+      throw vtkm::cont::ErrorBadValue("MapperPathTracer: checkpoints must be >= 1 and strictly increasing");
+  auto* canvas = Internals->Canvas;
+  const vtkm::Id nx = canvas->GetWidth(), ny = canvas->GetHeight();
+  for (const auto& camera : cameras)
+    Internals->RayCamera.SetParameters(camera, *canvas); // validates every view like the reference (:372)
+  auto tup = extract(cellset);
+  auto SphereIds = std::get<0>(tup);
+  auto SphereRadii = std::get<1>(tup);
+  auto QuadIds = std::get<3>(tup);
+  vtkm::cont::ArrayHandle<vtkm::Int32> matIdArray, texIdArray;
+  matIdArray.Allocate(nx * ny);
+  texIdArray.Allocate(nx * ny);
+  buildBVH(coords, QuadIds, SphereIds, SphereRadii, matIdArray, texIdArray, MatIdx, TexIdx);
+  const std::vector<float> views = packViews(cameras);
+  const size_t n = checkpoints.size() * cameras.size() * static_cast<size_t>(nx * ny) * 4;
+  albedo.assign(n, 0.f);
+  normalDepth.assign(n, 0.f);
+  b2pt_ctx* ctx = b2pt_facade::Context(Devices.empty() ? -1 : Devices[0]);
+  b2pt_facade::Check(b2pt_seed(ctx, 0)); // the streams RenderCellsViews* render with
+  const unsigned int buildFlags =
+    B2PT_FLAG_FORCE_BVH | B2PT_FLAG_NO_DEDUP | B2PT_FLAG_NO_AA | B2PT_FLAG_GPU_LBVH | B2PT_FLAG_WIDE_BVH;
+  b2pt_facade::Check(b2pt_render_views_features(ctx, static_cast<int>(cameras.size()), views.data(),
+                                                static_cast<int>(nx), static_cast<int>(ny),
+                                                static_cast<int>(checkpoints.size()), checkpoints.data(),
+                                                RenderFlags & buildFlags, albedo.data(), normalDepth.data()));
+}
+
 void MapperPathTracer::SetCompositeBackground(bool on) { Internals->CompositeBackground = on; }
 
 void MapperPathTracer::StartScene()

@@ -116,6 +116,13 @@ public:
                                       const vtkm::cont::CoordinateSystem& coords,
                                       const std::vector<vtkm::rendering::Camera>& cameras,
                                       const std::vector<int>& checkpoints, std::vector<unsigned short>& pnm);
+  // Denoiser guides of the same sweep (b2pt_render_views_features, on the first device of SetDevices): for every
+  // checkpoint c (strictly increasing, ending with samplecount, else ErrorBadValue) and view v, the float4 sums over the
+  // primary hits of path samples 0 .. c-1, the samples RenderCellsViewsCheckpointsPnm renders:
+  // albedo[((k * V + v) * W*H + i) * 4 + ...] = (albedo rgb, hit count), normalDepth = (normal xyz, depth).
+  void RenderCellsViewsFeatures(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
+                                const std::vector<vtkm::rendering::Camera>& cameras, const std::vector<int>& checkpoints,
+                                std::vector<float>& albedo, std::vector<float>& normalDepth);
   // The -direct G-buffers of main.cc:402-422 (what MapperQuadNormals / MapperQuadAlbedo leave in the canvas colour
   // buffer, raytracing/RayTracerNormals.cxx / RayTracerAlbedo.cxx, and a depth image) for the canvas set with
   // SetCanvas: one un-jittered ray per pixel, closest quad hit, the reference's two Shade rules (b2pt_render_direct).

@@ -21,6 +21,13 @@
 // sweep with -samplecount c writes, next to the usual <out>-<phi>-<theta>.pnm of samplecount samples (a denoiser
 // dataset's noisy inputs and target from one sweep).  A malformed or non-increasing list, an entry >= samplecount,
 // -direct, or no sweep is an error (exit 1).
+// -features (with -hemisphere or -fibonacci, path-traced) also writes denoiser guide images of the same path samples,
+// for the default sample count and every -checkpoints count c: <stem>-albedo-<phi>-<theta>.pfm (PF, mean first-hit
+// albedo), <stem>-normal-<phi>-<theta>.pfm (PF, mean first-hit normal, not renormalised) and
+// <stem>-depth-<phi>-<theta>.pfm (Pf, mean hit distance of the samples that hit, 0 where none does), with <stem> =
+// <out> for samplecount samples and <out>-s<c> for a checkpoint.  PFM (little-endian float32, scale -1.0, rows bottom
+// first as the buffers are) because PNM cannot hold negative normals or distances beyond 255.  The radiance files
+// stay byte-identical to a run without -features.  -features with -direct, or without a sweep, is an error (exit 1).
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
@@ -54,6 +61,7 @@ struct Options
   bool checkpointsGiven = false;
   std::string checkpointsArg;
   std::vector<int> checkpoints; // -checkpoints, parsed and checked by checkCheckpoints
+  bool features = false;
 };
 
 Options parse(int argc, char** argv)
@@ -91,6 +99,8 @@ Options parse(int argc, char** argv)
       next(o.viewCount);
     else if (!std::strcmp(argv[i], "-viewseed"))
       next(o.viewSeed);
+    else if (!std::strcmp(argv[i], "-features"))
+      o.features = true;
     else if (!std::strcmp(argv[i], "-checkpoints"))
     {
       o.checkpointsGiven = true;
@@ -125,6 +135,18 @@ std::string checkCheckpoints(Options& o)
   }
   if (o.checkpoints.back() >= o.samples)
     return "-checkpoints entries must be below -samplecount (" + std::to_string(o.samples) + ")";
+  return "";
+}
+
+// Returns an error message for an unusable -features, empty when it is usable or absent.
+std::string checkFeatures(const Options& o)
+{
+  if (!o.features)
+    return "";
+  if (o.direct)
+    return "-features cannot be combined with -direct";
+  if (!o.hemi && !o.fibonacci)
+    return "-features needs -hemisphere or -fibonacci";
   return "";
 }
 
@@ -250,6 +272,20 @@ void savePnm16(const std::string& stem, int nx, int ny, const unsigned short* rg
   fs.write(buf.data(), static_cast<std::streamsize>(buf.size()));
 }
 
+// Portable float map: "PF" (rgb) or "Pf" (grey), scale -1.0 (little-endian float32: the host's own layout on the
+// x86-64 and aarch64 hosts of a B200), rows bottom first.
+void savePfm(const std::string& stem, int nx, int ny, int channels, const std::vector<float>& values)
+{
+  std::ofstream fs(stem + ".pfm", std::ios::binary);
+  if (!fs)
+  {
+    std::cout << "Couldn't save pfm." << std::endl;
+    return;
+  }
+  fs << (channels == 3 ? "PF" : "Pf") << "\n" << nx << " " << ny << "\n-1.0\n";
+  fs.write(reinterpret_cast<const char*>(values.data()), static_cast<std::streamsize>(values.size() * sizeof(float)));
+}
+
 std::string viewName(const std::string& stem, float phi, float theta)
 { // generate(): "output-" << fixed << setw(4) << setprecision(4) << phi << "-" << theta
   std::stringstream name;
@@ -305,12 +341,40 @@ int renderViews(CornellBox& cb, const Options& o, const std::vector<vtkm::render
               << "  path samples/s = " << double(o.x) * o.y * o.samples * double(cameras.size()) /
         (mapper.GetLastRenderMilliseconds() * 1e-3)
               << "  segments = " << mapper.GetLastSegments() << std::endl;
-  const size_t n3 = static_cast<size_t>(o.x) * o.y * 3, V = cameras.size();
+  const size_t n = static_cast<size_t>(o.x) * o.y, n3 = n * 3, V = cameras.size();
+  auto stemOf = [&](size_t k) { // slice k: counts[k] samples; the last is the ordinary image
+    return k + 1 < counts.size() ? o.out + "-s" + std::to_string(counts[k]) : o.out;
+  };
   for (size_t k = 0; k < counts.size(); ++k)
-  { // slice k of pnm: counts[k] samples; the last is the ordinary image
-    const std::string stem = k + 1 < counts.size() ? o.out + "-s" + std::to_string(counts[k]) : o.out;
     for (size_t v = 0; v < V; ++v)
-      savePnm16(viewName(stem, angles[v].first, angles[v].second), o.x, o.y, &pnm[(k * V + v) * n3]);
+      savePnm16(viewName(stemOf(k), angles[v].first, angles[v].second), o.x, o.y, &pnm[(k * V + v) * n3]);
+  if (o.features)
+  { // the guide images: sums over the samples of each count, as means
+    std::vector<float> albedo, normalDepth;
+    mapper.RenderCellsViewsFeatures(cb.ds.GetCellSet(), cb.coord, cameras, counts, albedo, normalDepth);
+    std::vector<float> alb(n3), nrm(n3), dep(n);
+    for (size_t k = 0; k < counts.size(); ++k)
+    {
+      const float c = static_cast<float>(counts[k]);
+      for (size_t v = 0; v < V; ++v)
+      {
+        const float* a = &albedo[(k * V + v) * n * 4];
+        const float* nd = &normalDepth[(k * V + v) * n * 4];
+        for (size_t i = 0; i < n; ++i)
+        {
+          for (int ch = 0; ch < 3; ++ch)
+          {
+            alb[3 * i + ch] = a[4 * i + ch] / c;
+            nrm[3 * i + ch] = nd[4 * i + ch] / c;
+          }
+          dep[i] = a[4 * i + 3] > 0.f ? nd[4 * i + 3] / a[4 * i + 3] : 0.f;
+        }
+        const std::string stem = stemOf(k);
+        savePfm(viewName(stem + "-albedo", angles[v].first, angles[v].second), o.x, o.y, 3, alb);
+        savePfm(viewName(stem + "-normal", angles[v].first, angles[v].second), o.x, o.y, 3, nrm);
+        savePfm(viewName(stem + "-depth", angles[v].first, angles[v].second), o.x, o.y, 1, dep);
+      }
+    }
   }
   return static_cast<int>(cameras.size());
 }
@@ -387,7 +451,9 @@ int fibonacciHemisphere(CornellBox& cb, const Options& o)
 int main(int argc, char* argv[])
 {
   Options o = parse(argc, argv);
-  const std::string bad = checkCheckpoints(o);
+  std::string bad = checkCheckpoints(o);
+  if (bad.empty())
+    bad = checkFeatures(o);
   if (!bad.empty())
   {
     std::cerr << "error: " << bad << std::endl;
