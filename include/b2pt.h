@@ -58,6 +58,10 @@ typedef enum b2pt_status
 #define B2PT_FLAG_SPLIT_TRACE 0x4000u        /* BVH scenes, binary tree, sorted rays: a lean traversal kernel (k_bvh_hits) followed by k_resolve_hits instead of one k_trace per bounce; bit-identical, measured 0.4 % slower on configs[3] (A/B runs) */
 #define B2PT_FLAG_NO_RAY_SORT 0x2000u        /* BVH scenes: trace the ray queue in the order k_shade left it instead of sorted by origin cell and direction octant (A/B runs) */
 #define B2PT_FLAG_NO_AA 0x10u               /* do not use the axis-aligned quad specialisation (A/B parity checks) */
+/* The build flags: the ones that choose and shape the trace structures (b2pt_build_bvh_ex); every other flag only
+ * affects a render. */
+#define B2PT_BUILD_FLAGS \
+  (B2PT_FLAG_FORCE_BVH | B2PT_FLAG_NO_DEDUP | B2PT_FLAG_NO_AA | B2PT_FLAG_GPU_LBVH | B2PT_FLAG_WIDE_BVH)
 
 typedef struct b2pt_stats
 {
@@ -102,8 +106,7 @@ int b2pt_set_scene(b2pt_ctx* ctx, const float* pts, int64_t nPts, const int64_t*
  * (pathtracing/SphereIntersector.cxx:46-76), FindQuadAABBs / FindSphereAABBs (pathtracing/AABBSurface.h) and
  * VTK-m's LinearBVH::Construct.  One tree over quads and spheres; small scenes skip the tree. */
 int b2pt_build_bvh(b2pt_ctx* ctx);
-/* Same with build-affecting flags (B2PT_FLAG_FORCE_BVH, _NO_DEDUP, _NO_AA, _GPU_LBVH); a later render with other
- * build flags rebuilds. */
+/* Same with build-affecting flags (B2PT_BUILD_FLAGS); a later render with other build flags rebuilds. */
 int b2pt_build_bvh_ex(b2pt_ctx* ctx, uint32_t flags);
 
 /* Moved spheres: new centres (3 floats per sphere, the order of b2pt_set_scene) and, optionally, radii; counts and
@@ -177,7 +180,7 @@ int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views,
  * float32 sums over s = 0 .. c-1 in sample order from +0.0, c = checkpoints[k]; layout [k][view][j*W+i] float4,
  * K*nViews*W*H*4 floats each; either may be NULL.  Means are sum / c; the mean depth of the hitting samples is
  * sum depth / sum hit.  views holds 10 floats per view as in b2pt_render_views.  flags may hold only the build flags
- * FORCE_BVH, NO_DEDUP, NO_AA, GPU_LBVH, WIDE_BVH, and (re)builds the trace structures as a render would.
+ * (B2PT_BUILD_FLAGS), and (re)builds the trace structures as a render would.
  * B2PT_ERR_BAD_VALUE, before anything runs: a bad view list or view (b2pt_set_camera's message), a checkpoint list of
  * other than 1..32 strictly increasing counts >= 1, checkpoints[K-1] > 2^24 (the hit count must stay an exact float),
  * another flag, or K*W*H > 2^30.  nViews == 0 does nothing; no scene gives B2PT_ERR_STATE.  Views run in chunks of

@@ -641,9 +641,7 @@ int b2pt_set_scene(b2pt_ctx* ctx, const float* pts, int64_t nPts, const int64_t*
   return B2PT_OK;
 }
 
-// The flags that choose and shape the trace structures (every other flag only affects a render).
-static constexpr uint32_t kBuildFlags =
-  B2PT_FLAG_FORCE_BVH | B2PT_FLAG_NO_DEDUP | B2PT_FLAG_NO_AA | B2PT_FLAG_GPU_LBVH | B2PT_FLAG_WIDE_BVH;
+static constexpr uint32_t kBuildFlags = B2PT_BUILD_FLAGS;
 
 static int build_trace_structures(b2pt_ctx* ctx, uint32_t flags)
 {
@@ -1292,6 +1290,38 @@ static void stored_up(const float up[3], float out[3])
   hst(out, upv);
 }
 
+// Checks of the view-sweep entry points; fn names the entry point in the messages.
+static int check_view_list(const char* fn, int nViews, const float* views)
+{
+  if (nViews < 0 || (nViews > 0 && !views))
+    return fail(B2PT_ERR_BAD_VALUE, "%s: bad view list", fn);
+  return B2PT_OK;
+}
+
+static int check_checkpoints(const char* fn, int nCheckpoints, const int* checkpoints)
+{
+  if (nCheckpoints < 1 || nCheckpoints > b2pt::kMaxCheckpoints || !checkpoints)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: nCheckpoints must be in [1,%d] with a non-NULL list", fn,
+                b2pt::kMaxCheckpoints);
+  for (int k = 0; k < nCheckpoints; ++k)
+    if (checkpoints[k] < 1 || (k > 0 && checkpoints[k] <= checkpoints[k - 1]))
+      return fail(B2PT_ERR_BAD_VALUE, "%s: checkpoints must be >= 1 and strictly increasing", fn);
+  return B2PT_OK;
+}
+
+// The camera of every row (pos[3], lookAt[3], up[3], fovDeg) of a view list, all on a W x H canvas.
+static int make_view_cameras(int nViews, const float* views, int W, int H, std::vector<B2Camera>& cams)
+{
+  cams.resize((size_t)nViews);
+  for (int v = 0; v < nViews; ++v)
+  {
+    const float* p = views + 10 * (size_t)v;
+    if (int rc = make_camera(p, p + 3, p + 6, p[9], W, H, cams[(size_t)v]))
+      return rc;
+  }
+  return B2PT_OK;
+}
+
 int b2pt_set_camera(b2pt_ctx* ctx, const float pos[3], const float lookAt[3], const float up[3], float fovDeg, int W,
                     int H)
 {
@@ -1781,20 +1811,19 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
     // (view batches write disjoint canvases: no order needed)
     if (overlap && batch > 0 && !viewMode)
       CU(cudaStreamWaitEvent(bs, ctx->evAcc[(set + nSets - 1) % nSets], 0));
+    // view mode: nv views of sampleCount samples each; otherwise nb samples of the one canvas
+    float4* const canvas = viewMode ? ctx->viewColor.p + v0 * N : ctx->color();
+    const int accSamples = viewMode ? sampleCount : (int)nb, accViews = viewMode ? (int)nv : 1;
     if (ckpt)
     {
       b2pt::CheckpointArgs ck = *ckpt;
       ck.sampleBase = A.sampleBase;
       ck.entry0 += v0 * N;
-      CU(b2pt::launch_accumulate_checkpoints(viewMode ? ctx->viewColor.p + v0 * N : ctx->color(), bb.rad.p, (int)N,
-                                             viewMode ? sampleCount : (int)nb, viewMode ? (int)nv : 1,
-                                             ctx->nanCounter.p, ck, bs));
+      CU(b2pt::launch_accumulate_checkpoints(canvas, bb.rad.p, (int)N, accSamples, accViews, ctx->nanCounter.p, ck,
+                                             bs));
     }
-    else if (viewMode)
-      CU(b2pt::launch_accumulate(ctx->viewColor.p + v0 * N, bb.rad.p, (int)N, sampleCount, (int)nv,
-                                 ctx->nanCounter.p, bs));
     else
-      CU(b2pt::launch_accumulate(ctx->color(), bb.rad.p, (int)N, (int)nb, 1, ctx->nanCounter.p, bs));
+      CU(b2pt::launch_accumulate(canvas, bb.rad.p, (int)N, accSamples, accViews, ctx->nanCounter.p, bs));
     ++launches;
     if (overlap)
       CU(cudaEventRecord(ctx->evAcc[set], bs));
@@ -1919,146 +1948,24 @@ int b2pt_render_range(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxDe
   return render_impl(ctx, sampleBegin, sampleCount, maxDepth, flags, 0);
 }
 
-int b2pt_render_views(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int spp, int maxDepth,
-                      uint32_t flags, void* rgbaOut)
+// The view sweep of b2pt_render_views and b2pt_render_views_checkpoints once their arguments are checked: counts[K-1]
+// samples of every camera of `cams` (one canvas size) into ctx->viewColor, then for every count k the image its entry
+// point returns, converted per the view flags and copied to slice k of rgbaOut (NULL: no copy).  ck == nullptr
+// (b2pt_render_views, K == 1, no moments): the batches accumulate through k_accumulate.  Otherwise ck holds the
+// checkpoint list (n, count) and they accumulate through k_accumulate_checkpoints, which keeps the running sums at
+// every count and, when moment2Out is not NULL, the sums of squares.
+static int render_view_sweep(b2pt_ctx* ctx, const std::vector<B2Camera>& cams, const int* counts, int K, int maxDepth,
+                             uint32_t flags, b2pt::CheckpointArgs* ck, void* rgbaOut, float* moment2Out)
 {
-  if (int rc = bind(ctx))
-    return rc;
-  if (nViews < 0 || (nViews > 0 && !views))
-    return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views: bad view list");
-  if (spp < 0)
-    return fail(B2PT_ERR_BAD_VALUE, "negative sample range");
-  if (flags & B2PT_FLAG_REFERENCE_STREAM)
-    return fail(B2PT_ERR_BAD_VALUE, "REFERENCE_STREAM cannot be combined with a view-batched render");
-  if ((flags & B2PT_FLAG_VIEWS_PNM16) && spp <= 0)
-    return fail(B2PT_ERR_BAD_VALUE, "spp must be positive"); // the PNM integers divide by spp
-  std::vector<B2Camera> cams((size_t)nViews);
-  for (int v = 0; v < nViews; ++v)
-  {
-    const float* p = views + 10 * (size_t)v;
-    if (int rc = make_camera(p, p + 3, p + 6, p[9], W, H, cams[(size_t)v]))
-      return rc;
-  }
+  const int64_t nViews = (int64_t)cams.size();
   if (nViews == 0)
   {
     ctx->viewCount = 0;
     return B2PT_OK;
   }
-  const int64_t N = (int64_t)W * H;
-  if (N * nViews > (int64_t)1 << 30)
-    return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views: more than 2^30 output pixels (16 GiB); split the view list");
-  CU(ctx->viewColor.reserve((size_t)(N * nViews)));
-  CU(ctx->dViews.reserve((size_t)nViews));
-  ctx->viewCount = nViews;
-  ctx->viewPixels = N;
-  // the context's own camera gives the canvas shape to the launches; it is restored afterwards
-  const B2Camera savedCam = ctx->cam;
-  const bool savedHave = ctx->haveCamera;
-  float4* const savedExt = ctx->colorExt;
-  CU(cudaMemsetAsync(ctx->viewColor.p, 0, sizeof(float4) * (size_t)(N * nViews), ctx->stream));
-  ctx->cam = cams[0];
-  ctx->haveCamera = true;
-  int rc = B2PT_OK;
-  auto restore = [&]() {
-    ctx->cam = savedCam;
-    ctx->haveCamera = savedHave;
-    ctx->colorExt = savedExt;
-  };
-  bool perView = !(spp > 0 && N * spp <= std::min<int64_t>(batch_target_paths(ctx, true), 0xfffffff0LL));
-  if (!perView)
-  { // whole views fit a batch: (view, sample, pixel) is one flat index space, one set of launches per batch of views
-    // (pageable source: the copy is staged before the call returns, so `cams` may go out of scope)
-    cudaError_t e = cudaMemcpyAsync(ctx->dViews.p, cams.data(), sizeof(B2Camera) * (size_t)nViews,
-                                    cudaMemcpyHostToDevice, ctx->stream);
-    if (e != cudaSuccess)
-    {
-      restore();
-      return fail(B2PT_ERR_CUDA, "cudaMemcpyAsync(views): %s", cudaGetErrorString(e));
-    }
-    rc = render_impl(ctx, 0, spp, maxDepth, flags, nViews);
-    perView = rc == B2PT_ERR_ALLOC; // the buffers of a whole-view batch could not be allocated: views one by one
-  }
-  if (perView)
-  { // a single view already fills several batches: one ordinary render per view into its slice
-    rc = B2PT_OK;
-    if (cudaMemsetAsync(ctx->viewColor.p, 0, sizeof(float4) * (size_t)(N * nViews), ctx->stream) != cudaSuccess)
-      rc = fail(B2PT_ERR_CUDA, "clearing the view canvases failed");
-    int64_t paths = 0, launches = 0;
-    for (int v = 0; v < nViews && rc == B2PT_OK; ++v)
-    {
-      ctx->cam = cams[(size_t)v];
-      ctx->colorExt = ctx->viewColor.p + (size_t)v * N;
-      rc = render_impl(ctx, 0, spp, maxDepth, flags, 0);
-      paths += ctx->stats.paths;
-      launches += ctx->stats.launches;
-    }
-    ctx->stats.paths = paths;
-    ctx->stats.launches = launches;
-  }
-  restore();
-  if (rc != B2PT_OK)
-    return rc;
-  if (flags & B2PT_FLAG_VIEWS_PNM16)
-  { // the integers of the reference's P3 writer instead of the float sums: 6 B instead of 16 B per pixel to the host
-    CU(ctx->pnm.reserve((size_t)(N * nViews) * 3));
-    CU(b2pt::launch_pnm16(ctx->viewColor.p, N * nViews, spp, ctx->pnm.p, ctx->stream));
-    if (rgbaOut)
-    {
-      CU(cudaMemcpyAsync(rgbaOut, ctx->pnm.p, sizeof(uint16_t) * 3 * (size_t)(N * nViews), cudaMemcpyDeviceToHost,
-                         ctx->stream));
-      CU(cudaStreamSynchronize(ctx->stream));
-    }
-    return B2PT_OK;
-  }
-  if (flags & B2PT_FLAG_VIEWS_NORMALIZE)
-    CU(b2pt::launch_normalize(ctx->viewColor.p, N * nViews, spp, ctx->stream));
-  if (rgbaOut)
-  {
-    CU(cudaMemcpyAsync(rgbaOut, ctx->viewColor.p, sizeof(float4) * (size_t)(N * nViews), cudaMemcpyDeviceToHost,
-                       ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-  }
-  return B2PT_OK;
-}
-
-// b2pt_render_views at spp = checkpoints[K-1] through k_accumulate_checkpoints: sample s of a pixel is the same RNG
-// stream and is added in the same order at every spp, so the prefix sum after checkpoints[k] samples is the image
-// b2pt_render_views(spp = checkpoints[k]) returns, whatever the batching.
-int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
-                                  const int* checkpoints, int maxDepth, uint32_t flags, void* rgbaOut,
-                                  float* moment2Out)
-{
-  if (int rc = bind(ctx))
-    return rc;
-  if (nViews < 0 || (nViews > 0 && !views))
-    return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views_checkpoints: bad view list");
-  if (nCheckpoints < 1 || nCheckpoints > b2pt::kMaxCheckpoints || !checkpoints)
-    return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views_checkpoints: nCheckpoints must be in [1,%d] with a non-NULL list",
-                b2pt::kMaxCheckpoints);
-  for (int k = 0; k < nCheckpoints; ++k)
-    if (checkpoints[k] < 1 || (k > 0 && checkpoints[k] <= checkpoints[k - 1]))
-      return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views_checkpoints: checkpoints must be >= 1 and strictly increasing");
-  if (flags & B2PT_FLAG_REFERENCE_STREAM)
-    return fail(B2PT_ERR_BAD_VALUE, "REFERENCE_STREAM cannot be combined with a view-batched render");
-  std::vector<B2Camera> cams((size_t)nViews);
-  for (int v = 0; v < nViews; ++v)
-  {
-    const float* p = views + 10 * (size_t)v;
-    if (int rc = make_camera(p, p + 3, p + 6, p[9], W, H, cams[(size_t)v]))
-      return rc;
-  }
-  if (nViews == 0)
-  {
-    ctx->viewCount = 0;
-    return B2PT_OK;
-  }
-  const int K = nCheckpoints, spp = checkpoints[K - 1];
-  const int64_t N = (int64_t)W * H, NV = N * nViews;
+  const int spp = counts[K - 1];
+  const int64_t N = (int64_t)cams[0].W * cams[0].H, NV = N * nViews;
   const bool moments = moment2Out != nullptr;
-  const int64_t slices = (K - 1) + (moments ? K : 0) + 1; // snapshots, sums of squares, the last image
-  if (NV > ((int64_t)1 << 30) / slices)
-    return fail(B2PT_ERR_BAD_VALUE,
-                "b2pt_render_views_checkpoints: more than 2^30 float4 of device output (16 GiB); split the view list");
   CU(ctx->viewColor.reserve((size_t)NV));
   CU(ctx->dViews.reserve((size_t)nViews));
   if (K > 1)
@@ -2067,12 +1974,12 @@ int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views,
     CU(ctx->ckptMoment.reserve((size_t)(NV * K)));
   ctx->viewCount = nViews;
   ctx->viewPixels = N;
-  b2pt::CheckpointArgs ck{};
-  ck.n = K;
-  std::copy(checkpoints, checkpoints + K, ck.count);
-  ck.snap = ctx->ckptSnap.p;
-  ck.moment = moments ? ctx->ckptMoment.p : nullptr;
-  ck.sliceStride = NV;
+  if (ck)
+  {
+    ck->snap = ctx->ckptSnap.p;
+    ck->moment = moments ? ctx->ckptMoment.p : nullptr;
+    ck->sliceStride = NV;
+  }
   // the running sums start from zero: the image and the running sum of squares (slice K-1); every other slice is
   // written exactly once
   auto clear = [&]() -> cudaError_t {
@@ -2094,10 +2001,10 @@ int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views,
     ctx->haveCamera = savedHave;
     ctx->colorExt = savedExt;
   };
-  // b2pt_render_views' batching rule for spp = checkpoints[K-1]
-  bool perView = !(N * spp <= std::min<int64_t>(batch_target_paths(ctx, true), 0xfffffff0LL));
+  bool perView = !(spp > 0 && N * spp <= std::min<int64_t>(batch_target_paths(ctx, true), 0xfffffff0LL));
   if (!perView)
-  {
+  { // whole views fit a batch: (view, sample, pixel) is one flat index space, one set of launches per batch of views
+    // (pageable source: the copy is staged before the call returns, so `cams` may go out of scope)
     cudaError_t e = cudaMemcpyAsync(ctx->dViews.p, cams.data(), sizeof(B2Camera) * (size_t)nViews,
                                     cudaMemcpyHostToDevice, ctx->stream);
     if (e != cudaSuccess)
@@ -2105,22 +2012,23 @@ int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views,
       restore();
       return fail(B2PT_ERR_CUDA, "cudaMemcpyAsync(views): %s", cudaGetErrorString(e));
     }
-    rc = render_impl(ctx, 0, spp, maxDepth, flags, nViews, &ck);
-    perView = rc == B2PT_ERR_ALLOC;
+    rc = render_impl(ctx, 0, spp, maxDepth, flags, nViews, ck);
+    perView = rc == B2PT_ERR_ALLOC; // the buffers of a whole-view batch could not be allocated: views one by one
   }
   if (perView)
-  { // one render per view into its slice of every output; sample batches carry the running sums in viewColor and
-    // moment slice K-1
+  { // a single view already fills several batches: one ordinary render per view into its slice of every output;
+    // sample batches carry the running sums in viewColor and moment slice K-1
     rc = B2PT_OK;
     if (clear() != cudaSuccess)
       rc = fail(B2PT_ERR_CUDA, "clearing the view canvases failed");
     int64_t paths = 0, launches = 0;
-    for (int v = 0; v < nViews && rc == B2PT_OK; ++v)
+    for (int64_t v = 0; v < nViews && rc == B2PT_OK; ++v)
     {
       ctx->cam = cams[(size_t)v];
       ctx->colorExt = ctx->viewColor.p + (size_t)v * N;
-      ck.entry0 = v * N;
-      rc = render_impl(ctx, 0, spp, maxDepth, flags, 0, &ck);
+      if (ck)
+        ck->entry0 = v * N;
+      rc = render_impl(ctx, 0, spp, maxDepth, flags, 0, ck);
       paths += ctx->stats.paths;
       launches += ctx->stats.launches;
     }
@@ -2130,22 +2038,22 @@ int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views,
   restore();
   if (rc != B2PT_OK)
     return rc;
-  // per checkpoint, the conversion b2pt_render_views applies to its image (the last one is viewColor itself)
+  // per count, the conversion the view flags ask for (the last image is viewColor itself)
   for (int k = 0; k < K; ++k)
   {
     float4* const img = k + 1 < K ? ctx->ckptSnap.p + NV * k : ctx->viewColor.p;
     if (flags & B2PT_FLAG_VIEWS_PNM16)
-    {
+    { // the integers of the reference's P3 writer instead of the float sums: 6 B instead of 16 B per pixel to the host
       if (!rgbaOut)
         break;
       CU(ctx->pnm.reserve((size_t)NV * 3));
-      CU(b2pt::launch_pnm16(img, NV, checkpoints[k], ctx->pnm.p, ctx->stream));
+      CU(b2pt::launch_pnm16(img, NV, counts[k], ctx->pnm.p, ctx->stream));
       CU(cudaMemcpyAsync(static_cast<uint16_t*>(rgbaOut) + (size_t)(NV * k) * 3, ctx->pnm.p,
                          sizeof(uint16_t) * 3 * (size_t)NV, cudaMemcpyDeviceToHost, ctx->stream));
       continue;
     }
     if ((flags & B2PT_FLAG_VIEWS_NORMALIZE) && (rgbaOut || k + 1 == K))
-      CU(b2pt::launch_normalize(img, NV, checkpoints[k], ctx->stream));
+      CU(b2pt::launch_normalize(img, NV, counts[k], ctx->stream));
     if (rgbaOut)
       CU(cudaMemcpyAsync(static_cast<float4*>(rgbaOut) + NV * k, img, sizeof(float4) * (size_t)NV,
                          cudaMemcpyDeviceToHost, ctx->stream));
@@ -2156,6 +2064,56 @@ int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views,
   if (rgbaOut || moments)
     CU(cudaStreamSynchronize(ctx->stream));
   return B2PT_OK;
+}
+
+int b2pt_render_views(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int spp, int maxDepth,
+                      uint32_t flags, void* rgbaOut)
+{
+  if (int rc = bind(ctx))
+    return rc;
+  if (int rc = check_view_list("b2pt_render_views", nViews, views))
+    return rc;
+  if (spp < 0)
+    return fail(B2PT_ERR_BAD_VALUE, "negative sample range");
+  if (flags & B2PT_FLAG_REFERENCE_STREAM)
+    return fail(B2PT_ERR_BAD_VALUE, "REFERENCE_STREAM cannot be combined with a view-batched render");
+  if ((flags & B2PT_FLAG_VIEWS_PNM16) && spp <= 0)
+    return fail(B2PT_ERR_BAD_VALUE, "spp must be positive"); // the PNM integers divide by spp
+  std::vector<B2Camera> cams;
+  if (int rc = make_view_cameras(nViews, views, W, H, cams))
+    return rc;
+  if ((int64_t)W * H * nViews > (int64_t)1 << 30)
+    return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views: more than 2^30 output pixels (16 GiB); split the view list");
+  return render_view_sweep(ctx, cams, &spp, 1, maxDepth, flags, nullptr, rgbaOut, nullptr);
+}
+
+// b2pt_render_views at spp = checkpoints[K-1] through k_accumulate_checkpoints: sample s of a pixel is the same RNG
+// stream and is added in the same order at every spp, so the prefix sum after checkpoints[k] samples is the image
+// b2pt_render_views(spp = checkpoints[k]) returns, whatever the batching.
+int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
+                                  const int* checkpoints, int maxDepth, uint32_t flags, void* rgbaOut,
+                                  float* moment2Out)
+{
+  if (int rc = bind(ctx))
+    return rc;
+  if (int rc = check_view_list("b2pt_render_views_checkpoints", nViews, views))
+    return rc;
+  if (int rc = check_checkpoints("b2pt_render_views_checkpoints", nCheckpoints, checkpoints))
+    return rc;
+  if (flags & B2PT_FLAG_REFERENCE_STREAM)
+    return fail(B2PT_ERR_BAD_VALUE, "REFERENCE_STREAM cannot be combined with a view-batched render");
+  std::vector<B2Camera> cams;
+  if (int rc = make_view_cameras(nViews, views, W, H, cams))
+    return rc;
+  const int K = nCheckpoints;
+  const int64_t slices = (K - 1) + (moment2Out ? K : 0) + 1; // snapshots, sums of squares, the last image
+  if ((int64_t)W * H * nViews > ((int64_t)1 << 30) / slices)
+    return fail(B2PT_ERR_BAD_VALUE,
+                "b2pt_render_views_checkpoints: more than 2^30 float4 of device output (16 GiB); split the view list");
+  b2pt::CheckpointArgs ck{};
+  ck.n = K;
+  std::copy(checkpoints, checkpoints + K, ck.count);
+  return render_view_sweep(ctx, cams, ck.count, K, maxDepth, flags, &ck, rgbaOut, moment2Out);
 }
 
 // Denoiser guides of a view sweep (k_view_features).  Sample s of a pixel is traced from the stream the render gives it
@@ -2169,27 +2127,19 @@ int b2pt_render_views_features(b2pt_ctx* ctx, int nViews, const float* views, in
 {
   if (int rc = bind(ctx))
     return rc;
-  if (nViews < 0 || (nViews > 0 && !views))
-    return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views_features: bad view list");
-  if (nCheckpoints < 1 || nCheckpoints > b2pt::kMaxCheckpoints || !checkpoints)
-    return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views_features: nCheckpoints must be in [1,%d] with a non-NULL list",
-                b2pt::kMaxCheckpoints);
-  for (int k = 0; k < nCheckpoints; ++k)
-    if (checkpoints[k] < 1 || (k > 0 && checkpoints[k] <= checkpoints[k - 1]))
-      return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views_features: checkpoints must be >= 1 and strictly increasing");
+  if (int rc = check_view_list("b2pt_render_views_features", nViews, views))
+    return rc;
+  if (int rc = check_checkpoints("b2pt_render_views_features", nCheckpoints, checkpoints))
+    return rc;
   if (checkpoints[nCheckpoints - 1] > (1 << 24))
     return fail(B2PT_ERR_BAD_VALUE,
                 "b2pt_render_views_features: more than 2^24 samples (the hit count must stay an exact float)");
   if (flags & ~kBuildFlags)
     return fail(B2PT_ERR_BAD_VALUE,
                 "b2pt_render_views_features: flags may only hold FORCE_BVH, NO_DEDUP, NO_AA, GPU_LBVH and WIDE_BVH");
-  std::vector<B2Camera> cams((size_t)nViews);
-  for (int v = 0; v < nViews; ++v)
-  {
-    const float* p = views + 10 * (size_t)v;
-    if (int rc = make_camera(p, p + 3, p + 6, p[9], W, H, cams[(size_t)v]))
-      return rc;
-  }
+  std::vector<B2Camera> cams;
+  if (int rc = make_view_cameras(nViews, views, W, H, cams))
+    return rc;
   if (nViews == 0)
     return B2PT_OK;
   const int K = nCheckpoints;
@@ -2464,15 +2414,17 @@ int b2pt_render_direct_views(b2pt_ctx* ctx, int nViews, const float* views, int 
 {
   if (int rc = bind(ctx))
     return rc;
-  if (nViews < 0 || (nViews > 0 && !views))
-    return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_direct_views: bad view list");
+  if (int rc = check_view_list("b2pt_render_direct_views", nViews, views))
+    return rc;
+  std::vector<B2Camera> cams;
+  if (int rc = make_view_cameras(nViews, views, W, H, cams))
+    return rc;
   std::vector<b2pt::DirectView> dv((size_t)nViews);
   for (int v = 0; v < nViews; ++v)
   {
     const float* p = views + 10 * (size_t)v;
     b2pt::DirectView& d = dv[(size_t)v];
-    if (int rc = make_camera(p, p + 3, p + 6, p[9], W, H, d.cam))
-      return rc;
+    d.cam = cams[(size_t)v];
     for (int c = 0; c < 3; ++c)
       d.lookAt[c] = p[3 + c];
     stored_up(p + 6, d.upN);

@@ -2166,21 +2166,30 @@ cudaError_t launch_sort_rays(const B2RenderArgs& args, const float lo[3], const 
   return cudaGetLastError();
 }
 
+// Calls f with the scene a launch traverses: the 8-wide tree when bvh->wide (a B2WideScene built from *bvh), else the
+// binary tree *bvh, else the small scene *small.  Returns what f returns.
+template <class F>
+static auto with_trace_scene(const B2SmallScene* small, const B2BvhScene* bvh, F&& f)
+{
+  if (bvh && bvh->wide)
+  {
+    B2WideScene ws;
+    static_cast<B2BvhScene&>(ws) = *bvh;
+    return f(static_cast<const B2WideScene&>(ws));
+  }
+  if (bvh)
+    return f(*bvh);
+  return f(*small);
+}
+
 cudaError_t launch_tail_loop(const B2Camera& cam, const B2SmallScene* small, const B2BvhScene* bvh,
                              const B2Lights& lights, const B2RenderArgs& args, cudaStream_t stream)
 {
   if (args.depth < 1)
     return cudaErrorInvalidValue;
-  if (bvh && bvh->wide)
-  {
-    B2WideScene ws;
-    static_cast<B2BvhScene&>(ws) = *bvh;
-    k_tail_loop<B2WideScene><<<kTailCluster, kTailBlock, 0, stream>>>(cam, ws, lights, args);
-  }
-  else if (bvh)
-    k_tail_loop<B2BvhScene><<<kTailCluster, kTailBlock, 0, stream>>>(cam, *bvh, lights, args);
-  else
-    k_tail_loop<B2SmallScene><<<kTailCluster, kTailBlock, 0, stream>>>(cam, *small, lights, args);
+  with_trace_scene(small, bvh, [&](const auto& S) {
+    k_tail_loop<std::decay_t<decltype(S)>><<<kTailCluster, kTailBlock, 0, stream>>>(cam, S, lights, args);
+  });
   return cudaGetLastError();
 }
 
@@ -2188,15 +2197,9 @@ cudaError_t launch_bounce(const LaunchCfg& cfg, bool primary, int mode, const B2
                           const B2BvhScene* bvh, const B2Lights& lights, const B2RenderArgs& args,
                           cudaStream_t stream, cudaEvent_t betweenStages)
 {
-  if (bvh && bvh->wide)
-  {
-    B2WideScene ws;
-    static_cast<B2BvhScene&>(ws) = *bvh;
-    return launch_bounce_t(cfg, primary, mode, cam, ws, lights, args, stream, betweenStages);
-  }
-  if (bvh)
-    return launch_bounce_t(cfg, primary, mode, cam, *bvh, lights, args, stream, betweenStages);
-  return launch_bounce_t(cfg, primary, mode, cam, *small, lights, args, stream, betweenStages);
+  return with_trace_scene(small, bvh, [&](const auto& S) {
+    return launch_bounce_t(cfg, primary, mode, cam, S, lights, args, stream, betweenStages);
+  });
 }
 
 int warps_per_block() { return kWarps; }
@@ -2248,16 +2251,9 @@ cudaError_t launch_primary_hits(const B2Camera& cam, const B2SmallScene* small, 
                                 uint32_t seedOffset, int32_t* primOut, float* tOut, cudaStream_t stream)
 {
   const int n = cam.W * cam.H;
-  if (bvh && bvh->wide)
-  {
-    B2WideScene ws;
-    static_cast<B2BvhScene&>(ws) = *bvh;
-    k_primary_hits<B2WideScene><<<(n + 255) / 256, 256, 0, stream>>>(cam, ws, seedOffset, primOut, tOut);
-  }
-  else if (bvh)
-    k_primary_hits<B2BvhScene><<<(n + 255) / 256, 256, 0, stream>>>(cam, *bvh, seedOffset, primOut, tOut);
-  else
-    k_primary_hits<B2SmallScene><<<(n + 255) / 256, 256, 0, stream>>>(cam, *small, seedOffset, primOut, tOut);
+  with_trace_scene(small, bvh, [&](const auto& S) {
+    k_primary_hits<std::decay_t<decltype(S)>><<<(n + 255) / 256, 256, 0, stream>>>(cam, S, seedOffset, primOut, tOut);
+  });
   return cudaGetLastError();
 }
 
@@ -2294,19 +2290,10 @@ cudaError_t launch_view_features(const B2SmallScene* small, const B2BvhScene* bv
   uint32_t magic, shift;
   make_fastdiv((uint32_t)nPixels, magic, shift);
   const unsigned grid = (unsigned)((n + 255) / 256);
-  if (bvh && bvh->wide)
-  {
-    B2WideScene ws;
-    static_cast<B2BvhScene&>(ws) = *bvh;
-    k_view_features<B2WideScene><<<grid, 256, 0, stream>>>(ws, cams, n, (uint32_t)nPixels, magic, shift, seedOffset,
-                                                           ck, albedo, normalDepth);
-  }
-  else if (bvh)
-    k_view_features<B2BvhScene><<<grid, 256, 0, stream>>>(*bvh, cams, n, (uint32_t)nPixels, magic, shift, seedOffset,
-                                                          ck, albedo, normalDepth);
-  else
-    k_view_features<B2SmallScene><<<grid, 256, 0, stream>>>(*small, cams, n, (uint32_t)nPixels, magic, shift,
-                                                            seedOffset, ck, albedo, normalDepth);
+  with_trace_scene(small, bvh, [&](const auto& S) {
+    k_view_features<std::decay_t<decltype(S)>><<<grid, 256, 0, stream>>>(S, cams, n, (uint32_t)nPixels, magic, shift,
+                                                                         seedOffset, ck, albedo, normalDepth);
+  });
   return cudaGetLastError();
 }
 
@@ -2326,19 +2313,10 @@ cudaError_t launch_intersect(const B2SmallScene* small, const B2BvhScene* bvh, i
   const unsigned grid = (unsigned)((n + 255) / 256);
   if (grid == 0)
     return cudaSuccess;
-  if (bvh && bvh->wide)
-  {
-    B2WideScene ws;
-    static_cast<B2BvhScene&>(ws) = *bvh;
-    k_intersect<B2WideScene>
-      <<<grid, 256, 0, stream>>>(ws, n, ox, oy, oz, dx, dy, dz, tmin, tmax, primId, hrec9, matId, texId);
-  }
-  else if (bvh)
-    k_intersect<B2BvhScene>
-      <<<grid, 256, 0, stream>>>(*bvh, n, ox, oy, oz, dx, dy, dz, tmin, tmax, primId, hrec9, matId, texId);
-  else
-    k_intersect<B2SmallScene>
-      <<<grid, 256, 0, stream>>>(*small, n, ox, oy, oz, dx, dy, dz, tmin, tmax, primId, hrec9, matId, texId);
+  with_trace_scene(small, bvh, [&](const auto& S) {
+    k_intersect<std::decay_t<decltype(S)>>
+      <<<grid, 256, 0, stream>>>(S, n, ox, oy, oz, dx, dy, dz, tmin, tmax, primId, hrec9, matId, texId);
+  });
   return cudaGetLastError();
 }
 

@@ -324,12 +324,19 @@ static std::vector<float> packViews(const std::vector<vtkm::rendering::Camera>& 
   return views;
 }
 
-void MapperPathTracer::RenderDirectBuffersViews(const vtkm::cont::DynamicCellSet& cellset,
-                                                const vtkm::cont::CoordinateSystem& coords,
-                                                const std::vector<vtkm::rendering::Camera>& cameras,
-                                                std::vector<vtkm::cont::ArrayHandle<vtkm::Vec<vtkm::Float32, 4>>>& normals,
-                                                std::vector<vtkm::cont::ArrayHandle<vtkm::Vec<vtkm::Float32, 4>>>& albedo,
-                                                std::vector<vtkm::cont::ArrayHandle<vtkm::Float32>>& depth)
+// A sweep's checkpoint list: strictly increasing counts >= 1 that end with the sample count.
+static void CheckCheckpoints(const std::vector<int>& checkpoints, int samplecount)
+{
+  if (checkpoints.empty() || checkpoints.back() != samplecount)
+    throw vtkm::cont::ErrorBadValue("MapperPathTracer: the checkpoint list must end with the sample count");
+  for (size_t k = 0; k < checkpoints.size(); ++k)
+    if (checkpoints[k] < 1 || (k > 0 && checkpoints[k] <= checkpoints[k - 1]))
+      throw vtkm::cont::ErrorBadValue("MapperPathTracer: checkpoints must be >= 1 and strictly increasing");
+}
+
+std::vector<float> MapperPathTracer::PrepareSweep(const vtkm::cont::DynamicCellSet& cellset,
+                                                  const vtkm::cont::CoordinateSystem& coords,
+                                                  const std::vector<vtkm::rendering::Camera>& cameras)
 {
   if (Internals->Canvas == nullptr)
     throw vtkm::cont::ErrorBadValue("MapperPathTracer: no canvas set");
@@ -345,7 +352,18 @@ void MapperPathTracer::RenderDirectBuffersViews(const vtkm::cont::DynamicCellSet
   matIdArray.Allocate(nx * ny);
   texIdArray.Allocate(nx * ny);
   buildBVH(coords, QuadIds, SphereIds, SphereRadii, matIdArray, texIdArray, MatIdx, TexIdx);
-  const std::vector<float> views = packViews(cameras);
+  return packViews(cameras);
+}
+
+void MapperPathTracer::RenderDirectBuffersViews(const vtkm::cont::DynamicCellSet& cellset,
+                                                const vtkm::cont::CoordinateSystem& coords,
+                                                const std::vector<vtkm::rendering::Camera>& cameras,
+                                                std::vector<vtkm::cont::ArrayHandle<vtkm::Vec<vtkm::Float32, 4>>>& normals,
+                                                std::vector<vtkm::cont::ArrayHandle<vtkm::Vec<vtkm::Float32, 4>>>& albedo,
+                                                std::vector<vtkm::cont::ArrayHandle<vtkm::Float32>>& depth)
+{
+  const std::vector<float> views = PrepareSweep(cellset, coords, cameras);
+  const vtkm::Id nx = Internals->Canvas->GetWidth(), ny = Internals->Canvas->GetHeight();
   const size_t n = static_cast<size_t>(nx * ny), V = cameras.size();
   std::vector<float> nrm(V * n * 4), alb(V * n * 4), dep(V * n);
   b2pt_ctx* ctx = b2pt_facade::Context(Devices.empty() ? -1 : Devices[0]);
@@ -370,22 +388,8 @@ void MapperPathTracer::RenderViewsImpl(const vtkm::cont::DynamicCellSet& cellset
                                        const std::vector<vtkm::rendering::Camera>& cameras, unsigned int flags,
                                        void* out, const std::vector<int>* checkpoints)
 {
-  if (Internals->Canvas == nullptr)
-    throw vtkm::cont::ErrorBadValue("MapperPathTracer: no canvas set");
-  auto* canvas = Internals->Canvas;
-  const vtkm::Id nx = canvas->GetWidth(), ny = canvas->GetHeight();
-  for (const auto& camera : cameras)
-    Internals->RayCamera.SetParameters(camera, *canvas); // validates every view like the reference (:372)
-  auto tup = extract(cellset);
-  auto SphereIds = std::get<0>(tup);
-  auto SphereRadii = std::get<1>(tup);
-  auto QuadIds = std::get<3>(tup);
-  vtkm::cont::ArrayHandle<vtkm::Int32> matIdArray, texIdArray;
-  matIdArray.Allocate(nx * ny);
-  texIdArray.Allocate(nx * ny);
-  buildBVH(coords, QuadIds, SphereIds, SphereRadii, matIdArray, texIdArray, MatIdx, TexIdx);
-
-  std::vector<float> views = packViews(cameras);
+  std::vector<float> views = PrepareSweep(cellset, coords, cameras);
+  const vtkm::Id nx = Internals->Canvas->GetWidth(), ny = Internals->Canvas->GetHeight();
   b2pt_ctx* ctx = b2pt_facade::Context();
   b2pt_facade::Check(b2pt_seed(ctx, 0)); // seeds[i] = i, MapperPathTracer.cxx:265-267
   if (checkpoints)
@@ -440,11 +444,7 @@ void MapperPathTracer::RenderCellsViewsCheckpointsPnm(const vtkm::cont::DynamicC
 {
   if (Internals->Canvas == nullptr)
     throw vtkm::cont::ErrorBadValue("MapperPathTracer: no canvas set");
-  if (checkpoints.empty() || checkpoints.back() != samplecount)
-    throw vtkm::cont::ErrorBadValue("MapperPathTracer: the checkpoint list must end with the sample count");
-  for (size_t k = 0; k < checkpoints.size(); ++k)
-    if (checkpoints[k] < 1 || (k > 0 && checkpoints[k] <= checkpoints[k - 1]))
-      throw vtkm::cont::ErrorBadValue("MapperPathTracer: checkpoints must be >= 1 and strictly increasing");
+  CheckCheckpoints(checkpoints, samplecount);
   const size_t n = static_cast<size_t>(Internals->Canvas->GetWidth()) * Internals->Canvas->GetHeight();
   pnm.assign(checkpoints.size() * cameras.size() * n * 3, 0);
   RenderViewsImpl(cellset, coords, cameras, B2PT_FLAG_VIEWS_PNM16, pnm.data(), &checkpoints);
@@ -458,35 +458,18 @@ void MapperPathTracer::RenderCellsViewsFeatures(const vtkm::cont::DynamicCellSet
 {
   if (Internals->Canvas == nullptr)
     throw vtkm::cont::ErrorBadValue("MapperPathTracer: no canvas set");
-  if (checkpoints.empty() || checkpoints.back() != samplecount)
-    throw vtkm::cont::ErrorBadValue("MapperPathTracer: the checkpoint list must end with the sample count");
-  for (size_t k = 0; k < checkpoints.size(); ++k)
-    if (checkpoints[k] < 1 || (k > 0 && checkpoints[k] <= checkpoints[k - 1]))
-      throw vtkm::cont::ErrorBadValue("MapperPathTracer: checkpoints must be >= 1 and strictly increasing");
-  auto* canvas = Internals->Canvas;
-  const vtkm::Id nx = canvas->GetWidth(), ny = canvas->GetHeight();
-  for (const auto& camera : cameras)
-    Internals->RayCamera.SetParameters(camera, *canvas); // validates every view like the reference (:372)
-  auto tup = extract(cellset);
-  auto SphereIds = std::get<0>(tup);
-  auto SphereRadii = std::get<1>(tup);
-  auto QuadIds = std::get<3>(tup);
-  vtkm::cont::ArrayHandle<vtkm::Int32> matIdArray, texIdArray;
-  matIdArray.Allocate(nx * ny);
-  texIdArray.Allocate(nx * ny);
-  buildBVH(coords, QuadIds, SphereIds, SphereRadii, matIdArray, texIdArray, MatIdx, TexIdx);
-  const std::vector<float> views = packViews(cameras);
+  CheckCheckpoints(checkpoints, samplecount);
+  const std::vector<float> views = PrepareSweep(cellset, coords, cameras);
+  const vtkm::Id nx = Internals->Canvas->GetWidth(), ny = Internals->Canvas->GetHeight();
   const size_t n = checkpoints.size() * cameras.size() * static_cast<size_t>(nx * ny) * 4;
   albedo.assign(n, 0.f);
   normalDepth.assign(n, 0.f);
   b2pt_ctx* ctx = b2pt_facade::Context(Devices.empty() ? -1 : Devices[0]);
   b2pt_facade::Check(b2pt_seed(ctx, 0)); // the streams RenderCellsViews* render with
-  const unsigned int buildFlags =
-    B2PT_FLAG_FORCE_BVH | B2PT_FLAG_NO_DEDUP | B2PT_FLAG_NO_AA | B2PT_FLAG_GPU_LBVH | B2PT_FLAG_WIDE_BVH;
   b2pt_facade::Check(b2pt_render_views_features(ctx, static_cast<int>(cameras.size()), views.data(),
                                                 static_cast<int>(nx), static_cast<int>(ny),
                                                 static_cast<int>(checkpoints.size()), checkpoints.data(),
-                                                RenderFlags & buildFlags, albedo.data(), normalDepth.data()));
+                                                RenderFlags & B2PT_BUILD_FLAGS, albedo.data(), normalDepth.data()));
 }
 
 void MapperPathTracer::SetCompositeBackground(bool on) { Internals->CompositeBackground = on; }

@@ -156,6 +156,10 @@ public:
 private:
   struct InternalsType;
   std::shared_ptr<InternalsType> Internals;
+  // The set-up every camera sweep shares: needs a canvas, validates every camera against it, uploads the scene
+  // (buildBVH) and returns the view list of the C-ABI (10 floats per camera).
+  std::vector<float> PrepareSweep(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
+                                  const std::vector<vtkm::rendering::Camera>& cameras);
   void RenderViewsImpl(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
                        const std::vector<vtkm::rendering::Camera>& cameras, unsigned int flags, void* out,
                        const std::vector<int>* checkpoints = nullptr);

@@ -5,6 +5,7 @@ Bar: every view's radiance sum is BIT-IDENTICAL to b2pt_set_camera(view) + b2pt_
 per-(pixel, sample) streams, same per-path arithmetic, same sample-order accumulation), whatever the split of the view
 list into batches; and -- through the single-view parity tests -- equal to the oracle.
 """
+import ctypes
 import math
 import os
 
@@ -121,6 +122,79 @@ def test_views_errors(gpu_ctx, b2pt):
         gpu_ctx.render_views(bad, 32, 32, 2, 3)
     with pytest.raises(b2pt.B2ptError):
         gpu_ctx.render_views(views, 0, 32, 2, 3)
+
+
+def test_contract(b2pt, monkeypatch):
+    """b2pt_render_views at the C level: the code and message of every argument fault (the first fault when a call has
+    several), nothing touched by a failing call, the context's own camera and canvas untouched by a sweep, the
+    normalised image left on the device without a host output, and the statistics of the per-view fallback."""
+    L, p = b2pt.lib(), b2pt._p
+    views = hemisphere_views(2, 2)
+    w, h, spp, depth = 32, 24, 4, 5
+    n, V = w * h, len(views)
+    with b2pt.Context(0) as ctx:
+        ctx.set_scene(b2pt.Scene.cornell())
+        ctx.build_bvh()
+        ctx.set_camera(b2pt.Camera(48, 16))
+        ctx.render(2, 3)
+        canvas, hits = ctx.read_color().copy(), ctx.primary_hits()
+        full = ctx.render_views(views, w, h, spp, depth)
+        st = ctx.stats()
+        assert st.paths == n * spp * V
+        ptr = L.b2pt_views_device_ptr(ctx._h)
+        assert ptr
+        # the context's own camera and canvas are untouched by the sweep
+        assert same_bits(ctx.read_color(), canvas)
+        after = ctx.primary_hits()
+        assert np.array_equal(after[0], hits[0]) and same_bits(after[1], hits[1])
+
+        def fails(message, nv, vp, W, H, s, flags=0):
+            assert L.b2pt_render_views(ctx._h, nv, vp, W, H, s, depth, flags, None) == b2pt.ERR_BAD_VALUE
+            assert L.b2pt_last_error() == message
+
+        vp, ref = p(views), b2pt.FLAG_REFERENCE_STREAM
+        bad = views.copy()
+        bad[2, 9] = 0.0  # Camera.cxx:720
+        fails(b"b2pt_render_views: bad view list", V, None, w, h, spp)
+        fails(b"b2pt_render_views: bad view list", -1, vp, w, h, spp)
+        fails(b"b2pt_render_views: bad view list", V, None, w, h, -1, ref)
+        fails(b"negative sample range", V, vp, w, h, -1)
+        fails(b"negative sample range", V, p(bad), w, h, -1, ref)
+        fails(b"spp must be positive", V, vp, w, h, 0, b2pt.FLAG_VIEWS_PNM16)
+        fails(b"REFERENCE_STREAM cannot be combined with a view-batched render", V, vp, w, h, spp, ref)
+        fails(b"REFERENCE_STREAM cannot be combined with a view-batched render", V, p(bad), w, h, 0,
+              ref | b2pt.FLAG_VIEWS_PNM16)
+        fails(b"Camera feild of view must be greater than zero.", V, p(bad), w, h, spp)
+        # more than 2^30 output pixels: 17 views of 8192^2 (2^26 pixels each, the largest canvas)
+        big = np.ascontiguousarray(np.repeat(views[:1], 17, axis=0))
+        fails(b"b2pt_render_views: more than 2^30 output pixels (16 GiB); split the view list", 17, p(big), 8192, 8192,
+              spp)
+        bigbad = big.copy()
+        bigbad[16, 9] = 0.0
+        fails(b"Camera feild of view must be greater than zero.", 17, p(bigbad), 8192, 8192, spp)
+        # nothing was rendered: same statistics, same device image
+        st2 = ctx.stats()
+        assert (st2.paths, st2.launches, st2.batches) == (st.paths, st.launches, st.batches)
+        assert L.b2pt_views_device_ptr(ctx._h) == ptr
+        # VIEWS_NORMALIZE without a host output: the normalised images stay on the device
+        want = ctx.render_views(views, w, h, spp, depth, flags=b2pt.FLAG_VIEWS_NORMALIZE)
+        assert L.b2pt_render_views(ctx._h, V, vp, w, h, spp, depth, b2pt.FLAG_VIEWS_NORMALIZE, None) == 0
+        ptr = L.b2pt_views_device_ptr(ctx._h)
+        ctx.set_camera(b2pt.Camera(w, h))
+        for v in range(V):
+            assert L.b2pt_set_color_buffer(ctx._h, ctypes.c_void_p(ptr + v * n * 16)) == 0
+            assert same_bits(ctx.read_color(), want[v]), v
+        assert L.b2pt_set_color_buffer(ctx._h, None) == 0
+        # per-view fallback (a view no longer fits a batch): same images, statistics summed over the views
+        monkeypatch.setenv("B2PT_BATCH_PATHS", str(n * 2))
+        split = ctx.render_views(views, w, h, spp, depth)
+        st3 = ctx.stats()
+        monkeypatch.delenv("B2PT_BATCH_PATHS")
+        assert same_bits(split, full)
+        assert st3.paths == n * spp * V and st3.launches > st.launches
+        # nViews == 0 renders nothing and leaves no view image
+        assert ctx.render_views(np.zeros((0, 10), np.float32), w, h, spp, depth).shape == (0, n, 4)
+        assert not L.b2pt_views_device_ptr(ctx._h)
 
 
 def pnm_integers(rgba_sum, spp, oracle):
