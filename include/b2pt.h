@@ -189,6 +189,46 @@ int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views,
  * reference has no counterpart. */
 int b2pt_render_views_features(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
                                const int* checkpoints, uint32_t flags, float* albedoOut, float* normalDepthOut);
+/* Parameters of b2pt_denoise_views.  A sigma may be +inf, which switches its term off. */
+typedef struct b2pt_denoise_params
+{
+  int32_t levels;    /* a-trous levels, 0..10; 0 = no filtering (the output is the mean) */
+  float sigmaLum;    /* colour edge-stop, in standard deviations of the mean luminance */
+  float sigmaAlbedo; /* albedo + hit-fraction edge-stop */
+  float sigmaNormal; /* mean-normal edge-stop */
+  float sigmaDepth;  /* relative depth edge-stop, per pixel footprint */
+} b2pt_denoise_params;
+/* levels 5, sigmaLum 4, sigmaAlbedo 0.1, sigmaNormal 0.3, sigmaDepth 2 (DESIGN.md 8e). */
+void b2pt_denoise_defaults(b2pt_denoise_params* p);
+/* Spatial denoiser of a view sweep: the edge-avoiding a-trous wavelet filter of SVGF (Schied et al. 2017; Dammertz et
+ * al. 2010), its colour edge-stop scaled by the per-pixel standard deviation, guided by the sweep's own buffers.  All
+ * inputs are host arrays [k][view][j*W+i] of float4, K*nViews*W*H*4 floats each: color = the radiance sums of
+ * b2pt_render_views_checkpoints (flags 0), moment2 = its sums of squares (may be NULL), albedo and normalDepth = the sums
+ * of b2pt_render_views_features.  Every (slice k, view v) image is filtered on its own; taps never cross a view, a slice
+ * or the image border (taps outside are skipped, the weights renormalised).  With c = checkpoints[k], a pixel's inputs
+ * S, Q, A = (a, h), ND = (N, D), dn(x) = x with NaN replaced by 0 and luminance L(x) = 0.2126 x.r + 0.7152 x.g +
+ * 0.0722 x.b:
+ *   m = dn(S.rgb) / c;  V0 = sum_ch w_ch max(0, dn(Q_ch)/c - m_ch^2) / (c - 1), w = the luminance weights; V0 exists
+ *   only when moment2 is given and c >= 2, otherwise the colour term e_l is left out and V is 0 throughout;
+ *   guides g_a = (a/c, h/c), g_n = N/c, z = D/h when h > 0.
+ * Level i = 0..levels-1, step s = 2^i, taps q = p + s (dx, dy), dx, dy in -2..2, h = (1,4,6,4,1)/16:
+ *   w = h[dx] h[dy] exp(-(e_l + e_a + e_n + e_z)),
+ *   e_l = |L(x_i(p)) - L(x_i(q))| / (sigmaLum sqrt(V_i(p)) + 1e-6),
+ *   e_a = |g_a(p) - g_a(q)|^2 / sigmaAlbedo^2,  e_n = |g_n(p) - g_n(q)|^2 / sigmaNormal^2,
+ *   e_z = |z_p - z_q| H / (sigmaDepth z_p s sqrt(dx^2 + dy^2) + 1e-6) when both pixels have h > 0, else 0,
+ *   x_{i+1}(p) = sum w x_i(q) / sum w,  V_{i+1}(p) = sum w^2 V_i(q) / (sum w)^2,  x_0 = m, V_0 = V0.
+ * out: float4 (x_L.rgb, V_L) per pixel in the input layout; with B2PT_FLAG_VIEWS_PNM16 instead uint16_t[K*nViews*W*H*3],
+ * the integers b2pt_read_pnm16 gives for x_L with spp = 1 (levels = 0: the integers of
+ * b2pt_render_views_checkpoints(..., B2PT_FLAG_VIEWS_PNM16)).  params NULL = b2pt_denoise_defaults.  A pure function
+ * of its inputs: needs no scene, leaves the context's camera, canvas, view images and statistics untouched, and the
+ * result depends neither on chunking nor on launch shape.  B2PT_ERR_BAD_VALUE, before anything runs: a bad checkpoint
+ * list, NULL color / albedo / normalDepth, W or H <= 0, nViews < 0, levels outside 0..10, a sigma that is NaN or
+ * <= 0, a flag other than B2PT_FLAG_VIEWS_PNM16, or one view's K*W*H above 2^30.  nViews == 0 does nothing.  Views run
+ * in chunks of whole views through library-owned staging of at most max(2^23, K*W*H) float4 per buffer (four buffers).
+ * Synchronises the stream.  The reference has no counterpart (it has no denoiser). */
+int b2pt_denoise_views(b2pt_ctx* ctx, int nViews, int W, int H, int nCheckpoints, const int* checkpoints,
+                       const float* color, const float* moment2, const float* albedo, const float* normalDepth,
+                       const b2pt_denoise_params* params, uint32_t flags, void* out);
 void* b2pt_views_device_ptr(b2pt_ctx* ctx);
 int b2pt_clear_color(b2pt_ctx* ctx);
 /* Host-side planning rule of the renders above, exposed for tests and capacity planning (no GPU needed): `units`

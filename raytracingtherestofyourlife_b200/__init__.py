@@ -13,7 +13,7 @@ import numpy as np
 
 from . import _build
 
-__all__ = ["lib", "Scene", "Camera", "Context", "B2ptError", "Stats", "FLAG_REFERENCE_STREAM",
+__all__ = ["lib", "Scene", "Camera", "Context", "B2ptError", "Stats", "DenoiseParams", "FLAG_REFERENCE_STREAM",
            "FLAG_KILL_ZERO_THROUGHPUT", "FLAG_NO_DEDUP", "FLAG_FORCE_BVH", "FLAG_NO_AA", "FLAG_NO_TAIL", "FLAG_NO_OVERLAP", "FLAG_GPU_LBVH", "LIB_PATH"]
 
 LIB_PATH = _build.LIB
@@ -50,6 +50,18 @@ class Stats(C.Structure):
                 ("loopDepth", C.c_int32)]
 
 
+class DenoiseParams(C.Structure):
+    """b2pt_denoise_params: a-trous levels and the four edge-stop sigmas (+inf switches a term off)."""
+    _fields_ = [("levels", C.c_int32), ("sigmaLum", C.c_float), ("sigmaAlbedo", C.c_float),
+                ("sigmaNormal", C.c_float), ("sigmaDepth", C.c_float)]
+
+    @staticmethod
+    def defaults():
+        p = DenoiseParams()
+        lib().b2pt_denoise_defaults(C.byref(p))
+        return p
+
+
 _lib = None
 _vp, _i64, _i32, _f = C.c_void_p, C.c_int64, C.c_int, C.c_float
 
@@ -73,6 +85,9 @@ SIGNATURES = {
     "b2pt_render_views": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _i32, C.c_uint32, _vp]),
     "b2pt_render_views_checkpoints": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, _i32, C.c_uint32, _vp, _vp]),
     "b2pt_render_views_features": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, C.c_uint32, _vp, _vp]),
+    "b2pt_denoise_defaults": (None, [C.POINTER(DenoiseParams)]),
+    "b2pt_denoise_views": (_i32, [_vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, C.POINTER(DenoiseParams),
+                                  C.c_uint32, _vp]),
     "b2pt_views_device_ptr": (_vp, [_vp]),
     "b2pt_plan_batches": (_i32, [_i64, _i64, _i64, _i32, _vp, _vp]),
     "b2pt_clear_color": (_i32, [_vp]),
@@ -310,6 +325,28 @@ class Context:
         _check(lib().b2pt_render_views_features(self._h, v.shape[0], _p(v), W, H, K, _p(c), flags, _p(albedo),
                                                 _p(normal_depth)))
         return albedo, normal_depth
+
+    def denoise_views(self, color, moment2, albedo, normal_depth, W, H, checkpoints, params=None, flags=0):
+        """b2pt_denoise_views: the edge-avoiding a-trous filter of every (checkpoint, view) image of a sweep, guided by
+        its variance (from moment2, may be None), albedo and normal/depth sums.  Inputs are float32 [K, nViews, H*W, 4]
+        as render_views_checkpoints (flags 0, moments=True) and render_views_features return them; params is a
+        DenoiseParams (None: the defaults).  Returns float32 [K, nViews, H*W, 4] (denoised mean rgb, filtered variance)
+        or, under FLAG_VIEWS_PNM16, uint16 [K, nViews, H*W, 3]."""
+        c = np.ascontiguousarray(checkpoints, np.int32).reshape(-1)
+        K = c.shape[0]
+
+        def arr(a):
+            return None if a is None else np.ascontiguousarray(a, np.float32).reshape(K, -1, W * H, 4)
+        color, moment2, albedo, normal_depth = arr(color), arr(moment2), arr(albedo), arr(normal_depth)
+        V = color.shape[1]
+        for a in (moment2, albedo, normal_depth):
+            assert a is None or a.shape == color.shape, "inputs must share the [K, nViews, H*W, 4] layout"
+        dt, ch = (np.uint16, 3) if flags & FLAG_VIEWS_PNM16 else (np.float32, 4)
+        out = np.empty((K, V, W * H, ch), dt)
+        _check(lib().b2pt_denoise_views(self._h, V, W, H, K, _p(c), _p(color), _p(moment2), _p(albedo),
+                                        _p(normal_depth), None if params is None else C.byref(params), flags,
+                                        _p(out)))
+        return out
 
     def clear_color(self):
         _check(lib().b2pt_clear_color(self._h))

@@ -208,6 +208,9 @@ struct b2pt_ctx
   DevBuf<float4> ckptSnap, ckptMoment;
   // b2pt_render_views_features: [K][chunk views][W*H] staging of one chunk's sums
   DevBuf<float4> featAlbedo, featNormalDepth;
+  // b2pt_denoise_views: [K][chunk views][W*H] staging of one chunk: the ping-pong (x, V) images (the colour sums and
+  // sums of squares arrive in them) and the two guides
+  DevBuf<float4> dnX[2], dnGuideA, dnGuideNZ;
   DevBuf<uint2> primMask;         // primary-ray specialisation: [views][tiles] candidate masks (k_primary_prep)
   DevBuf<B2PrimQuad> primQuads;   // ... and [views][B2PT_SMALL_MAX_QUADS] per-quad constants
   int64_t viewCount = 0, viewPixels = 0;
@@ -467,6 +470,7 @@ void b2pt_destroy(b2pt_ctx* ctx)
   ctx->counters.release(), ctx->binTotals.release(), ctx->seeds.release(), ctx->nanCounter.release();
   ctx->dViews.release(), ctx->viewColor.release(), ctx->pnm.release(), ctx->primMask.release(), ctx->primQuads.release(); // (DevBuf's destructor would free them too)
   ctx->ckptSnap.release(), ctx->ckptMoment.release(), ctx->featAlbedo.release(), ctx->featNormalDepth.release();
+  ctx->dnX[0].release(), ctx->dnX[1].release(), ctx->dnGuideA.release(), ctx->dnGuideNZ.release();
   ctx->dDirectViews.release(), ctx->directNormals.release(), ctx->directAlbedo.release(), ctx->directDepth.release(),
     ctx->directPrim.release();
   if (ctx->evFork)
@@ -2178,6 +2182,108 @@ int b2pt_render_views_features(b2pt_ctx* ctx, int nViews, const float* views, in
                            cudaMemcpyDeviceToHost, ctx->stream));
       if (normalDepthOut)
         CU(cudaMemcpyAsync(normalDepthOut + dst, ctx->featNormalDepth.p + k * n, sizeof(float4) * (size_t)n,
+                           cudaMemcpyDeviceToHost, ctx->stream));
+    }
+  }
+  CU(cudaStreamSynchronize(ctx->stream));
+  return B2PT_OK;
+}
+
+void b2pt_denoise_defaults(b2pt_denoise_params* p)
+{
+  if (!p)
+    return;
+  p->levels = 5;
+  p->sigmaLum = 4.f;
+  p->sigmaAlbedo = 0.1f;
+  p->sigmaNormal = 0.3f;
+  p->sigmaDepth = 2.f;
+}
+
+// Spatial denoiser of a sweep (k_denoise_prep, then one k_atrous per level).  Views run in chunks of whole views: per
+// chunk, K host-to-device copies of each input into the context's staging [k][chunk view][pixel] (at most
+// max(kDenoiseChunkFloat4, K*W*H) float4 per buffer), the launches, and K copies of the result back.  The colour sums
+// land in dnX[0] and the sums of squares in dnX[1]; the prep turns dnX[0] into (m, V0) and the guide sums into the
+// guides in place, and the levels ping-pong between dnX[0] and dnX[1].  Every image is filtered on its own, so the
+// result does not depend on the chunking.
+static constexpr int64_t kDenoiseChunkFloat4 = (int64_t)1 << 23;
+int b2pt_denoise_views(b2pt_ctx* ctx, int nViews, int W, int H, int nCheckpoints, const int* checkpoints,
+                       const float* color, const float* moment2, const float* albedo, const float* normalDepth,
+                       const b2pt_denoise_params* params, uint32_t flags, void* out)
+{
+  static const char* const fn = "b2pt_denoise_views";
+  if (int rc = bind(ctx))
+    return rc;
+  if (nViews < 0)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: negative view count", fn);
+  if (int rc = check_checkpoints(fn, nCheckpoints, checkpoints))
+    return rc;
+  if (!color || !albedo || !normalDepth || !out)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: color, albedo, normalDepth and out must not be NULL", fn);
+  if (W <= 0 || H <= 0)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: W and H must be positive", fn);
+  b2pt_denoise_params P;
+  if (params)
+    P = *params;
+  else
+    b2pt_denoise_defaults(&P);
+  if (P.levels < 0 || P.levels > 10)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: levels must be in [0,10], got %d", fn, P.levels);
+  const float sigma[4] = { P.sigmaLum, P.sigmaAlbedo, P.sigmaNormal, P.sigmaDepth };
+  const char* const sigmaName[4] = { "sigmaLum", "sigmaAlbedo", "sigmaNormal", "sigmaDepth" };
+  for (int s = 0; s < 4; ++s)
+    if (!(sigma[s] > 0.f)) // NaN fails too
+      return fail(B2PT_ERR_BAD_VALUE, "%s: %s must be > 0 (or +inf), got %g", fn, sigmaName[s], (double)sigma[s]);
+  if (flags & ~B2PT_FLAG_VIEWS_PNM16)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: flags may only hold VIEWS_PNM16", fn);
+  const int K = nCheckpoints;
+  const int64_t N = (int64_t)W * H, KN = N * K;
+  if (KN > ((int64_t)1 << 30))
+    return fail(B2PT_ERR_BAD_VALUE, "%s: one view's %d slices exceed 2^30 float4", fn, K);
+  if (nViews == 0)
+    return B2PT_OK;
+  const bool pnm = (flags & B2PT_FLAG_VIEWS_PNM16) != 0;
+  b2pt::DenoiseArgs a{};
+  a.n = K;
+  std::copy(checkpoints, checkpoints + K, a.count);
+  a.hasMoments = moment2 != nullptr;
+  a.sigmaLum = P.sigmaLum, a.sigmaAlbedo = P.sigmaAlbedo, a.sigmaNormal = P.sigmaNormal, a.sigmaDepth = P.sigmaDepth;
+  const int64_t perChunk = std::max<int64_t>(1, kDenoiseChunkFloat4 / KN);
+  const size_t cap = (size_t)(std::min<int64_t>(perChunk, nViews) * KN);
+  CU(ctx->dnX[0].reserve(cap));
+  CU(ctx->dnX[1].reserve(cap));
+  CU(ctx->dnGuideA.reserve(cap));
+  CU(ctx->dnGuideNZ.reserve(cap));
+  if (pnm)
+    CU(ctx->pnm.reserve(cap * 3));
+  const float* const in[4] = { color, moment2, albedo, normalDepth };
+  float4* const stage[4] = { ctx->dnX[0].p, ctx->dnX[1].p, ctx->dnGuideA.p, ctx->dnGuideNZ.p };
+  for (int64_t v0 = 0; v0 < nViews; v0 += perChunk)
+  {
+    const int nv = (int)std::min<int64_t>(perChunk, nViews - v0);
+    const int64_t n = nv * N; // one slice of the chunk
+    for (int b = 0; b < 4; ++b)
+      for (int k = 0; in[b] && k < K; ++k)
+        CU(cudaMemcpyAsync(stage[b] + k * n, in[b] + 4 * (size_t)((k * (int64_t)nViews + v0) * N),
+                           sizeof(float4) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    a.nViews = nv;
+    CU(b2pt::launch_denoise_prep(ctx->dnX[0].p, moment2 ? ctx->dnX[1].p : nullptr, ctx->dnGuideA.p, ctx->dnGuideNZ.p,
+                                 (int)N, a, ctx->stream));
+    int cur = 0;
+    for (int level = 0; level < P.levels; ++level, cur ^= 1)
+      CU(b2pt::launch_atrous(ctx->dnX[cur].p, ctx->dnX[cur ^ 1].p, ctx->dnGuideA.p, ctx->dnGuideNZ.p, W, H, 1 << level,
+                             a, ctx->stream));
+    const float4* res = ctx->dnX[cur].p;
+    if (pnm)
+      CU(b2pt::launch_pnm16(res, n * K, 1, ctx->pnm.p, ctx->stream));
+    for (int k = 0; k < K; ++k)
+    {
+      const size_t dst = (size_t)((k * (int64_t)nViews + v0) * N);
+      if (pnm)
+        CU(cudaMemcpyAsync(static_cast<uint16_t*>(out) + 3 * dst, ctx->pnm.p + 3 * k * n, sizeof(uint16_t) * 3 * (size_t)n,
+                           cudaMemcpyDeviceToHost, ctx->stream));
+      else
+        CU(cudaMemcpyAsync(static_cast<float4*>(out) + dst, res + k * n, sizeof(float4) * (size_t)n,
                            cudaMemcpyDeviceToHost, ctx->stream));
     }
   }

@@ -18,6 +18,8 @@
 //   k_primary_hits                parity hook: production raygen + trace, writes hit primitive id / t.
 //   k_view_features<Scene>        per (view, pixel): albedo, normal and depth of the primary hits of its path samples,
 //                                 summed in sample order and stored at chosen sample counts (denoiser guides).
+//   k_denoise_prep, k_atrous       spatial denoiser of a view sweep: per-pixel means, variance and guides, then one
+//                                 edge-avoiding a-trous level per launch (b2pt_denoise_views).
 //   k_create_rays, k_intersect, k_normalize, k_pnm16, k_fill_seeds, k_sum_peers: stage-level API kernels.
 //
 // Work distribution: queue and bins are statically partitioned into one region per persistent warp
@@ -2008,6 +2010,101 @@ __global__ void __launch_bounds__(256)
   }
 }
 
+// ---- spatial denoiser of a view sweep (b2pt_denoise_views) ----------------------------------------------------------
+__device__ __forceinline__ float dn_lum(float4 x) { return 0.2126f * x.x + 0.7152f * x.y + 0.0722f * x.z; }
+__device__ __forceinline__ float de_nan(float x) { return x == x ? x : 0.f; }
+
+// Per pixel of a chunk [k][view][pixel] (sliceLen = views * pixels), in place: the color sums S become (m, V0) with
+// m = dn(S)/c and V0 the variance of the mean luminance (0 where it does not exist), the albedo sums (a, h) become
+// g_a = (a/c, h/c) and the normal/depth sums (N, D) become (N/c, z), z = D/h when h > 0, else 0.
+__global__ void __launch_bounds__(256)
+  k_denoise_prep(float4* __restrict__ x, const float4* __restrict__ moment, float4* __restrict__ ga,
+                 float4* __restrict__ gnz, long long n, long long sliceLen, const __grid_constant__ DenoiseArgs a)
+{
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n)
+    return;
+  const int c = a.count[idx / sliceLen];
+  const float cf = (float)c;
+  const float4 S = x[idx];
+  const float m0 = de_nan(S.x) / cf, m1 = de_nan(S.y) / cf, m2 = de_nan(S.z) / cf;
+  float V = 0.f;
+  if (a.hasMoments && c >= 2)
+  {
+    const float4 Q = moment[idx];
+    const float v0 = fmaxf(0.f, de_nan(Q.x) / cf - m0 * m0), v1 = fmaxf(0.f, de_nan(Q.y) / cf - m1 * m1),
+                v2 = fmaxf(0.f, de_nan(Q.z) / cf - m2 * m2);
+    V = (0.2126f * v0 + 0.7152f * v1 + 0.0722f * v2) / (float)(c - 1);
+  }
+  x[idx] = make_float4(m0, m1, m2, V);
+  const float4 A = ga[idx], ND = gnz[idx];
+  ga[idx] = make_float4(A.x / cf, A.y / cf, A.z / cf, A.w / cf);
+  gnz[idx] = make_float4(ND.x / cf, ND.y / cf, ND.z / cf, A.w > 0.f ? ND.w / A.w : 0.f);
+}
+
+// One a-trous level (step s) of SVGF's edge-avoiding wavelet filter: one thread per pixel, 16 x 16 pixel tiles in
+// blockIdx.x and one image per blockIdx.y, so the 5 x 5 taps of a block hit the same lines of L1.  Taps outside the
+// image are skipped; the centre tap (weight 9/64) keeps the sum of weights positive.  No atomics: every output is one
+// thread's sum in a fixed tap order.
+constexpr int kAtrousTile = 16;
+__global__ void __launch_bounds__(kAtrousTile * kAtrousTile)
+  k_atrous(const float4* __restrict__ xIn, float4* __restrict__ xOut, const float4* __restrict__ ga,
+           const float4* __restrict__ gnz, int W, int H, int tilesX, int step, int image0,
+           const __grid_constant__ DenoiseArgs a)
+{
+  const int img = image0 + (int)blockIdx.y;
+  const int i = (int)(blockIdx.x % (unsigned)tilesX) * kAtrousTile + (int)threadIdx.x;
+  const int j = (int)(blockIdx.x / (unsigned)tilesX) * kAtrousTile + (int)threadIdx.y;
+  if (i >= W || j >= H)
+    return;
+  const long long base = (long long)img * W * H, p = base + (long long)j * W + i;
+  const bool useL = a.hasMoments && a.count[img / a.nViews] >= 2 && !isinf(a.sigmaLum);
+  const bool useA = !isinf(a.sigmaAlbedo), useN = !isinf(a.sigmaNormal), useZ = !isinf(a.sigmaDepth);
+  const float sa2 = a.sigmaAlbedo * a.sigmaAlbedo, sn2 = a.sigmaNormal * a.sigmaNormal;
+  const float4 xp = xIn[p], ap = ga[p], np = gnz[p];
+  const float lp = dn_lum(xp), lden = a.sigmaLum * sqrtf(xp.w) + 1e-6f;
+  const bool hitP = ap.w > 0.f;
+  const float zScale = a.sigmaDepth * np.w * (float)step;
+  const float kh[5] = { 1.f / 16.f, 4.f / 16.f, 6.f / 16.f, 4.f / 16.f, 1.f / 16.f };
+  float sw = 0.f, sx = 0.f, sy = 0.f, sz = 0.f, sv = 0.f;
+#pragma unroll
+  for (int dy = -2; dy <= 2; ++dy)
+  {
+    const int jj = j + step * dy;
+    if (jj < 0 || jj >= H)
+      continue;
+#pragma unroll
+    for (int dx = -2; dx <= 2; ++dx)
+    {
+      const int ii = i + step * dx;
+      if (ii < 0 || ii >= W)
+        continue;
+      const long long q = base + (long long)jj * W + ii;
+      const float4 xq = xIn[q], aq = ga[q], nq = gnz[q];
+      float e = 0.f;
+      if (useL)
+        e += fabsf(lp - dn_lum(xq)) / lden;
+      if (useA)
+      {
+        const float d0 = ap.x - aq.x, d1 = ap.y - aq.y, d2 = ap.z - aq.z, d3 = ap.w - aq.w;
+        e += (d0 * d0 + d1 * d1 + d2 * d2 + d3 * d3) / sa2;
+      }
+      if (useN)
+      {
+        const float d0 = np.x - nq.x, d1 = np.y - nq.y, d2 = np.z - nq.z;
+        e += (d0 * d0 + d1 * d1 + d2 * d2) / sn2;
+      }
+      if (useZ && hitP && aq.w > 0.f)
+        e += fabsf(np.w - nq.w) * (float)H / (zScale * sqrtf((float)(dx * dx + dy * dy)) + 1e-6f);
+      const float w = kh[dx + 2] * kh[dy + 2] * expf(-e);
+      sw += w;
+      sx += w * xq.x, sy += w * xq.y, sz += w * xq.z;
+      sv += w * w * xq.w;
+    }
+  }
+  xOut[p] = make_float4(sx / sw, sy / sw, sz / sw, sv / (sw * sw));
+}
+
 __global__ void __launch_bounds__(256) k_fill_seeds(uint32_t* seeds, int n, uint32_t seedOffset)
 {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -2333,6 +2430,29 @@ cudaError_t launch_pnm16(const float4* color, int64_t n, int spp, uint16_t* rgb,
   if (n <= 0)
     return cudaSuccess;
   k_pnm16<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(color, n, (float)spp, rgb);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_denoise_prep(float4* x, const float4* moment, float4* ga, float4* gnz, int nPixels,
+                                const DenoiseArgs& a, cudaStream_t stream)
+{
+  const long long sliceLen = (long long)a.nViews * nPixels, n = sliceLen * a.n;
+  if (n <= 0)
+    return cudaSuccess;
+  k_denoise_prep<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(x, moment, ga, gnz, n, sliceLen, a);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_atrous(const float4* xIn, float4* xOut, const float4* ga, const float4* gnz, int W, int H,
+                          int step, const DenoiseArgs& a, cudaStream_t stream)
+{
+  const int tilesX = (W + kAtrousTile - 1) / kAtrousTile, tilesY = (H + kAtrousTile - 1) / kAtrousTile;
+  const int images = a.n * a.nViews;
+  for (int z0 = 0; z0 < images; z0 += 65535) // gridDim.y limit
+  {
+    const dim3 grid((unsigned)(tilesX * tilesY), (unsigned)std::min(65535, images - z0));
+    k_atrous<<<grid, dim3(kAtrousTile, kAtrousTile), 0, stream>>>(xIn, xOut, ga, gnz, W, H, tilesX, step, z0, a);
+  }
   return cudaGetLastError();
 }
 

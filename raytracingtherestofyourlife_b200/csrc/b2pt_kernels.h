@@ -124,6 +124,23 @@ struct FeatureCheckpoints
 cudaError_t launch_view_features(const B2SmallScene* small, const B2BvhScene* bvh, const B2Camera* cams, int nViews,
                                  int nPixels, uint32_t seedOffset, const FeatureCheckpoints& ck, float4* albedo,
                                  float4* normalDepth, cudaStream_t stream);
+// Spatial denoiser of b2pt_denoise_views over one chunk of nImages = K * nViews images of W x H pixels, stored
+// [k][view][pixel] (image z = k * nViews + v; its checkpoint count is count[z / nViews]).
+// launch_denoise_prep: in place, x (color sums in, (m, V0) out), moment (sums of squares, may be null; read only),
+// ga (albedo sums in, (a/c, h/c) out), gnz (normal/depth sums in, (N/c, z) out).
+// launch_atrous: one level of step `step` from xIn to xOut (float4 (x.rgb, V)); guides as prep leaves them.
+struct DenoiseArgs
+{
+  int n;                      // checkpoints
+  int count[kMaxCheckpoints]; // strictly increasing
+  int nViews;                 // views in the chunk
+  int hasMoments;
+  float sigmaLum, sigmaAlbedo, sigmaNormal, sigmaDepth; // +inf switches a term off
+};
+cudaError_t launch_denoise_prep(float4* x, const float4* moment, float4* ga, float4* gnz, int nPixels,
+                                const DenoiseArgs& a, cudaStream_t stream);
+cudaError_t launch_atrous(const float4* xIn, float4* xOut, const float4* ga, const float4* gnz, int W, int H,
+                          int step, const DenoiseArgs& a, cudaStream_t stream);
 cudaError_t launch_create_rays(const B2Camera& cam, uint32_t* seeds, float* dx, float* dy, float* dz, float* ox,
                                float* oy, float* oz, long long* pixelIdx, cudaStream_t stream);
 cudaError_t launch_intersect(const B2SmallScene* small, const B2BvhScene* bvh, int64_t n, const float* ox,

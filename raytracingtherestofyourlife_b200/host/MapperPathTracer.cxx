@@ -386,7 +386,7 @@ void MapperPathTracer::RenderDirectBuffersViews(const vtkm::cont::DynamicCellSet
 void MapperPathTracer::RenderViewsImpl(const vtkm::cont::DynamicCellSet& cellset,
                                        const vtkm::cont::CoordinateSystem& coords,
                                        const std::vector<vtkm::rendering::Camera>& cameras, unsigned int flags,
-                                       void* out, const std::vector<int>* checkpoints)
+                                       void* out, const std::vector<int>* checkpoints, float* moment2)
 {
   std::vector<float> views = PrepareSweep(cellset, coords, cameras);
   const vtkm::Id nx = Internals->Canvas->GetWidth(), ny = Internals->Canvas->GetHeight();
@@ -395,7 +395,7 @@ void MapperPathTracer::RenderViewsImpl(const vtkm::cont::DynamicCellSet& cellset
   if (checkpoints)
     b2pt_facade::Check(b2pt_render_views_checkpoints(
       ctx, static_cast<int>(cameras.size()), views.data(), static_cast<int>(nx), static_cast<int>(ny),
-      static_cast<int>(checkpoints->size()), checkpoints->data(), depthcount, RenderFlags | flags, out, nullptr));
+      static_cast<int>(checkpoints->size()), checkpoints->data(), depthcount, RenderFlags | flags, out, moment2));
   else
     b2pt_facade::Check(b2pt_render_views(ctx, static_cast<int>(cameras.size()), views.data(), static_cast<int>(nx),
                                          static_cast<int>(ny), samplecount, depthcount, RenderFlags | flags, out));
@@ -470,6 +470,38 @@ void MapperPathTracer::RenderCellsViewsFeatures(const vtkm::cont::DynamicCellSet
                                                 static_cast<int>(nx), static_cast<int>(ny),
                                                 static_cast<int>(checkpoints.size()), checkpoints.data(),
                                                 RenderFlags & B2PT_BUILD_FLAGS, albedo.data(), normalDepth.data()));
+}
+
+void MapperPathTracer::RenderCellsViewsDenoisedPnm(const vtkm::cont::DynamicCellSet& cellset,
+                                                   const vtkm::cont::CoordinateSystem& coords,
+                                                   const std::vector<vtkm::rendering::Camera>& cameras,
+                                                   const std::vector<int>& checkpoints, std::vector<unsigned short>& pnm,
+                                                   std::vector<unsigned short>& denoisedPnm)
+{
+  if (Internals->Canvas == nullptr)
+    throw vtkm::cont::ErrorBadValue("MapperPathTracer: no canvas set");
+  CheckCheckpoints(checkpoints, samplecount);
+  std::vector<float> color, moment2, albedo, normalDepth;
+  const size_t n = static_cast<size_t>(Internals->Canvas->GetWidth()) * Internals->Canvas->GetHeight();
+  const size_t n4 = checkpoints.size() * cameras.size() * n * 4;
+  color.assign(n4, 0.f);
+  moment2.assign(n4, 0.f);
+  RenderViewsImpl(cellset, coords, cameras, 0, color.data(), &checkpoints, moment2.data());
+  RenderCellsViewsFeatures(cellset, coords, cameras, checkpoints, albedo, normalDepth);
+  b2pt_ctx* ctx = b2pt_facade::Context();
+  const int V = static_cast<int>(cameras.size()), K = static_cast<int>(checkpoints.size());
+  const int nx = static_cast<int>(Internals->Canvas->GetWidth()), ny = static_cast<int>(Internals->Canvas->GetHeight());
+  pnm.assign(n4 / 4 * 3, 0);
+  denoisedPnm.assign(n4 / 4 * 3, 0);
+  b2pt_denoise_params unfiltered;
+  b2pt_denoise_defaults(&unfiltered);
+  unfiltered.levels = 0;
+  b2pt_facade::Check(b2pt_denoise_views(ctx, V, nx, ny, K, checkpoints.data(), color.data(), moment2.data(),
+                                        albedo.data(), normalDepth.data(), &unfiltered, B2PT_FLAG_VIEWS_PNM16,
+                                        pnm.data()));
+  b2pt_facade::Check(b2pt_denoise_views(ctx, V, nx, ny, K, checkpoints.data(), color.data(), moment2.data(),
+                                        albedo.data(), normalDepth.data(), nullptr, B2PT_FLAG_VIEWS_PNM16,
+                                        denoisedPnm.data()));
 }
 
 void MapperPathTracer::SetCompositeBackground(bool on) { Internals->CompositeBackground = on; }

@@ -123,6 +123,13 @@ public:
   void RenderCellsViewsFeatures(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
                                 const std::vector<vtkm::rendering::Camera>& cameras, const std::vector<int>& checkpoints,
                                 std::vector<float>& albedo, std::vector<float>& normalDepth);
+  // RenderCellsViewsCheckpointsPnm's integers (same checkpoint rule, same bytes in pnm) and, in denoisedPnm, the same
+  // layout for the sweep denoised with b2pt_denoise_views' defaults: one render of the float sums and their squares,
+  // the guides of RenderCellsViewsFeatures, then the filter (levels 0 for pnm, which is the unfiltered mean).
+  void RenderCellsViewsDenoisedPnm(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
+                                   const std::vector<vtkm::rendering::Camera>& cameras,
+                                   const std::vector<int>& checkpoints, std::vector<unsigned short>& pnm,
+                                   std::vector<unsigned short>& denoisedPnm);
   // The -direct G-buffers of main.cc:402-422 (what MapperQuadNormals / MapperQuadAlbedo leave in the canvas colour
   // buffer, raytracing/RayTracerNormals.cxx / RayTracerAlbedo.cxx, and a depth image) for the canvas set with
   // SetCanvas: one un-jittered ray per pixel, closest quad hit, the reference's two Shade rules (b2pt_render_direct).
@@ -162,7 +169,7 @@ private:
                                   const std::vector<vtkm::rendering::Camera>& cameras);
   void RenderViewsImpl(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
                        const std::vector<vtkm::rendering::Camera>& cameras, unsigned int flags, void* out,
-                       const std::vector<int>* checkpoints = nullptr);
+                       const std::vector<int>* checkpoints = nullptr, float* moment2 = nullptr);
   void RenderCellsImpl(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
                        const vtkm::cont::Field& scalarField, const vtkm::rendering::Camera& camera);
   void UploadScene(const vtkm::cont::CoordinateSystem& coord, vtkm::cont::ArrayHandle<vtkm::Vec<vtkm::Id, 5>>& QuadIds,

@@ -28,6 +28,11 @@
 // <out> for samplecount samples and <out>-s<c> for a checkpoint.  PFM (little-endian float32, scale -1.0, rows bottom
 // first as the buffers are) because PNM cannot hold negative normals or distances beyond 255.  The radiance files
 // stay byte-identical to a run without -features.  -features with -direct, or without a sweep, is an error (exit 1).
+// -denoise (with -hemisphere or -fibonacci, path-traced) also writes <stem>-denoised-<phi>-<theta>.pnm next to every
+// radiance file <stem>-<phi>-<theta>.pnm: the same sweep through the edge-avoiding a-trous filter (b2pt_denoise_views
+// with its default parameters), guided by the sweep's per-pixel variance, albedo, normal and depth, written with save()'s
+// arithmetic.  The radiance files (and the -features PFMs) stay byte-identical to a run without -denoise.  -denoise with
+// -direct, or without a sweep, is an error (exit 1).
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
@@ -62,6 +67,7 @@ struct Options
   std::string checkpointsArg;
   std::vector<int> checkpoints; // -checkpoints, parsed and checked by checkCheckpoints
   bool features = false;
+  bool denoise = false;
 };
 
 Options parse(int argc, char** argv)
@@ -101,6 +107,8 @@ Options parse(int argc, char** argv)
       next(o.viewSeed);
     else if (!std::strcmp(argv[i], "-features"))
       o.features = true;
+    else if (!std::strcmp(argv[i], "-denoise"))
+      o.denoise = true;
     else if (!std::strcmp(argv[i], "-checkpoints"))
     {
       o.checkpointsGiven = true;
@@ -147,6 +155,18 @@ std::string checkFeatures(const Options& o)
     return "-features cannot be combined with -direct";
   if (!o.hemi && !o.fibonacci)
     return "-features needs -hemisphere or -fibonacci";
+  return "";
+}
+
+// Returns an error message for an unusable -denoise, empty when it is usable or absent.
+std::string checkDenoise(const Options& o)
+{
+  if (!o.denoise)
+    return "";
+  if (o.direct)
+    return "-denoise cannot be combined with -direct";
+  if (!o.hemi && !o.fibonacci)
+    return "-denoise needs -hemisphere or -fibonacci";
   return "";
 }
 
@@ -329,10 +349,12 @@ int renderViews(CornellBox& cb, const Options& o, const std::vector<vtkm::render
   vtkm::rendering::CanvasRayTracer canvas(o.x, o.y);
   vtkm::rendering::MapperPathTracer mapper(o.samples, o.depth, cb.matIdx, cb.texIdx, cb.matType, cb.texType, cb.tex);
   mapper.SetCanvas(&canvas);
-  std::vector<unsigned short> pnm;
+  std::vector<unsigned short> pnm, denoised;
   std::vector<int> counts = o.checkpoints; // -checkpoints: one render, its images at every count up to samplecount
   counts.push_back(o.samples);
-  if (counts.size() > 1)
+  if (o.denoise) // the same integers as below, from the float sums the filter needs
+    mapper.RenderCellsViewsDenoisedPnm(cb.ds.GetCellSet(), cb.coord, cameras, counts, pnm, denoised);
+  else if (counts.size() > 1)
     mapper.RenderCellsViewsCheckpointsPnm(cb.ds.GetCellSet(), cb.coord, cameras, counts, pnm);
   else
     mapper.RenderCellsViewsPnm(cb.ds.GetCellSet(), cb.coord, cameras, pnm);
@@ -348,6 +370,11 @@ int renderViews(CornellBox& cb, const Options& o, const std::vector<vtkm::render
   for (size_t k = 0; k < counts.size(); ++k)
     for (size_t v = 0; v < V; ++v)
       savePnm16(viewName(stemOf(k), angles[v].first, angles[v].second), o.x, o.y, &pnm[(k * V + v) * n3]);
+  if (o.denoise)
+    for (size_t k = 0; k < counts.size(); ++k)
+      for (size_t v = 0; v < V; ++v)
+        savePnm16(viewName(stemOf(k) + "-denoised", angles[v].first, angles[v].second), o.x, o.y,
+                  &denoised[(k * V + v) * n3]);
   if (o.features)
   { // the guide images: sums over the samples of each count, as means
     std::vector<float> albedo, normalDepth;
@@ -454,6 +481,8 @@ int main(int argc, char* argv[])
   std::string bad = checkCheckpoints(o);
   if (bad.empty())
     bad = checkFeatures(o);
+  if (bad.empty())
+    bad = checkDenoise(o);
   if (!bad.empty())
   {
     std::cerr << "error: " << bad << std::endl;

@@ -1,0 +1,338 @@
+"""Spatial denoiser of a view sweep (b2pt_denoise_views: k_denoise_prep + k_atrous).
+
+Bar: with levels = 0 the output is the mean bit for bit, and its PNM integers are those of
+b2pt_render_views_checkpoints(PNM16); one level and the default levels agree with the float64 restatement
+(tests/denoise_ref.py) within a stated tolerance, on synthetic inputs with hard edges, misses and NaNs and on rendered
+sweeps, with and without sums of squares; every image is filtered on its own, whatever the chunking, and two calls give
+the same bits; the filter lowers the error against a 4096-spp target, and its guides are what keeps edges; bad inputs
+fail before anything runs; the driver's -denoise files are the binding's pipeline."""
+import ctypes
+import math
+import os
+import subprocess
+import sys
+
+import numpy as np
+import pytest
+
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+import denoise_ref as R  # noqa: E402
+from test_gpu_features import driver_view_names, hemisphere_positions, view_row  # noqa: E402
+
+pytestmark = pytest.mark.gpu
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+HOST = os.path.join(ROOT, "raytracingtherestofyourlife_b200", "host")
+C = 278 / 555.0
+W, H = 64, 48
+CKPTS = (1, 2, 5, 7)
+INF = float("inf")
+
+
+@pytest.fixture(scope="module")
+def host_build(b2pt):
+    import runpy
+    runpy.run_path(os.path.join(HOST, "build_host.py"), run_name="__test_build__")["build_host"]()
+    return HOST
+
+
+def tilted_views(n, fov=40.0):
+    """n view points in front of the box opening, tilted up vectors and varying fields of view."""
+    c = np.array([C] * 3, np.float32)
+    out = []
+    for v in range(n):
+        ang, elev = 0.35 * (v - (n - 1) / 2.0) / n, 0.08 * (v % 3)
+        d = 1078 / 555.0 + 0.1 * v
+        pos = c + d * np.array([math.sin(ang) * math.cos(elev), math.sin(elev), -math.cos(ang) * math.cos(elev)])
+        out.append(np.concatenate([pos, c, [0.1 * v, 1, 0.05 * (v % 2)], [fov + 2 * v]]).astype(np.float32))
+    return np.stack(out)
+
+
+@pytest.fixture(scope="module")
+def ctx(b2pt):
+    c = b2pt.Context(0)
+    c.set_scene(b2pt.Scene.cornell())
+    c.build_bvh()
+    yield c
+    c.close()
+
+
+@pytest.fixture(scope="module")
+def sweep(ctx, b2pt):
+    """6 tilted views at 64 x 48, checkpoints (1, 2, 5, 7): sums, sums of squares, guides and PNM integers."""
+    views = tilted_views(6)
+    color, m2 = ctx.render_views_checkpoints(views, W, H, CKPTS, 5, 0, moments=True)
+    pnm = ctx.render_views_checkpoints(views, W, H, CKPTS, 5, b2pt.FLAG_VIEWS_PNM16)
+    alb, nd = ctx.render_views_features(views, W, H, CKPTS)
+    return dict(views=views, color=color, m2=m2, pnm=pnm, alb=alb, nd=nd)
+
+
+def params(b2pt, levels=None, sl=None, sa=None, sn=None, sz=None):
+    p = b2pt.DenoiseParams.defaults()
+    for name, v in (("levels", levels), ("sigmaLum", sl), ("sigmaAlbedo", sa), ("sigmaNormal", sn), ("sigmaDepth", sz)):
+        if v is not None:
+            setattr(p, name, v)
+    return p
+
+
+def pnm_of(mean):
+    """k_pnm16 with spp = 1: int(255.99 * sqrtf(de_nan(x))), Float64 product, truncated, saturating at 65535."""
+    x = np.where(np.isnan(mean), np.float32(0), mean).astype(np.float32)
+    p = 255.99 * np.sqrt(x).astype(np.float64)
+    return np.where(p >= 65535, 65535, np.trunc(p)).astype(np.uint16)
+
+
+def synthetic(K, V, h, w, seed=0):
+    """Noisy sums with hard edges: albedo blocks, a missed region, a depth step, a normal crease and NaN pixels."""
+    rng = np.random.default_rng(seed)
+    ck = np.array([3, 8][:K], np.int32)
+    N = h * w
+    j, i = np.divmod(np.arange(N), w)
+    region = (i >= w // 3).astype(int) + (j >= h // 2).astype(int)
+    base = np.array([[0.2, 0.3, 0.4], [0.9, 0.6, 0.1], [0.05, 0.05, 0.5]])[region]
+    S = np.zeros((K, V, N, 4), np.float32)
+    Q = np.zeros_like(S)
+    A = np.zeros_like(S)
+    ND = np.zeros_like(S)
+    for k, c in enumerate(ck):
+        samples = base[None, None, :, None, :] * rng.exponential(1.0, (1, V, N, c, 3))
+        S[k, ..., :3] = samples.sum(3)
+        Q[k, ..., :3] = (samples ** 2).sum(3)
+        miss = (i < 4) & (j < 4)
+        hits = np.where(miss, 0, c)
+        A[k, ..., :3] = (np.array([[0.1, 0.1, 0.1], [0.7, 0.7, 0.2], [0.3, 0.3, 0.9]])[region] * hits[:, None])
+        A[k, ..., 3] = hits
+        nrm = np.where((i < w // 2)[:, None], [0.0, 0.0, -1.0], [0.7071, 0.0, -0.7071])
+        ND[k, ..., :3] = nrm * hits[:, None]
+        ND[k, ..., 3] = np.where(i < 2 * w // 3, 2.0, 3.5) * hits
+    S[:, :, ::37, 1] = np.nan
+    Q[:, :, ::53, 2] = np.nan
+    return ck, S, Q, A, ND
+
+
+def rel_err(g, r):
+    """Largest |gpu - reference| over max(|reference|, 1e-3 of the image's largest value), per image."""
+    g, r = np.asarray(g, np.float64), np.asarray(r, np.float64)
+    scale = np.abs(r).reshape(r.shape[0], r.shape[1], -1).max(-1)[:, :, None, None] * 1e-3
+    return float((np.abs(g - r) / np.maximum(np.abs(r), scale)).max())
+
+
+def test_levels_zero_is_the_mean(ctx, b2pt, sweep):
+    s = sweep
+    p0 = params(b2pt, levels=0)
+    out = ctx.denoise_views(s["color"], s["m2"], s["alb"], s["nd"], W, H, CKPTS, p0)
+    m, V0, *_ = R.prep(s["color"], s["m2"], s["alb"], s["nd"], CKPTS)
+    assert np.array_equal(out[..., :3].view(np.uint32), m.view(np.uint32))
+    assert np.array_equal(out[..., 3], V0)
+    assert (V0[0] == 0).all() and (V0[1:] > 0).any()  # c = 1 has no variance
+    pnm = ctx.denoise_views(s["color"], s["m2"], s["alb"], s["nd"], W, H, CKPTS, p0, b2pt.FLAG_VIEWS_PNM16)
+    assert np.array_equal(pnm, s["pnm"])
+    # NaN-poisoned sums: the renderer's integers treat NaN as 0, and so does the mean
+    poisoned = s["color"].copy()
+    poisoned[:, :, ::11, 0] = np.nan
+    poisoned[:, :, ::13, 2] = np.nan
+    pnm = ctx.denoise_views(poisoned, None, s["alb"], s["nd"], W, H, CKPTS, p0, b2pt.FLAG_VIEWS_PNM16)
+    mp, *_ = R.prep(poisoned, None, s["alb"], s["nd"], CKPTS)
+    assert np.array_equal(pnm, pnm_of(mp))
+    assert not np.array_equal(pnm, s["pnm"])
+
+
+# One level: fp32 weights against float64 ones; the inputs of the level are the same (the prep is bit-exact), so the
+# difference is the rounding of the edge-stop terms, exp and the 25-tap sums.  Several levels feed each level's fp32
+# output into the next one's edge-stops, so the bound is looser; measured values are in DESIGN.md 8e.
+TOL_ONE, TOL_ALL = 1e-4, 1e-3
+
+
+@pytest.mark.parametrize("moments", [True, False])
+def test_synthetic_against_restatement(ctx, b2pt, moments):
+    ck, S, Q, A, ND = synthetic(2, 3, 20, 27)
+    Q = Q if moments else None
+    for levels, tol in ((1, TOL_ONE), (5, TOL_ALL)):
+        out = ctx.denoise_views(S, Q, A, ND, 27, 20, ck, params(b2pt, levels=levels))
+        x, V = R.denoise(S, Q, A, ND, 27, 20, ck, levels=levels)
+        e = rel_err(out[..., :3], x)
+        assert e < tol, (levels, e)
+        if moments:
+            assert rel_err(out[..., 3:], V[..., None]) < 10 * tol, levels
+        else:
+            assert (out[..., 3] == 0).all()
+
+
+@pytest.mark.parametrize("moments", [True, False])
+def test_rendered_against_restatement(ctx, b2pt, sweep, moments):
+    s = sweep
+    Q = s["m2"] if moments else None
+    for levels, tol in ((1, TOL_ONE), (5, TOL_ALL)):
+        out = ctx.denoise_views(s["color"], Q, s["alb"], s["nd"], W, H, CKPTS, params(b2pt, levels=levels))
+        x, V = R.denoise(s["color"], Q, s["alb"], s["nd"], W, H, CKPTS, levels=levels)
+        e = rel_err(out[..., :3], x)
+        assert e < tol, (levels, e)
+    # the terms switch off: sigma = +inf everywhere is the plain B3 wavelet
+    p = params(b2pt, levels=2, sl=INF, sa=INF, sn=INF, sz=INF)
+    out = ctx.denoise_views(s["color"], Q, s["alb"], s["nd"], W, H, CKPTS, p)
+    x, _ = R.denoise(s["color"], Q, s["alb"], s["nd"], W, H, CKPTS, 2, INF, INF, INF, INF)
+    assert rel_err(out[..., :3], x) < TOL_ONE
+
+
+def test_images_are_independent_of_chunking_and_deterministic(ctx, b2pt):
+    # 16 x 16 images in 2 slices: 512 float4 per view, 2^14 views per chunk of 2^23 float4; 2^14 + 5 views cross it
+    h = w = 16
+    V = (1 << 14) + 5
+    rng = np.random.default_rng(1)
+    ck = np.array([2, 6], np.int32)
+    S = rng.random((2, V, h * w, 4), np.float32) * ck[:, None, None, None]
+    Q = S * S
+    A = np.repeat(rng.random((2, V, 1, 4), np.float32), h * w, 2)
+    A[..., 3] = ck[:, None, None]
+    A[:, :, : h * w // 2, :3] *= 0.3
+    ND = rng.random((2, V, h * w, 4), np.float32)
+    ND[..., 3] += 1
+    out = ctx.denoise_views(S, Q, A, ND, w, h, ck)
+    again = ctx.denoise_views(S, Q, A, ND, w, h, ck)
+    assert np.array_equal(out.view(np.uint32), again.view(np.uint32))
+    for v in (0, (1 << 14) - 1, 1 << 14, V - 1):
+        for k in range(2):
+            one = ctx.denoise_views(S[k:k + 1, v:v + 1], Q[k:k + 1, v:v + 1], A[k:k + 1, v:v + 1],
+                                    ND[k:k + 1, v:v + 1], w, h, ck[k:k + 1])
+            assert np.array_equal(one[0, 0].view(np.uint32), out[k, v].view(np.uint32)), (k, v)
+
+
+def test_rendered_sweep_is_deterministic(ctx, b2pt, sweep):
+    s = sweep
+    a = ctx.denoise_views(s["color"], s["m2"], s["alb"], s["nd"], W, H, CKPTS)
+    b = ctx.denoise_views(s["color"], s["m2"], s["alb"], s["nd"], W, H, CKPTS)
+    assert np.array_equal(a.view(np.uint32), b.view(np.uint32))
+
+
+def rel_mse(x, target):
+    return float(((x - target) ** 2 / (target ** 2 + 1e-2)).mean())
+
+
+def edge_mask(alb, nd, h, w):
+    """Pixels whose guides (mean albedo + hit fraction, mean normal, depth) change within 2 pixels."""
+    K = alb.shape[0]
+    c = alb[..., 3:4].max()
+    ga = (alb / c).reshape(alb.shape[1], h, w, 4)
+    gn = (nd[..., :3] / c).reshape(alb.shape[1], h, w, 3)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        z = np.where(alb[..., 3] > 0, nd[..., 3] / alb[..., 3], 0).reshape(alb.shape[1], h, w)
+    edge = np.zeros((alb.shape[1], h, w), bool)
+    for dy in range(-2, 3):
+        for dx in range(-2, 3):
+            sh = lambda a: np.roll(np.roll(a, dy, 1), dx, 2)
+            edge |= (np.abs(ga - sh(ga)).max(-1) > 0.05) | (np.abs(gn - sh(gn)).max(-1) > 0.1) | \
+                (np.abs(z - sh(z)) > 0.05 * np.maximum(z, 1e-3))
+    assert K >= 1
+    return edge.reshape(alb.shape[1], h * w)
+
+
+# Measured on a B200 (DESIGN.md 8e): denoised / noisy rel-MSE 0.22 at 4 spp and 0.28 at 64 spp; the bound leaves 1.4x.
+RATIO_BOUND = 0.4
+
+
+def test_it_denoises(b2pt):
+    views = tilted_views(8)
+    w = h = 128
+    ck = (4, 16, 64)
+    with b2pt.Context(0) as ctx:
+        ctx.set_scene(b2pt.Scene.cornell())
+        color, m2 = ctx.render_views_checkpoints(views, w, h, ck, 5, 0, moments=True)
+        alb, nd = ctx.render_views_features(views, w, h, ck)
+        target = ctx.render_views(views, w, h, 4096, 5)[..., :3] / np.float32(4096)
+        den = ctx.denoise_views(color, m2, alb, nd, w, h, ck)
+        blind = ctx.denoise_views(color, m2, alb, nd, w, h, ck, params(b2pt, sa=INF, sn=INF, sz=INF))
+    target = np.nan_to_num(target.astype(np.float64))
+    edge = edge_mask(alb[-1:], nd[-1:], h, w)
+    assert 0.02 < edge.mean() < 0.8, edge.mean()
+    report = []
+    for k, c in enumerate(ck):
+        noisy = np.nan_to_num(color[k, ..., :3].astype(np.float64)) / c
+        rn, rd = rel_mse(noisy, target), rel_mse(den[k, ..., :3], target)
+        ed, eb = rel_mse(den[k][edge][:, :3], target[edge]), rel_mse(blind[k][edge][:, :3], target[edge])
+        report.append((c, rn, rd, rd / rn, ed, eb))
+    for c, rn, rd, ratio, ed, eb in report:
+        assert ratio < RATIO_BOUND, report
+    # the guides keep edges once they are means of enough samples: at 64 spp the edge rel-MSE with the guides was 0.62x
+    # the one without them; at 4 spp the 4-sample guides are themselves noisy and cost 5 % on edges (DESIGN.md 8e)
+    c, rn, rd, ratio, ed, eb = report[-1]
+    assert ed < 0.85 * eb, report
+
+
+def test_contract(b2pt, sweep):
+    L, p = b2pt.lib(), b2pt._p
+    s = sweep
+    color, m2, alb, nd = (np.ascontiguousarray(s[k][:, :2]) for k in ("color", "m2", "alb", "nd"))
+    ck = np.array(CKPTS, np.int32)
+    out = np.zeros((4, 2, W * H, 4), np.float32)
+    with b2pt.Context(0) as ctx:  # no scene: the filter needs none
+        good = ctx.denoise_views(color, m2, alb, nd, W, H, ck)
+        assert np.isfinite(good).all()
+
+        def call(nViews=2, w=W, h=H, K=4, cks=ck, c=color, q=m2, a=alb, n=nd, prm=None, flags=0, o=out):
+            return L.b2pt_denoise_views(ctx._h, nViews, w, h, K, p(cks), p(c), p(q), p(a), p(n),
+                                        None if prm is None else ctypes.byref(prm), flags, p(o))
+
+        def fails(message, **kw):
+            assert call(**kw) == b2pt.ERR_BAD_VALUE, kw
+            assert message.encode() in L.b2pt_last_error(), (message, L.b2pt_last_error())
+
+        fails("nCheckpoints must be in [1,32]", K=0)
+        fails("nCheckpoints must be in [1,32]", K=33, cks=np.arange(1, 34, dtype=np.int32))
+        fails("checkpoints must be >= 1 and strictly increasing", cks=np.array([1, 2, 2, 7], np.int32))
+        fails("checkpoints must be >= 1 and strictly increasing", cks=np.array([0, 2, 5, 7], np.int32))
+        fails("nCheckpoints must be in [1,32]", cks=None)
+        for kw in (dict(c=None), dict(a=None), dict(n=None), dict(o=None)):
+            fails("color, albedo, normalDepth and out must not be NULL", **kw)
+        fails("W and H must be positive", w=0)
+        fails("W and H must be positive", h=-3)
+        fails("negative view count", nViews=-1)
+        for lv in (-1, 11):
+            fails("levels must be in [0,10]", prm=params(b2pt, levels=lv))
+        for name in ("sl", "sa", "sn", "sz"):
+            for bad in (0.0, -1.0, float("nan"), -INF):
+                fails("must be > 0 (or +inf)", prm=params(b2pt, **{name: bad}))
+        for f in (b2pt.FLAG_VIEWS_NORMALIZE, b2pt.FLAG_FORCE_BVH, 1 << 20):
+            fails("flags may only hold VIEWS_PNM16", flags=f)
+        # one 8192^2 view in 17 slices is more than 2^30 float4
+        fails("slices exceed 2^30 float4", nViews=1, w=8192, h=8192, K=17, cks=np.arange(1, 18, dtype=np.int32))
+        assert (out == 0).all()  # nothing ran
+        # nViews == 0 does nothing
+        assert call(nViews=0) == 0 and (out == 0).all()
+        # NULL params = the defaults; NULL moment2 is allowed
+        assert call(prm=b2pt.DenoiseParams.defaults()) == 0 and np.array_equal(out, good)
+        assert call(q=None) == 0 and (out[..., 3] == 0).all()
+
+
+# ---- the driver: -hemisphere -checkpoints 2,4 -denoise
+def test_driver_denoise(b2pt, host_build, tmp_path):
+    exe = os.path.join(host_build, "CornellBox_b2pt")
+    w, h, spp = 24, 16, 6
+    args = ["-x", str(w), "-y", str(h), "-raydepth", "5", "-samplecount", str(spp), "-hemisphere", "-phicount", "2",
+            "-thetacount", "3", "-checkpoints", "2,4"]
+
+    def run(name, *extra):
+        d = tmp_path / name
+        d.mkdir()
+        out = subprocess.run([exe] + args + list(extra), cwd=d, capture_output=True, text=True, timeout=300)
+        assert out.returncode == 0, out.stdout + out.stderr
+        return d, sorted(os.listdir(d))
+
+    ddir, files = run("denoise", "-denoise")
+    pdir, plain = run("plain")
+    assert len(plain) == 18
+    for f in plain:  # the radiance files: byte-identical to a run without -denoise
+        assert open(ddir / f, "rb").read() == open(pdir / f, "rb").read(), f
+    counts = [2, 4, spp]
+    stems = ["output-s2", "output-s4", "output"]
+    order = driver_view_names("hemisphere", hemisphere_positions(2, 3))
+    assert files == sorted(plain + ["%s-denoised-%s.pnm" % (s, t) for s in stems for t in order])
+    views = np.stack([view_row(pos) for pos in hemisphere_positions(2, 3)])
+    with b2pt.Context(0) as ctx:
+        ctx.set_scene(b2pt.Scene.cornell())
+        color, m2 = ctx.render_views_checkpoints(views, w, h, counts, 5, 0, moments=True)
+        alb, nd = ctx.render_views_features(views, w, h, counts)
+        want = ctx.denoise_views(color, m2, alb, nd, w, h, counts, flags=b2pt.FLAG_VIEWS_PNM16)
+    for k, stem in enumerate(stems):
+        for v, tail in enumerate(order):
+            body = "".join("%d %d %d\n" % tuple(px) for px in want[k, v])
+            text = "P3\n%d %d 255\n" % (w, h) + body
+            assert open(ddir / ("%s-denoised-%s.pnm" % (stem, tail))).read() == text, (stem, tail)
