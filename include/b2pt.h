@@ -229,6 +229,41 @@ void b2pt_denoise_defaults(b2pt_denoise_params* p);
 int b2pt_denoise_views(b2pt_ctx* ctx, int nViews, int W, int H, int nCheckpoints, const int* checkpoints,
                        const float* color, const float* moment2, const float* albedo, const float* normalDepth,
                        const b2pt_denoise_params* params, uint32_t flags, void* out);
+/* Parameters of b2pt_render_views_adaptive. */
+typedef struct b2pt_adaptive_params
+{
+  float threshold; /* tau: target relative standard error of a pixel's mean luminance, >= 0 (0 = never converged;
+                      +inf = stop after round 0) */
+  float epsilon;   /* absolute floor added to the mean luminance, > 0 */
+  int32_t radius;  /* 0..4: a pixel keeps sampling while any pixel within this Chebyshev radius in its view is
+                      unconverged */
+} b2pt_adaptive_params;
+/* threshold 0.02, epsilon 0.01, radius 1 (DESIGN.md 8f). */
+void b2pt_adaptive_defaults(b2pt_adaptive_params* p);
+/* Adaptive sampling of a view sweep: every pixel stops at the first round its own variance calls converged.  views
+ * holds 10 floats per view as in b2pt_render_views; rounds is a list of K = nRounds sample counts as
+ * b2pt_render_views_checkpoints takes it (1..32 strictly increasing counts), with rounds[0] >= 2.
+ * Round 0 renders rounds[0] samples of every pixel (b2pt_render_views_checkpoints with sums of squares).  After round
+ * k < K-1, with c = rounds[k], a pixel is unconverged when its count is c and, in float32 in this order (no FMA),
+ *   m = dn(S)/c and V0 as b2pt_denoise_views computes them (dn: NaN -> 0; V0 with the luminance weights),
+ *   L = 0.2126 m.r + 0.7152 m.g + 0.0722 m.b,  e = tau (L + epsilon),
+ * the test V0 <= e*e fails (a NaN V0 or L fails it; tau = 0 converges nothing).  A pixel is active in round k+1 when
+ * its count is c and some pixel of its view within Chebyshev distance `radius` is unconverged; active pixels get
+ * samples [rounds[k], rounds[k+1]), the others keep their count n_p.  Sample s of a pixel is the stream of every
+ * render (p + seedOffset + s * GOLDEN), added in sample order, so at every pixel S is the bits of
+ * b2pt_render_views(spp = n_p, flags) and Q the sums of squares of b2pt_render_views_checkpoints(rounds) at n_p.
+ * Outputs, [view][j*W+i], any may be NULL: rgbaOut float4 S (VIEWS_NORMALIZE: normalised with each pixel's n_p;
+ * VIEWS_PNM16: uint16[3] computed with n_p), moment2Out float4 Q whatever the flags, countOut int32 n_p, activeOut K
+ * entries: the pixels sampled in round k (activeOut[0] = nViews*W*H).  params NULL = b2pt_adaptive_defaults.
+ * B2PT_ERR_BAD_VALUE, before anything runs: a bad view list, view or round list, REFERENCE_STREAM or
+ * ONE_KERNEL_BOUNCE, a NaN or negative threshold, epsilon <= 0 or NaN, a radius outside 0..4, or more than 2^30
+ * float4 of device state (2 nViews W H).  nViews == 0 does nothing.  The context's camera and canvas are untouched;
+ * afterwards b2pt_views_device_ptr holds the image (S, normalised in place under VIEWS_NORMALIZE as b2pt_render_views
+ * does); stats.paths counts the paths of every round.  One 4-byte device-to-host read per round.  Synchronises the
+ * stream.  The reference has no counterpart. */
+int b2pt_render_views_adaptive(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nRounds,
+                               const int* rounds, int maxDepth, const b2pt_adaptive_params* params, uint32_t flags,
+                               void* rgbaOut, float* moment2Out, int32_t* countOut, int64_t* activeOut);
 void* b2pt_views_device_ptr(b2pt_ctx* ctx);
 int b2pt_clear_color(b2pt_ctx* ctx);
 /* Host-side planning rule of the renders above, exposed for tests and capacity planning (no GPU needed): `units`

@@ -13,7 +13,7 @@ import numpy as np
 
 from . import _build
 
-__all__ = ["lib", "Scene", "Camera", "Context", "B2ptError", "Stats", "DenoiseParams", "FLAG_REFERENCE_STREAM",
+__all__ = ["lib", "Scene", "Camera", "Context", "B2ptError", "Stats", "DenoiseParams", "AdaptiveParams", "FLAG_REFERENCE_STREAM",
            "FLAG_KILL_ZERO_THROUGHPUT", "FLAG_NO_DEDUP", "FLAG_FORCE_BVH", "FLAG_NO_AA", "FLAG_NO_TAIL", "FLAG_NO_OVERLAP", "FLAG_GPU_LBVH", "LIB_PATH"]
 
 LIB_PATH = _build.LIB
@@ -62,6 +62,18 @@ class DenoiseParams(C.Structure):
         return p
 
 
+class AdaptiveParams(C.Structure):
+    """b2pt_adaptive_params: convergence threshold tau (relative standard error of the mean luminance), luminance
+    floor epsilon and the Chebyshev radius over which an unconverged pixel keeps its neighbours sampling."""
+    _fields_ = [("threshold", C.c_float), ("epsilon", C.c_float), ("radius", C.c_int32)]
+
+    @staticmethod
+    def defaults():
+        p = AdaptiveParams()
+        lib().b2pt_adaptive_defaults(C.byref(p))
+        return p
+
+
 _lib = None
 _vp, _i64, _i32, _f = C.c_void_p, C.c_int64, C.c_int, C.c_float
 
@@ -88,6 +100,9 @@ SIGNATURES = {
     "b2pt_denoise_defaults": (None, [C.POINTER(DenoiseParams)]),
     "b2pt_denoise_views": (_i32, [_vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, C.POINTER(DenoiseParams),
                                   C.c_uint32, _vp]),
+    "b2pt_adaptive_defaults": (None, [C.POINTER(AdaptiveParams)]),
+    "b2pt_render_views_adaptive": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, _i32, C.POINTER(AdaptiveParams),
+                                          C.c_uint32, _vp, _vp, _vp, _vp]),
     "b2pt_views_device_ptr": (_vp, [_vp]),
     "b2pt_plan_batches": (_i32, [_i64, _i64, _i64, _i32, _vp, _vp]),
     "b2pt_clear_color": (_i32, [_vp]),
@@ -347,6 +362,26 @@ class Context:
                                         _p(normal_depth), None if params is None else C.byref(params), flags,
                                         _p(out)))
         return out
+
+    def render_views_adaptive(self, views, W, H, rounds, max_depth, params=None, flags=0):
+        """b2pt_render_views_adaptive: round 0 renders rounds[0] samples of every pixel, and after round k every pixel
+        whose neighbourhood is not converged gets samples [rounds[k], rounds[k+1]).  params is an AdaptiveParams (None:
+        the defaults).  Returns (image, moment2, counts, active): image float32 [nViews, H*W, 4] sums (normalised per
+        pixel under FLAG_VIEWS_NORMALIZE; uint16 [nViews, H*W, 3] under FLAG_VIEWS_PNM16), each pixel bit-identical to
+        render_views(spp=counts[pixel], flags); moment2 float32 [nViews, H*W, 4] sums of squares; counts int32
+        [nViews, H*W]; active int64 [K], the pixels sampled in each round."""
+        v = np.ascontiguousarray(views, np.float32).reshape(-1, 10)
+        r = np.ascontiguousarray(rounds, np.int32).reshape(-1)
+        nv = v.shape[0]
+        dt, ch = (np.uint16, 3) if flags & FLAG_VIEWS_PNM16 else (np.float32, 4)
+        image = np.empty((nv, W * H, ch), dt)
+        moment2 = np.empty((nv, W * H, 4), np.float32)
+        counts = np.empty((nv, W * H), np.int32)
+        active = np.zeros(r.shape[0], np.int64)
+        _check(lib().b2pt_render_views_adaptive(self._h, nv, _p(v), W, H, r.shape[0], _p(r), max_depth,
+                                                None if params is None else C.byref(params), flags, _p(image),
+                                                _p(moment2), _p(counts), _p(active)))
+        return image, moment2, counts, active
 
     def clear_color(self):
         _check(lib().b2pt_clear_color(self._h))

@@ -211,6 +211,12 @@ struct b2pt_ctx
   // b2pt_denoise_views: [K][chunk views][W*H] staging of one chunk: the ping-pong (x, V) images (the colour sums and
   // sums of squares arrive in them) and the two guides
   DevBuf<float4> dnX[2], dnGuideA, dnGuideNZ;
+  // b2pt_render_views_adaptive: per canvas entry the sample count, the unconverged and active flags; the compacted list
+  // of the next round's entries (padded to whole tiles), its length and the cub scratch
+  DevBuf<int32_t> adCounts, adNum;
+  DevBuf<uint8_t> adUnconv, adActive;
+  DevBuf<uint32_t> adList;
+  DevBuf<unsigned char> adTemp;
   DevBuf<uint2> primMask;         // primary-ray specialisation: [views][tiles] candidate masks (k_primary_prep)
   DevBuf<B2PrimQuad> primQuads;   // ... and [views][B2PT_SMALL_MAX_QUADS] per-quad constants
   int64_t viewCount = 0, viewPixels = 0;
@@ -1489,14 +1495,27 @@ static int ensure_built_for(b2pt_ctx* ctx, uint32_t flags)
   return B2PT_OK;
 }
 
+// A listed round of b2pt_render_views_adaptive: the canvas entries entries[0 .. nReal) (view * viewPixels + pixel,
+// padded to nPad by repeating the last one) for the cameras of ctx->dViews; their running sums live in color and
+// moment.
+struct ListedRound
+{
+  const uint32_t* entries;
+  int64_t nReal, nPad;
+  int viewPixels;
+  float4 *color, *moment;
+};
+
 // One render of the current scene.  nViews == 0: the context's camera, samples [sampleBegin, sampleBegin+sampleCount)
 // accumulated into the context's canvas.  nViews > 0 (b2pt_render_views): the same sample range for every camera of
 // ctx->dViews, accumulated into ctx->viewColor[view]; a batch holds whole views (viewsPerBatch x sampleCount sample
 // slots), so the caller guarantees W*H*sampleCount <= the batch target.  ckpt (b2pt_render_views_checkpoints): the
 // batches accumulate through k_accumulate_checkpoints into these snapshot slices as well; entry0 is the first canvas
-// entry of the render (its view's slice offset when nViews == 0).
+// entry of the render (its view's slice offset when nViews == 0).  list (nViews == 0): the same sample range for the
+// listed entries only, batched as the samples of one view of nPad pixels and accumulated in batch order through
+// k_accumulate_list; the per-tile primary masks are off (a tile is no longer 32 neighbouring pixels).
 static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxDepth, uint32_t flags, int64_t nViews,
-                       const b2pt::CheckpointArgs* ckpt = nullptr)
+                       const b2pt::CheckpointArgs* ckpt = nullptr, const ListedRound* list = nullptr)
 {
   if (int rc = bind(ctx))
     return rc;
@@ -1516,11 +1535,11 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
   if (int rc = ensure_built_for(ctx, flags))
     return rc;
   const bool viewMode = nViews > 0;
-  if (!viewMode)
+  if (!viewMode && !list)
     if (int rc = ensure_color(ctx))
       return rc;
 
-  const int64_t N = (int64_t)ctx->cam.W * ctx->cam.H;
+  const int64_t N = list ? list->nPad : (int64_t)ctx->cam.W * ctx->cam.H;
   // B = sample slots per batch (view mode: whole views, viewsPerBatch x sampleCount slots).  The render is cut into
   // equal batches of `units` (samples, or views of unitPaths paths each): as few as the memory target allows, but up
   // to one per buffer set while every batch keeps at least 32 Mi paths -- four batches in flight beat two larger ones
@@ -1667,7 +1686,8 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
   }
   // Primary-ray specialisation (small scenes whose tiles of 32 path ids are tiles of 32 pixels of one view): candidate
   // masks per tile and quad constants per view, recomputed per render (a few microseconds).
-  const bool primMasks = !ctx->useBvh && (N % 32) == 0 && nBatches > 0 && !(flags & B2PT_FLAG_NO_PRIMARY_MASKS);
+  const bool primMasks =
+    !ctx->useBvh && !list && (N % 32) == 0 && nBatches > 0 && !(flags & B2PT_FLAG_NO_PRIMARY_MASKS);
   const int tilesPerView = (int)(N / 32);
   if (primMasks)
   {
@@ -1742,7 +1762,7 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
     A.nPaths = N * nb;
     A.nPixels = (int32_t)N;
     A.sampleBase = (int32_t)(sampleBegin + s0);
-    A.views = viewMode ? ctx->dViews.p + v0 : nullptr;
+    A.views = viewMode ? ctx->dViews.p + v0 : (list ? ctx->dViews.p : nullptr);
     A.sppPerView = viewMode ? sampleCount : 0;
     A.primMask = primMasks ? ctx->primMask.p + (viewMode ? v0 * tilesPerView : 0) : nullptr;
     A.primQuads = primMasks ? ctx->primQuads.p + (viewMode ? v0 * B2PT_SMALL_MAX_QUADS : 0) : nullptr;
@@ -1754,6 +1774,11 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
     A.nLightSph = ctx->lights.nLightSph;
     A.seedOffset = ctx->seedOffset;
     A.flags = flags;
+    if (list)
+    { // (bounce 0 reads the list through A.perm, see below)
+      A.sppPerView = list->viewPixels;
+      b2pt::make_fastdiv((uint32_t)list->viewPixels, A.divSppMagic, A.divSppShift);
+    }
     // fused: launches 0 (primary) .. maxDepth (the closing shade pass); split: bounces 0 .. maxDepth-1, two launches each
     for (int depth = 0; depth < maxDepth + (fused ? 1 : 0); ++depth)
     {
@@ -1797,7 +1822,7 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
         ++launches;
         break;
       }
-      A.perm = nullptr;
+      A.perm = (list && depth == 0) ? list->entries : nullptr; // listed round: bounce 0 traces the list (k_trace LISTED)
       A.hits = nullptr;
       if (raySort && depth >= 1 && mode != b2pt::B2PT_BOUNCE_TAIL)
       { // queue regions of k_shade(depth - 1) -> permutation by origin cell and direction octant
@@ -1818,7 +1843,10 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
     // view mode: nv views of sampleCount samples each; otherwise nb samples of the one canvas
     float4* const canvas = viewMode ? ctx->viewColor.p + v0 * N : ctx->color();
     const int accSamples = viewMode ? sampleCount : (int)nb, accViews = viewMode ? (int)nv : 1;
-    if (ckpt)
+    if (list)
+      CU(b2pt::launch_accumulate_list(list->color, list->moment, bb.rad.p, list->entries, (int)list->nReal, (int)N,
+                                      (int)nb, ctx->nanCounter.p, bs));
+    else if (ckpt)
     {
       b2pt::CheckpointArgs ck = *ckpt;
       ck.sampleBase = A.sampleBase;
@@ -1957,9 +1985,10 @@ int b2pt_render_range(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxDe
 // point returns, converted per the view flags and copied to slice k of rgbaOut (NULL: no copy).  ck == nullptr
 // (b2pt_render_views, K == 1, no moments): the batches accumulate through k_accumulate.  Otherwise ck holds the
 // checkpoint list (n, count) and they accumulate through k_accumulate_checkpoints, which keeps the running sums at
-// every count and, when moment2Out is not NULL, the sums of squares.
+// every count and, when moment2Out is not NULL or keepMoments is set, the sums of squares (in ctx->ckptMoment).
 static int render_view_sweep(b2pt_ctx* ctx, const std::vector<B2Camera>& cams, const int* counts, int K, int maxDepth,
-                             uint32_t flags, b2pt::CheckpointArgs* ck, void* rgbaOut, float* moment2Out)
+                             uint32_t flags, b2pt::CheckpointArgs* ck, void* rgbaOut, float* moment2Out,
+                             bool keepMoments = false)
 {
   const int64_t nViews = (int64_t)cams.size();
   if (nViews == 0)
@@ -1969,7 +1998,7 @@ static int render_view_sweep(b2pt_ctx* ctx, const std::vector<B2Camera>& cams, c
   }
   const int spp = counts[K - 1];
   const int64_t N = (int64_t)cams[0].W * cams[0].H, NV = N * nViews;
-  const bool moments = moment2Out != nullptr;
+  const bool moments = moment2Out != nullptr || keepMoments;
   CU(ctx->viewColor.reserve((size_t)NV));
   CU(ctx->dViews.reserve((size_t)nViews));
   if (K > 1)
@@ -2062,10 +2091,10 @@ static int render_view_sweep(b2pt_ctx* ctx, const std::vector<B2Camera>& cams, c
       CU(cudaMemcpyAsync(static_cast<float4*>(rgbaOut) + NV * k, img, sizeof(float4) * (size_t)NV,
                          cudaMemcpyDeviceToHost, ctx->stream));
   }
-  if (moments)
+  if (moment2Out)
     CU(cudaMemcpyAsync(moment2Out, ctx->ckptMoment.p, sizeof(float4) * (size_t)(NV * K), cudaMemcpyDeviceToHost,
                        ctx->stream));
-  if (rgbaOut || moments)
+  if (rgbaOut || moment2Out)
     CU(cudaStreamSynchronize(ctx->stream));
   return B2PT_OK;
 }
@@ -2118,6 +2147,165 @@ int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views,
   ck.n = K;
   std::copy(checkpoints, checkpoints + K, ck.count);
   return render_view_sweep(ctx, cams, ck.count, K, maxDepth, flags, &ck, rgbaOut, moment2Out);
+}
+
+void b2pt_adaptive_defaults(b2pt_adaptive_params* p)
+{
+  if (!p)
+    return;
+  p->threshold = 0.02f;
+  p->epsilon = 0.01f;
+  p->radius = 1;
+}
+
+// Adaptive sampling of a view sweep (DESIGN.md 8f).  Round 0 is render_view_sweep at rounds[0] with the sums of squares
+// kept on the device, so it is b2pt_render_views_checkpoints by construction.  After round k, k_adaptive_mark and
+// k_adaptive_select choose the canvas entries of round k+1 and cub compacts them into ctx->adList in ascending order;
+// the one host read per round is that list's length.  Round k+1 is render_impl over the list (samples
+// [rounds[k], rounds[k+1]) of every listed entry), which continues each entry's sums in sample order, so an entry
+// that ends with n samples holds the bits of a uniform render of n samples.
+int b2pt_render_views_adaptive(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nRounds,
+                               const int* rounds, int maxDepth, const b2pt_adaptive_params* params, uint32_t flags,
+                               void* rgbaOut, float* moment2Out, int32_t* countOut, int64_t* activeOut)
+{
+  static const char* const fn = "b2pt_render_views_adaptive";
+  if (int rc = bind(ctx))
+    return rc;
+  if (int rc = check_view_list(fn, nViews, views))
+    return rc;
+  if (int rc = check_checkpoints(fn, nRounds, rounds))
+    return rc;
+  if (rounds[0] < 2)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: rounds[0] must be >= 2 (a variance needs two samples)", fn);
+  if (maxDepth < 1 || maxDepth > 4096)
+    return fail(B2PT_ERR_BAD_VALUE, "maxDepth must be in [1,4096]");
+  if (flags & (B2PT_FLAG_REFERENCE_STREAM | B2PT_FLAG_ONE_KERNEL_BOUNCE))
+    return fail(B2PT_ERR_BAD_VALUE, "%s: REFERENCE_STREAM and ONE_KERNEL_BOUNCE cannot be combined with it", fn);
+  b2pt_adaptive_params P;
+  if (params)
+    P = *params;
+  else
+    b2pt_adaptive_defaults(&P);
+  if (!(P.threshold >= 0.f)) // NaN fails too
+    return fail(B2PT_ERR_BAD_VALUE, "%s: threshold must be >= 0 (or +inf), got %g", fn, (double)P.threshold);
+  if (!(P.epsilon > 0.f))
+    return fail(B2PT_ERR_BAD_VALUE, "%s: epsilon must be > 0, got %g", fn, (double)P.epsilon);
+  if (P.radius < 0 || P.radius > 4)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: radius must be in [0,4], got %d", fn, P.radius);
+  std::vector<B2Camera> cams;
+  if (int rc = make_view_cameras(nViews, views, W, H, cams))
+    return rc;
+  if (2 * (int64_t)W * H * nViews > (int64_t)1 << 30)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: more than 2^30 float4 of device state (16 GiB); split the view list", fn);
+  if (nViews == 0)
+    return B2PT_OK;
+  if (!ctx->haveScene)
+    return fail(B2PT_ERR_STATE, "render before b2pt_set_scene");
+
+  const int K = nRounds;
+  const int64_t N = (int64_t)W * H, NV = N * nViews;
+  const uint32_t renderFlags = flags & ~(uint32_t)(B2PT_FLAG_VIEWS_NORMALIZE | B2PT_FLAG_VIEWS_PNM16);
+  b2pt::CheckpointArgs ck{};
+  ck.n = 1;
+  ck.count[0] = rounds[0];
+  if (int rc = render_view_sweep(ctx, cams, rounds, 1, maxDepth, renderFlags, &ck, nullptr, nullptr, true))
+    return rc;
+  int64_t paths = ctx->stats.paths, launches = ctx->stats.launches;
+  std::vector<int64_t> active((size_t)K, 0);
+  active[0] = NV;
+
+  const size_t tempBytes = b2pt::adaptive_select_temp_bytes(NV);
+  CU(ctx->adCounts.reserve((size_t)NV));
+  CU(ctx->adUnconv.reserve((size_t)NV));
+  CU(ctx->adActive.reserve((size_t)NV));
+  CU(ctx->adList.reserve((size_t)NV + 32));
+  CU(ctx->adNum.reserve(1));
+  CU(ctx->adTemp.reserve(std::max<size_t>(tempBytes, 1)));
+  // (the whole-view path of round 0 uploads the cameras too, its per-view fallback does not)
+  CU(cudaMemcpyAsync(ctx->dViews.p, cams.data(), sizeof(B2Camera) * (size_t)nViews, cudaMemcpyHostToDevice,
+                     ctx->stream));
+  b2pt::AdaptiveArgs a{};
+  a.tau = P.threshold;
+  a.eps = P.epsilon;
+  a.radius = P.radius;
+  a.W = W;
+  a.H = H;
+
+  // the listed rounds take the canvas shape from the context's camera, which is restored afterwards
+  const B2Camera savedCam = ctx->cam;
+  const bool savedHave = ctx->haveCamera;
+  ctx->cam = cams[0];
+  ctx->haveCamera = true;
+  int rc = B2PT_OK;
+  for (int k = 0; k + 1 < K && rc == B2PT_OK; ++k)
+  {
+    a.c = rounds[k];
+    a.next = rounds[k + 1];
+    a.first = k == 0;
+    int32_t n = 0;
+    cudaError_t e = b2pt::launch_adaptive_mark(ctx->viewColor.p, ctx->ckptMoment.p, ctx->adCounts.p, ctx->adUnconv.p,
+                                               NV, a, ctx->stream);
+    if (e == cudaSuccess)
+      e = b2pt::launch_adaptive_select(ctx->adUnconv.p, ctx->adCounts.p, ctx->adActive.p, NV, a, ctx->adList.p,
+                                       ctx->adNum.p, ctx->adTemp.p, tempBytes, ctx->stream);
+    if (e == cudaSuccess)
+      e = cudaMemcpyAsync(&n, ctx->adNum.p, sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess)
+      e = cudaStreamSynchronize(ctx->stream);
+    const int64_t nPad = ((int64_t)n + 31) / 32 * 32;
+    if (e == cudaSuccess && n > 0)
+      e = b2pt::launch_list_pad(ctx->adList.p, n, (int)nPad, ctx->stream);
+    if (e != cudaSuccess)
+    {
+      rc = fail(B2PT_ERR_CUDA, "%s: selecting round %d failed: %s", fn, k + 1, cudaGetErrorString(e));
+      break;
+    }
+    active[(size_t)k + 1] = n;
+    if (n == 0)
+      break; // nothing has rounds[k+1] samples, so nothing can reach the later rounds either
+    const ListedRound L{ ctx->adList.p, n, nPad, (int)N, ctx->viewColor.p, ctx->ckptMoment.p };
+    rc = render_impl(ctx, rounds[k], rounds[k + 1] - rounds[k], maxDepth, renderFlags, 0, nullptr, &L);
+    paths += (int64_t)n * (rounds[k + 1] - rounds[k]);
+    launches += ctx->stats.launches;
+  }
+  ctx->cam = savedCam;
+  ctx->haveCamera = savedHave;
+  if (rc != B2PT_OK)
+    return rc;
+  if (K == 1) // no selection ran: every entry has rounds[0] samples
+  {
+    a.c = rounds[0];
+    a.first = 1;
+    CU(b2pt::launch_adaptive_mark(ctx->viewColor.p, ctx->ckptMoment.p, ctx->adCounts.p, ctx->adUnconv.p, NV, a,
+                                  ctx->stream));
+  }
+  if (flags & B2PT_FLAG_VIEWS_PNM16)
+  {
+    if (rgbaOut)
+    {
+      CU(ctx->pnm.reserve((size_t)NV * 3));
+      CU(b2pt::launch_pnm16_counts(ctx->viewColor.p, NV, ctx->adCounts.p, ctx->pnm.p, ctx->stream));
+      CU(cudaMemcpyAsync(rgbaOut, ctx->pnm.p, sizeof(uint16_t) * 3 * (size_t)NV, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+  }
+  else
+  {
+    if (flags & B2PT_FLAG_VIEWS_NORMALIZE)
+      CU(b2pt::launch_normalize_counts(ctx->viewColor.p, NV, ctx->adCounts.p, ctx->stream));
+    if (rgbaOut)
+      CU(cudaMemcpyAsync(rgbaOut, ctx->viewColor.p, sizeof(float4) * (size_t)NV, cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  if (moment2Out)
+    CU(cudaMemcpyAsync(moment2Out, ctx->ckptMoment.p, sizeof(float4) * (size_t)NV, cudaMemcpyDeviceToHost,
+                       ctx->stream));
+  if (countOut)
+    CU(cudaMemcpyAsync(countOut, ctx->adCounts.p, sizeof(int32_t) * (size_t)NV, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  if (activeOut)
+    std::copy(active.begin(), active.end(), activeOut);
+  ctx->stats.paths = paths;
+  ctx->stats.launches = launches;
+  return B2PT_OK;
 }
 
 // Denoiser guides of a view sweep (k_view_features).  Sample s of a pixel is traced from the stream the render gives it

@@ -20,6 +20,9 @@
 //                                 summed in sample order and stored at chosen sample counts (denoiser guides).
 //   k_denoise_prep, k_atrous       spatial denoiser of a view sweep: per-pixel means, variance and guides, then one
 //                                 edge-avoiding a-trous level per launch (b2pt_denoise_views).
+//   k_accumulate_list, k_adaptive_mark, k_adaptive_select, k_list_pad, k_normalize_counts, k_pnm16_counts
+//                                 adaptive sampling of a view sweep: accumulate a listed round, choose the next
+//                                 round's pixels from each pixel's variance, per-pixel-count conversions.
 //   k_create_rays, k_intersect, k_normalize, k_pnm16, k_fill_seeds, k_sum_peers: stage-level API kernels.
 //
 // Work distribution: queue and bins are statically partitioned into one region per persistent warp
@@ -33,6 +36,8 @@
 #include <algorithm>
 #include <cooperative_groups.h>
 #include <cub/device/device_scan.cuh>
+#include <cub/device/device_select.cuh>
+#include <thrust/iterator/counting_iterator.h>
 #include <type_traits>
 
 namespace b2pt
@@ -148,12 +153,26 @@ __device__ __forceinline__ uint32_t fastdiv(uint32_t n, uint32_t magic, uint32_t
   return (t + ((n - t) >> 1)) >> shift;
 }
 
-// Ray `idx` of the warp's region.  PRIMARY: generated from (pixel, sample) -- idx is the path id.
-template <bool PRIMARY>
+// Ray `idx` of the warp's region.  PRIMARY: generated from (pixel, sample) -- idx is the path id.  LISTED (with
+// PRIMARY): path id b * nPixels + e is sample sampleBase + b of canvas entry A.perm[e] (B2RenderArgs::perm).
+template <bool PRIMARY, bool LISTED = false>
 __device__ __forceinline__ void load_ray(const B2Camera& cam, const B2RenderArgs& A, int64_t idx, f3& o, f3& d, f3& T,
                                          uint32_t& pid, uint32_t& rng, uint32_t* slotOut = nullptr)
 {
-  if (PRIMARY)
+  if constexpr (PRIMARY && LISTED)
+  {
+    pid = (uint32_t)idx;
+    const uint32_t b = fastdiv(pid, A.divPixelsMagic, A.divPixelsShift); // sample slot of the batch
+    const uint32_t entry = __ldg(A.perm + (pid - b * (uint32_t)A.nPixels));
+    const uint32_t view = fastdiv(entry, A.divSppMagic, A.divSppShift);
+    const uint32_t pixel = entry - view * (uint32_t)A.sppPerView;
+    const B2Camera vc = A.views[view];
+    rng = pixel + A.seedOffset + (uint32_t)(A.sampleBase + (int)b) * B2PT_GOLDEN;
+    d = raygen(vc, (int)pixel, rng);
+    o = ld3(vc.pos);
+    T = mk3(1.f, 1.f, 1.f);
+  }
+  else if (PRIMARY)
   {
     pid = (uint32_t)idx; // path id chosen by the caller (tile-interleaved over the warps' regions)
     uint32_t b = fastdiv(pid, A.divPixelsMagic, A.divPixelsShift); // sample slot of the batch
@@ -303,7 +322,7 @@ constexpr int kInnerSteps = B2PT_BVH_INNER_STEPS;
 #endif
 constexpr int kLeafChunk = B2PT_BVH_LEAF_CHUNK;
 
-template <bool PRIMARY, bool TAIL>
+template <bool PRIMARY, bool TAIL, bool LISTED = false>
 __device__ __forceinline__ void trace_body_bvh(const B2Camera& cam, const B2BvhScene& S, const B2RenderArgs& A,
                                                int depth, int w, int lane, int64_t nIn, int64_t tailWarps)
 {
@@ -349,7 +368,7 @@ __device__ __forceinline__ void trace_body_bvh(const B2Camera& cam, const B2BvhS
                                             : (A.perm ? (int64_t)__ldg(A.perm + permBase + r) : base + r));
         if (PRIMARY ? idx < A.nPaths : (TAIL ? idx < nIn : true))
         {
-          load_ray<PRIMARY>(cam, A, idx, o, d, T, pid, rng);
+          load_ray<PRIMARY, LISTED>(cam, A, idx, o, d, T, pid, rng);
           inv = mk3(rcp_safe(d.x), rcp_safe(d.y), rcp_safe(d.z));
           od = mk3(o.x * inv.x, o.y * inv.y, o.z * inv.z);
           closest = FLT_MAX;
@@ -848,7 +867,7 @@ __global__ void __launch_bounds__(kBlock, kMinBlocksPerSM)
 #endif
 constexpr int kWideRefillLanes = B2PT_WIDE_REFILL;
 
-template <bool PRIMARY, bool TAIL>
+template <bool PRIMARY, bool TAIL, bool LISTED = false>
 __device__ __forceinline__ void trace_body_wide(const B2Camera& cam, const B2BvhScene& S, const B2RenderArgs& A, int depth,
                                                 int w, int lane, int64_t nIn, int64_t tailWarps)
 {
@@ -893,7 +912,7 @@ __device__ __forceinline__ void trace_body_wide(const B2Camera& cam, const B2Bvh
         {
           f3 T;
           uint32_t pid;
-          load_ray<PRIMARY>(cam, A, idx, o, d, T, pid, rngP);
+          load_ray<PRIMARY, LISTED>(cam, A, idx, o, d, T, pid, rngP);
           inv = mk3(rcp_safe(d.x), rcp_safe(d.y), rcp_safe(d.z));
           od = mk3(o.x * inv.x, o.y * inv.y, o.z * inv.z);
           oct = wide_octant(inv);
@@ -1036,18 +1055,19 @@ __device__ __forceinline__ void trace_body_wide(const B2Camera& cam, const B2Bvh
 }
 
 // Work of one warp in k_trace: rays [.., nIn) of its region (TAIL: tiles w, w+tailWarps, ... of the flat queue).
-template <bool PRIMARY, class SceneT, bool TAIL>
+// LISTED: primary rays of listed path ids (load_ray), traced without the per-tile primary masks.
+template <bool PRIMARY, class SceneT, bool TAIL, bool LISTED = false>
 __device__ __forceinline__ void trace_body(const B2Camera& cam, const SceneT& S, const B2RenderArgs& A, int depth,
                                            int w, int lane, int64_t nIn, int64_t tailWarps)
 {
   if constexpr (std::is_same<SceneT, B2WideScene>::value)
   {
-    trace_body_wide<PRIMARY, TAIL>(cam, S, A, depth, w, lane, nIn, tailWarps);
+    trace_body_wide<PRIMARY, TAIL, LISTED>(cam, S, A, depth, w, lane, nIn, tailWarps);
     return;
   }
   if constexpr (std::is_same<SceneT, B2BvhScene>::value)
   {
-    trace_body_bvh<PRIMARY, TAIL>(cam, S, A, depth, w, lane, nIn, tailWarps);
+    trace_body_bvh<PRIMARY, TAIL, LISTED>(cam, S, A, depth, w, lane, nIn, tailWarps);
     return;
   }
   const int64_t base = TAIL ? 0 : (int64_t)w * A.regionCap;
@@ -1074,11 +1094,11 @@ __device__ __forceinline__ void trace_body(const B2Camera& cam, const SceneT& S,
     if (PRIMARY ? idx < A.nPaths : i < nIn)
     {
       uint32_t slotB = 0; // PRIMARY: sample slot of the path; the same for the 32 paths of a tile (nPixels % 32 == 0)
-      load_ray<PRIMARY>(cam, A, idx, o, d, T, pid, rng, &slotB);
+      load_ray<PRIMARY, LISTED>(cam, A, idx, o, d, T, pid, rng, &slotB);
       bool masked = false;
-      if constexpr (PRIMARY && std::is_same<SceneT, B2SmallScene>::value)
+      if constexpr (PRIMARY && !LISTED && std::is_same<SceneT, B2SmallScene>::value)
         masked = A.primMask != nullptr;
-      if constexpr (PRIMARY && std::is_same<SceneT, B2SmallScene>::value)
+      if constexpr (PRIMARY && !LISTED && std::is_same<SceneT, B2SmallScene>::value)
         if (masked)
       { // the tile's candidate mask and the view's per-quad constants (warp-uniform; nPixels % 32 == 0)
         const uint32_t tileBase = (uint32_t)idx - (uint32_t)lane;
@@ -1158,12 +1178,13 @@ __device__ __forceinline__ void trace_body(const B2Camera& cam, const SceneT& S,
   }
 }
 
-template <bool PRIMARY, class SceneT, bool TAIL>
+template <bool PRIMARY, class SceneT, bool TAIL, bool LISTED = false>
 __global__ void __launch_bounds__(kBlock, kTraceMinBlocksPerSM)
   k_trace(const __grid_constant__ B2Camera cam, const __grid_constant__ SceneT scene,
           const __grid_constant__ B2RenderArgs A)
 {
   static_assert(!(PRIMARY && TAIL), "primary rays are never traced in tail mode");
+  static_assert(PRIMARY || !LISTED, "only primary rays are listed");
   const int w = blockIdx.x * kWarps + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   // PRIMARY: the batch's 32-path tiles are dealt round by round to the warps, skewed by one slot per round
@@ -1204,7 +1225,7 @@ __global__ void __launch_bounds__(kBlock, kTraceMinBlocksPerSM)
   __syncthreads();
   if (!TAIL && w >= A.numWarps)
     return;
-  trace_body<PRIMARY, SceneT, TAIL>(cam, S, A, A.depth, w, lane, nIn, tailWarps);
+  trace_body<PRIMARY, SceneT, TAIL, LISTED>(cam, S, A, A.depth, w, lane, nIn, tailWarps);
 }
 
 // K3+K5: material response, direction generator, light pdfs, mixture pdf and the next ray for every binned hit
@@ -1975,11 +1996,8 @@ __global__ void __launch_bounds__(256)
 }
 
 // main.cc:253-287 NormalizeFunctor: sqrt(de_nan(sum)/spp); the alpha lane goes through the same sqrt.
-__global__ void __launch_bounds__(256) k_normalize(float4* color, long long n, float spp)
+__device__ __forceinline__ void normalize_pixel(float4* color, long long i, float spp)
 {
-  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n)
-    return;
   float4 c = color[i];
   if (!(c.x == c.x))
     c.x = 0.f;
@@ -1989,16 +2007,20 @@ __global__ void __launch_bounds__(256) k_normalize(float4* color, long long n, f
     c.z = 0.f;
   color[i] = make_float4(sqrtf(c.x / spp), sqrtf(c.y / spp), sqrtf(c.z / spp), sqrtf(c.w / spp));
 }
-
-// main.cc:325-384 save(): the three integers the reference prints per pixel of a P3 file, int(255.99 * col[k]) with
-// col = NormalizeFunctor(sum) (de_nan, /spp, sqrt); the product is Float64 as in the reference (255.99 is a double
-// literal), truncated toward zero; values past 65535 (radiance sums beyond 6.5e4 x spp) saturate.
-__global__ void __launch_bounds__(256)
-  k_pnm16(const float4* __restrict__ color, long long n, float spp, uint16_t* __restrict__ rgb)
+__global__ void __launch_bounds__(256) k_normalize(float4* color, long long n, float spp)
 {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n)
     return;
+  normalize_pixel(color, i, spp);
+}
+
+// main.cc:325-384 save(): the three integers the reference prints per pixel of a P3 file, int(255.99 * col[k]) with
+// col = NormalizeFunctor(sum) (de_nan, /spp, sqrt); the product is Float64 as in the reference (255.99 is a double
+// literal), truncated toward zero; values past 65535 (radiance sums beyond 6.5e4 x spp) saturate.
+__device__ __forceinline__ void pnm16_pixel(const float4* __restrict__ color, long long i, float spp,
+                                            uint16_t* __restrict__ rgb)
+{
   const float4 c = color[i];
   const float v[3] = { c.x, c.y, c.z };
 #pragma unroll
@@ -2008,6 +2030,33 @@ __global__ void __launch_bounds__(256)
     const double p = 255.99 * (double)sqrtf(x / spp);
     rgb[3 * i + k] = (uint16_t)(p >= 65535.0 ? 65535 : __double2int_rz(p));
   }
+}
+__global__ void __launch_bounds__(256)
+  k_pnm16(const float4* __restrict__ color, long long n, float spp, uint16_t* __restrict__ rgb)
+{
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n)
+    return;
+  pnm16_pixel(color, i, spp, rgb);
+}
+
+// k_normalize and k_pnm16 with every pixel's own sample count (b2pt_render_views_adaptive): the same float operations
+// with spp = (float)counts[i], so a pixel of n samples gets the bits of the uniform kernels at spp = n.
+__global__ void __launch_bounds__(256) k_normalize_counts(float4* color, long long n, const int32_t* __restrict__ counts)
+{
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n)
+    return;
+  normalize_pixel(color, i, (float)counts[i]);
+}
+__global__ void __launch_bounds__(256)
+  k_pnm16_counts(const float4* __restrict__ color, long long n, const int32_t* __restrict__ counts,
+                 uint16_t* __restrict__ rgb)
+{
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n)
+    return;
+  pnm16_pixel(color, i, (float)counts[i], rgb);
 }
 
 // ---- spatial denoiser of a view sweep (b2pt_denoise_views) ----------------------------------------------------------
@@ -2105,6 +2154,105 @@ __global__ void __launch_bounds__(kAtrousTile * kAtrousTile)
   xOut[p] = make_float4(sx / sw, sy / sw, sz / sw, sv / (sw * sw));
 }
 
+// ---- adaptive sampling of a view sweep (b2pt_render_views_adaptive) --------------------------------------------------
+// k_accumulate_checkpoints' loop over one batch of a listed round: entry e < nReal of the list adds the samples
+// rad[b * nPad + e], b = 0 .. nSamples-1, of canvas entry P = list[e] onto the running sum S[P] and their squares onto
+// Q[P], in sample order.  The padding entries [nReal, nPad) were traced and are not accumulated.
+__global__ void __launch_bounds__(256)
+  k_accumulate_list(float4* __restrict__ color, float4* __restrict__ moment, const float4* __restrict__ rad,
+                    const uint32_t* __restrict__ list, int nReal, int nPad, int nSamples,
+                    unsigned long long* nanCounter)
+{
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= nReal)
+    return;
+  const uint32_t P = list[e];
+  float4 c = color[P], m = moment[P];
+  int nan = 0;
+  for (int b = 0; b < nSamples; ++b)
+  {
+    const float4 r = rad[(size_t)b * nPad + e];
+    nan += (r.x != r.x || r.y != r.y || r.z != r.z) ? 1 : 0;
+    c.x += r.x;
+    c.y += r.y;
+    c.z += r.z;
+    m.x += r.x * r.x;
+    m.y += r.y * r.y;
+    m.z += r.z * r.z;
+  }
+  color[P] = c;
+  moment[P] = m;
+  if (nan)
+    atomicAdd(nanCounter, (unsigned long long)nan);
+}
+
+// After round k (c = a.c samples): unconv[P] = 1 when canvas entry P has c samples and its variance of the mean
+// luminance V0 exceeds (tau (L + eps))^2 -- m and V0 exactly as k_denoise_prep computes them, L = the luminance of m;
+// NaN fails the test, and tau = 0 converges nothing.  a.first (round 0): the counts are set to c.
+__global__ void __launch_bounds__(256)
+  k_adaptive_mark(const float4* __restrict__ color, const float4* __restrict__ moment, int32_t* __restrict__ counts,
+                  uint8_t* __restrict__ unconv, long long n, const __grid_constant__ AdaptiveArgs a)
+{
+  const long long P = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (P >= n)
+    return;
+  int cnt = a.c;
+  if (a.first)
+    counts[P] = a.c;
+  else
+    cnt = counts[P];
+  bool u = false;
+  if (cnt == a.c)
+  {
+    const float cf = (float)a.c;
+    const float4 S = color[P], Q = moment[P];
+    const float m0 = de_nan(S.x) / cf, m1 = de_nan(S.y) / cf, m2 = de_nan(S.z) / cf;
+    const float v0 = fmaxf(0.f, de_nan(Q.x) / cf - m0 * m0), v1 = fmaxf(0.f, de_nan(Q.y) / cf - m1 * m1),
+                v2 = fmaxf(0.f, de_nan(Q.z) / cf - m2 * m2);
+    const float V = (0.2126f * v0 + 0.7152f * v1 + 0.0722f * v2) / (float)(a.c - 1);
+    const float L = 0.2126f * m0 + 0.7152f * m1 + 0.0722f * m2;
+    const float e = a.tau * (L + a.eps);
+    u = !(a.tau > 0.f && V <= e * e);
+  }
+  unconv[P] = u ? 1 : 0;
+}
+
+// active[P] = 1 when canvas entry P has a.c samples and an unconverged entry lies within Chebyshev distance a.radius of
+// it in its own view; its count becomes a.next.  Reads only unconv, so no entry sees another's new count.
+__global__ void __launch_bounds__(256)
+  k_adaptive_select(const uint8_t* __restrict__ unconv, int32_t* __restrict__ counts, uint8_t* __restrict__ active,
+                    long long n, const __grid_constant__ AdaptiveArgs a)
+{
+  const long long P = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (P >= n)
+    return;
+  bool act = false;
+  if (counts[P] == a.c)
+  {
+    const long long N = (long long)a.W * a.H, view = P / N;
+    const int pix = (int)(P - view * N), j = pix / a.W, i = pix - j * a.W;
+    const uint8_t* u = unconv + view * N;
+    for (int y = max(0, j - a.radius); y <= min(a.H - 1, j + a.radius) && !act; ++y)
+      for (int x = max(0, i - a.radius); x <= min(a.W - 1, i + a.radius); ++x)
+        if (u[y * a.W + x])
+        {
+          act = true;
+          break;
+        }
+  }
+  active[P] = act ? 1 : 0;
+  if (act)
+    counts[P] = a.next;
+}
+
+// Pads a list of n >= 1 entries to nPad (a multiple of 32) by repeating its last entry.
+__global__ void k_list_pad(uint32_t* list, int n, int nPad)
+{
+  const int t = n + (int)threadIdx.x;
+  if (t < nPad)
+    list[t] = list[n - 1];
+}
+
 __global__ void __launch_bounds__(256) k_fill_seeds(uint32_t* seeds, int n, uint32_t seedOffset)
 {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -2175,7 +2323,8 @@ static cudaError_t launch_bounce_t(const LaunchCfg& cfg, bool primary, int mode,
     k_trace<false, SceneT, true><<<tailGrid, kBlock, 0, stream>>>(cam, S, args);
   }
   else if (primary)
-    k_trace<true, SceneT, false><<<grid, kBlock, 0, stream>>>(cam, S, args);
+    args.perm ? k_trace<true, SceneT, false, true><<<grid, kBlock, 0, stream>>>(cam, S, args)
+              : k_trace<true, SceneT, false><<<grid, kBlock, 0, stream>>>(cam, S, args);
   else if (std::is_same<SceneT, B2BvhScene>::value && args.perm && args.hits)
   { // split bounce: lean traversal over the sorted order, then the bookkeeping in queue order
     const B2BvhScene& BS = reinterpret_cast<const B2BvhScene&>(S);
@@ -2453,6 +2602,72 @@ cudaError_t launch_atrous(const float4* xIn, float4* xOut, const float4* ga, con
     const dim3 grid((unsigned)(tilesX * tilesY), (unsigned)std::min(65535, images - z0));
     k_atrous<<<grid, dim3(kAtrousTile, kAtrousTile), 0, stream>>>(xIn, xOut, ga, gnz, W, H, tilesX, step, z0, a);
   }
+  return cudaGetLastError();
+}
+
+cudaError_t launch_accumulate_list(float4* color, float4* moment, const float4* rad, const uint32_t* list, int nReal,
+                                   int nPad, int nSamples, unsigned long long* nanCounter, cudaStream_t stream)
+{
+  if (nReal <= 0)
+    return cudaSuccess;
+  k_accumulate_list<<<(unsigned)((nReal + 255) / 256), 256, 0, stream>>>(color, moment, rad, list, nReal, nPad,
+                                                                         nSamples, nanCounter);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_adaptive_mark(const float4* color, const float4* moment, int32_t* counts, uint8_t* unconv, int64_t n,
+                                 const AdaptiveArgs& a, cudaStream_t stream)
+{
+  if (n <= 0)
+    return cudaSuccess;
+  k_adaptive_mark<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(color, moment, counts, unconv, n, a);
+  return cudaGetLastError();
+}
+
+size_t adaptive_select_temp_bytes(int64_t n)
+{
+  size_t bytes = 0;
+  cub::DeviceSelect::Flagged(nullptr, bytes, thrust::counting_iterator<uint32_t>(0), (const uint8_t*)nullptr,
+                             (uint32_t*)nullptr, (int32_t*)nullptr, n);
+  return bytes;
+}
+
+cudaError_t launch_adaptive_select(const uint8_t* unconv, int32_t* counts, uint8_t* active, int64_t n,
+                                   const AdaptiveArgs& a, uint32_t* list, int32_t* numActive, void* temp,
+                                   size_t tempBytes, cudaStream_t stream)
+{
+  if (n <= 0)
+    return cudaSuccess;
+  k_adaptive_select<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(unconv, counts, active, n, a);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess)
+    return e;
+  return cub::DeviceSelect::Flagged(temp, tempBytes, thrust::counting_iterator<uint32_t>(0), active, list, numActive,
+                                    n, stream);
+}
+
+cudaError_t launch_list_pad(uint32_t* list, int n, int nPad, cudaStream_t stream)
+{
+  if (n < 1 || nPad - n <= 0 || nPad - n >= 32)
+    return n >= 1 && nPad == n ? cudaSuccess : cudaErrorInvalidValue;
+  k_list_pad<<<1, 32, 0, stream>>>(list, n, nPad);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_normalize_counts(float4* color, int64_t n, const int32_t* counts, cudaStream_t stream)
+{
+  if (n <= 0)
+    return cudaSuccess;
+  k_normalize_counts<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(color, n, counts);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_pnm16_counts(const float4* color, int64_t n, const int32_t* counts, uint16_t* rgb,
+                                cudaStream_t stream)
+{
+  if (n <= 0)
+    return cudaSuccess;
+  k_pnm16_counts<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(color, n, counts, rgb);
   return cudaGetLastError();
 }
 

@@ -141,6 +141,34 @@ cudaError_t launch_denoise_prep(float4* x, const float4* moment, float4* ga, flo
                                 const DenoiseArgs& a, cudaStream_t stream);
 cudaError_t launch_atrous(const float4* xIn, float4* xOut, const float4* ga, const float4* gnz, int W, int H,
                           int step, const DenoiseArgs& a, cudaStream_t stream);
+// Adaptive sampling of a view sweep (b2pt_render_views_adaptive).  Canvas entries P = view * W*H + pixel, n of them.
+// launch_accumulate_list: for e < nReal, the samples rad[b * nPad + e] (b < nSamples) onto color[list[e]] and their
+// squares onto moment[list[e]], in sample order (k_accumulate_checkpoints' operations).
+// launch_adaptive_mark: after round a.c, unconv[P] = the convergence test failed (first: counts set to a.c first).
+// launch_adaptive_select: active[P] = count a.c and an unconverged entry within a.radius in its view, counts of the
+// active entries set to a.next; then the active P in ascending order into list and their number into *numActive
+// (device), through cub (temp: adaptive_select_temp_bytes(n)).
+// launch_list_pad: list[n .. nPad) = list[n-1], nPad - n < 32.
+struct AdaptiveArgs
+{
+  float tau, eps; // threshold and luminance floor (b2pt_adaptive_params)
+  int radius, W, H;
+  int c, next; // samples of the round just finished, samples after the next one
+  int first;   // round 0: the counts are not yet written
+};
+cudaError_t launch_accumulate_list(float4* color, float4* moment, const float4* rad, const uint32_t* list, int nReal,
+                                   int nPad, int nSamples, unsigned long long* nanCounter, cudaStream_t stream);
+cudaError_t launch_adaptive_mark(const float4* color, const float4* moment, int32_t* counts, uint8_t* unconv, int64_t n,
+                                 const AdaptiveArgs& a, cudaStream_t stream);
+size_t adaptive_select_temp_bytes(int64_t n);
+cudaError_t launch_adaptive_select(const uint8_t* unconv, int32_t* counts, uint8_t* active, int64_t n,
+                                   const AdaptiveArgs& a, uint32_t* list, int32_t* numActive, void* temp,
+                                   size_t tempBytes, cudaStream_t stream);
+cudaError_t launch_list_pad(uint32_t* list, int n, int nPad, cudaStream_t stream);
+// launch_normalize / launch_pnm16 with spp = counts[i] per entry
+cudaError_t launch_normalize_counts(float4* color, int64_t n, const int32_t* counts, cudaStream_t stream);
+cudaError_t launch_pnm16_counts(const float4* color, int64_t n, const int32_t* counts, uint16_t* rgb,
+                                cudaStream_t stream);
 cudaError_t launch_create_rays(const B2Camera& cam, uint32_t* seeds, float* dx, float* dy, float* dz, float* ox,
                                float* oy, float* oz, long long* pixelIdx, cudaStream_t stream);
 cudaError_t launch_intersect(const B2SmallScene* small, const B2BvhScene* bvh, int64_t n, const float* ox,

@@ -298,6 +298,9 @@ struct B2RenderArgs
   // BVH pipeline, bounces >= 1 in region mode: the rays of the queue in spatially sorted order (k_sort_keys /
   // k_sort_scatter: perm[j] = queue entry of the j-th ray by origin cell and direction octant); warp w traces the
   // chunk [w*chunk, (w+1)*chunk) of it, chunk = total / numWarps rounded up to whole tiles.  nullptr = queue order.
+  // Bounce 0 of a listed round (k_trace LISTED, b2pt_render_views_adaptive): the list instead -- path id b * nPixels
+  // + e traces sample sampleBase + b of canvas entry perm[e] = view * sppPerView + pixel with camera views[view];
+  // nPixels is the padded list length, and sppPerView / divSpp* hold the pixels per view.
   const uint32_t* perm;
   // BVH pipeline with a binary tree and sorted rays: the closest hit of queue entry r, written by k_bvh_hits
   // (x = bits of t, y = primitive code or B2PT_MISS) and consumed by k_resolve_hits.  nullptr = k_trace does both.

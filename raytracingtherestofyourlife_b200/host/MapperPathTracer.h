@@ -130,6 +130,13 @@ public:
                                    const std::vector<vtkm::rendering::Camera>& cameras,
                                    const std::vector<int>& checkpoints, std::vector<unsigned short>& pnm,
                                    std::vector<unsigned short>& denoisedPnm);
+  // Adaptive sampling of the sweep (b2pt_render_views_adaptive with its default epsilon and radius): rounds is a
+  // checkpoint list ending with the sample count; every pixel stops at the first round whose variance test it passes.
+  // pnm: [view][pixel] the integers of RenderCellsViewsPnm computed with each pixel's own count; counts: [view][pixel]
+  // the samples each pixel received.
+  void RenderCellsViewsAdaptivePnm(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
+                                   const std::vector<vtkm::rendering::Camera>& cameras, const std::vector<int>& rounds,
+                                   float threshold, std::vector<unsigned short>& pnm, std::vector<int>& counts);
   // The -direct G-buffers of main.cc:402-422 (what MapperQuadNormals / MapperQuadAlbedo leave in the canvas colour
   // buffer, raytracing/RayTracerNormals.cxx / RayTracerAlbedo.cxx, and a depth image) for the canvas set with
   // SetCanvas: one un-jittered ray per pixel, closest quad hit, the reference's two Shade rules (b2pt_render_direct).

@@ -33,6 +33,12 @@
 // with its default parameters), guided by the sweep's per-pixel variance, albedo, normal and depth, written with save()'s
 // arithmetic.  The radiance files (and the -features PFMs) stay byte-identical to a run without -denoise.  -denoise with
 // -direct, or without a sweep, is an error (exit 1).
+// -adaptive <tau> (with -hemisphere or -fibonacci and -checkpoints) renders the sweep adaptively instead: the
+// checkpoints and samplecount are the rounds, and after each round a pixel stops when the relative standard error of
+// its mean luminance is below tau (b2pt_render_views_adaptive, default epsilon and radius).  It writes
+// <out>-adaptive-<phi>-<theta>.pnm (save()'s arithmetic with each pixel's own sample count) and
+// <out>-spp-<phi>-<theta>.pfm (Pf, the sample count of every pixel).  -adaptive without -checkpoints, with -direct,
+// -features or -denoise, or with a tau that is not a number >= 0 is an error (exit 1).
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
@@ -68,6 +74,9 @@ struct Options
   std::vector<int> checkpoints; // -checkpoints, parsed and checked by checkCheckpoints
   bool features = false;
   bool denoise = false;
+  bool adaptiveGiven = false;
+  std::string adaptiveArg;
+  float adaptive = 0.f; // -adaptive, parsed and checked by checkAdaptive
 };
 
 Options parse(int argc, char** argv)
@@ -109,6 +118,12 @@ Options parse(int argc, char** argv)
       o.features = true;
     else if (!std::strcmp(argv[i], "-denoise"))
       o.denoise = true;
+    else if (!std::strcmp(argv[i], "-adaptive"))
+    {
+      o.adaptiveGiven = true;
+      if (i + 1 < argc)
+        o.adaptiveArg = argv[++i];
+    }
     else if (!std::strcmp(argv[i], "-checkpoints"))
     {
       o.checkpointsGiven = true;
@@ -167,6 +182,27 @@ std::string checkDenoise(const Options& o)
     return "-denoise cannot be combined with -direct";
   if (!o.hemi && !o.fibonacci)
     return "-denoise needs -hemisphere or -fibonacci";
+  return "";
+}
+
+// Parses -adaptive into o.adaptive; returns an error message, empty when it is usable or absent.
+std::string checkAdaptive(Options& o)
+{
+  if (!o.adaptiveGiven)
+    return "";
+  if (o.direct)
+    return "-adaptive cannot be combined with -direct";
+  if (o.features || o.denoise)
+    return "-adaptive cannot be combined with -features or -denoise";
+  if (!o.hemi && !o.fibonacci)
+    return "-adaptive needs -hemisphere or -fibonacci";
+  if (!o.checkpointsGiven)
+    return "-adaptive needs -checkpoints (the rounds before samplecount)";
+  char* end = nullptr;
+  const float tau = std::strtof(o.adaptiveArg.c_str(), &end);
+  if (o.adaptiveArg.empty() || *end != '\0' || !(tau >= 0.f))
+    return "-adaptive takes a threshold >= 0, got '" + o.adaptiveArg + "'";
+  o.adaptive = tau;
   return "";
 }
 
@@ -352,6 +388,21 @@ int renderViews(CornellBox& cb, const Options& o, const std::vector<vtkm::render
   std::vector<unsigned short> pnm, denoised;
   std::vector<int> counts = o.checkpoints; // -checkpoints: one render, its images at every count up to samplecount
   counts.push_back(o.samples);
+  if (o.adaptiveGiven)
+  { // the rounds are the counts; one image and one sample-count map per view
+    std::vector<int> spp;
+    mapper.RenderCellsViewsAdaptivePnm(cb.ds.GetCellSet(), cb.coord, cameras, counts, o.adaptive, pnm, spp);
+    const size_t n = static_cast<size_t>(o.x) * o.y;
+    std::vector<float> map(n);
+    for (size_t v = 0; v < cameras.size(); ++v)
+    {
+      savePnm16(viewName(o.out + "-adaptive", angles[v].first, angles[v].second), o.x, o.y, &pnm[v * n * 3]);
+      for (size_t i = 0; i < n; ++i)
+        map[i] = static_cast<float>(spp[v * n + i]);
+      savePfm(viewName(o.out + "-spp", angles[v].first, angles[v].second), o.x, o.y, 1, map);
+    }
+    return static_cast<int>(cameras.size());
+  }
   if (o.denoise) // the same integers as below, from the float sums the filter needs
     mapper.RenderCellsViewsDenoisedPnm(cb.ds.GetCellSet(), cb.coord, cameras, counts, pnm, denoised);
   else if (counts.size() > 1)
@@ -483,6 +534,8 @@ int main(int argc, char* argv[])
     bad = checkFeatures(o);
   if (bad.empty())
     bad = checkDenoise(o);
+  if (bad.empty())
+    bad = checkAdaptive(o);
   if (!bad.empty())
   {
     std::cerr << "error: " << bad << std::endl;
