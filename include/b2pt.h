@@ -110,14 +110,20 @@ int b2pt_build_bvh(b2pt_ctx* ctx);
 int b2pt_build_bvh_ex(b2pt_ctx* ctx, uint32_t flags);
 
 /* Moved spheres: new centres (3 floats per sphere, the order of b2pt_set_scene) and, optionally, radii; counts and
- * materials stay.  The reference has no counterpart (its scene is static); this is the input side of
- * b2pt_refit_bvh.  Waits for renders in flight. */
+ * materials stay.  A light sphere moves with its scene sphere and takes its new radius.  The reference has no
+ * counterpart (its scene is static); this is the input side of b2pt_refit_bvh.  Waits for renders in flight.  Every
+ * later trace sees the moved spheres: the kernel-parameter path takes them at once, and on a BVH the next trace call
+ * first refits the binary tree (as b2pt_refit_bvh does) or rebuilds the 8-wide one with its build flags, unless
+ * b2pt_refit_bvh ran in between.  NULL centres: B2PT_ERR_BAD_VALUE; before b2pt_set_scene: B2PT_ERR_STATE. */
 int b2pt_update_spheres(b2pt_ctx* ctx, const float* centers, const float* radii);
 /* Refit instead of rebuild: the tree built by b2pt_build_bvh keeps its topology and every node box is recomputed
  * bottom-up on the device from the primitives' current geometry (one kernel, atomic arrival counters as in the LBVH
  * build).  The reference's equivalent is a full LinearBVH::Construct on every RenderCells (QuadIntersector.cxx:134,
  * SphereIntersector.cxx:75).  Closest hits equal a fresh build's (they do not depend on the tree); traversal slows
- * down as primitives drift away from the positions the tree was built for.  Binary tree only. */
+ * down as primitives drift away from the positions the tree was built for.  Optional after b2pt_update_spheres (the
+ * next trace refits a tree the update left behind); calling it keeps the refit out of the next trace call.  Binary
+ * tree only: B2PT_ERR_UNSUPPORTED under B2PT_FLAG_WIDE_BVH, whose tree the next trace rebuilds.  B2PT_ERR_STATE before
+ * b2pt_build_bvh. */
 int b2pt_refit_bvh(b2pt_ctx* ctx);
 
 /* ---- camera -------------------------------------------------------------------------------- */

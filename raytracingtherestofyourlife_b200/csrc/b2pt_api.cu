@@ -154,6 +154,8 @@ struct b2pt_ctx
   int32_t tracedQuads = 0, tracedSph = 0, bvhNodes = 0;
   float sortLo[3] = { 0.f, 0.f, 0.f }, sortHi[3] = { 1.f, 1.f, 1.f }; // scene box (cells of the ray sort)
   uint32_t builtFlags = 0;
+  size_t treeSlots = 0;   // primitives in the binary tree (B2PT_VALIDATE_BVH)
+  bool treeStale = false; // b2pt_update_spheres moved spheres since the BVH was last built or refitted
 
   // camera
   B2Camera cam{};
@@ -653,9 +655,79 @@ int b2pt_set_scene(b2pt_ctx* ctx, const float* pts, int64_t nPts, const int64_t*
 
 static constexpr uint32_t kBuildFlags = B2PT_BUILD_FLAGS;
 
+// B2PT_VALIDATE_BVH debug self-check of the binary tree on the device, after a build and after a refit: every primitive
+// reachable exactly once, its padded box inside the boxes of all its ancestors.
+static int validate_binary_tree(b2pt_ctx* ctx, size_t nNodes)
+{
+  if (!getenv("B2PT_VALIDATE_BVH") || nNodes == 0)
+    return B2PT_OK;
+  CU(cudaStreamSynchronize(ctx->stream));
+  const size_t nSlots = ctx->treeSlots;
+  std::vector<B2BvhNode> hn(nNodes);
+  std::vector<int32_t> hs(nSlots);
+  CU(cudaMemcpy(hn.data(), ctx->dNodes.p, nNodes * sizeof(B2BvhNode), cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(hs.data(), ctx->dSlots.p, nSlots * sizeof(int32_t), cudaMemcpyDeviceToHost));
+  std::vector<int> seen(nSlots, 0);
+  struct W
+  {
+    int32_t node;
+    float lo[3], hi[3];
+  };
+  std::vector<W> st;
+  W r{};
+  r.node = 0;
+  for (int c = 0; c < 3; ++c)
+    r.lo[c] = hn[0].bmin[c], r.hi[c] = hn[0].bmax[c];
+  st.push_back(r);
+  size_t bad = 0, visited = 0;
+  while (!st.empty())
+  {
+    const W w = st.back();
+    st.pop_back();
+    const B2BvhNode& nd = hn[(size_t)w.node];
+    for (int c = 0; c < 3; ++c)
+      if (nd.bmin[c] < w.lo[c] || nd.bmax[c] > w.hi[c])
+        ++bad;
+    if (nd.count > 0)
+    {
+      for (int k = 0; k < nd.count; ++k)
+      {
+        const int32_t enc = hs[(size_t)nd.left + k];
+        ++seen[(size_t)nd.left + k];
+        ++visited;
+        float a[3], b[3];
+        if (enc >= 0)
+          b2pt::quad_aabb(ctx->quads[(size_t)enc], a, b);
+        else
+          b2pt::sphere_aabb(ctx->sph[(size_t)(~enc)], a, b);
+        for (int c = 0; c < 3; ++c)
+          if (a[c] < nd.bmin[c] || b[c] > nd.bmax[c])
+            ++bad;
+      }
+    }
+    else
+      for (int k = 0; k < 2; ++k)
+      {
+        W ch{};
+        ch.node = nd.left + k;
+        for (int c = 0; c < 3; ++c)
+          ch.lo[c] = nd.bmin[c], ch.hi[c] = nd.bmax[c];
+        st.push_back(ch);
+      }
+  }
+  size_t once = 0;
+  for (int v : seen)
+    once += v == 1;
+  if (bad || once != nSlots || visited != nSlots)
+    return fail(B2PT_ERR_STATE, "BVH validation failed: %zu box violations, %zu of %zu slots reached once", bad, once,
+                nSlots);
+  return B2PT_OK;
+}
+
 static int build_trace_structures(b2pt_ctx* ctx, uint32_t flags)
 {
   ctx->haveParents = false;
+  ctx->treeStale = false;
   ctx->builtFlags = flags & kBuildFlags;
   // Drop bit-identical duplicate quads: a later copy computes the same t and loses the strict t<tmax
   // comparison (Surface.h:178-179), so removing it cannot change any result.
@@ -1024,68 +1096,9 @@ static int build_trace_structures(b2pt_ctx* ctx, uint32_t flags)
     CU(cudaStreamSynchronize(ctx->stream)); // host vectors go out of scope
   }
   CU(cudaStreamSynchronize(ctx->stream));
-  if (getenv("B2PT_VALIDATE_BVH") && nNodes > 0)
-  { // debug self-check: every primitive reachable exactly once, its padded box inside the boxes of all its ancestors
-    const size_t nSlots = treeQuads.size() + ctx->sph.size();
-    std::vector<B2BvhNode> hn(nNodes);
-    std::vector<int32_t> hs(nSlots);
-    CU(cudaMemcpy(hn.data(), ctx->dNodes.p, nNodes * sizeof(B2BvhNode), cudaMemcpyDeviceToHost));
-    CU(cudaMemcpy(hs.data(), ctx->dSlots.p, nSlots * sizeof(int32_t), cudaMemcpyDeviceToHost));
-    std::vector<int> seen(nSlots, 0);
-    struct W
-    {
-      int32_t node;
-      float lo[3], hi[3];
-    };
-    std::vector<W> st;
-    W r{};
-    r.node = 0;
-    for (int c = 0; c < 3; ++c)
-      r.lo[c] = hn[0].bmin[c], r.hi[c] = hn[0].bmax[c];
-    st.push_back(r);
-    size_t bad = 0, visited = 0;
-    while (!st.empty())
-    {
-      const W w = st.back();
-      st.pop_back();
-      const B2BvhNode& nd = hn[(size_t)w.node];
-      for (int c = 0; c < 3; ++c)
-        if (nd.bmin[c] < w.lo[c] || nd.bmax[c] > w.hi[c])
-          ++bad;
-      if (nd.count > 0)
-      {
-        for (int k = 0; k < nd.count; ++k)
-        {
-          const int32_t enc = hs[(size_t)nd.left + k];
-          ++seen[(size_t)nd.left + k];
-          ++visited;
-          float a[3], b[3];
-          if (enc >= 0)
-            b2pt::quad_aabb(ctx->quads[(size_t)enc], a, b);
-          else
-            b2pt::sphere_aabb(ctx->sph[(size_t)(~enc)], a, b);
-          for (int c = 0; c < 3; ++c)
-            if (a[c] < nd.bmin[c] || b[c] > nd.bmax[c])
-              ++bad;
-        }
-      }
-      else
-        for (int k = 0; k < 2; ++k)
-        {
-          W ch{};
-          ch.node = nd.left + k;
-          for (int c = 0; c < 3; ++c)
-            ch.lo[c] = nd.bmin[c], ch.hi[c] = nd.bmax[c];
-          st.push_back(ch);
-        }
-    }
-    size_t once = 0;
-    for (int v : seen)
-      once += v == 1;
-    if (bad || once != nSlots || visited != nSlots)
-      return fail(B2PT_ERR_STATE, "BVH validation failed: %zu box violations, %zu of %zu slots reached once", bad, once,
-                  nSlots);
-  }
+  ctx->treeSlots = treeQuads.size() + ctx->sph.size();
+  if (int rc = validate_binary_tree(ctx, nNodes))
+    return rc;
   // B2PT_FLAG_WIDE_BVH: the traversal kernels walk the 8-wide compressed tree collapsed from the binary one
   // (b2pt_wide.h); primSlots and leafSph are rewritten in its leaf order.  Opt-in (B2PT_FLAG_WIDE_BVH): the binary tree measured faster.
   ctx->bvh.wide = nullptr;
@@ -1207,22 +1220,21 @@ int b2pt_update_spheres(b2pt_ctx* ctx, const float* centers, const float* radii)
     CU(cudaMemcpyAsync(ctx->dSph.p, ctx->sph.data(), ctx->sph.size() * sizeof(B2Sphere), cudaMemcpyHostToDevice,
                        ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
+  // The node boxes and the leaf-ordered sphere copies (leafSph) still hold the old geometry: the next trace refits or
+  // rebuilds the tree first (refresh_stale_tree) unless b2pt_refit_bvh does it before.
+  ctx->treeStale = true;
   return B2PT_OK;
 }
 
-int b2pt_refit_bvh(b2pt_ctx* ctx)
+// The binary tree's boxes and leafSph recomputed from the current geometry, topology kept (b2pt_refit_bvh).
+static int refit_tree(b2pt_ctx* ctx)
 {
-  if (int rc = bind(ctx))
-    return rc;
-  if (!ctx->haveScene || !ctx->haveBvh)
-    return fail(B2PT_ERR_STATE, "b2pt_refit_bvh before b2pt_build_bvh");
-  if (!ctx->useBvh)
-    return B2PT_OK; // no tree on the kernel-parameter path (b2pt_update_spheres refreshed its tables)
-  if (ctx->bvh.wide)
-    return fail(B2PT_ERR_UNSUPPORTED, "b2pt_refit_bvh refits the binary tree; rebuild when B2PT_FLAG_WIDE_BVH is in use");
   const int nNodes = ctx->bvhNodes;
   if (nNodes <= 0)
+  {
+    ctx->treeStale = false;
     return B2PT_OK;
+  }
   if (!ctx->haveParents)
   { // one-time: parent links of the tree as it sits on the device (either builder's layout)
     std::vector<B2BvhNode> hn((size_t)nNodes);
@@ -1252,7 +1264,30 @@ int b2pt_refit_bvh(b2pt_ctx* ctx)
   }
   CU(b2pt::refit_bvh_device(ctx->dNodes.p, ctx->dParent.p, ctx->dArrived.p, nNodes, ctx->dSlots.p, ctx->dQuads.p,
                             ctx->dSph.p, ctx->dLeafSph.p, ctx->stream));
-  return B2PT_OK;
+  ctx->treeStale = false;
+  return validate_binary_tree(ctx, (size_t)nNodes);
+}
+
+int b2pt_refit_bvh(b2pt_ctx* ctx)
+{
+  if (int rc = bind(ctx))
+    return rc;
+  if (!ctx->haveScene || !ctx->haveBvh)
+    return fail(B2PT_ERR_STATE, "b2pt_refit_bvh before b2pt_build_bvh");
+  if (!ctx->useBvh)
+    return B2PT_OK; // no tree on the kernel-parameter path (b2pt_update_spheres refreshed its tables)
+  if (ctx->bvh.wide)
+    return fail(B2PT_ERR_UNSUPPORTED, "b2pt_refit_bvh refits the binary tree; rebuild when B2PT_FLAG_WIDE_BVH is in use");
+  return refit_tree(ctx);
+}
+
+// Before a trace: a tree that b2pt_update_spheres left behind the spheres is brought up to date -- the binary tree is
+// refitted, the 8-wide tree (which has no refit) rebuilt with the flags it was built with.
+static int refresh_stale_tree(b2pt_ctx* ctx)
+{
+  if (!ctx->treeStale)
+    return B2PT_OK;
+  return ctx->bvh.wide ? build_trace_structures(ctx, ctx->builtFlags) : refit_tree(ctx);
 }
 
 // Camera.cxx:913-914 Look; :803-811 SetUp; RayGen ctor :438-476 with fovX = fovY (:936-938), zoom off.
@@ -1482,7 +1517,8 @@ static void plan_batches(int64_t units, int64_t unitPaths, int64_t maxPathsPerBa
 }
 
 // MapperPathTracer::RenderCellsImpl builds its acceleration structures on every call (:275-276); here
-// they are rebuilt only when the scene or the build-affecting flags changed.
+// they are rebuilt only when the scene or the build-affecting flags changed, and brought up to date after
+// b2pt_update_spheres (refresh_stale_tree).
 static int ensure_built_for(b2pt_ctx* ctx, uint32_t flags)
 {
   const uint32_t buildFlags = flags & kBuildFlags;
@@ -1492,7 +1528,7 @@ static int ensure_built_for(b2pt_ctx* ctx, uint32_t flags)
       return rc;
     ctx->haveBvh = true;
   }
-  return B2PT_OK;
+  return refresh_stale_tree(ctx);
 }
 
 // A listed round of b2pt_render_views_adaptive: the canvas entries entries[0 .. nReal) (view * viewPixels + pixel,
@@ -2728,6 +2764,8 @@ int b2pt_render_direct_views(b2pt_ctx* ctx, int nViews, const float* views, int 
   return render_direct_chunks(ctx, nViews, dv.data(), (int64_t)W * H, normals, albedo, depth, primId);
 }
 
+// The trace structures for a call without build flags: the ones built last (the default ones if none were), up to
+// date with b2pt_update_spheres.
 static int ensure_trace(b2pt_ctx* ctx)
 {
   if (!ctx->haveScene)
@@ -2738,7 +2776,7 @@ static int ensure_trace(b2pt_ctx* ctx)
       return rc;
     ctx->haveBvh = true;
   }
-  return B2PT_OK;
+  return refresh_stale_tree(ctx);
 }
 
 int b2pt_primary_hits(b2pt_ctx* ctx, int32_t* primId, float* t)
