@@ -270,6 +270,27 @@ void b2pt_adaptive_defaults(b2pt_adaptive_params* p);
 int b2pt_render_views_adaptive(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nRounds,
                                const int* rounds, int maxDepth, const b2pt_adaptive_params* params, uint32_t flags,
                                void* rgbaOut, float* moment2Out, int32_t* countOut, int64_t* activeOut);
+/* An adaptive sweep denoised on the device: b2pt_render_views_adaptive, then b2pt_denoise_views' filter at every
+ * pixel's own sample count n_p, from the sums the render leaves on the device (only the outputs are copied).
+ * rgbaOut and countOut are, bit for bit, what b2pt_render_views_adaptive returns for the same arguments (flags 0,
+ * VIEWS_NORMALIZE or VIEWS_PNM16), and afterwards b2pt_views_device_ptr and the statistics are as it leaves them.
+ * Guides, [view][j*W+i] float4, either may be NULL: albedoOut = (sum albedo.rgb, sum hit) and normalDepthOut =
+ * (sum normal.xyz, sum depth) over the pixel's own samples s = 0 .. n_p-1 with b2pt_render_views_features' per-sample
+ * rule, so a pixel holds the bits of b2pt_render_views_features(views, rounds) in the slice k with rounds[k] == n_p.
+ * denoisedOut: b2pt_denoise_views' filter with checkpoints[k] replaced by n_p in the prep (c = n_p >= rounds[0] >= 2,
+ * so V0 always exists): m = dn(S)/n_p, V0 = sum_ch w_ch max(0, dn(Q_ch)/n_p - m_ch^2)/(n_p - 1), g_a = (a/n_p, h/n_p),
+ * g_n = N/n_p, z = D/h where h > 0, from S before any VIEWS_NORMALIZE conversion; then `levels` a-trous levels.  Per
+ * pixel float4 (x_L.rgb, V_L), or under VIEWS_PNM16 uint16_t[3], the integers b2pt_read_pnm16 gives for x_L with
+ * spp = 1 (levels = 0: the adaptive rgbaOut integers).  adaptive NULL = b2pt_adaptive_defaults, denoise NULL =
+ * b2pt_denoise_defaults.  B2PT_ERR_BAD_VALUE, before anything runs: whatever b2pt_render_views_adaptive rejects,
+ * levels outside 0..10, a sigma that is NaN or <= 0, or rounds[K-1] > 2^24.  nViews == 0 does nothing; no scene gives
+ * B2PT_ERR_STATE.  Views are denoised in chunks of whole views through library-owned staging of at most
+ * max(2^23, W*H) float4 per buffer; the result depends neither on the chunking nor on the launch shape.  The context's
+ * camera and canvas are untouched.  Synchronises the stream.  The reference has no counterpart. */
+int b2pt_render_views_adaptive_denoised(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nRounds,
+                                        const int* rounds, int maxDepth, const b2pt_adaptive_params* adaptive,
+                                        const b2pt_denoise_params* denoise, uint32_t flags, void* rgbaOut,
+                                        int32_t* countOut, float* albedoOut, float* normalDepthOut, void* denoisedOut);
 void* b2pt_views_device_ptr(b2pt_ctx* ctx);
 int b2pt_clear_color(b2pt_ctx* ctx);
 /* Host-side planning rule of the renders above, exposed for tests and capacity planning (no GPU needed): `units`

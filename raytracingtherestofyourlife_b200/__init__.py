@@ -103,6 +103,9 @@ SIGNATURES = {
     "b2pt_adaptive_defaults": (None, [C.POINTER(AdaptiveParams)]),
     "b2pt_render_views_adaptive": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, _i32, C.POINTER(AdaptiveParams),
                                           C.c_uint32, _vp, _vp, _vp, _vp]),
+    "b2pt_render_views_adaptive_denoised": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, _i32,
+                                                   C.POINTER(AdaptiveParams), C.POINTER(DenoiseParams), C.c_uint32,
+                                                   _vp, _vp, _vp, _vp, _vp]),
     "b2pt_views_device_ptr": (_vp, [_vp]),
     "b2pt_plan_batches": (_i32, [_i64, _i64, _i64, _i32, _vp, _vp]),
     "b2pt_clear_color": (_i32, [_vp]),
@@ -382,6 +385,31 @@ class Context:
                                                 None if params is None else C.byref(params), flags, _p(image),
                                                 _p(moment2), _p(counts), _p(active)))
         return image, moment2, counts, active
+
+    def render_views_adaptive_denoised(self, views, W, H, rounds, max_depth, adaptive=None, denoise=None, flags=0,
+                                       features=False):
+        """b2pt_render_views_adaptive_denoised: render_views_adaptive, then the a-trous filter of denoise_views with
+        every pixel's own sample count, on the device.  adaptive is an AdaptiveParams and denoise a DenoiseParams
+        (None: the defaults).  Returns (image, counts, denoised): image and counts as render_views_adaptive returns
+        them, denoised float32 [nViews, H*W, 4] (denoised mean rgb, filtered variance) or uint16 [nViews, H*W, 3] under
+        FLAG_VIEWS_PNM16; with features=True also (albedo, normal_depth), float32 [nViews, H*W, 4] sums over each
+        pixel's own samples."""
+        v = np.ascontiguousarray(views, np.float32).reshape(-1, 10)
+        r = np.ascontiguousarray(rounds, np.int32).reshape(-1)
+        nv = v.shape[0]
+        dt, ch = (np.uint16, 3) if flags & FLAG_VIEWS_PNM16 else (np.float32, 4)
+        image = np.empty((nv, W * H, ch), dt)
+        counts = np.empty((nv, W * H), np.int32)
+        denoised = np.empty((nv, W * H, ch), dt)
+        albedo = np.empty((nv, W * H, 4), np.float32) if features else None
+        normal_depth = np.empty((nv, W * H, 4), np.float32) if features else None
+        _check(lib().b2pt_render_views_adaptive_denoised(
+            self._h, nv, _p(v), W, H, r.shape[0], _p(r), max_depth, None if adaptive is None else C.byref(adaptive),
+            None if denoise is None else C.byref(denoise), flags, _p(image), _p(counts), _p(albedo),
+            _p(normal_depth), _p(denoised)))
+        if features:
+            return image, counts, denoised, albedo, normal_depth
+        return image, counts, denoised
 
     def clear_color(self):
         _check(lib().b2pt_clear_color(self._h))

@@ -2194,17 +2194,42 @@ void b2pt_adaptive_defaults(b2pt_adaptive_params* p)
   p->radius = 1;
 }
 
+// b2pt_denoise_views' checks of its parameters (fn: the entry point named in the messages).
+static int check_denoise_params(const char* fn, const b2pt_denoise_params& P)
+{
+  if (P.levels < 0 || P.levels > 10)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: levels must be in [0,10], got %d", fn, P.levels);
+  const float sigma[4] = { P.sigmaLum, P.sigmaAlbedo, P.sigmaNormal, P.sigmaDepth };
+  const char* const sigmaName[4] = { "sigmaLum", "sigmaAlbedo", "sigmaNormal", "sigmaDepth" };
+  for (int s = 0; s < 4; ++s)
+    if (!(sigma[s] > 0.f)) // NaN fails too
+      return fail(B2PT_ERR_BAD_VALUE, "%s: %s must be > 0 (or +inf), got %g", fn, sigmaName[s], (double)sigma[s]);
+  return B2PT_OK;
+}
+
+// The denoising stage of b2pt_render_views_adaptive_denoised: its parameters and outputs.
+struct AdaptiveDenoise
+{
+  b2pt_denoise_params P;
+  float *albedoOut, *normalDepthOut;
+  void* out;
+};
+static int denoise_adaptive_sweep(b2pt_ctx* ctx, int64_t nViews, int W, int H, int rounds0, uint32_t flags,
+                                  const AdaptiveDenoise& dn);
+
 // Adaptive sampling of a view sweep (DESIGN.md 8f).  Round 0 is render_view_sweep at rounds[0] with the sums of squares
 // kept on the device, so it is b2pt_render_views_checkpoints by construction.  After round k, k_adaptive_mark and
 // k_adaptive_select choose the canvas entries of round k+1 and cub compacts them into ctx->adList in ascending order;
 // the one host read per round is that list's length.  Round k+1 is render_impl over the list (samples
 // [rounds[k], rounds[k+1]) of every listed entry), which continues each entry's sums in sample order, so an entry
-// that ends with n samples holds the bits of a uniform render of n samples.
-int b2pt_render_views_adaptive(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nRounds,
-                               const int* rounds, int maxDepth, const b2pt_adaptive_params* params, uint32_t flags,
-                               void* rgbaOut, float* moment2Out, int32_t* countOut, int64_t* activeOut)
+// that ends with n samples holds the bits of a uniform render of n samples.  dn (b2pt_render_views_adaptive_denoised,
+// DESIGN.md 8g): after the last round and before the image's conversions, the sweep is denoised from its sums on the
+// device (denoise_adaptive_sweep).  fn names the entry point in the messages.
+static int render_adaptive(b2pt_ctx* ctx, const char* fn, int nViews, const float* views, int W, int H, int nRounds,
+                           const int* rounds, int maxDepth, const b2pt_adaptive_params* params, uint32_t flags,
+                           void* rgbaOut, float* moment2Out, int32_t* countOut, int64_t* activeOut,
+                           const AdaptiveDenoise* dn)
 {
-  static const char* const fn = "b2pt_render_views_adaptive";
   if (int rc = bind(ctx))
     return rc;
   if (int rc = check_view_list(fn, nViews, views))
@@ -2228,6 +2253,13 @@ int b2pt_render_views_adaptive(b2pt_ctx* ctx, int nViews, const float* views, in
     return fail(B2PT_ERR_BAD_VALUE, "%s: epsilon must be > 0, got %g", fn, (double)P.epsilon);
   if (P.radius < 0 || P.radius > 4)
     return fail(B2PT_ERR_BAD_VALUE, "%s: radius must be in [0,4], got %d", fn, P.radius);
+  if (dn)
+  {
+    if (int rc = check_denoise_params(fn, dn->P))
+      return rc;
+    if (rounds[nRounds - 1] > (1 << 24))
+      return fail(B2PT_ERR_BAD_VALUE, "%s: more than 2^24 samples (the hit count must stay an exact float)", fn);
+  }
   std::vector<B2Camera> cams;
   if (int rc = make_view_cameras(nViews, views, W, H, cams))
     return rc;
@@ -2315,6 +2347,9 @@ int b2pt_render_views_adaptive(b2pt_ctx* ctx, int nViews, const float* views, in
     CU(b2pt::launch_adaptive_mark(ctx->viewColor.p, ctx->ckptMoment.p, ctx->adCounts.p, ctx->adUnconv.p, NV, a,
                                   ctx->stream));
   }
+  if (dn) // reads the sums before the conversions below
+    if (int rc = denoise_adaptive_sweep(ctx, nViews, W, H, rounds[0], flags, *dn))
+      return rc;
   if (flags & B2PT_FLAG_VIEWS_PNM16)
   {
     if (rgbaOut)
@@ -2342,6 +2377,31 @@ int b2pt_render_views_adaptive(b2pt_ctx* ctx, int nViews, const float* views, in
   ctx->stats.paths = paths;
   ctx->stats.launches = launches;
   return B2PT_OK;
+}
+
+int b2pt_render_views_adaptive(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nRounds,
+                               const int* rounds, int maxDepth, const b2pt_adaptive_params* params, uint32_t flags,
+                               void* rgbaOut, float* moment2Out, int32_t* countOut, int64_t* activeOut)
+{
+  return render_adaptive(ctx, "b2pt_render_views_adaptive", nViews, views, W, H, nRounds, rounds, maxDepth, params,
+                         flags, rgbaOut, moment2Out, countOut, activeOut, nullptr);
+}
+
+int b2pt_render_views_adaptive_denoised(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nRounds,
+                                        const int* rounds, int maxDepth, const b2pt_adaptive_params* adaptive,
+                                        const b2pt_denoise_params* denoise, uint32_t flags, void* rgbaOut,
+                                        int32_t* countOut, float* albedoOut, float* normalDepthOut, void* denoisedOut)
+{
+  AdaptiveDenoise dn{};
+  if (denoise)
+    dn.P = *denoise;
+  else
+    b2pt_denoise_defaults(&dn.P);
+  dn.albedoOut = albedoOut;
+  dn.normalDepthOut = normalDepthOut;
+  dn.out = denoisedOut;
+  return render_adaptive(ctx, "b2pt_render_views_adaptive_denoised", nViews, views, W, H, nRounds, rounds, maxDepth,
+                         adaptive, flags, rgbaOut, nullptr, countOut, nullptr, &dn);
 }
 
 // Denoiser guides of a view sweep (k_view_features).  Sample s of a pixel is traced from the stream the render gives it
@@ -2451,13 +2511,8 @@ int b2pt_denoise_views(b2pt_ctx* ctx, int nViews, int W, int H, int nCheckpoints
     P = *params;
   else
     b2pt_denoise_defaults(&P);
-  if (P.levels < 0 || P.levels > 10)
-    return fail(B2PT_ERR_BAD_VALUE, "%s: levels must be in [0,10], got %d", fn, P.levels);
-  const float sigma[4] = { P.sigmaLum, P.sigmaAlbedo, P.sigmaNormal, P.sigmaDepth };
-  const char* const sigmaName[4] = { "sigmaLum", "sigmaAlbedo", "sigmaNormal", "sigmaDepth" };
-  for (int s = 0; s < 4; ++s)
-    if (!(sigma[s] > 0.f)) // NaN fails too
-      return fail(B2PT_ERR_BAD_VALUE, "%s: %s must be > 0 (or +inf), got %g", fn, sigmaName[s], (double)sigma[s]);
+  if (int rc = check_denoise_params(fn, P))
+    return rc;
   if (flags & ~B2PT_FLAG_VIEWS_PNM16)
     return fail(B2PT_ERR_BAD_VALUE, "%s: flags may only hold VIEWS_PNM16", fn);
   const int K = nCheckpoints;
@@ -2512,6 +2567,66 @@ int b2pt_denoise_views(b2pt_ctx* ctx, int nViews, int W, int H, int nCheckpoints
     }
   }
   CU(cudaStreamSynchronize(ctx->stream));
+  return B2PT_OK;
+}
+
+// The denoising stage of render_adaptive, on the sweep it leaves on the device: the sums S (ctx->viewColor), the sums
+// of squares Q (ctx->ckptMoment), the counts n_p (ctx->adCounts) and the cameras (ctx->dViews).  Views run in chunks of
+// whole views through b2pt_denoise_views' staging (at most max(kDenoiseChunkFloat4, W*H) float4 per buffer): per
+// chunk, the guides at every pixel's own count into dnGuideA / dnGuideNZ (copied out when asked for), the prep with
+// c = n_p into dnX[0], the levels (k_atrous with one slice of count rounds[0] >= 2, so the colour term is on), the
+// PNM integers under VIEWS_PNM16, and the copy of the result.
+static int denoise_adaptive_sweep(b2pt_ctx* ctx, int64_t nViews, int W, int H, int rounds0, uint32_t flags,
+                                  const AdaptiveDenoise& dn)
+{
+  const int64_t N = (int64_t)W * H;
+  const bool pnm = (flags & B2PT_FLAG_VIEWS_PNM16) != 0;
+  b2pt::DenoiseArgs a{};
+  a.n = 1;
+  a.count[0] = rounds0;
+  a.hasMoments = 1;
+  a.sigmaLum = dn.P.sigmaLum, a.sigmaAlbedo = dn.P.sigmaAlbedo, a.sigmaNormal = dn.P.sigmaNormal;
+  a.sigmaDepth = dn.P.sigmaDepth;
+  const int64_t perChunk = std::max<int64_t>(1, kDenoiseChunkFloat4 / N);
+  const size_t cap = (size_t)(std::min<int64_t>(perChunk, nViews) * N);
+  CU(ctx->dnX[0].reserve(cap));
+  CU(ctx->dnX[1].reserve(cap));
+  CU(ctx->dnGuideA.reserve(cap));
+  CU(ctx->dnGuideNZ.reserve(cap));
+  if (pnm)
+    CU(ctx->pnm.reserve(cap * 3));
+  for (int64_t v0 = 0; v0 < nViews; v0 += perChunk)
+  {
+    const int nv = (int)std::min<int64_t>(perChunk, nViews - v0);
+    const int64_t n = nv * N, off = v0 * N;
+    CU(b2pt::launch_view_features_counts(ctx->useBvh ? nullptr : &ctx->small, ctx->useBvh ? &ctx->bvh : nullptr,
+                                         ctx->dViews.p + v0, nv, (int)N, ctx->seedOffset, ctx->adCounts.p + off,
+                                         ctx->dnGuideA.p, ctx->dnGuideNZ.p, ctx->stream));
+    if (dn.albedoOut)
+      CU(cudaMemcpyAsync(dn.albedoOut + 4 * off, ctx->dnGuideA.p, sizeof(float4) * (size_t)n, cudaMemcpyDeviceToHost,
+                         ctx->stream));
+    if (dn.normalDepthOut)
+      CU(cudaMemcpyAsync(dn.normalDepthOut + 4 * off, ctx->dnGuideNZ.p, sizeof(float4) * (size_t)n,
+                         cudaMemcpyDeviceToHost, ctx->stream));
+    CU(b2pt::launch_denoise_prep_counts(ctx->viewColor.p + off, ctx->ckptMoment.p + off, ctx->adCounts.p + off,
+                                        ctx->dnX[0].p, ctx->dnGuideA.p, ctx->dnGuideNZ.p, n, ctx->stream));
+    a.nViews = nv;
+    int cur = 0;
+    for (int level = 0; level < dn.P.levels; ++level, cur ^= 1)
+      CU(b2pt::launch_atrous(ctx->dnX[cur].p, ctx->dnX[cur ^ 1].p, ctx->dnGuideA.p, ctx->dnGuideNZ.p, W, H, 1 << level,
+                             a, ctx->stream));
+    const float4* res = ctx->dnX[cur].p;
+    if (pnm)
+    {
+      CU(b2pt::launch_pnm16(res, n, 1, ctx->pnm.p, ctx->stream));
+      if (dn.out)
+        CU(cudaMemcpyAsync(static_cast<uint16_t*>(dn.out) + 3 * off, ctx->pnm.p, sizeof(uint16_t) * 3 * (size_t)n,
+                           cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    else if (dn.out)
+      CU(cudaMemcpyAsync(static_cast<float4*>(dn.out) + off, res, sizeof(float4) * (size_t)n, cudaMemcpyDeviceToHost,
+                         ctx->stream));
+  }
   return B2PT_OK;
 }
 

@@ -23,6 +23,8 @@
 //   k_accumulate_list, k_adaptive_mark, k_adaptive_select, k_list_pad, k_normalize_counts, k_pnm16_counts
 //                                 adaptive sampling of a view sweep: accumulate a listed round, choose the next
 //                                 round's pixels from each pixel's variance, per-pixel-count conversions.
+//   k_view_features_counts<Scene>, k_denoise_prep_counts
+//                                 guides and denoiser prep of an adaptive sweep at each pixel's own sample count.
 //   k_create_rays, k_intersect, k_normalize, k_pnm16, k_fill_seeds, k_sum_peers: stage-level API kernels.
 //
 // Work distribution: queue and bins are statically partitioned into one region per persistent warp
@@ -1898,6 +1900,28 @@ __global__ void __launch_bounds__(256)
 // colour clamped to [0,1]), a hit flag, the shading normal and t; all zero on a miss.  The sums run in registers in
 // sample order (plain adds under -fmad=false) and slice k receives them after count[k] samples.
 template <class SceneT>
+__device__ __forceinline__ void add_feature_sample(const SceneT& scene, const B2Camera& cam, f3 o, int p,
+                                                   uint32_t seedOffset, int s, float4& alb, float4& nd)
+{
+  uint32_t rng = (uint32_t)p + seedOffset + (uint32_t)s * B2PT_GOLDEN;
+  const f3 d = raygen(cam, p, rng);
+  Hit hit;
+  f3 a = mk3(0.f, 0.f, 0.f), nrm = a;
+  float h = 0.f, t = 0.f;
+  if (trace(scene, o, d, 0.001f, FLT_MAX, hit))
+  {
+    a = hit.kind == 2 ? mk3(1.f, 1.f, 1.f)
+      : hit.kind == 1 ? mk3(fminf(fmaxf(hit.alb.x, 0.f), 1.f), fminf(fmaxf(hit.alb.y, 0.f), 1.f),
+                            fminf(fmaxf(hit.alb.z, 0.f), 1.f))
+                      : hit.alb;
+    nrm = hit.n;
+    h = 1.f;
+    t = hit.t;
+  }
+  alb.x += a.x, alb.y += a.y, alb.z += a.z, alb.w += h;
+  nd.x += nrm.x, nd.y += nrm.y, nd.z += nrm.z, nd.w += t;
+}
+template <class SceneT>
 __global__ void __launch_bounds__(256)
   k_view_features(const __grid_constant__ SceneT scene, const B2Camera* __restrict__ cams, int64_t n,
                   uint32_t nPixels, uint32_t divMagic, uint32_t divShift, uint32_t seedOffset,
@@ -1915,23 +1939,7 @@ __global__ void __launch_bounds__(256)
   int k = 0, next = ck.count[0];
   for (int s = 0; s < last; ++s)
   {
-    uint32_t rng = (uint32_t)p + seedOffset + (uint32_t)s * B2PT_GOLDEN;
-    const f3 d = raygen(cam, p, rng);
-    Hit hit;
-    f3 a = mk3(0.f, 0.f, 0.f), nrm = a;
-    float h = 0.f, t = 0.f;
-    if (trace(scene, o, d, 0.001f, FLT_MAX, hit))
-    {
-      a = hit.kind == 2 ? mk3(1.f, 1.f, 1.f)
-        : hit.kind == 1 ? mk3(fminf(fmaxf(hit.alb.x, 0.f), 1.f), fminf(fmaxf(hit.alb.y, 0.f), 1.f),
-                              fminf(fmaxf(hit.alb.z, 0.f), 1.f))
-                        : hit.alb;
-      nrm = hit.n;
-      h = 1.f;
-      t = hit.t;
-    }
-    alb.x += a.x, alb.y += a.y, alb.z += a.z, alb.w += h;
-    nd.x += nrm.x, nd.y += nrm.y, nd.z += nrm.z, nd.w += t;
+    add_feature_sample(scene, cam, o, p, seedOffset, s, alb, nd);
     if (s + 1 == next)
     {
       const int64_t e = (int64_t)k * n + idx;
@@ -1943,6 +1951,29 @@ __global__ void __launch_bounds__(256)
       next = k < ck.n ? ck.count[k] : 0;
     }
   }
+}
+
+// k_view_features with every (view, pixel) entry's own sample count (b2pt_render_views_adaptive_denoised): the sums
+// over samples s < counts[idx], stored once, so an entry of count c holds the bits of k_view_features' slice at c.
+template <class SceneT>
+__global__ void __launch_bounds__(256)
+  k_view_features_counts(const __grid_constant__ SceneT scene, const B2Camera* __restrict__ cams, int64_t n,
+                         uint32_t nPixels, uint32_t divMagic, uint32_t divShift, uint32_t seedOffset,
+                         const int32_t* __restrict__ counts, float4* albedoOut, float4* normalDepthOut)
+{
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n)
+    return;
+  const uint32_t view = fastdiv((uint32_t)idx, divMagic, divShift);
+  const int p = (int)((uint32_t)idx - view * nPixels);
+  const B2Camera cam = cams[view];
+  const f3 o = ld3(cam.pos);
+  float4 alb = make_float4(0.f, 0.f, 0.f, 0.f), nd = alb;
+  const int c = counts[idx];
+  for (int s = 0; s < c; ++s)
+    add_feature_sample(scene, cam, o, p, seedOffset, s, alb, nd);
+  albedoOut[idx] = alb;
+  normalDepthOut[idx] = nd;
 }
 
 // pathtracing/Camera.cxx:894-953: fills + RayGen + origin broadcast, fused.
@@ -2063,9 +2094,31 @@ __global__ void __launch_bounds__(256)
 __device__ __forceinline__ float dn_lum(float4 x) { return 0.2126f * x.x + 0.7152f * x.y + 0.0722f * x.z; }
 __device__ __forceinline__ float de_nan(float x) { return x == x ? x : 0.f; }
 
-// Per pixel of a chunk [k][view][pixel] (sliceLen = views * pixels), in place: the color sums S become (m, V0) with
-// m = dn(S)/c and V0 the variance of the mean luminance (0 where it does not exist), the albedo sums (a, h) become
-// g_a = (a/c, h/c) and the normal/depth sums (N, D) become (N/c, z), z = D/h when h > 0, else 0.
+// Entry idx of c samples: its color sums S[idx] become (m, V0) in x[idx] with m = dn(S)/c and V0 the variance of the
+// mean luminance from its sums of squares Q[idx] (when hasQ and c >= 2; otherwise 0), the albedo sums (a, h) in
+// ga[idx] become g_a = (a/c, h/c) and the normal/depth sums (N, D) in gnz[idx] become (N/c, z), z = D/h when h > 0,
+// else 0.  S may be x.
+__device__ __forceinline__ void denoise_prep_pixel(const float4* S, const float4* Q, float4* x, float4* ga, float4* gnz,
+                                                   long long idx, int c, int hasQ)
+{
+  const float cf = (float)c;
+  const float4 s = S[idx];
+  const float m0 = de_nan(s.x) / cf, m1 = de_nan(s.y) / cf, m2 = de_nan(s.z) / cf;
+  float V = 0.f;
+  if (hasQ && c >= 2)
+  {
+    const float4 q = Q[idx];
+    const float v0 = fmaxf(0.f, de_nan(q.x) / cf - m0 * m0), v1 = fmaxf(0.f, de_nan(q.y) / cf - m1 * m1),
+                v2 = fmaxf(0.f, de_nan(q.z) / cf - m2 * m2);
+    V = (0.2126f * v0 + 0.7152f * v1 + 0.0722f * v2) / (float)(c - 1);
+  }
+  x[idx] = make_float4(m0, m1, m2, V);
+  const float4 A = ga[idx], ND = gnz[idx];
+  ga[idx] = make_float4(A.x / cf, A.y / cf, A.z / cf, A.w / cf);
+  gnz[idx] = make_float4(ND.x / cf, ND.y / cf, ND.z / cf, A.w > 0.f ? ND.w / A.w : 0.f);
+}
+
+// Per pixel of a chunk [k][view][pixel] (sliceLen = views * pixels), in place, c = the slice's checkpoint count.
 __global__ void __launch_bounds__(256)
   k_denoise_prep(float4* __restrict__ x, const float4* __restrict__ moment, float4* __restrict__ ga,
                  float4* __restrict__ gnz, long long n, long long sliceLen, const __grid_constant__ DenoiseArgs a)
@@ -2074,21 +2127,20 @@ __global__ void __launch_bounds__(256)
   if (idx >= n)
     return;
   const int c = a.count[idx / sliceLen];
-  const float cf = (float)c;
-  const float4 S = x[idx];
-  const float m0 = de_nan(S.x) / cf, m1 = de_nan(S.y) / cf, m2 = de_nan(S.z) / cf;
-  float V = 0.f;
-  if (a.hasMoments && c >= 2)
-  {
-    const float4 Q = moment[idx];
-    const float v0 = fmaxf(0.f, de_nan(Q.x) / cf - m0 * m0), v1 = fmaxf(0.f, de_nan(Q.y) / cf - m1 * m1),
-                v2 = fmaxf(0.f, de_nan(Q.z) / cf - m2 * m2);
-    V = (0.2126f * v0 + 0.7152f * v1 + 0.0722f * v2) / (float)(c - 1);
-  }
-  x[idx] = make_float4(m0, m1, m2, V);
-  const float4 A = ga[idx], ND = gnz[idx];
-  ga[idx] = make_float4(A.x / cf, A.y / cf, A.z / cf, A.w / cf);
-  gnz[idx] = make_float4(ND.x / cf, ND.y / cf, ND.z / cf, A.w > 0.f ? ND.w / A.w : 0.f);
+  denoise_prep_pixel(x, moment, x, ga, gnz, idx, c, a.hasMoments);
+}
+
+// The same per pixel of a chunk of whole views with c = counts[idx] >= 2 (b2pt_render_views_adaptive_denoised): S and
+// Q are read from the sweep's own sums, (m, V0) written to x, the guides converted in place.
+__global__ void __launch_bounds__(256)
+  k_denoise_prep_counts(const float4* __restrict__ color, const float4* __restrict__ moment,
+                        const int32_t* __restrict__ counts, float4* __restrict__ x, float4* __restrict__ ga,
+                        float4* __restrict__ gnz, long long n)
+{
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n)
+    return;
+  denoise_prep_pixel(color, moment, x, ga, gnz, idx, counts[idx], 1);
 }
 
 // One a-trous level (step s) of SVGF's edge-avoiding wavelet filter: one thread per pixel, 16 x 16 pixel tiles in
@@ -2543,6 +2595,25 @@ cudaError_t launch_view_features(const B2SmallScene* small, const B2BvhScene* bv
   return cudaGetLastError();
 }
 
+cudaError_t launch_view_features_counts(const B2SmallScene* small, const B2BvhScene* bvh, const B2Camera* cams,
+                                        int nViews, int nPixels, uint32_t seedOffset, const int32_t* counts,
+                                        float4* albedo, float4* normalDepth, cudaStream_t stream)
+{
+  const int64_t n = (int64_t)nViews * nPixels;
+  if (n <= 0)
+    return cudaSuccess;
+  if (n > 0xffffffffLL)
+    return cudaErrorInvalidValue;
+  uint32_t magic, shift;
+  make_fastdiv((uint32_t)nPixels, magic, shift);
+  const unsigned grid = (unsigned)((n + 255) / 256);
+  with_trace_scene(small, bvh, [&](const auto& S) {
+    k_view_features_counts<std::decay_t<decltype(S)>><<<grid, 256, 0, stream>>>(
+      S, cams, n, (uint32_t)nPixels, magic, shift, seedOffset, counts, albedo, normalDepth);
+  });
+  return cudaGetLastError();
+}
+
 cudaError_t launch_create_rays(const B2Camera& cam, uint32_t* seeds, float* dx, float* dy, float* dz, float* ox,
                                float* oy, float* oz, long long* pixelIdx, cudaStream_t stream)
 {
@@ -2589,6 +2660,15 @@ cudaError_t launch_denoise_prep(float4* x, const float4* moment, float4* ga, flo
   if (n <= 0)
     return cudaSuccess;
   k_denoise_prep<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(x, moment, ga, gnz, n, sliceLen, a);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_denoise_prep_counts(const float4* color, const float4* moment, const int32_t* counts, float4* x,
+                                       float4* ga, float4* gnz, int64_t n, cudaStream_t stream)
+{
+  if (n <= 0)
+    return cudaSuccess;
+  k_denoise_prep_counts<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(color, moment, counts, x, ga, gnz, n);
   return cudaGetLastError();
 }
 

@@ -169,6 +169,16 @@ cudaError_t launch_list_pad(uint32_t* list, int n, int nPad, cudaStream_t stream
 cudaError_t launch_normalize_counts(float4* color, int64_t n, const int32_t* counts, cudaStream_t stream);
 cudaError_t launch_pnm16_counts(const float4* color, int64_t n, const int32_t* counts, uint16_t* rgb,
                                 cudaStream_t stream);
+// Denoising an adaptive sweep (b2pt_render_views_adaptive_denoised), over one chunk of whole views with each
+// (view, pixel) entry's own sample count counts[idx] (the chunk's slice of the adaptive counts).
+// launch_view_features_counts: launch_view_features' sums over samples s < counts[idx], stored once per entry (both
+// outputs required).  launch_denoise_prep_counts: launch_denoise_prep's arithmetic with c = counts[idx] >= 2 and the
+// sums of squares always used; color and moment are read only, (m, V0) goes to x, ga and gnz are converted in place.
+cudaError_t launch_view_features_counts(const B2SmallScene* small, const B2BvhScene* bvh, const B2Camera* cams,
+                                        int nViews, int nPixels, uint32_t seedOffset, const int32_t* counts,
+                                        float4* albedo, float4* normalDepth, cudaStream_t stream);
+cudaError_t launch_denoise_prep_counts(const float4* color, const float4* moment, const int32_t* counts, float4* x,
+                                       float4* ga, float4* gnz, int64_t n, cudaStream_t stream);
 cudaError_t launch_create_rays(const B2Camera& cam, uint32_t* seeds, float* dx, float* dy, float* dz, float* ox,
                                float* oy, float* oz, long long* pixelIdx, cudaStream_t stream);
 cudaError_t launch_intersect(const B2SmallScene* small, const B2BvhScene* bvh, int64_t n, const float* ox,

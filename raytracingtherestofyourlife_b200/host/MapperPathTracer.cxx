@@ -534,6 +534,37 @@ void MapperPathTracer::RenderCellsViewsAdaptivePnm(const vtkm::cont::DynamicCell
   LastSegments = st.segments;
 }
 
+void MapperPathTracer::RenderCellsViewsAdaptiveDenoisedPnm(const vtkm::cont::DynamicCellSet& cellset,
+                                                           const vtkm::cont::CoordinateSystem& coords,
+                                                           const std::vector<vtkm::rendering::Camera>& cameras,
+                                                           const std::vector<int>& rounds, float threshold,
+                                                           std::vector<unsigned short>& pnm, std::vector<int>& counts,
+                                                           std::vector<unsigned short>& denoisedPnm)
+{
+  if (Internals->Canvas == nullptr)
+    throw vtkm::cont::ErrorBadValue("MapperPathTracer: no canvas set");
+  CheckCheckpoints(rounds, samplecount);
+  const std::vector<float> views = PrepareSweep(cellset, coords, cameras);
+  const vtkm::Id nx = Internals->Canvas->GetWidth(), ny = Internals->Canvas->GetHeight();
+  const size_t n = cameras.size() * static_cast<size_t>(nx * ny);
+  pnm.assign(n * 3, 0);
+  counts.assign(n, 0);
+  denoisedPnm.assign(n * 3, 0);
+  b2pt_ctx* ctx = b2pt_facade::Context();
+  b2pt_facade::Check(b2pt_seed(ctx, 0)); // the streams RenderCellsViews* render with
+  b2pt_adaptive_params params;
+  b2pt_adaptive_defaults(&params);
+  params.threshold = threshold;
+  b2pt_facade::Check(b2pt_render_views_adaptive_denoised(
+    ctx, static_cast<int>(cameras.size()), views.data(), static_cast<int>(nx), static_cast<int>(ny),
+    static_cast<int>(rounds.size()), rounds.data(), depthcount, &params, nullptr, RenderFlags | B2PT_FLAG_VIEWS_PNM16,
+    pnm.data(), counts.data(), nullptr, nullptr, denoisedPnm.data()));
+  b2pt_stats st;
+  b2pt_facade::Check(b2pt_get_stats(ctx, &st));
+  LastRenderMs = st.renderMs;
+  LastSegments = st.segments;
+}
+
 void MapperPathTracer::SetCompositeBackground(bool on) { Internals->CompositeBackground = on; }
 
 void MapperPathTracer::StartScene()

@@ -137,6 +137,15 @@ public:
   void RenderCellsViewsAdaptivePnm(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
                                    const std::vector<vtkm::rendering::Camera>& cameras, const std::vector<int>& rounds,
                                    float threshold, std::vector<unsigned short>& pnm, std::vector<int>& counts);
+  // RenderCellsViewsAdaptivePnm's integers and counts (same rounds rule, same bytes) and, in denoisedPnm, the same
+  // layout for the adaptive sweep denoised on the GPU at every pixel's own count with b2pt_denoise_views' defaults
+  // (b2pt_render_views_adaptive_denoised).
+  void RenderCellsViewsAdaptiveDenoisedPnm(const vtkm::cont::DynamicCellSet& cellset,
+                                           const vtkm::cont::CoordinateSystem& coords,
+                                           const std::vector<vtkm::rendering::Camera>& cameras,
+                                           const std::vector<int>& rounds, float threshold,
+                                           std::vector<unsigned short>& pnm, std::vector<int>& counts,
+                                           std::vector<unsigned short>& denoisedPnm);
   // The -direct G-buffers of main.cc:402-422 (what MapperQuadNormals / MapperQuadAlbedo leave in the canvas colour
   // buffer, raytracing/RayTracerNormals.cxx / RayTracerAlbedo.cxx, and a depth image) for the canvas set with
   // SetCanvas: one un-jittered ray per pixel, closest quad hit, the reference's two Shade rules (b2pt_render_direct).

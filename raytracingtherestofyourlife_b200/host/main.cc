@@ -39,6 +39,10 @@
 // <out>-adaptive-<phi>-<theta>.pnm (save()'s arithmetic with each pixel's own sample count) and
 // <out>-spp-<phi>-<theta>.pfm (Pf, the sample count of every pixel).  -adaptive without -checkpoints, with -direct,
 // -features or -denoise, or with a tau that is not a number >= 0 is an error (exit 1).
+// -adaptive-denoise <tau> is -adaptive <tau> with the adaptive sweep also denoised on the GPU at every pixel's own
+// sample count (b2pt_render_views_adaptive_denoised, default filter parameters): the files of -adaptive <tau>,
+// byte-identical, and <out>-adaptive-denoised-<phi>-<theta>.pnm.  The same uses as -adaptive are errors, and so is
+// -adaptive-denoise with -adaptive.
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
@@ -76,7 +80,9 @@ struct Options
   bool denoise = false;
   bool adaptiveGiven = false;
   std::string adaptiveArg;
-  float adaptive = 0.f; // -adaptive, parsed and checked by checkAdaptive
+  bool adaptiveDenoiseGiven = false;
+  std::string adaptiveDenoiseArg;
+  float adaptive = 0.f; // -adaptive or -adaptive-denoise, parsed and checked by checkAdaptive
 };
 
 Options parse(int argc, char** argv)
@@ -123,6 +129,12 @@ Options parse(int argc, char** argv)
       o.adaptiveGiven = true;
       if (i + 1 < argc)
         o.adaptiveArg = argv[++i];
+    }
+    else if (!std::strcmp(argv[i], "-adaptive-denoise"))
+    {
+      o.adaptiveDenoiseGiven = true;
+      if (i + 1 < argc)
+        o.adaptiveDenoiseArg = argv[++i];
     }
     else if (!std::strcmp(argv[i], "-checkpoints"))
     {
@@ -185,24 +197,35 @@ std::string checkDenoise(const Options& o)
   return "";
 }
 
-// Parses -adaptive into o.adaptive; returns an error message, empty when it is usable or absent.
+// Parses the threshold arg of the adaptive switch `flag` into o.adaptive; returns an error message, empty when the
+// switch is usable.
+std::string checkAdaptiveSwitch(Options& o, const std::string& flag, const std::string& arg)
+{
+  if (o.direct)
+    return flag + " cannot be combined with -direct";
+  if (o.features || o.denoise)
+    return flag + " cannot be combined with -features or -denoise";
+  if (!o.hemi && !o.fibonacci)
+    return flag + " needs -hemisphere or -fibonacci";
+  if (!o.checkpointsGiven)
+    return flag + " needs -checkpoints (the rounds before samplecount)";
+  char* end = nullptr;
+  const float tau = std::strtof(arg.c_str(), &end);
+  if (arg.empty() || *end != '\0' || !(tau >= 0.f))
+    return flag + " takes a threshold >= 0, got '" + arg + "'";
+  o.adaptive = tau;
+  return "";
+}
+
+// Parses -adaptive or -adaptive-denoise; returns an error message, empty when it is usable or absent.
 std::string checkAdaptive(Options& o)
 {
-  if (!o.adaptiveGiven)
-    return "";
-  if (o.direct)
-    return "-adaptive cannot be combined with -direct";
-  if (o.features || o.denoise)
-    return "-adaptive cannot be combined with -features or -denoise";
-  if (!o.hemi && !o.fibonacci)
-    return "-adaptive needs -hemisphere or -fibonacci";
-  if (!o.checkpointsGiven)
-    return "-adaptive needs -checkpoints (the rounds before samplecount)";
-  char* end = nullptr;
-  const float tau = std::strtof(o.adaptiveArg.c_str(), &end);
-  if (o.adaptiveArg.empty() || *end != '\0' || !(tau >= 0.f))
-    return "-adaptive takes a threshold >= 0, got '" + o.adaptiveArg + "'";
-  o.adaptive = tau;
+  if (o.adaptiveGiven && o.adaptiveDenoiseGiven)
+    return "-adaptive-denoise cannot be combined with -adaptive";
+  if (o.adaptiveGiven)
+    return checkAdaptiveSwitch(o, "-adaptive", o.adaptiveArg);
+  if (o.adaptiveDenoiseGiven)
+    return checkAdaptiveSwitch(o, "-adaptive-denoise", o.adaptiveDenoiseArg);
   return "";
 }
 
@@ -388,15 +411,22 @@ int renderViews(CornellBox& cb, const Options& o, const std::vector<vtkm::render
   std::vector<unsigned short> pnm, denoised;
   std::vector<int> counts = o.checkpoints; // -checkpoints: one render, its images at every count up to samplecount
   counts.push_back(o.samples);
-  if (o.adaptiveGiven)
-  { // the rounds are the counts; one image and one sample-count map per view
+  if (o.adaptiveGiven || o.adaptiveDenoiseGiven)
+  { // the rounds are the counts; one image and one sample-count map per view (and one denoised image)
     std::vector<int> spp;
-    mapper.RenderCellsViewsAdaptivePnm(cb.ds.GetCellSet(), cb.coord, cameras, counts, o.adaptive, pnm, spp);
+    if (o.adaptiveDenoiseGiven)
+      mapper.RenderCellsViewsAdaptiveDenoisedPnm(cb.ds.GetCellSet(), cb.coord, cameras, counts, o.adaptive, pnm, spp,
+                                                 denoised);
+    else
+      mapper.RenderCellsViewsAdaptivePnm(cb.ds.GetCellSet(), cb.coord, cameras, counts, o.adaptive, pnm, spp);
     const size_t n = static_cast<size_t>(o.x) * o.y;
     std::vector<float> map(n);
     for (size_t v = 0; v < cameras.size(); ++v)
     {
       savePnm16(viewName(o.out + "-adaptive", angles[v].first, angles[v].second), o.x, o.y, &pnm[v * n * 3]);
+      if (o.adaptiveDenoiseGiven)
+        savePnm16(viewName(o.out + "-adaptive-denoised", angles[v].first, angles[v].second), o.x, o.y,
+                  &denoised[v * n * 3]);
       for (size_t i = 0; i < n; ++i)
         map[i] = static_cast<float>(spp[v * n + i]);
       savePfm(viewName(o.out + "-spp", angles[v].first, angles[v].second), o.x, o.y, 1, map);
