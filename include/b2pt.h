@@ -137,6 +137,33 @@ int b2pt_set_camera(b2pt_ctx* ctx, const float pos[3], const float lookAt[3], co
 int b2pt_set_memory_budget(b2pt_ctx* ctx, int64_t bytes);
 /* seeds[i] = i + seedOffset (0 = the reference, MapperPathTracer.cxx:265-267). */
 int b2pt_seed(b2pt_ctx* ctx, uint32_t seedOffset);
+/* Thin-lens depth of field (DESIGN.md 8h; the book's camera with an aperture and a focus distance, which the reference's
+ * camera dropped).  aperture = lens diameter in scene units, finite and >= 0; 0 (the default) is the pinhole: the
+ * current behaviour bit for bit, with no extra RNG draws.  focusDistance, finite: > 0 is the distance from the camera
+ * position to the plane of focus along the view direction; <= 0 (the default) focuses every camera at its own
+ * |lookAt - pos| (a hemisphere sweep that looks at the box centre keeps the box in focus in every view).  NaN, +-inf or
+ * a negative aperture gives B2PT_ERR_BAD_VALUE and leaves the state unchanged; the state persists until the next call
+ * ((0, 0) restores the pinhole).  With aperture > 0, the primary ray of pixel p, sample s (rng = p + seedOffset +
+ * s*0x9E3779B9) of a camera with basis nlook, dx, dy, pos is, in float32 with no FMA and in this order:
+ *   1. d0 = the pinhole ray (two jitter draws, unchanged);
+ *   2. for k = 0..15: a = 2 randf - 1, b = 2 randf - 1, stop at the first pair with a*a + b*b < 1; after 16 rejections
+ *      a = b = 0 (the book's random_in_unit_disk, bounded);
+ *   3. per camera: u = dx/|dx|, v = dy/|dy| (|x| = sqrtf((x0*x0 + x1*x1) + x2*x2)), r = aperture/2, f = focusDistance
+ *      or |lookAt - pos|;
+ *   4. o = (pos + u*(r*a)) + v*(r*b);
+ *   5. F = pos + d0*(f / ((d0.x*nlook.x + d0.y*nlook.y) + d0.z*nlook.z)), where the pinhole ray meets the plane of focus;
+ *   6. d = F - o, zero components nudged by 1e-7 and normalised by division as the pinhole raygen does;
+ *   7. the path continues from (o, d) with the stream after the lens draws.
+ * The lens applies to b2pt_render, b2pt_render_range, b2pt_render_views and its _checkpoints, _features, _adaptive and
+ * _adaptive_denoised forms, and b2pt_primary_hits (sample 0's lens ray; t, like the features' depth, is measured from
+ * o).  View v of a sweep stays bit-identical to b2pt_set_camera(view v) + b2pt_render under the same lens.  It does not
+ * apply to the reference's stage hooks b2pt_create_rays and b2pt_intersect, to the -direct G-buffers
+ * (b2pt_render_direct, b2pt_render_direct_views: un-jittered corner rays as in the reference), or to
+ * b2pt_denoise_views (a pure function of its inputs).  Every render flag works under a lens except
+ * B2PT_FLAG_REFERENCE_STREAM, which the reference's lens-less camera defines: b2pt_render and b2pt_render_range with it
+ * and aperture > 0 fail with B2PT_ERR_BAD_VALUE before anything runs.  Small scenes trace lens rays without the per-tile
+ * primary masks (as under B2PT_FLAG_NO_PRIMARY_MASKS), which assume one ray origin per view. */
+int b2pt_set_lens(b2pt_ctx* ctx, float aperture, float focusDistance);
 
 /* ---- render -------------------------------------------------------------------------------- */
 /* Replaces MapperPathTracer::RenderCellsImpl's sample x depth loop (MapperPathTracer.cxx:278-350):
@@ -176,7 +203,8 @@ int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views,
 /* Denoiser guide buffers of a view sweep: per pixel, the first-hit albedo, normal and depth of the SAME path samples
  * b2pt_render_views_checkpoints averages, summed over the first checkpoints[k] samples.  For view v, pixel
  * p = j*W+i (j = 0 bottom row) and sample s, the primary ray is the renderer's: rng = p + seedOffset + s*0x9E3779B9
- * (b2pt_seed), the jittered raygen of the path tracer, origin at the camera, closest hit in (0.001, FLT_MAX) through
+ * (b2pt_seed), the jittered raygen of the path tracer, origin at the camera (under b2pt_set_lens: the lens ray, depth
+ * measured from its origin on the lens), closest hit in (0.001, FLT_MAX) through
  * the trace structure a render with `flags` uses (quads and spheres).  Per sample, on a hit:
  *   albedo = lambertian (matType 0): the primitive's texture colour; dielectric (2): (1,1,1), the attenuation of the
  *            specular bounce; emitter (1): its colour clamped per channel to [0,1];
@@ -326,7 +354,8 @@ int b2pt_get_stage_profile(b2pt_ctx* ctx, int maxEntries, float* traceMs, float*
 /* ---- parity hooks and stage-level entry points --------------------------------------------- */
 /* Sample-0 primary rays with seeds[i] = i + seedOffset through the production raygen + trace device
  * code: hit primitive id per pixel (quad q -> q, sphere s -> nQuads+s, miss -> -1) and hit t.
- * Either output may be NULL. */
+ * Either output may be NULL.  Under b2pt_set_lens the rays are sample 0's lens rays and t is measured from their
+ * origin on the lens. */
 int b2pt_primary_hits(b2pt_ctx* ctx, int32_t* primId, float* t);
 /* Replaces the -direct G-buffer passes of main.cc:402-422 (runNorms / runAlbedo through MapperQuadNormals / MapperQuadAlbedo,
  * raytracing/RayTracerNormals.cxx:47-143 and :234-281, RayTracerAlbedo.cxx:100-143, MapperQuad.cxx:86-150) and the

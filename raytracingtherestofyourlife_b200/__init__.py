@@ -91,6 +91,7 @@ SIGNATURES = {
     "b2pt_refit_bvh": (_i32, [_vp]),
     "b2pt_set_camera": (_i32, [_vp, _vp, _vp, _vp, _f, _i32, _i32]),
     "b2pt_seed": (_i32, [_vp, C.c_uint32]),
+    "b2pt_set_lens": (_i32, [_vp, _f, _f]),
     "b2pt_set_memory_budget": (_i32, [_vp, _i64]),
     "b2pt_render": (_i32, [_vp, _i32, _i32, C.c_uint32]),
     "b2pt_render_range": (_i32, [_vp, _i32, _i32, _i32, C.c_uint32]),
@@ -297,6 +298,12 @@ class Context:
 
     def seed(self, offset):
         _check(lib().b2pt_seed(self._h, offset))
+
+    def set_lens(self, aperture, focus_distance=0.0):
+        """Thin-lens depth of field for every later path-traced render, sweep and primary_hits (b2pt_set_lens):
+        aperture = lens diameter (0 = pinhole); focus_distance > 0 = distance to the plane of focus along the view
+        direction, <= 0 = each camera focuses at its look-at point."""
+        _check(lib().b2pt_set_lens(self._h, aperture, focus_distance))
 
     def render(self, spp, max_depth, flags=0):
         _check(lib().b2pt_render(self._h, spp, max_depth, flags))

@@ -161,6 +161,10 @@ struct b2pt_ctx
   B2Camera cam{};
   float camLookAt[3] = { 0.f, 0.f, 0.f }, camUpN[3] = { 0.f, 1.f, 0.f }; // look-at point, up as Camera::SetUp stores it
   uint32_t seedOffset = 0;
+  // thin lens (b2pt_set_lens): aperture 0 is the pinhole.  dLens: one record per camera of the sweep in dViews;
+  // dLensCam: the record of the single camera a render_impl call without views traces
+  float lensAperture = 0.f, lensFocus = 0.f;
+  DevBuf<B2Lens> dLens, dLensCam;
 
   // buffers
   DevBuf<float4> colorOwn;
@@ -1367,6 +1371,60 @@ static int make_view_cameras(int nViews, const float* views, int W, int H, std::
   return B2PT_OK;
 }
 
+// The thin-lens record of camera c (DESIGN.md 8h), in float32 in the order include/b2pt.h fixes: u = dx/|dx|,
+// v = dy/|dy|, r = aperture/2, f = the context's focus distance if it is > 0, else |lookAt - pos|.
+static B2Lens make_lens(const b2pt_ctx* ctx, const B2Camera& c, const float lookAt[3])
+{
+  B2Lens L{};
+  const H3 dx = { c.dx[0], c.dx[1], c.dx[2] }, dy = { c.dy[0], c.dy[1], c.dy[2] };
+  const float lu = std::sqrt(hdot(dx, dx)), lv = std::sqrt(hdot(dy, dy));
+  hst(L.u, { dx.x / lu, dx.y / lu, dx.z / lu });
+  hst(L.v, { dy.x / lv, dy.y / lv, dy.z / lv });
+  L.r = ctx->lensAperture / 2.f;
+  if (ctx->lensFocus > 0.f)
+    L.f = ctx->lensFocus;
+  else
+  {
+    const H3 e = hsub({ lookAt[0], lookAt[1], lookAt[2] }, { c.pos[0], c.pos[1], c.pos[2] });
+    L.f = std::sqrt(hdot(e, e));
+  }
+  return L;
+}
+
+// The lens records of the cameras of a view list (make_view_cameras); empty for the pinhole.
+static std::vector<B2Lens> make_view_lenses(const b2pt_ctx* ctx, const float* views, const std::vector<B2Camera>& cams)
+{
+  std::vector<B2Lens> lenses;
+  if (ctx->lensAperture > 0.f)
+    for (size_t v = 0; v < cams.size(); ++v)
+      lenses.push_back(make_lens(ctx, cams[v], views + 10 * v + 3));
+  return lenses;
+}
+
+// ctx->dLens = lenses (nothing for the pinhole)
+static int upload_lenses(b2pt_ctx* ctx, const std::vector<B2Lens>& lenses)
+{
+  if (lenses.empty())
+    return B2PT_OK;
+  CU(ctx->dLens.reserve(lenses.size()));
+  CU(cudaMemcpyAsync(ctx->dLens.p, lenses.data(), sizeof(B2Lens) * lenses.size(), cudaMemcpyHostToDevice,
+                     ctx->stream));
+  return B2PT_OK;
+}
+
+int b2pt_set_lens(b2pt_ctx* ctx, float aperture, float focusDistance)
+{
+  if (int rc = bind(ctx))
+    return rc;
+  if (!std::isfinite(aperture) || aperture < 0.f)
+    return fail(B2PT_ERR_BAD_VALUE, "b2pt_set_lens: aperture must be finite and >= 0, got %g", (double)aperture);
+  if (!std::isfinite(focusDistance))
+    return fail(B2PT_ERR_BAD_VALUE, "b2pt_set_lens: focusDistance must be finite, got %g", (double)focusDistance);
+  ctx->lensAperture = aperture;
+  ctx->lensFocus = focusDistance;
+  return B2PT_OK;
+}
+
 int b2pt_set_camera(b2pt_ctx* ctx, const float pos[3], const float lookAt[3], const float up[3], float fovDeg, int W,
                     int H)
 {
@@ -1549,9 +1607,13 @@ struct ListedRound
 // batches accumulate through k_accumulate_checkpoints into these snapshot slices as well; entry0 is the first canvas
 // entry of the render (its view's slice offset when nViews == 0).  list (nViews == 0): the same sample range for the
 // listed entries only, batched as the samples of one view of nPad pixels and accumulated in batch order through
-// k_accumulate_list; the per-tile primary masks are off (a tile is no longer 32 neighbouring pixels).
+// k_accumulate_list; the per-tile primary masks are off (a tile is no longer 32 neighbouring pixels).  Under a lens
+// (b2pt_set_lens) the primary rays run through k_trace_lens, without the masks: with views or a list the caller has put
+// one lens record per camera of ctx->dViews into ctx->dLens; otherwise camLens is the record of ctx->cam (nullptr: made
+// from ctx->cam and ctx->camLookAt).
 static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxDepth, uint32_t flags, int64_t nViews,
-                       const b2pt::CheckpointArgs* ckpt = nullptr, const ListedRound* list = nullptr)
+                       const b2pt::CheckpointArgs* ckpt = nullptr, const ListedRound* list = nullptr,
+                       const B2Lens* camLens = nullptr)
 {
   if (int rc = bind(ctx))
     return rc;
@@ -1568,6 +1630,9 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
     return fail(B2PT_ERR_BAD_VALUE, "KILL_ZERO_THROUGHPUT cannot be combined with REFERENCE_STREAM");
   if (refStream && sampleBegin != 0)
     return fail(B2PT_ERR_BAD_VALUE, "REFERENCE_STREAM renders samples from 0 (one persistent stream per pixel)");
+  const bool lens = ctx->lensAperture > 0.f;
+  if (refStream && lens)
+    return fail(B2PT_ERR_BAD_VALUE, "REFERENCE_STREAM cannot be combined with a lens (the reference has none)");
   if (int rc = ensure_built_for(ctx, flags))
     return rc;
   const bool viewMode = nViews > 0;
@@ -1723,7 +1788,7 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
   // Primary-ray specialisation (small scenes whose tiles of 32 path ids are tiles of 32 pixels of one view): candidate
   // masks per tile and quad constants per view, recomputed per render (a few microseconds).
   const bool primMasks =
-    !ctx->useBvh && !list && (N % 32) == 0 && nBatches > 0 && !(flags & B2PT_FLAG_NO_PRIMARY_MASKS);
+    !ctx->useBvh && !list && !lens && (N % 32) == 0 && nBatches > 0 && !(flags & B2PT_FLAG_NO_PRIMARY_MASKS);
   const int tilesPerView = (int)(N / 32);
   if (primMasks)
   {
@@ -1733,6 +1798,16 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
     CU(b2pt::launch_primary_prep(ctx->small, ctx->cam, viewMode ? ctx->dViews.p : nullptr, nv, tilesPerView,
                                  ctx->primMask.p, ctx->primQuads.p, ctx->stream));
     ++launches0;
+  }
+  const B2Lens* dLens = nullptr;
+  if (lens && (viewMode || list))
+    dLens = ctx->dLens.p;
+  else if (lens)
+  { // (pageable source: staged before the call returns)
+    const B2Lens rec = camLens ? *camLens : make_lens(ctx, ctx->cam, ctx->camLookAt);
+    CU(ctx->dLensCam.reserve(1));
+    CU(cudaMemcpyAsync(ctx->dLensCam.p, &rec, sizeof(B2Lens), cudaMemcpyHostToDevice, ctx->stream));
+    dLens = ctx->dLensCam.p;
   }
 
   // An error return while batches are in flight on the extra streams must not leave them running behind the caller's
@@ -1782,6 +1857,7 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
     const int set = (int)(batch % nSets);
     b2pt_ctx::BatchBufs& bb = ctx->bufs[set];
     cudaStream_t bs = set ? ctx->extra[set] : ctx->stream;
+    const B2Lens* const batchLens = dLens ? dLens + (viewMode ? v0 : 0) : nullptr;
     B2RenderArgs A{};
     A.depthTotals = ctx->counters.p + batch * maxDepth;
     A.binTotals = ctx->binTotals.p + batch * maxDepth * 4;
@@ -1837,7 +1913,7 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
       if (fused)
       {
         if (depth == 0)
-          CU(b2pt::launch_primary(ctx->cfg, ctx->cam, ctx->small, A, bs));
+          CU(b2pt::launch_primary(ctx->cfg, ctx->cam, ctx->small, A, bs, batchLens));
         else if (depth >= loopDepth)
         { // every remaining bounce and the closing pass in one cluster launch
           CU(b2pt::launch_bounce_tail_loop(ctx->small, ctx->lights, A, bs));
@@ -1869,7 +1945,8 @@ static int render_impl(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxD
         launches += splitTrace ? 4 : 3;
       }
       CU(b2pt::launch_bounce(ctx->cfg, depth == 0, mode, ctx->cam, ctx->useBvh ? nullptr : &ctx->small,
-                             ctx->useBvh ? &ctx->bvh : nullptr, ctx->lights, A, bs, mid));
+                             ctx->useBvh ? &ctx->bvh : nullptr, ctx->lights, A, bs, mid,
+                             depth == 0 ? batchLens : nullptr));
       launches += 2;
     }
     // the canvas is accumulated in batch order (sample-order sums): wait for the previous batch's accumulate
@@ -2022,9 +2099,10 @@ int b2pt_render_range(b2pt_ctx* ctx, int sampleBegin, int sampleCount, int maxDe
 // (b2pt_render_views, K == 1, no moments): the batches accumulate through k_accumulate.  Otherwise ck holds the
 // checkpoint list (n, count) and they accumulate through k_accumulate_checkpoints, which keeps the running sums at
 // every count and, when moment2Out is not NULL or keepMoments is set, the sums of squares (in ctx->ckptMoment).
-static int render_view_sweep(b2pt_ctx* ctx, const std::vector<B2Camera>& cams, const int* counts, int K, int maxDepth,
-                             uint32_t flags, b2pt::CheckpointArgs* ck, void* rgbaOut, float* moment2Out,
-                             bool keepMoments = false)
+// lenses: the lens record of every camera (make_view_lenses; empty for the pinhole).
+static int render_view_sweep(b2pt_ctx* ctx, const std::vector<B2Camera>& cams, const std::vector<B2Lens>& lenses,
+                             const int* counts, int K, int maxDepth, uint32_t flags, b2pt::CheckpointArgs* ck,
+                             void* rgbaOut, float* moment2Out, bool keepMoments = false)
 {
   const int64_t nViews = (int64_t)cams.size();
   if (nViews == 0)
@@ -2081,6 +2159,12 @@ static int render_view_sweep(b2pt_ctx* ctx, const std::vector<B2Camera>& cams, c
       restore();
       return fail(B2PT_ERR_CUDA, "cudaMemcpyAsync(views): %s", cudaGetErrorString(e));
     }
+    rc = upload_lenses(ctx, lenses);
+    if (rc != B2PT_OK)
+    {
+      restore();
+      return rc;
+    }
     rc = render_impl(ctx, 0, spp, maxDepth, flags, nViews, ck);
     perView = rc == B2PT_ERR_ALLOC; // the buffers of a whole-view batch could not be allocated: views one by one
   }
@@ -2097,7 +2181,7 @@ static int render_view_sweep(b2pt_ctx* ctx, const std::vector<B2Camera>& cams, c
       ctx->colorExt = ctx->viewColor.p + (size_t)v * N;
       if (ck)
         ck->entry0 = v * N;
-      rc = render_impl(ctx, 0, spp, maxDepth, flags, 0, ck);
+      rc = render_impl(ctx, 0, spp, maxDepth, flags, 0, ck, nullptr, lenses.empty() ? nullptr : &lenses[(size_t)v]);
       paths += ctx->stats.paths;
       launches += ctx->stats.launches;
     }
@@ -2153,7 +2237,8 @@ int b2pt_render_views(b2pt_ctx* ctx, int nViews, const float* views, int W, int 
     return rc;
   if ((int64_t)W * H * nViews > (int64_t)1 << 30)
     return fail(B2PT_ERR_BAD_VALUE, "b2pt_render_views: more than 2^30 output pixels (16 GiB); split the view list");
-  return render_view_sweep(ctx, cams, &spp, 1, maxDepth, flags, nullptr, rgbaOut, nullptr);
+  return render_view_sweep(ctx, cams, make_view_lenses(ctx, views, cams), &spp, 1, maxDepth, flags, nullptr, rgbaOut,
+                           nullptr);
 }
 
 // b2pt_render_views at spp = checkpoints[K-1] through k_accumulate_checkpoints: sample s of a pixel is the same RNG
@@ -2182,7 +2267,8 @@ int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views,
   b2pt::CheckpointArgs ck{};
   ck.n = K;
   std::copy(checkpoints, checkpoints + K, ck.count);
-  return render_view_sweep(ctx, cams, ck.count, K, maxDepth, flags, &ck, rgbaOut, moment2Out);
+  return render_view_sweep(ctx, cams, make_view_lenses(ctx, views, cams), ck.count, K, maxDepth, flags, &ck, rgbaOut,
+                           moment2Out);
 }
 
 void b2pt_adaptive_defaults(b2pt_adaptive_params* p)
@@ -2276,7 +2362,8 @@ static int render_adaptive(b2pt_ctx* ctx, const char* fn, int nViews, const floa
   b2pt::CheckpointArgs ck{};
   ck.n = 1;
   ck.count[0] = rounds[0];
-  if (int rc = render_view_sweep(ctx, cams, rounds, 1, maxDepth, renderFlags, &ck, nullptr, nullptr, true))
+  const std::vector<B2Lens> lenses = make_view_lenses(ctx, views, cams);
+  if (int rc = render_view_sweep(ctx, cams, lenses, rounds, 1, maxDepth, renderFlags, &ck, nullptr, nullptr, true))
     return rc;
   int64_t paths = ctx->stats.paths, launches = ctx->stats.launches;
   std::vector<int64_t> active((size_t)K, 0);
@@ -2292,6 +2379,8 @@ static int render_adaptive(b2pt_ctx* ctx, const char* fn, int nViews, const floa
   // (the whole-view path of round 0 uploads the cameras too, its per-view fallback does not)
   CU(cudaMemcpyAsync(ctx->dViews.p, cams.data(), sizeof(B2Camera) * (size_t)nViews, cudaMemcpyHostToDevice,
                      ctx->stream));
+  if (int rc = upload_lenses(ctx, lenses))
+    return rc;
   b2pt::AdaptiveArgs a{};
   a.tau = P.threshold;
   a.eps = P.epsilon;
@@ -2446,6 +2535,9 @@ int b2pt_render_views_features(b2pt_ctx* ctx, int nViews, const float* views, in
   CU(ctx->dViews.reserve((size_t)nViews));
   CU(cudaMemcpyAsync(ctx->dViews.p, cams.data(), sizeof(B2Camera) * (size_t)nViews, cudaMemcpyHostToDevice,
                      ctx->stream));
+  const std::vector<B2Lens> lenses = make_view_lenses(ctx, views, cams);
+  if (int rc = upload_lenses(ctx, lenses))
+    return rc;
   if (albedoOut)
     CU(ctx->featAlbedo.reserve(cap));
   if (normalDepthOut)
@@ -2457,7 +2549,8 @@ int b2pt_render_views_features(b2pt_ctx* ctx, int nViews, const float* views, in
     CU(b2pt::launch_view_features(ctx->useBvh ? nullptr : &ctx->small, ctx->useBvh ? &ctx->bvh : nullptr,
                                   ctx->dViews.p + v0, nv, (int)N, ctx->seedOffset, ck,
                                   albedoOut ? ctx->featAlbedo.p : nullptr,
-                                  normalDepthOut ? ctx->featNormalDepth.p : nullptr, ctx->stream));
+                                  normalDepthOut ? ctx->featNormalDepth.p : nullptr, ctx->stream,
+                                  lenses.empty() ? nullptr : ctx->dLens.p + v0));
     for (int k = 0; k < K; ++k)
     {
       const size_t dst = 4 * (size_t)((k * (int64_t)nViews + v0) * N);
@@ -2601,7 +2694,8 @@ static int denoise_adaptive_sweep(b2pt_ctx* ctx, int64_t nViews, int W, int H, i
     const int64_t n = nv * N, off = v0 * N;
     CU(b2pt::launch_view_features_counts(ctx->useBvh ? nullptr : &ctx->small, ctx->useBvh ? &ctx->bvh : nullptr,
                                          ctx->dViews.p + v0, nv, (int)N, ctx->seedOffset, ctx->adCounts.p + off,
-                                         ctx->dnGuideA.p, ctx->dnGuideNZ.p, ctx->stream));
+                                         ctx->dnGuideA.p, ctx->dnGuideNZ.p, ctx->stream,
+                                         ctx->lensAperture > 0.f ? ctx->dLens.p + v0 : nullptr));
     if (dn.albedoOut)
       CU(cudaMemcpyAsync(dn.albedoOut + 4 * off, ctx->dnGuideA.p, sizeof(float4) * (size_t)n, cudaMemcpyDeviceToHost,
                          ctx->stream));
@@ -2907,9 +3001,10 @@ int b2pt_primary_hits(b2pt_ctx* ctx, int32_t* primId, float* t)
   DevBuf<float> dT;
   CU(dPrim.reserve(N));
   CU(dT.reserve(N));
+  const B2Lens lens = make_lens(ctx, ctx->cam, ctx->camLookAt);
   cudaError_t e = b2pt::launch_primary_hits(ctx->cam, ctx->useBvh ? nullptr : &ctx->small,
                                             ctx->useBvh ? &ctx->bvh : nullptr, ctx->seedOffset, dPrim.p, dT.p,
-                                            ctx->stream);
+                                            ctx->stream, ctx->lensAperture > 0.f ? &lens : nullptr);
   if (e == cudaSuccess && primId)
     e = cudaMemcpyAsync(primId, dPrim.p, N * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream);
   if (e == cudaSuccess && t)

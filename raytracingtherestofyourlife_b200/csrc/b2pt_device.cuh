@@ -129,6 +129,42 @@ __device__ __forceinline__ f3 raygen(const B2Camera& cam, int pixel, uint32_t& s
   return mk3(d.x / m, d.y / m, d.z / m);
 }
 
+// Thin lens (b2pt_set_lens, DESIGN.md 8h) applied to the pinhole ray d0 = raygen(...): a point (a, b) of the unit disk
+// by bounded rejection (at most 16 pairs of draws; (0, 0) after 16 rejections), the origin o = pos + u*(r*a) + v*(r*b)
+// on the lens, and the direction from o to the point F = pos + d0 * (f / (d0 . nlook)) where the pinhole ray meets
+// the plane of focus; zero components nudged and normalised as raygen does.  Consumes 2k draws for k pairs.  The float
+// operations and their order are the ones include/b2pt.h fixes (b2pt_set_lens), so the CPU restatement agrees bit for
+// bit under -fmad=false.
+__device__ __forceinline__ void lens_ray(const B2Camera& cam, const B2Lens& L, f3 d0, uint32_t& seed, f3& o, f3& d)
+{
+  float a = 0.f, b = 0.f;
+#pragma unroll 1
+  for (int k = 0; k < 16; ++k)
+  {
+    const float x = 2.f * randf(seed) - 1.f;
+    const float y = 2.f * randf(seed) - 1.f;
+    if (x * x + y * y < 1.f)
+    {
+      a = x, b = y;
+      break;
+    }
+  }
+  const f3 pos = ld3(cam.pos);
+  const float ra = L.r * a, rb = L.r * b;
+  o = (pos + ld3(L.u) * ra) + ld3(L.v) * rb;
+  const float k = L.f / dot3(d0, ld3(cam.nlook));
+  const f3 F = pos + d0 * k;
+  d = F - o;
+  if (d.x == 0.f)
+    d.x += 0.0000001f;
+  if (d.y == 0.f)
+    d.y += 0.0000001f;
+  if (d.z == 0.f)
+    d.z += 0.0000001f;
+  const float m = sqrtf(dot3(d, d));
+  d = mk3(d.x / m, d.y / m, d.z / m);
+}
+
 // pathtracing/Camera.cxx:394-423 (Camera::PerspectiveRayGen, the generator of the -direct modes): the un-jittered ray
 // through the pixel's lower-left corner.
 __device__ __forceinline__ f3 raygen_corner(const B2Camera& cam, int pixel)

@@ -25,6 +25,8 @@
 //                                 round's pixels from each pixel's variance, per-pixel-count conversions.
 //   k_view_features_counts<Scene>, k_denoise_prep_counts
 //                                 guides and denoiser prep of an adaptive sweep at each pixel's own sample count.
+//   k_trace_lens<Scene,LISTED>, k_primary_hits_lens, k_view_features_lens, k_view_features_counts_lens
+//                                 the primary-ray kernels with every camera ray through a thin lens (b2pt_set_lens).
 //   k_create_rays, k_intersect, k_normalize, k_pnm16, k_fill_seeds, k_sum_peers: stage-level API kernels.
 //
 // Work distribution: queue and bins are statically partitioned into one region per persistent warp
@@ -156,10 +158,12 @@ __device__ __forceinline__ uint32_t fastdiv(uint32_t n, uint32_t magic, uint32_t
 }
 
 // Ray `idx` of the warp's region.  PRIMARY: generated from (pixel, sample) -- idx is the path id.  LISTED (with
-// PRIMARY): path id b * nPixels + e is sample sampleBase + b of canvas entry A.perm[e] (B2RenderArgs::perm).
-template <bool PRIMARY, bool LISTED = false>
+// PRIMARY): path id b * nPixels + e is sample sampleBase + b of canvas entry A.perm[e] (B2RenderArgs::perm).  LENS (with
+// PRIMARY): the ray goes through the thin lens of its camera, lens[view] (lens[0] for the camera parameter).
+template <bool PRIMARY, bool LISTED = false, bool LENS = false>
 __device__ __forceinline__ void load_ray(const B2Camera& cam, const B2RenderArgs& A, int64_t idx, f3& o, f3& d, f3& T,
-                                         uint32_t& pid, uint32_t& rng, uint32_t* slotOut = nullptr)
+                                         uint32_t& pid, uint32_t& rng, uint32_t* slotOut = nullptr,
+                                         const B2Lens* lens = nullptr)
 {
   if constexpr (PRIMARY && LISTED)
   {
@@ -172,6 +176,8 @@ __device__ __forceinline__ void load_ray(const B2Camera& cam, const B2RenderArgs
     rng = pixel + A.seedOffset + (uint32_t)(A.sampleBase + (int)b) * B2PT_GOLDEN;
     d = raygen(vc, (int)pixel, rng);
     o = ld3(vc.pos);
+    if constexpr (LENS)
+      lens_ray(vc, lens[view], d, rng, o, d);
     T = mk3(1.f, 1.f, 1.f);
   }
   else if (PRIMARY)
@@ -189,6 +195,8 @@ __device__ __forceinline__ void load_ray(const B2Camera& cam, const B2RenderArgs
       rng = pixel + A.seedOffset + (uint32_t)(A.sampleBase + (int)b) * B2PT_GOLDEN;
       d = raygen(vc, (int)pixel, rng);
       o = ld3(vc.pos);
+      if constexpr (LENS)
+        lens_ray(vc, lens[view], d, rng, o, d);
     }
     else
     {
@@ -198,6 +206,8 @@ __device__ __forceinline__ void load_ray(const B2Camera& cam, const B2RenderArgs
         : pixel + A.seedOffset + (uint32_t)(A.sampleBase + (int)b) * B2PT_GOLDEN;
       d = raygen(cam, (int)pixel, rng);
       o = ld3(cam.pos);
+      if constexpr (LENS)
+        lens_ray(cam, lens[0], d, rng, o, d);
     }
     T = mk3(1.f, 1.f, 1.f);
   }
@@ -324,9 +334,10 @@ constexpr int kInnerSteps = B2PT_BVH_INNER_STEPS;
 #endif
 constexpr int kLeafChunk = B2PT_BVH_LEAF_CHUNK;
 
-template <bool PRIMARY, bool TAIL, bool LISTED = false>
+template <bool PRIMARY, bool TAIL, bool LISTED = false, bool LENS = false>
 __device__ __forceinline__ void trace_body_bvh(const B2Camera& cam, const B2BvhScene& S, const B2RenderArgs& A,
-                                               int depth, int w, int lane, int64_t nIn, int64_t tailWarps)
+                                               int depth, int w, int lane, int64_t nIn, int64_t tailWarps,
+                                               const B2Lens* lens = nullptr)
 {
   const int64_t base = TAIL ? 0 : (int64_t)w * A.regionCap;
   const bool refStream = (A.flags & B2PT_FLAG_REFERENCE_STREAM_DEV) != 0;
@@ -370,7 +381,7 @@ __device__ __forceinline__ void trace_body_bvh(const B2Camera& cam, const B2BvhS
                                             : (A.perm ? (int64_t)__ldg(A.perm + permBase + r) : base + r));
         if (PRIMARY ? idx < A.nPaths : (TAIL ? idx < nIn : true))
         {
-          load_ray<PRIMARY, LISTED>(cam, A, idx, o, d, T, pid, rng);
+          load_ray<PRIMARY, LISTED, LENS>(cam, A, idx, o, d, T, pid, rng, nullptr, lens);
           inv = mk3(rcp_safe(d.x), rcp_safe(d.y), rcp_safe(d.z));
           od = mk3(o.x * inv.x, o.y * inv.y, o.z * inv.z);
           closest = FLT_MAX;
@@ -869,9 +880,10 @@ __global__ void __launch_bounds__(kBlock, kMinBlocksPerSM)
 #endif
 constexpr int kWideRefillLanes = B2PT_WIDE_REFILL;
 
-template <bool PRIMARY, bool TAIL, bool LISTED = false>
+template <bool PRIMARY, bool TAIL, bool LISTED = false, bool LENS = false>
 __device__ __forceinline__ void trace_body_wide(const B2Camera& cam, const B2BvhScene& S, const B2RenderArgs& A, int depth,
-                                                int w, int lane, int64_t nIn, int64_t tailWarps)
+                                                int w, int lane, int64_t nIn, int64_t tailWarps,
+                                                const B2Lens* lens = nullptr)
 {
   const int64_t base = TAIL ? 0 : (int64_t)w * A.regionCap;
   const bool refStream = (A.flags & B2PT_FLAG_REFERENCE_STREAM_DEV) != 0;
@@ -914,7 +926,7 @@ __device__ __forceinline__ void trace_body_wide(const B2Camera& cam, const B2Bvh
         {
           f3 T;
           uint32_t pid;
-          load_ray<PRIMARY, LISTED>(cam, A, idx, o, d, T, pid, rngP);
+          load_ray<PRIMARY, LISTED, LENS>(cam, A, idx, o, d, T, pid, rngP, nullptr, lens);
           inv = mk3(rcp_safe(d.x), rcp_safe(d.y), rcp_safe(d.z));
           od = mk3(o.x * inv.x, o.y * inv.y, o.z * inv.z);
           oct = wide_octant(inv);
@@ -1057,19 +1069,21 @@ __device__ __forceinline__ void trace_body_wide(const B2Camera& cam, const B2Bvh
 }
 
 // Work of one warp in k_trace: rays [.., nIn) of its region (TAIL: tiles w, w+tailWarps, ... of the flat queue).
-// LISTED: primary rays of listed path ids (load_ray), traced without the per-tile primary masks.
-template <bool PRIMARY, class SceneT, bool TAIL, bool LISTED = false>
+// LISTED: primary rays of listed path ids (load_ray), traced without the per-tile primary masks.  LENS: primary rays
+// through the thin lenses `lens` (load_ray), also without the masks, which assume one ray origin per view.
+template <bool PRIMARY, class SceneT, bool TAIL, bool LISTED = false, bool LENS = false>
 __device__ __forceinline__ void trace_body(const B2Camera& cam, const SceneT& S, const B2RenderArgs& A, int depth,
-                                           int w, int lane, int64_t nIn, int64_t tailWarps)
+                                           int w, int lane, int64_t nIn, int64_t tailWarps,
+                                           const B2Lens* lens = nullptr)
 {
   if constexpr (std::is_same<SceneT, B2WideScene>::value)
   {
-    trace_body_wide<PRIMARY, TAIL, LISTED>(cam, S, A, depth, w, lane, nIn, tailWarps);
+    trace_body_wide<PRIMARY, TAIL, LISTED, LENS>(cam, S, A, depth, w, lane, nIn, tailWarps, lens);
     return;
   }
   if constexpr (std::is_same<SceneT, B2BvhScene>::value)
   {
-    trace_body_bvh<PRIMARY, TAIL, LISTED>(cam, S, A, depth, w, lane, nIn, tailWarps);
+    trace_body_bvh<PRIMARY, TAIL, LISTED, LENS>(cam, S, A, depth, w, lane, nIn, tailWarps, lens);
     return;
   }
   const int64_t base = TAIL ? 0 : (int64_t)w * A.regionCap;
@@ -1096,11 +1110,11 @@ __device__ __forceinline__ void trace_body(const B2Camera& cam, const SceneT& S,
     if (PRIMARY ? idx < A.nPaths : i < nIn)
     {
       uint32_t slotB = 0; // PRIMARY: sample slot of the path; the same for the 32 paths of a tile (nPixels % 32 == 0)
-      load_ray<PRIMARY, LISTED>(cam, A, idx, o, d, T, pid, rng, &slotB);
+      load_ray<PRIMARY, LISTED, LENS>(cam, A, idx, o, d, T, pid, rng, &slotB, lens);
       bool masked = false;
-      if constexpr (PRIMARY && !LISTED && std::is_same<SceneT, B2SmallScene>::value)
+      if constexpr (PRIMARY && !LISTED && !LENS && std::is_same<SceneT, B2SmallScene>::value)
         masked = A.primMask != nullptr;
-      if constexpr (PRIMARY && !LISTED && std::is_same<SceneT, B2SmallScene>::value)
+      if constexpr (PRIMARY && !LISTED && !LENS && std::is_same<SceneT, B2SmallScene>::value)
         if (masked)
       { // the tile's candidate mask and the view's per-quad constants (warp-uniform; nPixels % 32 == 0)
         const uint32_t tileBase = (uint32_t)idx - (uint32_t)lane;
@@ -1228,6 +1242,33 @@ __global__ void __launch_bounds__(kBlock, kTraceMinBlocksPerSM)
   if (!TAIL && w >= A.numWarps)
     return;
   trace_body<PRIMARY, SceneT, TAIL, LISTED>(cam, S, A, A.depth, w, lane, nIn, tailWarps);
+}
+
+// k_trace<PRIMARY> (LISTED or not) with every primary ray through the thin lens of its camera (b2pt_set_lens):
+// lens[view] of the cameras in A.views, or lens[0] for the camera parameter.  A kernel of its own, so that k_trace's
+// instantiations and parameter block stay as they are.
+template <class SceneT, bool LISTED>
+__global__ void __launch_bounds__(kBlock, kTraceMinBlocksPerSM)
+  k_trace_lens(const __grid_constant__ B2Camera cam, const __grid_constant__ SceneT scene,
+               const __grid_constant__ B2RenderArgs A, const B2Lens* __restrict__ lens)
+{
+  const int w = blockIdx.x * kWarps + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  const int64_t tilesTotal = (A.nPaths + 31) >> 5;
+  const int64_t nIn = w < A.numWarps ? ((tilesTotal + A.numWarps - 1) / A.numWarps) * 32 : 0;
+  if (!__syncthreads_or(nIn > 0))
+  {
+    if (w < A.numWarps && lane == 0)
+      for (int k = 0; k < 4; ++k)
+        A.bins[0].count[k * A.numWarps + w] = 0;
+    return;
+  }
+  __shared__ StageArea<SceneT> sStage;
+  const SceneT& S = stage_scene(scene, sStage);
+  __syncthreads();
+  if (w >= A.numWarps)
+    return;
+  trace_body<true, SceneT, false, LISTED, true>(cam, S, A, A.depth, w, lane, nIn, 0, lens);
 }
 
 // K3+K5: material response, direction generator, light pdfs, mixture pdf and the next ray for every binned hit
@@ -1839,6 +1880,25 @@ __global__ void __launch_bounds__(256)
   if (tOut)
     tOut[p] = h ? hit.t : FLT_MAX;
 }
+// k_primary_hits through the thin lens of the camera: t is measured from the ray's origin on the lens.
+template <class SceneT>
+__global__ void __launch_bounds__(256)
+  k_primary_hits_lens(const __grid_constant__ B2Camera cam, const __grid_constant__ SceneT scene, uint32_t seedOffset,
+                      const __grid_constant__ B2Lens lens, int32_t* primOut, float* tOut)
+{
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= cam.W * cam.H)
+    return;
+  uint32_t rng = (uint32_t)p + seedOffset;
+  f3 o, d = raygen(cam, p, rng);
+  lens_ray(cam, lens, d, rng, o, d);
+  Hit hit;
+  bool h = trace(scene, o, d, 0.001f, FLT_MAX, hit);
+  if (primOut)
+    primOut[p] = h ? hit.prim : -1;
+  if (tOut)
+    tOut[p] = h ? hit.t : FLT_MAX;
+}
 
 // -direct G-buffers (main.cc:402-422: runNorms / runAlbedo + the depth buffer): one un-jittered ray per pixel
 // (Camera::PerspectiveRayGen), closest QUAD hit (MapperQuad.cxx:103-113 extracts quads only) beyond t = 0, the two
@@ -1898,13 +1958,17 @@ __global__ void __launch_bounds__(256)
 // the features describe the same rays the radiance image averages.  Per sample: albedo = the reflectance the path's
 // first bounce applies (lambertian: the texture colour; dielectric: 1, shade_specular's attenuation; emitter: its
 // colour clamped to [0,1]), a hit flag, the shading normal and t; all zero on a miss.  The sums run in registers in
-// sample order (plain adds under -fmad=false) and slice k receives them after count[k] samples.
-template <class SceneT>
+// sample order (plain adds under -fmad=false) and slice k receives them after count[k] samples.  LENS: the primary rays
+// go through the camera's thin lens *lens as the render's do, and t is measured from the ray's origin on the lens.
+template <class SceneT, bool LENS = false>
 __device__ __forceinline__ void add_feature_sample(const SceneT& scene, const B2Camera& cam, f3 o, int p,
-                                                   uint32_t seedOffset, int s, float4& alb, float4& nd)
+                                                   uint32_t seedOffset, int s, float4& alb, float4& nd,
+                                                   const B2Lens* lens = nullptr)
 {
   uint32_t rng = (uint32_t)p + seedOffset + (uint32_t)s * B2PT_GOLDEN;
-  const f3 d = raygen(cam, p, rng);
+  f3 d = raygen(cam, p, rng);
+  if constexpr (LENS)
+    lens_ray(cam, *lens, d, rng, o, d);
   Hit hit;
   f3 a = mk3(0.f, 0.f, 0.f), nrm = a;
   float h = 0.f, t = 0.f;
@@ -1952,6 +2016,40 @@ __global__ void __launch_bounds__(256)
     }
   }
 }
+// k_view_features through the thin lens of every view, lenses[view] (b2pt_set_lens)
+template <class SceneT>
+__global__ void __launch_bounds__(256)
+  k_view_features_lens(const __grid_constant__ SceneT scene, const B2Camera* __restrict__ cams, int64_t n,
+                       uint32_t nPixels, uint32_t divMagic, uint32_t divShift, uint32_t seedOffset,
+                       const __grid_constant__ FeatureCheckpoints ck, float4* albedoOut, float4* normalDepthOut,
+                       const B2Lens* __restrict__ lenses)
+{
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n)
+    return;
+  const uint32_t view = fastdiv((uint32_t)idx, divMagic, divShift);
+  const int p = (int)((uint32_t)idx - view * nPixels);
+  const B2Camera cam = cams[view];
+  const B2Lens lens = lenses[view];
+  const f3 o = ld3(cam.pos);
+  float4 alb = make_float4(0.f, 0.f, 0.f, 0.f), nd = alb;
+  const int last = ck.count[ck.n - 1];
+  int k = 0, next = ck.count[0];
+  for (int s = 0; s < last; ++s)
+  {
+    add_feature_sample<SceneT, true>(scene, cam, o, p, seedOffset, s, alb, nd, &lens);
+    if (s + 1 == next)
+    {
+      const int64_t e = (int64_t)k * n + idx;
+      if (albedoOut)
+        albedoOut[e] = alb;
+      if (normalDepthOut)
+        normalDepthOut[e] = nd;
+      ++k;
+      next = k < ck.n ? ck.count[k] : 0;
+    }
+  }
+}
 
 // k_view_features with every (view, pixel) entry's own sample count (b2pt_render_views_adaptive_denoised): the sums
 // over samples s < counts[idx], stored once, so an entry of count c holds the bits of k_view_features' slice at c.
@@ -1972,6 +2070,29 @@ __global__ void __launch_bounds__(256)
   const int c = counts[idx];
   for (int s = 0; s < c; ++s)
     add_feature_sample(scene, cam, o, p, seedOffset, s, alb, nd);
+  albedoOut[idx] = alb;
+  normalDepthOut[idx] = nd;
+}
+// k_view_features_counts through the thin lens of every view, lenses[view] (b2pt_set_lens)
+template <class SceneT>
+__global__ void __launch_bounds__(256)
+  k_view_features_counts_lens(const __grid_constant__ SceneT scene, const B2Camera* __restrict__ cams, int64_t n,
+                              uint32_t nPixels, uint32_t divMagic, uint32_t divShift, uint32_t seedOffset,
+                              const int32_t* __restrict__ counts, float4* albedoOut, float4* normalDepthOut,
+                              const B2Lens* __restrict__ lenses)
+{
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n)
+    return;
+  const uint32_t view = fastdiv((uint32_t)idx, divMagic, divShift);
+  const int p = (int)((uint32_t)idx - view * nPixels);
+  const B2Camera cam = cams[view];
+  const B2Lens lens = lenses[view];
+  const f3 o = ld3(cam.pos);
+  float4 alb = make_float4(0.f, 0.f, 0.f, 0.f), nd = alb;
+  const int c = counts[idx];
+  for (int s = 0; s < c; ++s)
+    add_feature_sample<SceneT, true>(scene, cam, o, p, seedOffset, s, alb, nd, &lens);
   albedoOut[idx] = alb;
   normalDepthOut[idx] = nd;
 }
@@ -2364,7 +2485,7 @@ cudaError_t query_launch_cfg(LaunchCfg* cfg)
 template <class SceneT>
 static cudaError_t launch_bounce_t(const LaunchCfg& cfg, bool primary, int mode, const B2Camera& cam, const SceneT& S,
                                    const B2Lights& lights, const B2RenderArgs& args, cudaStream_t stream,
-                                   cudaEvent_t betweenStages)
+                                   cudaEvent_t betweenStages, const B2Lens* lens)
 {
   const int grid = (args.numWarps + kWarps - 1) / kWarps;
   const int tailGrid = std::max(1, std::min(grid, cfg.numSMs * 2));
@@ -2374,6 +2495,9 @@ static cudaError_t launch_bounce_t(const LaunchCfg& cfg, bool primary, int mode,
       return cudaErrorInvalidValue;
     k_trace<false, SceneT, true><<<tailGrid, kBlock, 0, stream>>>(cam, S, args);
   }
+  else if (primary && lens)
+    args.perm ? k_trace_lens<SceneT, true><<<grid, kBlock, 0, stream>>>(cam, S, args, lens)
+              : k_trace_lens<SceneT, false><<<grid, kBlock, 0, stream>>>(cam, S, args, lens);
   else if (primary)
     args.perm ? k_trace<true, SceneT, false, true><<<grid, kBlock, 0, stream>>>(cam, S, args)
               : k_trace<true, SceneT, false><<<grid, kBlock, 0, stream>>>(cam, S, args);
@@ -2402,10 +2526,13 @@ static cudaError_t launch_bounce_t(const LaunchCfg& cfg, bool primary, int mode,
 // One-kernel pipeline of small scenes.  Bounce 0 = k_trace<PRIMARY> (raygen + closest hit, bins into set 0); bounce
 // d >= 1 = k_bounce (shade the hits of bounce d-1, trace, bin into set d&1); d == maxDepth = the closing shade pass.
 cudaError_t launch_primary(const LaunchCfg& cfg, const B2Camera& cam, const B2SmallScene& S, const B2RenderArgs& args,
-                           cudaStream_t stream)
+                           cudaStream_t stream, const B2Lens* lens)
 {
   const int grid = (args.numWarps + kWarps - 1) / kWarps;
-  k_trace<true, B2SmallScene, false><<<grid, kBlock, 0, stream>>>(cam, S, args);
+  if (lens)
+    k_trace_lens<B2SmallScene, false><<<grid, kBlock, 0, stream>>>(cam, S, args, lens);
+  else
+    k_trace<true, B2SmallScene, false><<<grid, kBlock, 0, stream>>>(cam, S, args);
   return cudaGetLastError();
 }
 
@@ -2493,10 +2620,10 @@ cudaError_t launch_tail_loop(const B2Camera& cam, const B2SmallScene* small, con
 
 cudaError_t launch_bounce(const LaunchCfg& cfg, bool primary, int mode, const B2Camera& cam, const B2SmallScene* small,
                           const B2BvhScene* bvh, const B2Lights& lights, const B2RenderArgs& args,
-                          cudaStream_t stream, cudaEvent_t betweenStages)
+                          cudaStream_t stream, cudaEvent_t betweenStages, const B2Lens* lens)
 {
   return with_trace_scene(small, bvh, [&](const auto& S) {
-    return launch_bounce_t(cfg, primary, mode, cam, S, lights, args, stream, betweenStages);
+    return launch_bounce_t(cfg, primary, mode, cam, S, lights, args, stream, betweenStages, lens);
   });
 }
 
@@ -2546,11 +2673,16 @@ cudaError_t launch_accumulate_checkpoints(float4* color, const float4* rad, int 
 }
 
 cudaError_t launch_primary_hits(const B2Camera& cam, const B2SmallScene* small, const B2BvhScene* bvh,
-                                uint32_t seedOffset, int32_t* primOut, float* tOut, cudaStream_t stream)
+                                uint32_t seedOffset, int32_t* primOut, float* tOut, cudaStream_t stream,
+                                const B2Lens* lens)
 {
   const int n = cam.W * cam.H;
   with_trace_scene(small, bvh, [&](const auto& S) {
-    k_primary_hits<std::decay_t<decltype(S)>><<<(n + 255) / 256, 256, 0, stream>>>(cam, S, seedOffset, primOut, tOut);
+    if (lens)
+      k_primary_hits_lens<std::decay_t<decltype(S)>>
+        <<<(n + 255) / 256, 256, 0, stream>>>(cam, S, seedOffset, *lens, primOut, tOut);
+    else
+      k_primary_hits<std::decay_t<decltype(S)>><<<(n + 255) / 256, 256, 0, stream>>>(cam, S, seedOffset, primOut, tOut);
   });
   return cudaGetLastError();
 }
@@ -2578,7 +2710,7 @@ cudaError_t launch_direct_views(const B2SmallScene* small, const B2BvhScene* bvh
 
 cudaError_t launch_view_features(const B2SmallScene* small, const B2BvhScene* bvh, const B2Camera* cams, int nViews,
                                  int nPixels, uint32_t seedOffset, const FeatureCheckpoints& ck, float4* albedo,
-                                 float4* normalDepth, cudaStream_t stream)
+                                 float4* normalDepth, cudaStream_t stream, const B2Lens* lenses)
 {
   const int64_t n = (int64_t)nViews * nPixels;
   if (n <= 0)
@@ -2589,15 +2721,20 @@ cudaError_t launch_view_features(const B2SmallScene* small, const B2BvhScene* bv
   make_fastdiv((uint32_t)nPixels, magic, shift);
   const unsigned grid = (unsigned)((n + 255) / 256);
   with_trace_scene(small, bvh, [&](const auto& S) {
-    k_view_features<std::decay_t<decltype(S)>><<<grid, 256, 0, stream>>>(S, cams, n, (uint32_t)nPixels, magic, shift,
-                                                                         seedOffset, ck, albedo, normalDepth);
+    if (lenses)
+      k_view_features_lens<std::decay_t<decltype(S)>><<<grid, 256, 0, stream>>>(
+        S, cams, n, (uint32_t)nPixels, magic, shift, seedOffset, ck, albedo, normalDepth, lenses);
+    else
+      k_view_features<std::decay_t<decltype(S)>><<<grid, 256, 0, stream>>>(S, cams, n, (uint32_t)nPixels, magic, shift,
+                                                                           seedOffset, ck, albedo, normalDepth);
   });
   return cudaGetLastError();
 }
 
 cudaError_t launch_view_features_counts(const B2SmallScene* small, const B2BvhScene* bvh, const B2Camera* cams,
                                         int nViews, int nPixels, uint32_t seedOffset, const int32_t* counts,
-                                        float4* albedo, float4* normalDepth, cudaStream_t stream)
+                                        float4* albedo, float4* normalDepth, cudaStream_t stream,
+                                        const B2Lens* lenses)
 {
   const int64_t n = (int64_t)nViews * nPixels;
   if (n <= 0)
@@ -2608,8 +2745,12 @@ cudaError_t launch_view_features_counts(const B2SmallScene* small, const B2BvhSc
   make_fastdiv((uint32_t)nPixels, magic, shift);
   const unsigned grid = (unsigned)((n + 255) / 256);
   with_trace_scene(small, bvh, [&](const auto& S) {
-    k_view_features_counts<std::decay_t<decltype(S)>><<<grid, 256, 0, stream>>>(
-      S, cams, n, (uint32_t)nPixels, magic, shift, seedOffset, counts, albedo, normalDepth);
+    if (lenses)
+      k_view_features_counts_lens<std::decay_t<decltype(S)>><<<grid, 256, 0, stream>>>(
+        S, cams, n, (uint32_t)nPixels, magic, shift, seedOffset, counts, albedo, normalDepth, lenses);
+    else
+      k_view_features_counts<std::decay_t<decltype(S)>><<<grid, 256, 0, stream>>>(
+        S, cams, n, (uint32_t)nPixels, magic, shift, seedOffset, counts, albedo, normalDepth);
   });
   return cudaGetLastError();
 }

@@ -34,12 +34,14 @@ enum
 };
 cudaError_t launch_bounce(const LaunchCfg& cfg, bool primary, int mode, const B2Camera& cam, const B2SmallScene* small,
                           const B2BvhScene* bvh, const B2Lights& lights, const B2RenderArgs& args,
-                          cudaStream_t stream, cudaEvent_t betweenStages = nullptr);
+                          cudaStream_t stream, cudaEvent_t betweenStages = nullptr, const B2Lens* lens = nullptr);
 // One-kernel pipeline of small scenes (b2pt_kernels.cu k_bounce): bounce 0, bounce args.depth >= 1 (the closing shade
 // pass when args.depth == args.maxDepth) in one of the three modes above, and every bounce from args.depth >= 2
 // (global bins) to the closing pass inside one cluster launch.
+// lens (device array, nullptr = pinhole) in launch_bounce (primary) and launch_primary: the thin-lens records of the
+// cameras, [view] of args.views or [0] for cam; the primary rays then run through k_trace_lens.
 cudaError_t launch_primary(const LaunchCfg& cfg, const B2Camera& cam, const B2SmallScene& S, const B2RenderArgs& args,
-                           cudaStream_t stream);
+                           cudaStream_t stream, const B2Lens* lens = nullptr);
 cudaError_t launch_bounce_fused(const LaunchCfg& cfg, int mode, const B2SmallScene& S, const B2Lights& lights,
                                 const B2RenderArgs& args, cudaStream_t stream);
 cudaError_t launch_bounce_tail_loop(const B2SmallScene& S, const B2Lights& lights, const B2RenderArgs& args,
@@ -97,8 +99,10 @@ struct CheckpointArgs
 };
 cudaError_t launch_accumulate_checkpoints(float4* color, const float4* rad, int nPixels, int samplesPerView, int nViews,
                                           unsigned long long* nanCounter, const CheckpointArgs& ck, cudaStream_t stream);
+// lens (host pointer, nullptr = pinhole): sample 0's ray through this thin lens, t measured from its origin.
 cudaError_t launch_primary_hits(const B2Camera& cam, const B2SmallScene* small, const B2BvhScene* bvh,
-                                uint32_t seedOffset, int32_t* primOut, float* tOut, cudaStream_t stream);
+                                uint32_t seedOffset, int32_t* primOut, float* tOut, cudaStream_t stream,
+                                const B2Lens* lens = nullptr);
 // -direct G-buffers of nViews views (k_direct_views): per view the camera basis, its look-at point and its up vector
 // as Camera::SetUp stores it.  Outputs [view][pixel]: normals / albedo float4, depth float, prim ids; any may be null.
 // bvh != nullptr traverses its binary tree (nodes / primSlots in binary leaf order), else the small scene.
@@ -115,7 +119,8 @@ cudaError_t launch_direct_views(const B2SmallScene* small, const B2BvhScene* bvh
 // samples s = 0 .. count[n-1]-1 (the render's streams: rng = pixel + seedOffset + s * B2PT_GOLDEN), summed in sample
 // order; at s + 1 == count[k] the sums go to slice k, outputs [k][view][pixel] with slices nViews * nPixels apart.
 // albedo: (albedo rgb, hit); normalDepth: (normal xyz, t); either may be null.  The trace structure is the one the
-// renders use (bvh->wide: the 8-wide tree).  nViews * nPixels must stay below 2^32.
+// renders use (bvh->wide: the 8-wide tree).  nViews * nPixels must stay below 2^32.  lenses (device, nullptr = pinhole):
+// the thin-lens record of every camera, the rays then go through lenses[view] as the render's do.
 struct FeatureCheckpoints
 {
   int n;
@@ -123,7 +128,7 @@ struct FeatureCheckpoints
 };
 cudaError_t launch_view_features(const B2SmallScene* small, const B2BvhScene* bvh, const B2Camera* cams, int nViews,
                                  int nPixels, uint32_t seedOffset, const FeatureCheckpoints& ck, float4* albedo,
-                                 float4* normalDepth, cudaStream_t stream);
+                                 float4* normalDepth, cudaStream_t stream, const B2Lens* lenses = nullptr);
 // Spatial denoiser of b2pt_denoise_views over one chunk of nImages = K * nViews images of W x H pixels, stored
 // [k][view][pixel] (image z = k * nViews + v; its checkpoint count is count[z / nViews]).
 // launch_denoise_prep: in place, x (color sums in, (m, V0) out), moment (sums of squares, may be null; read only),
@@ -176,7 +181,8 @@ cudaError_t launch_pnm16_counts(const float4* color, int64_t n, const int32_t* c
 // sums of squares always used; color and moment are read only, (m, V0) goes to x, ga and gnz are converted in place.
 cudaError_t launch_view_features_counts(const B2SmallScene* small, const B2BvhScene* bvh, const B2Camera* cams,
                                         int nViews, int nPixels, uint32_t seedOffset, const int32_t* counts,
-                                        float4* albedo, float4* normalDepth, cudaStream_t stream);
+                                        float4* albedo, float4* normalDepth, cudaStream_t stream,
+                                        const B2Lens* lenses = nullptr);
 cudaError_t launch_denoise_prep_counts(const float4* color, const float4* moment, const int32_t* counts, float4* x,
                                        float4* ga, float4* gnz, int64_t n, cudaStream_t stream);
 cudaError_t launch_create_rays(const B2Camera& cam, uint32_t* seeds, float* dx, float* dy, float* dz, float* ox,

@@ -115,6 +115,15 @@ struct B2Camera // RayGen members, pathtracing/Camera.cxx:431-438
   int32_t W, H;
 };
 
+// Thin lens of one camera (b2pt_set_lens, DESIGN.md 8h), built on the host in float32: u = dx/|dx|, v = dy/|dy|,
+// r = aperture/2, f = the focus distance along nlook.  Kept apart from B2Camera so that no existing kernel parameter
+// block changes; the lens launches take one extra pointer to these records, one per camera.
+struct alignas(16) B2Lens
+{
+  float u[3], v[3];
+  float r, f;
+};
+
 struct alignas(16) B2Lights
 {
   int32_t nLightQuads, nLightSph;

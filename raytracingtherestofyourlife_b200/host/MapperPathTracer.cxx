@@ -243,6 +243,7 @@ void MapperPathTracer::RenderCellsImpl(const vtkm::cont::DynamicCellSet& cellset
     b2pt_facade::Check(
       b2pt_set_camera(ctx, p, a, u, camera.GetFieldOfView(), static_cast<int>(nx), static_cast<int>(ny)));
     b2pt_facade::Check(b2pt_seed(ctx, 0)); // seeds[i] = i, MapperPathTracer.cxx:265-267
+    b2pt_facade::Check(b2pt_set_lens(ctx, LensAperture, LensFocus));
     const int begin = static_cast<int>(static_cast<long long>(samplecount) * g / G);
     const int end = static_cast<int>(static_cast<long long>(samplecount) * (g + 1) / G);
     b2pt_facade::Check(b2pt_clear_color(ctx)); // MapperPathTracer.cxx:222-223
@@ -392,6 +393,7 @@ void MapperPathTracer::RenderViewsImpl(const vtkm::cont::DynamicCellSet& cellset
   const vtkm::Id nx = Internals->Canvas->GetWidth(), ny = Internals->Canvas->GetHeight();
   b2pt_ctx* ctx = b2pt_facade::Context();
   b2pt_facade::Check(b2pt_seed(ctx, 0)); // seeds[i] = i, MapperPathTracer.cxx:265-267
+  b2pt_facade::Check(b2pt_set_lens(ctx, LensAperture, LensFocus));
   if (checkpoints)
     b2pt_facade::Check(b2pt_render_views_checkpoints(
       ctx, static_cast<int>(cameras.size()), views.data(), static_cast<int>(nx), static_cast<int>(ny),
@@ -466,6 +468,7 @@ void MapperPathTracer::RenderCellsViewsFeatures(const vtkm::cont::DynamicCellSet
   normalDepth.assign(n, 0.f);
   b2pt_ctx* ctx = b2pt_facade::Context(Devices.empty() ? -1 : Devices[0]);
   b2pt_facade::Check(b2pt_seed(ctx, 0)); // the streams RenderCellsViews* render with
+  b2pt_facade::Check(b2pt_set_lens(ctx, LensAperture, LensFocus));
   b2pt_facade::Check(b2pt_render_views_features(ctx, static_cast<int>(cameras.size()), views.data(),
                                                 static_cast<int>(nx), static_cast<int>(ny),
                                                 static_cast<int>(checkpoints.size()), checkpoints.data(),
@@ -520,6 +523,7 @@ void MapperPathTracer::RenderCellsViewsAdaptivePnm(const vtkm::cont::DynamicCell
   counts.assign(n, 0);
   b2pt_ctx* ctx = b2pt_facade::Context();
   b2pt_facade::Check(b2pt_seed(ctx, 0)); // the streams RenderCellsViews* render with
+  b2pt_facade::Check(b2pt_set_lens(ctx, LensAperture, LensFocus));
   b2pt_adaptive_params params;
   b2pt_adaptive_defaults(&params);
   params.threshold = threshold;
@@ -552,6 +556,7 @@ void MapperPathTracer::RenderCellsViewsAdaptiveDenoisedPnm(const vtkm::cont::Dyn
   denoisedPnm.assign(n * 3, 0);
   b2pt_ctx* ctx = b2pt_facade::Context();
   b2pt_facade::Check(b2pt_seed(ctx, 0)); // the streams RenderCellsViews* render with
+  b2pt_facade::Check(b2pt_set_lens(ctx, LensAperture, LensFocus));
   b2pt_adaptive_params params;
   b2pt_adaptive_defaults(&params);
   params.threshold = threshold;

@@ -91,6 +91,14 @@ public:
 
   // B200 additions (not in the reference): render flags (B2PT_FLAG_*) and the statistics of the last render.
   void SetRenderFlags(unsigned int flags) { RenderFlags = flags; }
+  // Thin-lens depth of field (b2pt_set_lens): lens diameter and focus distance (<= 0: each camera focuses at its
+  // look-at point), passed to the context before every path-traced render and sweep.  (0, 0), the default, is the
+  // reference's pinhole; the reference has no counterpart.  The -direct buffers never use it.
+  void SetLens(float aperture, float focusDistance)
+  {
+    LensAperture = aperture;
+    LensFocus = focusDistance;
+  }
   // The GPUs RenderCells uses (CUDA device ordinals; default: the one of B2PT_DEVICE).  With G > 1 devices the samples
   // of every pixel are partitioned over them -- device g renders a contiguous range of the global sample indices with
   // the same per-(pixel, sample) streams a single GPU would use -- and the radiance sums are added over NVLink
@@ -196,6 +204,7 @@ private:
   [[noreturn]] static void FusedStage(const char* name);
 
   unsigned int RenderFlags = 0;
+  float LensAperture = 0.f, LensFocus = 0.f;
   std::vector<int> Devices; // empty = the default device
   double LastRenderMs = 0.0;
   long long LastSegments = 0;

@@ -43,6 +43,11 @@
 // sample count (b2pt_render_views_adaptive_denoised, default filter parameters): the files of -adaptive <tau>,
 // byte-identical, and <out>-adaptive-denoised-<phi>-<theta>.pnm.  The same uses as -adaptive are errors, and so is
 // -adaptive-denoise with -adaptive.
+// -aperture <a> [-focusdist <f>] renders every path-traced image -- the single render, -hemisphere, -fibonacci and
+// every sweep option above -- through a thin lens of diameter a (b2pt_set_lens; the reference's camera has none):
+// defocus blur away from the plane of focus, f scene units in front of each camera, or, with f <= 0 (the default), at
+// each camera's look-at point (the box centre in the sweeps).  a = 0 is the pinhole; without the flags every file is
+// what it was.  With -direct, or with a value that is not a finite number (a < 0 too), they are an error (exit 1).
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
@@ -83,6 +88,9 @@ struct Options
   bool adaptiveDenoiseGiven = false;
   std::string adaptiveDenoiseArg;
   float adaptive = 0.f; // -adaptive or -adaptive-denoise, parsed and checked by checkAdaptive
+  bool apertureGiven = false, focusGiven = false;
+  std::string apertureArg, focusArg;
+  float aperture = 0.f, focus = 0.f; // -aperture / -focusdist, parsed and checked by checkLens
 };
 
 Options parse(int argc, char** argv)
@@ -141,6 +149,18 @@ Options parse(int argc, char** argv)
       o.checkpointsGiven = true;
       if (i + 1 < argc)
         o.checkpointsArg = argv[++i];
+    }
+    else if (!std::strcmp(argv[i], "-aperture"))
+    {
+      o.apertureGiven = true;
+      if (i + 1 < argc)
+        o.apertureArg = argv[++i];
+    }
+    else if (!std::strcmp(argv[i], "-focusdist"))
+    {
+      o.focusGiven = true;
+      if (i + 1 < argc)
+        o.focusArg = argv[++i];
     }
   }
   return o;
@@ -229,6 +249,26 @@ std::string checkAdaptive(Options& o)
   return "";
 }
 
+// Parses -aperture and -focusdist into o.aperture / o.focus; returns an error message, empty when they are usable or
+// absent.
+std::string checkLens(Options& o)
+{
+  if (!o.apertureGiven && !o.focusGiven)
+    return "";
+  if (o.direct)
+    return "-aperture and -focusdist cannot be combined with -direct (its G-buffers use the pinhole corner rays)";
+  auto number = [](const std::string& arg, float& out) {
+    char* end = nullptr;
+    out = std::strtof(arg.c_str(), &end);
+    return !arg.empty() && *end == '\0' && std::isfinite(out);
+  };
+  if (o.apertureGiven && (!number(o.apertureArg, o.aperture) || o.aperture < 0.f))
+    return "-aperture takes a finite lens diameter >= 0, got '" + o.apertureArg + "'";
+  if (o.focusGiven && !number(o.focusArg, o.focus))
+    return "-focusdist takes a finite distance, got '" + o.focusArg + "'";
+  return "";
+}
+
 // NormalizeFunctor (main.cc:253-287): sqrt(de_nan(sum) / samplecount), alpha through the same sqrt
 void normalizeColors(vtkm::cont::ArrayHandle<vtkm::Vec<vtkm::Float32, 4>>& colors, int samplecount)
 {
@@ -247,12 +287,14 @@ void normalizeColors(vtkm::cont::ArrayHandle<vtkm::Vec<vtkm::Float32, 4>>& color
 }
 
 // the reference's runPath (main.cc:289-323): this body is what a reference user already has
+// (plus the -aperture / -focusdist lens, an extension)
 void runPath(CornellBox& cb, int samplecount, int depthcount, vtkm::rendering::Canvas& canvas,
-             vtkm::rendering::Camera& cam, bool stats)
+             vtkm::rendering::Camera& cam, bool stats, float aperture, float focus)
 {
   vtkm::rendering::MapperPathTracer mapper(samplecount, depthcount, cb.matIdx, cb.texIdx, cb.matType, cb.texType,
                                            cb.tex);
   mapper.SetCanvas(&canvas);
+  mapper.SetLens(aperture, focus);
   vtkm::cont::Field field;
   vtkm::cont::ColorTable ct;
   vtkm::Range sr;
@@ -408,6 +450,7 @@ int renderViews(CornellBox& cb, const Options& o, const std::vector<vtkm::render
   vtkm::rendering::CanvasRayTracer canvas(o.x, o.y);
   vtkm::rendering::MapperPathTracer mapper(o.samples, o.depth, cb.matIdx, cb.texIdx, cb.matType, cb.texType, cb.tex);
   mapper.SetCanvas(&canvas);
+  mapper.SetLens(o.aperture, o.focus);
   std::vector<unsigned short> pnm, denoised;
   std::vector<int> counts = o.checkpoints; // -checkpoints: one render, its images at every count up to samplecount
   counts.push_back(o.samples);
@@ -566,6 +609,8 @@ int main(int argc, char* argv[])
     bad = checkDenoise(o);
   if (bad.empty())
     bad = checkAdaptive(o);
+  if (bad.empty())
+    bad = checkLens(o);
   if (!bad.empty())
   {
     std::cerr << "error: " << bad << std::endl;
@@ -596,7 +641,7 @@ int main(int argc, char* argv[])
       runDirect(*cb, o, canvas, cam);
     else
     {
-      runPath(*cb, o.samples, o.depth, canvas, cam, o.stats);
+      runPath(*cb, o.samples, o.depth, canvas, cam, o.stats, o.aperture, o.focus);
       savePnm(o.out, o.x, o.y, canvas.GetColorBuffer());
     }
   }
