@@ -223,6 +223,37 @@ int b2pt_render_views_checkpoints(b2pt_ctx* ctx, int nViews, const float* views,
  * reference has no counterpart. */
 int b2pt_render_views_features(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
                                const int* checkpoints, uint32_t flags, float* albedoOut, float* normalDepthOut);
+/* Motion vectors and disocclusion between the views of a sweep (DESIGN.md 8i), from the primary hits of the SAME path
+ * samples b2pt_render_views_features traces.  views and prevViews hold 10 floats per view as in b2pt_render_views, on
+ * one W x H canvas; prevViews[v] is the camera view v is reprojected into (for a sweep, view v-1).  For view v with
+ * camera C and C' = prevViews[v], pixel p = j*W+i (j = 0 bottom row) and sample s:
+ *   1. (o, d) = the primary ray of b2pt_render_views_features (same stream, jittered raygen, under b2pt_set_lens the
+ *      lens ray), t = its closest hit in (0.001, FLT_MAX) through the trace structure `flags` selects; on a miss the
+ *      sample adds nothing;
+ *   2. X = o + d*t per component;
+ *   3. proj(C, X): D = X - pos, w = (D.x*nlook.x + D.y*nlook.y) + D.z*nlook.z, x = (D.dx) / (w * (dx.dx)) + W*0.5,
+ *      y = (D.dy) / (w * (dy.dy)) + H*0.5, every dot product in that order, with the camera basis of b2pt_set_camera
+ *      (nlook unit, |dx| = 2 tan(fov/2) / W, |dy| = 2 tan(fov/2) / H).  Raygen's sample of pixel (i, j) with jitter
+ *      (fx, fy) sits at (i + fx, j + fy); the projection ignores any lens (the camera's centre of projection);
+ *   4. the sample is valid when w > 0 for C and w' > 0 for C' (NaN is not > 0); an invalid sample adds nothing;
+ *   5. motion m = (x' - x, y' - y) in pixels, x to the right and y up;
+ *   6. visible = 1 when 0 <= x' < W and 0 <= y' < H and the closest hit from pos' along e = X - pos' (components equal
+ *      to 0 nudged by 1e-7, then L = sqrtf((e.x*e.x + e.y*e.y) + e.z*e.z) and e / L per component, as raygen
+ *      normalises) in (0.001, FLT_MAX) is absent or has t' >= L * 0.999755859375f (L*(1 - 2^-12)); else 0.  Off the
+ *      canvas no visibility ray is traced.
+ * motionOut = (sum m.x, sum m.y, sum visible, sum valid) over the valid samples s < checkpoints[k], float32 sums in
+ * sample order from +0.0, every operation in float32 without FMA; layout [k][view][j*W+i] float4, K*nViews*W*H*4
+ * floats.  Means are sum / sum valid; with prevViews == views the motion sums are exactly 0 and sum valid is the
+ * features' hit count.  The scene is the context's, static within the call (spheres moved by b2pt_update_spheres are
+ * not tracked: visibility is tested against the current scene).  flags may hold only the build flags.
+ * B2PT_ERR_BAD_VALUE, before anything runs: a bad view list or view in either list (b2pt_set_camera's message), a NULL
+ * prevViews or motionOut with nViews > 0, a checkpoint list of other than 1..32 strictly increasing counts >= 1,
+ * checkpoints[K-1] > 2^24, another flag, or K*W*H > 2^30.  nViews == 0 does nothing; no scene gives B2PT_ERR_STATE.
+ * Views run in chunks of whole views through library-owned staging of at most max(2^23, K*W*H) float4; the result does
+ * not depend on the chunking.  The context's camera, canvas, b2pt_views_device_ptr image and statistics are left
+ * untouched.  Synchronises the stream.  The reference has no counterpart. */
+int b2pt_render_views_motion(b2pt_ctx* ctx, int nViews, const float* views, const float* prevViews, int W, int H,
+                             int nCheckpoints, const int* checkpoints, uint32_t flags, float* motionOut);
 /* Parameters of b2pt_denoise_views.  A sigma may be +inf, which switches its term off. */
 typedef struct b2pt_denoise_params
 {

@@ -98,6 +98,7 @@ SIGNATURES = {
     "b2pt_render_views": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _i32, C.c_uint32, _vp]),
     "b2pt_render_views_checkpoints": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, _i32, C.c_uint32, _vp, _vp]),
     "b2pt_render_views_features": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, C.c_uint32, _vp, _vp]),
+    "b2pt_render_views_motion": (_i32, [_vp, _i32, _vp, _vp, _i32, _i32, _i32, _vp, C.c_uint32, _vp]),
     "b2pt_denoise_defaults": (None, [C.POINTER(DenoiseParams)]),
     "b2pt_denoise_views": (_i32, [_vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, C.POINTER(DenoiseParams),
                                   C.c_uint32, _vp]),
@@ -350,6 +351,22 @@ class Context:
         _check(lib().b2pt_render_views_features(self._h, v.shape[0], _p(v), W, H, K, _p(c), flags, _p(albedo),
                                                 _p(normal_depth)))
         return albedo, normal_depth
+
+    def render_views_motion(self, views, prev_views, W, H, checkpoints, flags=0):
+        """b2pt_render_views_motion: motion vectors from every view into prev_views (same shape as views: the camera
+        each view is reprojected into) over the path samples render_views_features traces; returns float32
+        [K, nViews, H*W, 4] sums over the first checkpoints[k] samples of (motion x, motion y, visible, valid), motion in
+        pixels with y up.  Means are sums / valid."""
+        v = np.ascontiguousarray(views, np.float32).reshape(-1, 10)
+        pv = np.ascontiguousarray(prev_views, np.float32).reshape(-1, 10)
+        if pv.shape != v.shape:
+            raise ValueError("prev_views must hold one camera per view")
+        c = np.ascontiguousarray(checkpoints, np.int32).reshape(-1)
+        K = c.shape[0]
+        motion = np.empty((K, v.shape[0], W * H, 4), np.float32)
+        _check(lib().b2pt_render_views_motion(self._h, v.shape[0], _p(v), _p(pv), W, H, K, _p(c), flags,
+                                              _p(motion)))
+        return motion
 
     def denoise_views(self, color, moment2, albedo, normal_depth, W, H, checkpoints, params=None, flags=0):
         """b2pt_denoise_views: the edge-avoiding a-trous filter of every (checkpoint, view) image of a sweep, guided by

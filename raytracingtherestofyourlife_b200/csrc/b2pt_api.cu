@@ -214,6 +214,8 @@ struct b2pt_ctx
   DevBuf<float4> ckptSnap, ckptMoment;
   // b2pt_render_views_features: [K][chunk views][W*H] staging of one chunk's sums
   DevBuf<float4> featAlbedo, featNormalDepth;
+  // b2pt_render_views_motion: [K][chunk views][W*H] staging of one chunk's sums
+  DevBuf<float4> motionSums;
   // b2pt_denoise_views: [K][chunk views][W*H] staging of one chunk: the ping-pong (x, V) images (the colour sums and
   // sums of squares arrive in them) and the two guides
   DevBuf<float4> dnX[2], dnGuideA, dnGuideNZ;
@@ -482,6 +484,7 @@ void b2pt_destroy(b2pt_ctx* ctx)
   ctx->counters.release(), ctx->binTotals.release(), ctx->seeds.release(), ctx->nanCounter.release();
   ctx->dViews.release(), ctx->viewColor.release(), ctx->pnm.release(), ctx->primMask.release(), ctx->primQuads.release(); // (DevBuf's destructor would free them too)
   ctx->ckptSnap.release(), ctx->ckptMoment.release(), ctx->featAlbedo.release(), ctx->featNormalDepth.release();
+  ctx->motionSums.release();
   ctx->dnX[0].release(), ctx->dnX[1].release(), ctx->dnGuideA.release(), ctx->dnGuideNZ.release();
   ctx->dDirectViews.release(), ctx->directNormals.release(), ctx->directAlbedo.release(), ctx->directDepth.release(),
     ctx->directPrim.release();
@@ -2561,6 +2564,72 @@ int b2pt_render_views_features(b2pt_ctx* ctx, int nViews, const float* views, in
         CU(cudaMemcpyAsync(normalDepthOut + dst, ctx->featNormalDepth.p + k * n, sizeof(float4) * (size_t)n,
                            cudaMemcpyDeviceToHost, ctx->stream));
     }
+  }
+  CU(cudaStreamSynchronize(ctx->stream));
+  return B2PT_OK;
+}
+
+// Motion vectors and disocclusion of a view sweep (k_view_motion) over the primary rays b2pt_render_views_features
+// traces.  The previous cameras go into ctx->dViews right after the cameras; views run in chunks of whole views by the
+// features' rule, each chunk one launch into ctx->motionSums and K copies into the caller's array.  The context's
+// camera, canvas, view images and statistics are not touched.
+int b2pt_render_views_motion(b2pt_ctx* ctx, int nViews, const float* views, const float* prevViews, int W, int H,
+                             int nCheckpoints, const int* checkpoints, uint32_t flags, float* motionOut)
+{
+  const char* fn = "b2pt_render_views_motion";
+  if (int rc = bind(ctx))
+    return rc;
+  if (int rc = check_view_list(fn, nViews, views))
+    return rc;
+  if (int rc = check_view_list(fn, nViews, prevViews))
+    return rc;
+  if (nViews > 0 && !motionOut)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: NULL motionOut", fn);
+  if (int rc = check_checkpoints(fn, nCheckpoints, checkpoints))
+    return rc;
+  if (checkpoints[nCheckpoints - 1] > (1 << 24))
+    return fail(B2PT_ERR_BAD_VALUE, "%s: more than 2^24 samples (the valid count must stay an exact float)", fn);
+  if (flags & ~kBuildFlags)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: flags may only hold FORCE_BVH, NO_DEDUP, NO_AA, GPU_LBVH and WIDE_BVH", fn);
+  std::vector<B2Camera> cams, prevCams;
+  if (int rc = make_view_cameras(nViews, views, W, H, cams))
+    return rc;
+  if (int rc = make_view_cameras(nViews, prevViews, W, H, prevCams))
+    return rc;
+  if (nViews == 0)
+    return B2PT_OK;
+  const int K = nCheckpoints;
+  const int64_t N = (int64_t)W * H, KN = N * K;
+  if (KN > ((int64_t)1 << 30))
+    return fail(B2PT_ERR_BAD_VALUE, "%s: one view's %d slices exceed 2^30 float4", fn, K);
+  if (!ctx->haveScene)
+    return fail(B2PT_ERR_STATE, "%s before b2pt_set_scene", fn);
+  if (int rc = ensure_built_for(ctx, flags))
+    return rc;
+  b2pt::FeatureCheckpoints ck{};
+  ck.n = K;
+  std::copy(checkpoints, checkpoints + K, ck.count);
+  const int64_t perChunk = std::max<int64_t>(1, kFeatureChunkFloat4 / KN);
+  CU(ctx->dViews.reserve(2 * (size_t)nViews));
+  CU(cudaMemcpyAsync(ctx->dViews.p, cams.data(), sizeof(B2Camera) * (size_t)nViews, cudaMemcpyHostToDevice,
+                     ctx->stream));
+  const B2Camera* dPrev = ctx->dViews.p + nViews;
+  CU(cudaMemcpyAsync(ctx->dViews.p + nViews, prevCams.data(), sizeof(B2Camera) * (size_t)nViews,
+                     cudaMemcpyHostToDevice, ctx->stream));
+  const std::vector<B2Lens> lenses = make_view_lenses(ctx, views, cams);
+  if (int rc = upload_lenses(ctx, lenses))
+    return rc;
+  CU(ctx->motionSums.reserve((size_t)(std::min<int64_t>(perChunk, nViews) * KN)));
+  for (int64_t v0 = 0; v0 < nViews; v0 += perChunk)
+  {
+    const int nv = (int)std::min<int64_t>(perChunk, nViews - v0);
+    const int64_t n = nv * N; // one slice of the chunk
+    CU(b2pt::launch_view_motion(ctx->useBvh ? nullptr : &ctx->small, ctx->useBvh ? &ctx->bvh : nullptr,
+                                ctx->dViews.p + v0, dPrev + v0, nv, (int)N, ctx->seedOffset, ck, ctx->motionSums.p,
+                                ctx->stream, lenses.empty() ? nullptr : ctx->dLens.p + v0));
+    for (int k = 0; k < K; ++k)
+      CU(cudaMemcpyAsync(motionOut + 4 * (size_t)((k * (int64_t)nViews + v0) * N), ctx->motionSums.p + k * n,
+                         sizeof(float4) * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
   }
   CU(cudaStreamSynchronize(ctx->stream));
   return B2PT_OK;

@@ -165,6 +165,21 @@ __device__ __forceinline__ void lens_ray(const B2Camera& cam, const B2Lens& L, f
   d = mk3(d.x / m, d.y / m, d.z / m);
 }
 
+// Pinhole projection of a world point X into camera cam, the inverse of raygen (b2pt_render_views_motion, DESIGN.md
+// 8i): D = X - pos, w = D . nlook, x = (D . dx) / (w * (dx . dx)) + W/2, y likewise with dy and H, continuous pixel
+// coordinates in which raygen's sample of pixel (i, j) with jitter (fx, fy) sits at (i + fx, j + fy).  Returns w; X is in
+// front of the camera when w > 0.  The float operations and their order are the ones include/b2pt.h fixes, so the CPU
+// restatement agrees bit for bit under -fmad=false.
+__device__ __forceinline__ float project(const B2Camera& cam, f3 X, float& x, float& y)
+{
+  const f3 D = X - ld3(cam.pos);
+  const f3 dx = ld3(cam.dx), dy = ld3(cam.dy);
+  const float w = dot3(D, ld3(cam.nlook));
+  x = dot3(D, dx) / (w * dot3(dx, dx)) + 0.5f * (float)cam.W;
+  y = dot3(D, dy) / (w * dot3(dy, dy)) + 0.5f * (float)cam.H;
+  return w;
+}
+
 // pathtracing/Camera.cxx:394-423 (Camera::PerspectiveRayGen, the generator of the -direct modes): the un-jittered ray
 // through the pixel's lower-left corner.
 __device__ __forceinline__ f3 raygen_corner(const B2Camera& cam, int pixel)

@@ -27,6 +27,8 @@
 //                                 guides and denoiser prep of an adaptive sweep at each pixel's own sample count.
 //   k_trace_lens<Scene,LISTED>, k_primary_hits_lens, k_view_features_lens, k_view_features_counts_lens
 //                                 the primary-ray kernels with every camera ray through a thin lens (b2pt_set_lens).
+//   k_view_motion<Scene,LENS>     per (view, pixel): motion vectors and disocclusion of its primary hits towards a
+//                                 previous camera (a projection and one visibility trace per hit), at chosen counts.
 //   k_create_rays, k_intersect, k_normalize, k_pnm16, k_fill_seeds, k_sum_peers: stage-level API kernels.
 //
 // Work distribution: queue and bins are statically partitioned into one region per persistent warp
@@ -2097,6 +2099,78 @@ __global__ void __launch_bounds__(256)
   normalDepthOut[idx] = nd;
 }
 
+// Motion vectors and disocclusion of a chunk of whole views (b2pt_render_views_motion): one thread per (view, pixel),
+// idx = view * nPixels + pixel as in k_view_features, and the same primary rays (LENS: through lenses[view]).  A sample
+// that hits at X = o + d*t is valid when X is in front of both cams[view] and prevCams[view] (project's w > 0); it adds
+// the motion (x' - x, y' - y) from its projection (x, y) into the view to its projection (x', y') into the previous
+// camera, and visible = 1 when (x', y') lies on the canvas and the closest hit from the previous camera's position
+// towards X is absent or no nearer than L*(1 - 2^-12), L = |X - pos'| (the ray nudged and normalised as raygen's is, L
+// the magnitude it is divided by).  The sums (motion.x, motion.y, visible, valid) run in sample order; slice k receives
+// them after count[k] samples.
+template <class SceneT, bool LENS>
+__global__ void __launch_bounds__(256)
+  k_view_motion(const __grid_constant__ SceneT scene, const B2Camera* __restrict__ cams,
+                const B2Camera* __restrict__ prevCams, int64_t n, uint32_t nPixels, uint32_t divMagic,
+                uint32_t divShift, uint32_t seedOffset, const __grid_constant__ FeatureCheckpoints ck,
+                float4* motionOut, const B2Lens* __restrict__ lenses)
+{
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n)
+    return;
+  const uint32_t view = fastdiv((uint32_t)idx, divMagic, divShift);
+  const int p = (int)((uint32_t)idx - view * nPixels);
+  const B2Camera cam = cams[view], prev = prevCams[view];
+  B2Lens lens;
+  if constexpr (LENS)
+    lens = lenses[view];
+  const f3 pos = ld3(cam.pos), prevPos = ld3(prev.pos);
+  const float W = (float)cam.W, H = (float)cam.H;
+  float4 sum = make_float4(0.f, 0.f, 0.f, 0.f);
+  const int last = ck.count[ck.n - 1];
+  int k = 0, next = ck.count[0];
+  for (int s = 0; s < last; ++s)
+  {
+    uint32_t rng = (uint32_t)p + seedOffset + (uint32_t)s * B2PT_GOLDEN;
+    f3 o = pos, d = raygen(cam, p, rng);
+    if constexpr (LENS)
+      lens_ray(cam, lens, d, rng, o, d);
+    Hit hit;
+    if (trace(scene, o, d, 0.001f, FLT_MAX, hit))
+    {
+      const f3 X = o + d * hit.t;
+      float x, y, xp, yp;
+      const float w = project(cam, X, x, y);
+      const float wp = project(prev, X, xp, yp);
+      if (w > 0.f && wp > 0.f)
+      {
+        float visible = 0.f;
+        if (xp >= 0.f && xp < W && yp >= 0.f && yp < H)
+        {
+          f3 e = X - prevPos;
+          if (e.x == 0.f)
+            e.x += 0.0000001f;
+          if (e.y == 0.f)
+            e.y += 0.0000001f;
+          if (e.z == 0.f)
+            e.z += 0.0000001f;
+          const float L = sqrtf(dot3(e, e));
+          e = mk3(e.x / L, e.y / L, e.z / L);
+          Hit occ;
+          if (!trace(scene, prevPos, e, 0.001f, FLT_MAX, occ) || occ.t >= L * 0.999755859375f)
+            visible = 1.f;
+        }
+        sum.x += xp - x, sum.y += yp - y, sum.z += visible, sum.w += 1.f;
+      }
+    }
+    if (s + 1 == next)
+    {
+      motionOut[(int64_t)k * n + idx] = sum;
+      ++k;
+      next = k < ck.n ? ck.count[k] : 0;
+    }
+  }
+}
+
 // pathtracing/Camera.cxx:894-953: fills + RayGen + origin broadcast, fused.
 __global__ void __launch_bounds__(256)
   k_create_rays(const __grid_constant__ B2Camera cam, uint32_t* seeds, float* dx, float* dy, float* dz, float* ox,
@@ -2751,6 +2825,30 @@ cudaError_t launch_view_features_counts(const B2SmallScene* small, const B2BvhSc
     else
       k_view_features_counts<std::decay_t<decltype(S)>><<<grid, 256, 0, stream>>>(
         S, cams, n, (uint32_t)nPixels, magic, shift, seedOffset, counts, albedo, normalDepth);
+  });
+  return cudaGetLastError();
+}
+
+cudaError_t launch_view_motion(const B2SmallScene* small, const B2BvhScene* bvh, const B2Camera* cams,
+                               const B2Camera* prevCams, int nViews, int nPixels, uint32_t seedOffset,
+                               const FeatureCheckpoints& ck, float4* motion, cudaStream_t stream, const B2Lens* lenses)
+{
+  const int64_t n = (int64_t)nViews * nPixels;
+  if (n <= 0)
+    return cudaSuccess;
+  if (n > 0xffffffffLL || ck.n < 1 || ck.n > kMaxCheckpoints)
+    return cudaErrorInvalidValue;
+  uint32_t magic, shift;
+  make_fastdiv((uint32_t)nPixels, magic, shift);
+  const unsigned grid = (unsigned)((n + 255) / 256);
+  with_trace_scene(small, bvh, [&](const auto& S) {
+    using SceneT = std::decay_t<decltype(S)>;
+    if (lenses)
+      k_view_motion<SceneT, true><<<grid, 256, 0, stream>>>(S, cams, prevCams, n, (uint32_t)nPixels, magic, shift,
+                                                            seedOffset, ck, motion, lenses);
+    else
+      k_view_motion<SceneT, false><<<grid, 256, 0, stream>>>(S, cams, prevCams, n, (uint32_t)nPixels, magic, shift,
+                                                             seedOffset, ck, motion, nullptr);
   });
   return cudaGetLastError();
 }

@@ -129,6 +129,14 @@ struct FeatureCheckpoints
 cudaError_t launch_view_features(const B2SmallScene* small, const B2BvhScene* bvh, const B2Camera* cams, int nViews,
                                  int nPixels, uint32_t seedOffset, const FeatureCheckpoints& ck, float4* albedo,
                                  float4* normalDepth, cudaStream_t stream, const B2Lens* lenses = nullptr);
+// Motion vectors of nViews views towards prevCams (k_view_motion): the primary rays of launch_view_features (same
+// streams, trace structure and lenses), per sample that hits the motion to prevCams[view] in pixels, its visibility
+// there and a valid flag; motion = (sum dx, sum dy, sum visible, sum valid) over the valid samples, stored at the
+// checkpoints as launch_view_features stores its sums.  nViews * nPixels must stay below 2^32.
+cudaError_t launch_view_motion(const B2SmallScene* small, const B2BvhScene* bvh, const B2Camera* cams,
+                               const B2Camera* prevCams, int nViews, int nPixels, uint32_t seedOffset,
+                               const FeatureCheckpoints& ck, float4* motion, cudaStream_t stream,
+                               const B2Lens* lenses = nullptr);
 // Spatial denoiser of b2pt_denoise_views over one chunk of nImages = K * nViews images of W x H pixels, stored
 // [k][view][pixel] (image z = k * nViews + v; its checkpoint count is count[z / nViews]).
 // launch_denoise_prep: in place, x (color sums in, (m, V0) out), moment (sums of squares, may be null; read only),

@@ -475,6 +475,29 @@ void MapperPathTracer::RenderCellsViewsFeatures(const vtkm::cont::DynamicCellSet
                                                 RenderFlags & B2PT_BUILD_FLAGS, albedo.data(), normalDepth.data()));
 }
 
+void MapperPathTracer::RenderCellsViewsMotion(const vtkm::cont::DynamicCellSet& cellset,
+                                              const vtkm::cont::CoordinateSystem& coords,
+                                              const std::vector<vtkm::rendering::Camera>& cameras,
+                                              const std::vector<vtkm::rendering::Camera>& prevCameras,
+                                              const std::vector<int>& checkpoints, std::vector<float>& motion)
+{
+  if (Internals->Canvas == nullptr)
+    throw vtkm::cont::ErrorBadValue("MapperPathTracer: no canvas set");
+  if (prevCameras.size() != cameras.size())
+    throw vtkm::cont::ErrorBadValue("MapperPathTracer: one previous camera per camera");
+  CheckCheckpoints(checkpoints, samplecount);
+  const std::vector<float> views = PrepareSweep(cellset, coords, cameras), prevViews = packViews(prevCameras);
+  const vtkm::Id nx = Internals->Canvas->GetWidth(), ny = Internals->Canvas->GetHeight();
+  motion.assign(checkpoints.size() * cameras.size() * static_cast<size_t>(nx * ny) * 4, 0.f);
+  b2pt_ctx* ctx = b2pt_facade::Context(Devices.empty() ? -1 : Devices[0]);
+  b2pt_facade::Check(b2pt_seed(ctx, 0)); // the streams RenderCellsViews* render with
+  b2pt_facade::Check(b2pt_set_lens(ctx, LensAperture, LensFocus));
+  b2pt_facade::Check(b2pt_render_views_motion(ctx, static_cast<int>(cameras.size()), views.data(), prevViews.data(),
+                                              static_cast<int>(nx), static_cast<int>(ny),
+                                              static_cast<int>(checkpoints.size()), checkpoints.data(),
+                                              RenderFlags & B2PT_BUILD_FLAGS, motion.data()));
+}
+
 void MapperPathTracer::RenderCellsViewsDenoisedPnm(const vtkm::cont::DynamicCellSet& cellset,
                                                    const vtkm::cont::CoordinateSystem& coords,
                                                    const std::vector<vtkm::rendering::Camera>& cameras,

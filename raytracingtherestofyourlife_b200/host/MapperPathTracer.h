@@ -131,6 +131,14 @@ public:
   void RenderCellsViewsFeatures(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
                                 const std::vector<vtkm::rendering::Camera>& cameras, const std::vector<int>& checkpoints,
                                 std::vector<float>& albedo, std::vector<float>& normalDepth);
+  // Motion vectors of the same sweep (b2pt_render_views_motion, on the first device of SetDevices): prevCameras[v]
+  // (one per camera, else ErrorBadValue) is the camera view v is reprojected into; same checkpoint rule.
+  // motion[((k * V + v) * W*H + i) * 4 + ...] = the sums over the primary hits of path samples 0 .. c-1 of
+  // (motion x, motion y, visible, valid), motion in pixels from view v to prevCameras[v], y up.
+  void RenderCellsViewsMotion(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
+                              const std::vector<vtkm::rendering::Camera>& cameras,
+                              const std::vector<vtkm::rendering::Camera>& prevCameras,
+                              const std::vector<int>& checkpoints, std::vector<float>& motion);
   // RenderCellsViewsCheckpointsPnm's integers (same checkpoint rule, same bytes in pnm) and, in denoisedPnm, the same
   // layout for the sweep denoised with b2pt_denoise_views' defaults: one render of the float sums and their squares,
   // the guides of RenderCellsViewsFeatures, then the filter (levels 0 for pnm, which is the unfiltered mean).

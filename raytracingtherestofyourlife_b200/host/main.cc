@@ -48,6 +48,13 @@
 // defocus blur away from the plane of focus, f scene units in front of each camera, or, with f <= 0 (the default), at
 // each camera's look-at point (the box centre in the sweeps).  a = 0 is the pinhole; without the flags every file is
 // what it was.  With -direct, or with a value that is not a finite number (a < 0 too), they are an error (exit 1).
+// -motion (with -hemisphere, path-traced) also writes <stem>-motion-<phi>-<theta>.pfm for every <stem> of -features:
+// motion vectors and disocclusion of the same path samples towards the previous view of the sweep (the first view
+// towards itself), b2pt_render_views_motion: PF with the mean motion x and y in pixels (y up) and the fraction of the
+// samples whose surface the previous view sees, over the samples whose hit lies in front of both cameras; 0 where there
+// is none.  It works with -checkpoints, -features, -denoise and -aperture, and every other file stays byte-identical to
+// a run without -motion.  -motion with -direct, without a sweep, with -fibonacci (consecutive lattice points are a
+// golden angle apart, not neighbours) or with -adaptive / -adaptive-denoise is an error (exit 1).
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
@@ -83,6 +90,7 @@ struct Options
   std::vector<int> checkpoints; // -checkpoints, parsed and checked by checkCheckpoints
   bool features = false;
   bool denoise = false;
+  bool motion = false;
   bool adaptiveGiven = false;
   std::string adaptiveArg;
   bool adaptiveDenoiseGiven = false;
@@ -132,6 +140,8 @@ Options parse(int argc, char** argv)
       o.features = true;
     else if (!std::strcmp(argv[i], "-denoise"))
       o.denoise = true;
+    else if (!std::strcmp(argv[i], "-motion"))
+      o.motion = true;
     else if (!std::strcmp(argv[i], "-adaptive"))
     {
       o.adaptiveGiven = true;
@@ -214,6 +224,22 @@ std::string checkDenoise(const Options& o)
     return "-denoise cannot be combined with -direct";
   if (!o.hemi && !o.fibonacci)
     return "-denoise needs -hemisphere or -fibonacci";
+  return "";
+}
+
+// Returns an error message for an unusable -motion, empty when it is usable or absent.
+std::string checkMotion(const Options& o)
+{
+  if (!o.motion)
+    return "";
+  if (o.direct)
+    return "-motion cannot be combined with -direct";
+  if (o.fibonacci)
+    return "-motion cannot be combined with -fibonacci (consecutive lattice points are not neighbouring views)";
+  if (!o.hemi)
+    return "-motion needs -hemisphere";
+  if (o.adaptiveGiven || o.adaptiveDenoiseGiven)
+    return "-motion cannot be combined with -adaptive or -adaptive-denoise";
   return "";
 }
 
@@ -527,6 +553,25 @@ int renderViews(CornellBox& cb, const Options& o, const std::vector<vtkm::render
       }
     }
   }
+  if (o.motion)
+  { // every view towards the one before it in sweep order, the first towards itself; sums as means over valid samples
+    std::vector<vtkm::rendering::Camera> prevCameras(cameras.begin(), cameras.end() - 1);
+    prevCameras.insert(prevCameras.begin(), cameras.front());
+    std::vector<float> motion, mv(n3);
+    mapper.RenderCellsViewsMotion(cb.ds.GetCellSet(), cb.coord, cameras, prevCameras, counts, motion);
+    for (size_t k = 0; k < counts.size(); ++k)
+      for (size_t v = 0; v < V; ++v)
+      {
+        const float* m = &motion[(k * V + v) * n * 4];
+        for (size_t i = 0; i < n; ++i)
+        {
+          const float valid = m[4 * i + 3];
+          for (int ch = 0; ch < 3; ++ch)
+            mv[3 * i + ch] = valid > 0.f ? m[4 * i + ch] / valid : 0.f;
+        }
+        savePfm(viewName(stemOf(k) + "-motion", angles[v].first, angles[v].second), o.x, o.y, 3, mv);
+      }
+  }
   return static_cast<int>(cameras.size());
 }
 
@@ -609,6 +654,8 @@ int main(int argc, char* argv[])
     bad = checkDenoise(o);
   if (bad.empty())
     bad = checkAdaptive(o);
+  if (bad.empty())
+    bad = checkMotion(o);
   if (bad.empty())
     bad = checkLens(o);
   if (!bad.empty())
