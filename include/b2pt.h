@@ -294,6 +294,59 @@ void b2pt_denoise_defaults(b2pt_denoise_params* p);
 int b2pt_denoise_views(b2pt_ctx* ctx, int nViews, int W, int H, int nCheckpoints, const int* checkpoints,
                        const float* color, const float* moment2, const float* albedo, const float* normalDepth,
                        const b2pt_denoise_params* params, uint32_t flags, void* out);
+/* Parameters of b2pt_denoise_views_temporal.  A tolerance may be +inf, which switches its test off. */
+typedef struct b2pt_temporal_params
+{
+  float alpha;      /* least weight of the new view, (0, 1]; 1 = no history at all */
+  float minVisible; /* a pixel takes history only when sum visible >= minVisible * sum valid, [0, 1] */
+  float normalTol;  /* tap consistent when |g_n(p) - g_n(q)|^2 <= normalTol^2 */
+  float albedoTol;  /* ... and |g_a(p) - g_a(q)|^2 <= albedoTol^2 (four lanes, as the a-trous filter) */
+  float depthTol;   /* ... and |z_q - d'| <= depthTol * d' (relative) */
+} b2pt_temporal_params;
+/* alpha 0.1, minVisible 0.5, normalTol 0.3, albedoTol 0.03, depthTol 0.05 (DESIGN.md 8j). */
+void b2pt_temporal_defaults(b2pt_temporal_params* p);
+/* Temporal accumulation of a view sweep (the temporal half of SVGF, Schied et al. 2017), then b2pt_denoise_views'
+ * a-trous filter.  The inputs are those of b2pt_denoise_views plus views (10 floats per view, the sweep in order, as in
+ * b2pt_render_views) and motion = the sums of b2pt_render_views_motion(views, prevViews) with prevViews[v] = views[v-1]
+ * for v >= 1 (row 0 of motion is not read), [k][view][j*W+i] float4 like the other inputs.  Every slice k is its own
+ * chain: view v takes its history from view v-1 of the same slice, view 0 has none.  The history is the UNFILTERED
+ * temporal result (x_bar, V_bar, n) of view v-1 (SVGF feeds back its first filtered level instead; DESIGN.md 8j).
+ * Float32 in this order, without FMA.  Pixel p = (i, j) of view v, slice k, c = checkpoints[k]: m, V0, g_a = (a, h),
+ * g_n and z as b2pt_denoise_views computes them, (Sx, Sy, Svis, Sval) its motion sums; the state of view v-1 at pixel
+ * q is (x_bar_q, V_bar_q), n_q and that view's g_a, g_n, z.
+ *   p takes history when v >= 1, alpha < 1, h_p > 0, Sval > 0 and Svis >= minVisible * Sval; otherwise
+ *   x_bar = m, V_bar = V0, n = 1.
+ *   Reprojection (pixel centres): u = (float)i + Sx/Sval, y = (float)j + Sy/Sval, u0 = floorf(u), y0 = floorf(y),
+ *   fu = u - u0, fy = y - y0; taps in the order (0,0), (1,0), (0,1), (1,1) at (u0 + dx, y0 + dy) with the bilinear
+ *   weights b = (1-fu)*(1-fy), fu*(1-fy), (1-fu)*fy, fu*fy.  A tap's column and row are tested for [0, W-1] x [0, H-1]
+ *   in float before any conversion to int, so NaN or huge motion only gives inconsistent taps.
+ *   Expected distance from the previous camera: d_hat = raygen's pinhole direction of camera C for pixel p at jitter
+ *   (0.5, 0.5), i.e. sx = (2*((float)i + 0.5f) - W)/2, sy = (2*((float)j + 0.5f) - H)/2, d = (nlook + dx*sx) + dy*sy,
+ *   zero components nudged by 1e-7, divided by sqrtf((d.x*d.x + d.y*d.y) + d.z*d.z); X_hat = pos + d_hat*z_p;
+ *   e = X_hat - pos' (pos' = the position of views[v-1]); d' = sqrtf((e.x*e.x + e.y*e.y) + e.z*e.z).
+ *   Tap q is consistent when it is inside the canvas, h_q > 0, ((dn0*dn0 + dn1*dn1) + dn2*dn2) <= normalTol^2 with
+ *   dn = g_n(p) - g_n(q), (((da0*da0 + da1*da1) + da2*da2) + da3*da3) <= albedoTol^2 with da = g_a(p) - g_a(q), and
+ *   fabsf(z_q - d') <= depthTol * d'; a tolerance of +inf switches its test off.
+ *   Over the consistent taps in tap order, sums from +0: sb = sum b, sx = sum b*x_bar_q (per channel),
+ *   sv = sum (b*b)*V_bar_q, sn = sum b*n_q.  If sb > 0: xh = sx/sb, Vh = sv/(sb*sb), nh = sn/sb, n = nh + 1,
+ *   a = fmaxf(alpha, 1/n), x_bar = (1-a)*xh + a*m, V_bar = ((1-a)*(1-a))*Vh + (a*a)*V0; if sb = 0, no history.
+ * Then denoise.levels levels of b2pt_denoise_views' filter with x_0 = x_bar, V_0 = V_bar and view v's own guides.
+ * out: float4 (x_L.rgb, V_L), or under B2PT_FLAG_VIEWS_PNM16 the uint16_t integers of b2pt_denoise_views;
+ * historyOut (may be NULL): float32 n per pixel, [k][view][j*W+i].  Guarantees: with alpha = 1, out is bit for bit
+ * b2pt_denoise_views(...) with the same denoise parameters and the history is 1 everywhere; with levels = 0, out is
+ * (x_bar, V_bar).  temporal NULL = b2pt_temporal_defaults, denoise NULL = b2pt_denoise_defaults.  A pure function of
+ * its inputs: needs no scene, leaves the context's camera, canvas, view images and statistics untouched, and the
+ * result depends neither on chunking nor on launch shape.  B2PT_ERR_BAD_VALUE, before anything runs: whatever
+ * b2pt_denoise_views rejects, a NULL views or motion with nViews > 0, a bad view (b2pt_set_camera's message), alpha NaN
+ * or outside (0, 1], minVisible NaN or outside [0, 1], a tolerance NaN or <= 0.  nViews == 0 does nothing.  Views run
+ * in chunks of whole views through library-owned staging of at most max(2^23, K*W*H) float4 per buffer (five buffers,
+ * plus max(2^23, K*W*H) floats of history); the state of the last view of a chunk (K*W*H float4 of (x_bar, V_bar), two
+ * of guides and K*W*H floats of n) is carried into the next.  Steady state allocates nothing.  One small launch per view
+ * (view v reads view v-1's result).  Synchronises the stream.  The reference has no counterpart. */
+int b2pt_denoise_views_temporal(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
+                                const int* checkpoints, const float* color, const float* moment2, const float* albedo,
+                                const float* normalDepth, const float* motion, const b2pt_temporal_params* temporal,
+                                const b2pt_denoise_params* denoise, uint32_t flags, void* out, float* historyOut);
 /* Parameters of b2pt_render_views_adaptive. */
 typedef struct b2pt_adaptive_params
 {

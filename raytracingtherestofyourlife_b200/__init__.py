@@ -13,7 +13,7 @@ import numpy as np
 
 from . import _build
 
-__all__ = ["lib", "Scene", "Camera", "Context", "B2ptError", "Stats", "DenoiseParams", "AdaptiveParams", "FLAG_REFERENCE_STREAM",
+__all__ = ["lib", "Scene", "Camera", "Context", "B2ptError", "Stats", "DenoiseParams", "TemporalParams", "AdaptiveParams", "FLAG_REFERENCE_STREAM",
            "FLAG_KILL_ZERO_THROUGHPUT", "FLAG_NO_DEDUP", "FLAG_FORCE_BVH", "FLAG_NO_AA", "FLAG_NO_TAIL", "FLAG_NO_OVERLAP", "FLAG_GPU_LBVH", "LIB_PATH"]
 
 LIB_PATH = _build.LIB
@@ -62,6 +62,19 @@ class DenoiseParams(C.Structure):
         return p
 
 
+class TemporalParams(C.Structure):
+    """b2pt_temporal_params: the least weight alpha of the new view, the visible fraction a pixel needs to take history,
+    and the normal, albedo and relative depth tolerances of a history tap (+inf switches a test off)."""
+    _fields_ = [("alpha", C.c_float), ("minVisible", C.c_float), ("normalTol", C.c_float), ("albedoTol", C.c_float),
+                ("depthTol", C.c_float)]
+
+    @staticmethod
+    def defaults():
+        p = TemporalParams()
+        lib().b2pt_temporal_defaults(C.byref(p))
+        return p
+
+
 class AdaptiveParams(C.Structure):
     """b2pt_adaptive_params: convergence threshold tau (relative standard error of the mean luminance), luminance
     floor epsilon and the Chebyshev radius over which an unconverged pixel keeps its neighbours sampling."""
@@ -102,6 +115,10 @@ SIGNATURES = {
     "b2pt_denoise_defaults": (None, [C.POINTER(DenoiseParams)]),
     "b2pt_denoise_views": (_i32, [_vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, C.POINTER(DenoiseParams),
                                   C.c_uint32, _vp]),
+    "b2pt_temporal_defaults": (None, [C.POINTER(TemporalParams)]),
+    "b2pt_denoise_views_temporal": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp,
+                                           C.POINTER(TemporalParams), C.POINTER(DenoiseParams), C.c_uint32, _vp,
+                                           _vp]),
     "b2pt_adaptive_defaults": (None, [C.POINTER(AdaptiveParams)]),
     "b2pt_render_views_adaptive": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, _i32, C.POINTER(AdaptiveParams),
                                           C.c_uint32, _vp, _vp, _vp, _vp]),
@@ -389,6 +406,36 @@ class Context:
                                         _p(normal_depth), None if params is None else C.byref(params), flags,
                                         _p(out)))
         return out
+
+    def denoise_views_temporal(self, color, moment2, albedo, normal_depth, motion, views, W, H, checkpoints,
+                               temporal=None, params=None, flags=0, history=False):
+        """b2pt_denoise_views_temporal: every view of a sweep blended with the previous view's unfiltered result,
+        reprojected along motion (render_views_motion(views, prev_views) with prev_views[v] = views[v-1]; row 0 is not
+        read), then the a-trous filter of denoise_views.  Inputs as denoise_views takes them plus motion
+        [K, nViews, H*W, 4] and views [nViews, 10] in sweep order; temporal is a TemporalParams and params a
+        DenoiseParams (None: the defaults).  Returns float32 [K, nViews, H*W, 4] (denoised mean rgb, filtered variance)
+        or, under FLAG_VIEWS_PNM16, uint16 [K, nViews, H*W, 3]; with history=True also the float32 [K, nViews, H*W]
+        history lengths n."""
+        c = np.ascontiguousarray(checkpoints, np.int32).reshape(-1)
+        K = c.shape[0]
+
+        def arr(a):
+            return None if a is None else np.ascontiguousarray(a, np.float32).reshape(K, -1, W * H, 4)
+        color, moment2, albedo, normal_depth, motion = (arr(a) for a in (color, moment2, albedo, normal_depth, motion))
+        V = color.shape[1]
+        for a in (moment2, albedo, normal_depth, motion):
+            assert a is None or a.shape == color.shape, "inputs must share the [K, nViews, H*W, 4] layout"
+        v = np.ascontiguousarray(views, np.float32).reshape(-1, 10)
+        if v.shape[0] != V:
+            raise ValueError("views must hold one camera per view")
+        dt, ch = (np.uint16, 3) if flags & FLAG_VIEWS_PNM16 else (np.float32, 4)
+        out = np.empty((K, V, W * H, ch), dt)
+        hist = np.empty((K, V, W * H), np.float32) if history else None
+        _check(lib().b2pt_denoise_views_temporal(
+            self._h, V, _p(v), W, H, K, _p(c), _p(color), _p(moment2), _p(albedo), _p(normal_depth), _p(motion),
+            None if temporal is None else C.byref(temporal), None if params is None else C.byref(params), flags,
+            _p(out), _p(hist)))
+        return (out, hist) if history else out
 
     def render_views_adaptive(self, views, W, H, rounds, max_depth, params=None, flags=0):
         """b2pt_render_views_adaptive: round 0 renders rounds[0] samples of every pixel, and after round k every pixel

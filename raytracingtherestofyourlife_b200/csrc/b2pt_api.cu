@@ -219,6 +219,10 @@ struct b2pt_ctx
   // b2pt_denoise_views: [K][chunk views][W*H] staging of one chunk: the ping-pong (x, V) images (the colour sums and
   // sums of squares arrive in them) and the two guides
   DevBuf<float4> dnX[2], dnGuideA, dnGuideNZ;
+  // b2pt_denoise_views_temporal: the chunk's motion sums and history n next to the buffers above, and the state of the
+  // last view of the previous chunk ([k][W*H]: (x_bar, V_bar), the two guides, n)
+  DevBuf<float4> tmMotion, tmCarryX, tmCarryA, tmCarryNZ;
+  DevBuf<float> tmHist, tmCarryN;
   // b2pt_render_views_adaptive: per canvas entry the sample count, the unconverged and active flags; the compacted list
   // of the next round's entries (padded to whole tiles), its length and the cub scratch
   DevBuf<int32_t> adCounts, adNum;
@@ -486,6 +490,8 @@ void b2pt_destroy(b2pt_ctx* ctx)
   ctx->ckptSnap.release(), ctx->ckptMoment.release(), ctx->featAlbedo.release(), ctx->featNormalDepth.release();
   ctx->motionSums.release();
   ctx->dnX[0].release(), ctx->dnX[1].release(), ctx->dnGuideA.release(), ctx->dnGuideNZ.release();
+  ctx->tmMotion.release(), ctx->tmCarryX.release(), ctx->tmCarryA.release(), ctx->tmCarryNZ.release();
+  ctx->tmHist.release(), ctx->tmCarryN.release();
   ctx->dDirectViews.release(), ctx->directNormals.release(), ctx->directAlbedo.release(), ctx->directDepth.release(),
     ctx->directPrim.release();
   if (ctx->evFork)
@@ -2726,6 +2732,174 @@ int b2pt_denoise_views(b2pt_ctx* ctx, int nViews, int W, int H, int nCheckpoints
       else
         CU(cudaMemcpyAsync(static_cast<float4*>(out) + dst, res + k * n, sizeof(float4) * (size_t)n,
                            cudaMemcpyDeviceToHost, ctx->stream));
+    }
+  }
+  CU(cudaStreamSynchronize(ctx->stream));
+  return B2PT_OK;
+}
+
+void b2pt_temporal_defaults(b2pt_temporal_params* p)
+{
+  if (!p)
+    return;
+  p->alpha = 0.1f;
+  p->minVisible = 0.5f;
+  p->normalTol = 0.3f;
+  p->albedoTol = 0.03f;
+  p->depthTol = 0.05f;
+}
+
+// Temporal accumulation of a sweep, then b2pt_denoise_views' filter (DESIGN.md 8j).  Views run in chunks of whole
+// views through b2pt_denoise_views' staging plus the motion and history buffers: per chunk, K host-to-device copies of
+// each input, the prep, one k_temporal launch per view in sweep order (view v reads view v-1's unfiltered result: the
+// view before it in the chunk, or for the chunk's first view the state carried over from the previous chunk), the
+// carry of the chunk's last view, the a-trous levels and the copies of the result and the history.  Every slice is its
+// own chain and every pixel's result depends only on its inputs and the previous view's state, so the result does not
+// depend on the chunking.
+int b2pt_denoise_views_temporal(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
+                                const int* checkpoints, const float* color, const float* moment2, const float* albedo,
+                                const float* normalDepth, const float* motion, const b2pt_temporal_params* temporal,
+                                const b2pt_denoise_params* denoise, uint32_t flags, void* out, float* historyOut)
+{
+  static const char* const fn = "b2pt_denoise_views_temporal";
+  if (int rc = bind(ctx))
+    return rc;
+  if (nViews < 0)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: negative view count", fn);
+  if (int rc = check_checkpoints(fn, nCheckpoints, checkpoints))
+    return rc;
+  if (!color || !albedo || !normalDepth || !out)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: color, albedo, normalDepth and out must not be NULL", fn);
+  if (W <= 0 || H <= 0)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: W and H must be positive", fn);
+  b2pt_denoise_params P;
+  if (denoise)
+    P = *denoise;
+  else
+    b2pt_denoise_defaults(&P);
+  if (int rc = check_denoise_params(fn, P))
+    return rc;
+  if (flags & ~B2PT_FLAG_VIEWS_PNM16)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: flags may only hold VIEWS_PNM16", fn);
+  const int K = nCheckpoints;
+  const int64_t N = (int64_t)W * H, KN = N * K;
+  if (KN > ((int64_t)1 << 30))
+    return fail(B2PT_ERR_BAD_VALUE, "%s: one view's %d slices exceed 2^30 float4", fn, K);
+  if (int rc = check_view_list(fn, nViews, views))
+    return rc;
+  if (nViews > 0 && !motion)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: NULL motion", fn);
+  b2pt_temporal_params T;
+  if (temporal)
+    T = *temporal;
+  else
+    b2pt_temporal_defaults(&T);
+  if (!(T.alpha > 0.f && T.alpha <= 1.f))
+    return fail(B2PT_ERR_BAD_VALUE, "%s: alpha must be in (0,1], got %g", fn, (double)T.alpha);
+  if (!(T.minVisible >= 0.f && T.minVisible <= 1.f))
+    return fail(B2PT_ERR_BAD_VALUE, "%s: minVisible must be in [0,1], got %g", fn, (double)T.minVisible);
+  const float tol[3] = { T.normalTol, T.albedoTol, T.depthTol };
+  const char* const tolName[3] = { "normalTol", "albedoTol", "depthTol" };
+  for (int s = 0; s < 3; ++s)
+    if (!(tol[s] > 0.f)) // NaN fails too
+      return fail(B2PT_ERR_BAD_VALUE, "%s: %s must be > 0 (or +inf), got %g", fn, tolName[s], (double)tol[s]);
+  std::vector<B2Camera> cams;
+  if (int rc = make_view_cameras(nViews, views, W, H, cams))
+    return rc;
+  if (nViews == 0)
+    return B2PT_OK;
+  const bool pnm = (flags & B2PT_FLAG_VIEWS_PNM16) != 0;
+  b2pt::DenoiseArgs a{};
+  a.n = K;
+  std::copy(checkpoints, checkpoints + K, a.count);
+  a.hasMoments = moment2 != nullptr;
+  a.sigmaLum = P.sigmaLum, a.sigmaAlbedo = P.sigmaAlbedo, a.sigmaNormal = P.sigmaNormal, a.sigmaDepth = P.sigmaDepth;
+  b2pt::TemporalArgs t{};
+  t.alpha = T.alpha, t.minVisible = T.minVisible, t.normalTol = T.normalTol, t.albedoTol = T.albedoTol;
+  t.depthTol = T.depthTol;
+  const int64_t perChunk = std::max<int64_t>(1, kDenoiseChunkFloat4 / KN);
+  const size_t cap = (size_t)(std::min<int64_t>(perChunk, nViews) * KN);
+  CU(ctx->dnX[0].reserve(cap));
+  CU(ctx->dnX[1].reserve(cap));
+  CU(ctx->dnGuideA.reserve(cap));
+  CU(ctx->dnGuideNZ.reserve(cap));
+  CU(ctx->tmMotion.reserve(cap));
+  CU(ctx->tmHist.reserve(cap));
+  if (perChunk < nViews)
+  {
+    CU(ctx->tmCarryX.reserve((size_t)KN));
+    CU(ctx->tmCarryA.reserve((size_t)KN));
+    CU(ctx->tmCarryNZ.reserve((size_t)KN));
+    CU(ctx->tmCarryN.reserve((size_t)KN));
+  }
+  if (pnm)
+    CU(ctx->pnm.reserve(cap * 3));
+  const float* const in[5] = { color, moment2, albedo, normalDepth, motion };
+  float4* const stage[5] = { ctx->dnX[0].p, ctx->dnX[1].p, ctx->dnGuideA.p, ctx->dnGuideNZ.p, ctx->tmMotion.p };
+  for (int64_t v0 = 0; v0 < nViews; v0 += perChunk)
+  {
+    const int nv = (int)std::min<int64_t>(perChunk, nViews - v0);
+    const int64_t n = nv * N; // one slice of the chunk
+    for (int b = 0; b < 5; ++b)
+      for (int k = 0; in[b] && k < K; ++k)
+        CU(cudaMemcpyAsync(stage[b] + k * n, in[b] + 4 * (size_t)((k * (int64_t)nViews + v0) * N),
+                           sizeof(float4) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    a.nViews = nv;
+    CU(b2pt::launch_denoise_prep(ctx->dnX[0].p, moment2 ? ctx->dnX[1].p : nullptr, ctx->dnGuideA.p, ctx->dnGuideNZ.p,
+                                 (int)N, a, ctx->stream));
+    for (int v = 0; v < nv; ++v)
+    {
+      const int64_t g = v0 + v, off = v * N;
+      t.cam = cams[(size_t)g];
+      const B2Camera& prev = cams[(size_t)(g > 0 ? g - 1 : g)];
+      t.prevPos[0] = prev.pos[0], t.prevPos[1] = prev.pos[1], t.prevPos[2] = prev.pos[2];
+      float4* const x = ctx->dnX[0].p + off;
+      const float4 *ga = ctx->dnGuideA.p + off, *gnz = ctx->dnGuideNZ.p + off;
+      float* const hist = ctx->tmHist.p + off;
+      if (g == 0) // no history
+        CU(b2pt::launch_temporal(x, ga, gnz, ctx->tmMotion.p + off, hist, n, nullptr, nullptr, nullptr, nullptr, 0, K,
+                                 t, ctx->stream));
+      else if (v > 0) // the view before it in this chunk
+        CU(b2pt::launch_temporal(x, ga, gnz, ctx->tmMotion.p + off, hist, n, x - N, ga - N, gnz - N, hist - N, n, K, t,
+                                 ctx->stream));
+      else // the last view of the previous chunk
+        CU(b2pt::launch_temporal(x, ga, gnz, ctx->tmMotion.p + off, hist, n, ctx->tmCarryX.p, ctx->tmCarryA.p,
+                                 ctx->tmCarryNZ.p, ctx->tmCarryN.p, N, K, t, ctx->stream));
+    }
+    if (v0 + nv < nViews)
+    { // carry the chunk's last view into the next chunk, before the levels overwrite (x_bar, V_bar)
+      const int64_t last = (nv - 1) * N;
+      for (int k = 0; k < K; ++k)
+      {
+        CU(cudaMemcpyAsync(ctx->tmCarryX.p + k * N, ctx->dnX[0].p + k * n + last, sizeof(float4) * (size_t)N,
+                           cudaMemcpyDeviceToDevice, ctx->stream));
+        CU(cudaMemcpyAsync(ctx->tmCarryA.p + k * N, ctx->dnGuideA.p + k * n + last, sizeof(float4) * (size_t)N,
+                           cudaMemcpyDeviceToDevice, ctx->stream));
+        CU(cudaMemcpyAsync(ctx->tmCarryNZ.p + k * N, ctx->dnGuideNZ.p + k * n + last, sizeof(float4) * (size_t)N,
+                           cudaMemcpyDeviceToDevice, ctx->stream));
+        CU(cudaMemcpyAsync(ctx->tmCarryN.p + k * N, ctx->tmHist.p + k * n + last, sizeof(float) * (size_t)N,
+                           cudaMemcpyDeviceToDevice, ctx->stream));
+      }
+    }
+    int cur = 0;
+    for (int level = 0; level < P.levels; ++level, cur ^= 1)
+      CU(b2pt::launch_atrous(ctx->dnX[cur].p, ctx->dnX[cur ^ 1].p, ctx->dnGuideA.p, ctx->dnGuideNZ.p, W, H, 1 << level,
+                             a, ctx->stream));
+    const float4* res = ctx->dnX[cur].p;
+    if (pnm)
+      CU(b2pt::launch_pnm16(res, n * K, 1, ctx->pnm.p, ctx->stream));
+    for (int k = 0; k < K; ++k)
+    {
+      const size_t dst = (size_t)((k * (int64_t)nViews + v0) * N);
+      if (pnm)
+        CU(cudaMemcpyAsync(static_cast<uint16_t*>(out) + 3 * dst, ctx->pnm.p + 3 * k * n, sizeof(uint16_t) * 3 * (size_t)n,
+                           cudaMemcpyDeviceToHost, ctx->stream));
+      else
+        CU(cudaMemcpyAsync(static_cast<float4*>(out) + dst, res + k * n, sizeof(float4) * (size_t)n,
+                           cudaMemcpyDeviceToHost, ctx->stream));
+      if (historyOut)
+        CU(cudaMemcpyAsync(historyOut + dst, ctx->tmHist.p + k * n, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost,
+                           ctx->stream));
     }
   }
   CU(cudaStreamSynchronize(ctx->stream));

@@ -196,6 +196,22 @@ __device__ __forceinline__ f3 raygen_corner(const B2Camera& cam, int pixel)
   const float m = sqrtf(dot3(d, d));
   return mk3(d.x / m, d.y / m, d.z / m);
 }
+// raygen's direction for pixel (i, j) at jitter (0.5, 0.5), the pixel centre, with no draws (the expected distance of
+// b2pt_denoise_views_temporal): the same float operations as raygen with ru = rv = 0.5.
+__device__ __forceinline__ f3 raygen_centre(const B2Camera& cam, int i, int j)
+{
+  const float sx = (2.f * ((float)i + 0.5f) - (float)cam.W) / 2.0f;
+  const float sy = (2.f * ((float)j + 0.5f) - (float)cam.H) / 2.0f;
+  f3 d = (ld3(cam.nlook) + ld3(cam.dx) * sx) + ld3(cam.dy) * sy;
+  if (d.x == 0.f)
+    d.x += 0.0000001f;
+  if (d.y == 0.f)
+    d.y += 0.0000001f;
+  if (d.z == 0.f)
+    d.z += 0.0000001f;
+  const float m = sqrtf(dot3(d, d));
+  return mk3(d.x / m, d.y / m, d.z / m);
+}
 // The per-pixel colour rules of the -direct G-buffers: raytracing/RayTracerNormals.cxx:137-140 (the hit normal) and
 // RayTracerAlbedo.cxx:100-143 (cosPhi * R / (cosTheta * L) per channel, with the light at camera + 2 up, :154-155).
 // Same float operations in the same order as the reference's worklets (pinned through the oracle, tests/).

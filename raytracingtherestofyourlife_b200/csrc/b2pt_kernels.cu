@@ -29,6 +29,8 @@
 //                                 the primary-ray kernels with every camera ray through a thin lens (b2pt_set_lens).
 //   k_view_motion<Scene,LENS>     per (view, pixel): motion vectors and disocclusion of its primary hits towards a
 //                                 previous camera (a projection and one visibility trace per hit), at chosen counts.
+//   k_temporal                    per (slice, pixel) of one view: temporal accumulation of a sweep, the previous
+//                                 view's unfiltered result reprojected along the motion sums (one launch per view).
 //   k_create_rays, k_intersect, k_normalize, k_pnm16, k_fill_seeds, k_sum_peers: stage-level API kernels.
 //
 // Work distribution: queue and bins are statically partitioned into one region per persistent warp
@@ -2401,6 +2403,79 @@ __global__ void __launch_bounds__(kAtrousTile * kAtrousTile)
   xOut[p] = make_float4(sx / sw, sy / sw, sz / sw, sv / (sw * sw));
 }
 
+// Temporal accumulation of one view (b2pt_denoise_views_temporal, include/b2pt.h fixes the float operations and their
+// order): one thread per pixel, the slice in blockIdx.y.  The pixel's (m, V0) in x becomes (x_bar, V_bar) in place and
+// its history n goes to hist; the four bilinear taps read only the previous view (px, pga, pgnz, phist), which no
+// thread of this launch writes.  No atomics: every output is one thread's sum in a fixed tap order.
+__global__ void __launch_bounds__(256)
+  k_temporal(float4* x, const float4* __restrict__ ga, const float4* __restrict__ gnz,
+             const float4* __restrict__ motion, float* hist, long long stride, const float4* __restrict__ px,
+             const float4* __restrict__ pga, const float4* __restrict__ pgnz, const float* __restrict__ phist,
+             long long pstride, const __grid_constant__ TemporalArgs t)
+{
+  const int W = t.cam.W, H = t.cam.H;
+  const int p = (int)(blockIdx.x * blockDim.x + threadIdx.x);
+  if (p >= W * H)
+    return;
+  const long long o = (long long)blockIdx.y * stride + p, po = (long long)blockIdx.y * pstride;
+  const float4 cur = x[o], ap = ga[o], np = gnz[o], M = motion[o];
+  float4 res = cur;
+  float n = 1.f;
+  if (px && t.alpha < 1.f && ap.w > 0.f && M.w > 0.f && M.z >= t.minVisible * M.w)
+  {
+    const int i = p % W, j = p / W;
+    const float u = (float)i + M.x / M.w, y = (float)j + M.y / M.w;
+    const float u0 = floorf(u), y0 = floorf(y), fu = u - u0, fy = y - y0;
+    const f3 d = raygen_centre(t.cam, i, j);
+    const f3 e = (ld3(t.cam.pos) + d * np.w) - ld3(t.prevPos);
+    const float dprev = sqrtf(dot3(e, e));
+    const bool useN = !isinf(t.normalTol), useA = !isinf(t.albedoTol), useZ = !isinf(t.depthTol);
+    const float nt2 = t.normalTol * t.normalTol, at2 = t.albedoTol * t.albedoTol, zt = t.depthTol * dprev;
+    float sb = 0.f, s0 = 0.f, s1 = 0.f, s2 = 0.f, sv = 0.f, sn = 0.f;
+#pragma unroll
+    for (int tap = 0; tap < 4; ++tap)
+    {
+      const int dx = tap & 1, dy = tap >> 1;
+      const float cu = u0 + (float)dx, cy = y0 + (float)dy;
+      if (!(cu >= 0.f && cu <= (float)(W - 1) && cy >= 0.f && cy <= (float)(H - 1)))
+        continue;
+      const long long q = po + (long long)((int)cy * W + (int)cu);
+      const float4 aq = pga[q], nq = pgnz[q];
+      if (!(aq.w > 0.f))
+        continue;
+      if (useN)
+      {
+        const float d0 = np.x - nq.x, d1 = np.y - nq.y, d2 = np.z - nq.z;
+        if (!(d0 * d0 + d1 * d1 + d2 * d2 <= nt2))
+          continue;
+      }
+      if (useA)
+      {
+        const float d0 = ap.x - aq.x, d1 = ap.y - aq.y, d2 = ap.z - aq.z, d3 = ap.w - aq.w;
+        if (!(d0 * d0 + d1 * d1 + d2 * d2 + d3 * d3 <= at2))
+          continue;
+      }
+      if (useZ && !(fabsf(nq.w - dprev) <= zt))
+        continue;
+      const float b = (dx ? fu : 1.f - fu) * (dy ? fy : 1.f - fy);
+      const float4 xq = px[q];
+      sb += b;
+      s0 += b * xq.x, s1 += b * xq.y, s2 += b * xq.z;
+      sv += (b * b) * xq.w;
+      sn += b * phist[q];
+    }
+    if (sb > 0.f)
+    {
+      n = sn / sb + 1.f;
+      const float a = fmaxf(t.alpha, 1.f / n), r = 1.f - a, sb2 = sb * sb;
+      res = make_float4(r * (s0 / sb) + a * cur.x, r * (s1 / sb) + a * cur.y, r * (s2 / sb) + a * cur.z,
+                        (r * r) * (sv / sb2) + (a * a) * cur.w);
+    }
+  }
+  x[o] = res;
+  hist[o] = n;
+}
+
 // ---- adaptive sampling of a view sweep (b2pt_render_views_adaptive) --------------------------------------------------
 // k_accumulate_checkpoints' loop over one batch of a listed round: entry e < nReal of the list adds the samples
 // rad[b * nPad + e], b = 0 .. nSamples-1, of canvas entry P = list[e] onto the running sum S[P] and their squares onto
@@ -2921,6 +2996,20 @@ cudaError_t launch_atrous(const float4* xIn, float4* xOut, const float4* ga, con
     const dim3 grid((unsigned)(tilesX * tilesY), (unsigned)std::min(65535, images - z0));
     k_atrous<<<grid, dim3(kAtrousTile, kAtrousTile), 0, stream>>>(xIn, xOut, ga, gnz, W, H, tilesX, step, z0, a);
   }
+  return cudaGetLastError();
+}
+
+cudaError_t launch_temporal(float4* x, const float4* ga, const float4* gnz, const float4* motion, float* hist,
+                            int64_t stride, const float4* px, const float4* pga, const float4* pgnz, const float* phist,
+                            int64_t pstride, int nSlices, const TemporalArgs& t, cudaStream_t stream)
+{
+  const int64_t n = (int64_t)t.cam.W * t.cam.H;
+  if (n <= 0 || nSlices <= 0)
+    return cudaSuccess;
+  if (n > 0x7fffffffLL || nSlices > 65535)
+    return cudaErrorInvalidValue;
+  const dim3 grid((unsigned)((n + 255) / 256), (unsigned)nSlices);
+  k_temporal<<<grid, 256, 0, stream>>>(x, ga, gnz, motion, hist, stride, px, pga, pgnz, phist, pstride, t);
   return cudaGetLastError();
 }
 

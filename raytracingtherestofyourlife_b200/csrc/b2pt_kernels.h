@@ -154,6 +154,19 @@ cudaError_t launch_denoise_prep(float4* x, const float4* moment, float4* ga, flo
                                 const DenoiseArgs& a, cudaStream_t stream);
 cudaError_t launch_atrous(const float4* xIn, float4* xOut, const float4* ga, const float4* gnz, int W, int H,
                           int step, const DenoiseArgs& a, cudaStream_t stream);
+// Temporal accumulation of one view of a sweep (b2pt_denoise_views_temporal, k_temporal) in all nSlices slices: slice k
+// of the view's (m, V0) in x[k * stride .. + W*H), turned in place into (x_bar, V_bar), with its guides ga / gnz as
+// launch_denoise_prep leaves them, its motion sums and its history n written to hist, at the same offsets.  The
+// previous view's state px / pga / pgnz / phist sits at k * pstride; px == nullptr means there is no previous view.
+struct TemporalArgs
+{
+  B2Camera cam;   // camera of the view (pixel-centre ray of the expected distance)
+  float prevPos[3]; // position of the previous view's camera
+  float alpha, minVisible, normalTol, albedoTol, depthTol; // +inf switches a test off
+};
+cudaError_t launch_temporal(float4* x, const float4* ga, const float4* gnz, const float4* motion, float* hist,
+                            int64_t stride, const float4* px, const float4* pga, const float4* pgnz, const float* phist,
+                            int64_t pstride, int nSlices, const TemporalArgs& t, cudaStream_t stream);
 // Adaptive sampling of a view sweep (b2pt_render_views_adaptive).  Canvas entries P = view * W*H + pixel, n of them.
 // launch_accumulate_list: for e < nReal, the samples rad[b * nPad + e] (b < nSamples) onto color[list[e]] and their
 // squares onto moment[list[e]], in sample order (k_accumulate_checkpoints' operations).

@@ -530,6 +530,41 @@ void MapperPathTracer::RenderCellsViewsDenoisedPnm(const vtkm::cont::DynamicCell
                                         denoisedPnm.data()));
 }
 
+void MapperPathTracer::RenderCellsViewsTemporalPnm(const vtkm::cont::DynamicCellSet& cellset,
+                                                   const vtkm::cont::CoordinateSystem& coords,
+                                                   const std::vector<vtkm::rendering::Camera>& cameras,
+                                                   const std::vector<int>& checkpoints,
+                                                   std::vector<unsigned short>& temporalPnm)
+{
+  if (Internals->Canvas == nullptr)
+    throw vtkm::cont::ErrorBadValue("MapperPathTracer: no canvas set");
+  CheckCheckpoints(checkpoints, samplecount);
+  if (cameras.empty())
+  {
+    temporalPnm.clear();
+    return;
+  }
+  std::vector<float> color, moment2, albedo, normalDepth, motion;
+  const size_t n = static_cast<size_t>(Internals->Canvas->GetWidth()) * Internals->Canvas->GetHeight();
+  const size_t n4 = checkpoints.size() * cameras.size() * n * 4;
+  color.assign(n4, 0.f);
+  moment2.assign(n4, 0.f);
+  RenderViewsImpl(cellset, coords, cameras, 0, color.data(), &checkpoints, moment2.data());
+  RenderCellsViewsFeatures(cellset, coords, cameras, checkpoints, albedo, normalDepth);
+  // every view towards the one before it in sweep order (the first towards itself; its motion is not read)
+  std::vector<vtkm::rendering::Camera> prevCameras(cameras.begin(), cameras.end() - 1);
+  prevCameras.insert(prevCameras.begin(), cameras.front());
+  RenderCellsViewsMotion(cellset, coords, cameras, prevCameras, checkpoints, motion);
+  const std::vector<float> views = packViews(cameras);
+  b2pt_ctx* ctx = b2pt_facade::Context();
+  const int V = static_cast<int>(cameras.size()), K = static_cast<int>(checkpoints.size());
+  const int nx = static_cast<int>(Internals->Canvas->GetWidth()), ny = static_cast<int>(Internals->Canvas->GetHeight());
+  temporalPnm.assign(n4 / 4 * 3, 0);
+  b2pt_facade::Check(b2pt_denoise_views_temporal(ctx, V, views.data(), nx, ny, K, checkpoints.data(), color.data(),
+                                                 moment2.data(), albedo.data(), normalDepth.data(), motion.data(),
+                                                 nullptr, nullptr, B2PT_FLAG_VIEWS_PNM16, temporalPnm.data(), nullptr));
+}
+
 void MapperPathTracer::RenderCellsViewsAdaptivePnm(const vtkm::cont::DynamicCellSet& cellset,
                                                    const vtkm::cont::CoordinateSystem& coords,
                                                    const std::vector<vtkm::rendering::Camera>& cameras,

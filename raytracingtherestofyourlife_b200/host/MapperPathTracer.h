@@ -146,6 +146,13 @@ public:
                                    const std::vector<vtkm::rendering::Camera>& cameras,
                                    const std::vector<int>& checkpoints, std::vector<unsigned short>& pnm,
                                    std::vector<unsigned short>& denoisedPnm);
+  // The same sweep with temporal accumulation, in the layout of RenderCellsViewsCheckpointsPnm: the float sums and
+  // their squares, the guides of RenderCellsViewsFeatures and the motion of RenderCellsViewsMotion towards the view
+  // before each in the order of `cameras`, through b2pt_denoise_views_temporal with the default temporal and filter
+  // parameters (same checkpoint rule).
+  void RenderCellsViewsTemporalPnm(const vtkm::cont::DynamicCellSet& cellset, const vtkm::cont::CoordinateSystem& coords,
+                                   const std::vector<vtkm::rendering::Camera>& cameras,
+                                   const std::vector<int>& checkpoints, std::vector<unsigned short>& temporalPnm);
   // Adaptive sampling of the sweep (b2pt_render_views_adaptive with its default epsilon and radius): rounds is a
   // checkpoint list ending with the sample count; every pixel stops at the first round whose variance test it passes.
   // pnm: [view][pixel] the integers of RenderCellsViewsPnm computed with each pixel's own count; counts: [view][pixel]

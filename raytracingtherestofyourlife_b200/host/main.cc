@@ -55,6 +55,11 @@
 // is none.  It works with -checkpoints, -features, -denoise and -aperture, and every other file stays byte-identical to
 // a run without -motion.  -motion with -direct, without a sweep, with -fibonacci (consecutive lattice points are a
 // golden angle apart, not neighbours) or with -adaptive / -adaptive-denoise is an error (exit 1).
+// -temporal (with -hemisphere, path-traced) also writes <stem>-temporal-<phi>-<theta>.pnm next to every radiance file
+// <stem>-<phi>-<theta>.pnm: the sweep with temporal accumulation along the motion of -motion's view chain (every view
+// towards the one before it), then the a-trous filter (b2pt_denoise_views_temporal with its default parameters),
+// written with save()'s arithmetic.  Every other file stays byte-identical to a run without -temporal.  -temporal is
+// refused where -motion is: with -direct, without a sweep, with -fibonacci or with -adaptive / -adaptive-denoise.
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
@@ -91,6 +96,7 @@ struct Options
   bool features = false;
   bool denoise = false;
   bool motion = false;
+  bool temporal = false;
   bool adaptiveGiven = false;
   std::string adaptiveArg;
   bool adaptiveDenoiseGiven = false;
@@ -142,6 +148,8 @@ Options parse(int argc, char** argv)
       o.denoise = true;
     else if (!std::strcmp(argv[i], "-motion"))
       o.motion = true;
+    else if (!std::strcmp(argv[i], "-temporal"))
+      o.temporal = true;
     else if (!std::strcmp(argv[i], "-adaptive"))
     {
       o.adaptiveGiven = true;
@@ -227,19 +235,20 @@ std::string checkDenoise(const Options& o)
   return "";
 }
 
-// Returns an error message for an unusable -motion, empty when it is usable or absent.
-std::string checkMotion(const Options& o)
+// Returns an error message for an unusable -motion or -temporal (flag: the switch, given: whether it was), empty when
+// it is usable or absent: both need the view chain of a hemisphere sweep.
+std::string checkViewChain(const Options& o, const std::string& flag, bool given)
 {
-  if (!o.motion)
+  if (!given)
     return "";
   if (o.direct)
-    return "-motion cannot be combined with -direct";
+    return flag + " cannot be combined with -direct";
   if (o.fibonacci)
-    return "-motion cannot be combined with -fibonacci (consecutive lattice points are not neighbouring views)";
+    return flag + " cannot be combined with -fibonacci (consecutive lattice points are not neighbouring views)";
   if (!o.hemi)
-    return "-motion needs -hemisphere";
+    return flag + " needs -hemisphere";
   if (o.adaptiveGiven || o.adaptiveDenoiseGiven)
-    return "-motion cannot be combined with -adaptive or -adaptive-denoise";
+    return flag + " cannot be combined with -adaptive or -adaptive-denoise";
   return "";
 }
 
@@ -572,6 +581,15 @@ int renderViews(CornellBox& cb, const Options& o, const std::vector<vtkm::render
         savePfm(viewName(stemOf(k) + "-motion", angles[v].first, angles[v].second), o.x, o.y, 3, mv);
       }
   }
+  if (o.temporal)
+  { // the same render, guides and view chain as above, accumulated over the sweep and filtered
+    std::vector<unsigned short> temporal;
+    mapper.RenderCellsViewsTemporalPnm(cb.ds.GetCellSet(), cb.coord, cameras, counts, temporal);
+    for (size_t k = 0; k < counts.size(); ++k)
+      for (size_t v = 0; v < V; ++v)
+        savePnm16(viewName(stemOf(k) + "-temporal", angles[v].first, angles[v].second), o.x, o.y,
+                  &temporal[(k * V + v) * n3]);
+  }
   return static_cast<int>(cameras.size());
 }
 
@@ -655,7 +673,9 @@ int main(int argc, char* argv[])
   if (bad.empty())
     bad = checkAdaptive(o);
   if (bad.empty())
-    bad = checkMotion(o);
+    bad = checkViewChain(o, "-motion", o.motion);
+  if (bad.empty())
+    bad = checkViewChain(o, "-temporal", o.temporal);
   if (bad.empty())
     bad = checkLens(o);
   if (!bad.empty())
