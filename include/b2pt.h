@@ -347,6 +347,32 @@ int b2pt_denoise_views_temporal(b2pt_ctx* ctx, int nViews, const float* views, i
                                 const int* checkpoints, const float* color, const float* moment2, const float* albedo,
                                 const float* normalDepth, const float* motion, const b2pt_temporal_params* temporal,
                                 const b2pt_denoise_params* denoise, uint32_t flags, void* out, float* historyOut);
+/* A view sweep rendered and temporally denoised in one call, its state kept on the device (DESIGN.md 8k).  Defined as
+ * the chain of four calls, bit for bit: with prevViews = (views[0], views[0], views[1], ..., views[nViews-2]),
+ * rf = flags & ~B2PT_FLAG_VIEWS_PNM16 and bf = flags & B2PT_BUILD_FLAGS,
+ *   colorOut, moment2Out  = b2pt_render_views_checkpoints(views, checkpoints, maxDepth, rf): float4 sums and sums of
+ *                           squares;
+ *   albedoOut, normalDepthOut = b2pt_render_views_features(views, checkpoints, bf);
+ *   motionOut             = b2pt_render_views_motion(views, prevViews, checkpoints, bf);
+ *   out, historyOut       = b2pt_denoise_views_temporal(views, checkpoints, color, moment2, albedo, normalDepth,
+ *                           motion, temporal, denoise, flags & B2PT_FLAG_VIEWS_PNM16): float4 (x_L.rgb, V_L), or
+ *                           uint16_t[3] under B2PT_FLAG_VIEWS_PNM16; float32 n.
+ * Every array is [k][view][j*W+i], K*nViews*W*H entries.  out is required when nViews > 0; every other output may be
+ * NULL and is only a copy of a buffer the call computes anyway, so one call gives a whole denoiser-dataset record
+ * (noisy sums, variance, guides, motion, denoised target).  The seed offset (b2pt_seed) and the lens (b2pt_set_lens)
+ * apply as they do to the four calls.  Each primary ray of the guides and the motion is traced once for both.
+ * Afterwards b2pt_views_device_ptr and the statistics are what b2pt_render_views_checkpoints leaves, and the context's
+ * camera and canvas are untouched.  B2PT_ERR_BAD_VALUE, before anything runs: whatever one of the four calls rejects,
+ * B2PT_FLAG_VIEWS_NORMALIZE (the sums stay raw), B2PT_FLAG_REFERENCE_STREAM, a NULL out with nViews > 0,
+ * checkpoints[K-1] > 2^24, or more than 2^30 float4 of render state (2K nViews W H).  nViews == 0 does nothing; no
+ * scene gives B2PT_ERR_STATE.  Views are denoised in chunks of whole views through b2pt_denoise_views_temporal's
+ * staging; only the requested outputs are copied to the host.  Synchronises the stream once.  The reference has no
+ * counterpart. */
+int b2pt_render_views_temporal_denoised(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
+                                        const int* checkpoints, int maxDepth, const b2pt_temporal_params* temporal,
+                                        const b2pt_denoise_params* denoise, uint32_t flags, void* out,
+                                        float* historyOut, float* colorOut, float* moment2Out, float* albedoOut,
+                                        float* normalDepthOut, float* motionOut);
 /* Parameters of b2pt_render_views_adaptive. */
 typedef struct b2pt_adaptive_params
 {

@@ -119,6 +119,9 @@ SIGNATURES = {
     "b2pt_denoise_views_temporal": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp,
                                            C.POINTER(TemporalParams), C.POINTER(DenoiseParams), C.c_uint32, _vp,
                                            _vp]),
+    "b2pt_render_views_temporal_denoised": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, _i32,
+                                                   C.POINTER(TemporalParams), C.POINTER(DenoiseParams), C.c_uint32,
+                                                   _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "b2pt_adaptive_defaults": (None, [C.POINTER(AdaptiveParams)]),
     "b2pt_render_views_adaptive": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, _i32, C.POINTER(AdaptiveParams),
                                           C.c_uint32, _vp, _vp, _vp, _vp]),
@@ -436,6 +439,28 @@ class Context:
             None if temporal is None else C.byref(temporal), None if params is None else C.byref(params), flags,
             _p(out), _p(hist)))
         return (out, hist) if history else out
+
+    def render_views_temporal_denoised(self, views, W, H, checkpoints, max_depth, temporal=None, denoise=None, flags=0,
+                                       history=False, inputs=False):
+        """b2pt_render_views_temporal_denoised: render_views_checkpoints, render_views_features, render_views_motion
+        towards the previous view and denoise_views_temporal in one call, the sweep kept on the device; bit for bit
+        that chain.  views [nViews, 10] in sweep order; temporal a TemporalParams and denoise a DenoiseParams (None:
+        the defaults).  Returns the denoised float32 [K, nViews, H*W, 4] (uint16 [K, nViews, H*W, 3] under
+        FLAG_VIEWS_PNM16); with history=True also the float32 [K, nViews, H*W] history lengths; with inputs=True also
+        (color, moment2, albedo, normal_depth, motion), each float32 [K, nViews, H*W, 4] as the four calls return
+        them."""
+        v = np.ascontiguousarray(views, np.float32).reshape(-1, 10)
+        c = np.ascontiguousarray(checkpoints, np.int32).reshape(-1)
+        K, V = c.shape[0], v.shape[0]
+        dt, ch = (np.uint16, 3) if flags & FLAG_VIEWS_PNM16 else (np.float32, 4)
+        out = np.empty((K, V, W * H, ch), dt)
+        hist = np.empty((K, V, W * H), np.float32) if history else None
+        ins = tuple(np.empty((K, V, W * H, 4), np.float32) for _ in range(5)) if inputs else (None,) * 5
+        _check(lib().b2pt_render_views_temporal_denoised(
+            self._h, V, _p(v), W, H, K, _p(c), max_depth, None if temporal is None else C.byref(temporal),
+            None if denoise is None else C.byref(denoise), flags, _p(out), _p(hist), *(_p(a) for a in ins)))
+        res = (out,) + ((hist,) if history else ()) + ((ins,) if inputs else ())
+        return res[0] if len(res) == 1 else res
 
     def render_views_adaptive(self, views, W, H, rounds, max_depth, params=None, flags=0):
         """b2pt_render_views_adaptive: round 0 renders rounds[0] samples of every pixel, and after round k every pixel

@@ -8,6 +8,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <string>
 #include <limits>
 #include <vector>
@@ -2749,51 +2750,9 @@ void b2pt_temporal_defaults(b2pt_temporal_params* p)
   p->depthTol = 0.05f;
 }
 
-// Temporal accumulation of a sweep, then b2pt_denoise_views' filter (DESIGN.md 8j).  Views run in chunks of whole
-// views through b2pt_denoise_views' staging plus the motion and history buffers: per chunk, K host-to-device copies of
-// each input, the prep, one k_temporal launch per view in sweep order (view v reads view v-1's unfiltered result: the
-// view before it in the chunk, or for the chunk's first view the state carried over from the previous chunk), the
-// carry of the chunk's last view, the a-trous levels and the copies of the result and the history.  Every slice is its
-// own chain and every pixel's result depends only on its inputs and the previous view's state, so the result does not
-// depend on the chunking.
-int b2pt_denoise_views_temporal(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
-                                const int* checkpoints, const float* color, const float* moment2, const float* albedo,
-                                const float* normalDepth, const float* motion, const b2pt_temporal_params* temporal,
-                                const b2pt_denoise_params* denoise, uint32_t flags, void* out, float* historyOut)
+// b2pt_denoise_views_temporal's checks of its temporal parameters (fn: the entry point named in the messages).
+static int check_temporal_params(const char* fn, const b2pt_temporal_params& T)
 {
-  static const char* const fn = "b2pt_denoise_views_temporal";
-  if (int rc = bind(ctx))
-    return rc;
-  if (nViews < 0)
-    return fail(B2PT_ERR_BAD_VALUE, "%s: negative view count", fn);
-  if (int rc = check_checkpoints(fn, nCheckpoints, checkpoints))
-    return rc;
-  if (!color || !albedo || !normalDepth || !out)
-    return fail(B2PT_ERR_BAD_VALUE, "%s: color, albedo, normalDepth and out must not be NULL", fn);
-  if (W <= 0 || H <= 0)
-    return fail(B2PT_ERR_BAD_VALUE, "%s: W and H must be positive", fn);
-  b2pt_denoise_params P;
-  if (denoise)
-    P = *denoise;
-  else
-    b2pt_denoise_defaults(&P);
-  if (int rc = check_denoise_params(fn, P))
-    return rc;
-  if (flags & ~B2PT_FLAG_VIEWS_PNM16)
-    return fail(B2PT_ERR_BAD_VALUE, "%s: flags may only hold VIEWS_PNM16", fn);
-  const int K = nCheckpoints;
-  const int64_t N = (int64_t)W * H, KN = N * K;
-  if (KN > ((int64_t)1 << 30))
-    return fail(B2PT_ERR_BAD_VALUE, "%s: one view's %d slices exceed 2^30 float4", fn, K);
-  if (int rc = check_view_list(fn, nViews, views))
-    return rc;
-  if (nViews > 0 && !motion)
-    return fail(B2PT_ERR_BAD_VALUE, "%s: NULL motion", fn);
-  b2pt_temporal_params T;
-  if (temporal)
-    T = *temporal;
-  else
-    b2pt_temporal_defaults(&T);
   if (!(T.alpha > 0.f && T.alpha <= 1.f))
     return fail(B2PT_ERR_BAD_VALUE, "%s: alpha must be in (0,1], got %g", fn, (double)T.alpha);
   if (!(T.minVisible >= 0.f && T.minVisible <= 1.f))
@@ -2803,16 +2762,27 @@ int b2pt_denoise_views_temporal(b2pt_ctx* ctx, int nViews, const float* views, i
   for (int s = 0; s < 3; ++s)
     if (!(tol[s] > 0.f)) // NaN fails too
       return fail(B2PT_ERR_BAD_VALUE, "%s: %s must be > 0 (or +inf), got %g", fn, tolName[s], (double)tol[s]);
-  std::vector<B2Camera> cams;
-  if (int rc = make_view_cameras(nViews, views, W, H, cams))
-    return rc;
-  if (nViews == 0)
-    return B2PT_OK;
-  const bool pnm = (flags & B2PT_FLAG_VIEWS_PNM16) != 0;
+  return B2PT_OK;
+}
+
+// Temporal accumulation of a sweep, then b2pt_denoise_views' filter (DESIGN.md 8j), for b2pt_denoise_views_temporal
+// and b2pt_render_views_temporal_denoised once their arguments are checked.  Views run in chunks of whole views through
+// b2pt_denoise_views' staging plus the motion and history buffers: per chunk, stage(v0, nv, n) puts the inputs of views
+// [v0, v0+nv) into dnX[0] (colour sums), dnX[1] (sums of squares, when moments), dnGuideA, dnGuideNZ and tmMotion,
+// [k][chunk view][pixel] with n = nv*W*H entries per slice; then the prep, one k_temporal launch per view in sweep
+// order (view v reads view v-1's unfiltered result: the view before it in the chunk, or for the chunk's first view the
+// state carried over from the previous chunk), the carry of the chunk's last view, the a-trous levels and the copies of
+// the result and the history.  Every slice is its own chain and every pixel's result depends only on its inputs and the
+// previous view's state, so the result does not depend on the chunking.  Does not synchronise.
+static int temporal_sweep(b2pt_ctx* ctx, const std::vector<B2Camera>& cams, int W, int H, int K, const int* checkpoints,
+                          bool moments, const b2pt_temporal_params& T, const b2pt_denoise_params& P, bool pnm, void* out,
+                          float* historyOut, const std::function<int(int64_t v0, int nv, int64_t n)>& stage)
+{
+  const int64_t nViews = (int64_t)cams.size(), N = (int64_t)W * H, KN = N * K;
   b2pt::DenoiseArgs a{};
   a.n = K;
   std::copy(checkpoints, checkpoints + K, a.count);
-  a.hasMoments = moment2 != nullptr;
+  a.hasMoments = moments;
   a.sigmaLum = P.sigmaLum, a.sigmaAlbedo = P.sigmaAlbedo, a.sigmaNormal = P.sigmaNormal, a.sigmaDepth = P.sigmaDepth;
   b2pt::TemporalArgs t{};
   t.alpha = T.alpha, t.minVisible = T.minVisible, t.normalTol = T.normalTol, t.albedoTol = T.albedoTol;
@@ -2834,18 +2804,14 @@ int b2pt_denoise_views_temporal(b2pt_ctx* ctx, int nViews, const float* views, i
   }
   if (pnm)
     CU(ctx->pnm.reserve(cap * 3));
-  const float* const in[5] = { color, moment2, albedo, normalDepth, motion };
-  float4* const stage[5] = { ctx->dnX[0].p, ctx->dnX[1].p, ctx->dnGuideA.p, ctx->dnGuideNZ.p, ctx->tmMotion.p };
   for (int64_t v0 = 0; v0 < nViews; v0 += perChunk)
   {
     const int nv = (int)std::min<int64_t>(perChunk, nViews - v0);
     const int64_t n = nv * N; // one slice of the chunk
-    for (int b = 0; b < 5; ++b)
-      for (int k = 0; in[b] && k < K; ++k)
-        CU(cudaMemcpyAsync(stage[b] + k * n, in[b] + 4 * (size_t)((k * (int64_t)nViews + v0) * N),
-                           sizeof(float4) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    if (int rc = stage(v0, nv, n))
+      return rc;
     a.nViews = nv;
-    CU(b2pt::launch_denoise_prep(ctx->dnX[0].p, moment2 ? ctx->dnX[1].p : nullptr, ctx->dnGuideA.p, ctx->dnGuideNZ.p,
+    CU(b2pt::launch_denoise_prep(ctx->dnX[0].p, moments ? ctx->dnX[1].p : nullptr, ctx->dnGuideA.p, ctx->dnGuideNZ.p,
                                  (int)N, a, ctx->stream));
     for (int v = 0; v < nv; ++v)
     {
@@ -2890,7 +2856,7 @@ int b2pt_denoise_views_temporal(b2pt_ctx* ctx, int nViews, const float* views, i
       CU(b2pt::launch_pnm16(res, n * K, 1, ctx->pnm.p, ctx->stream));
     for (int k = 0; k < K; ++k)
     {
-      const size_t dst = (size_t)((k * (int64_t)nViews + v0) * N);
+      const size_t dst = (size_t)((k * nViews + v0) * N);
       if (pnm)
         CU(cudaMemcpyAsync(static_cast<uint16_t*>(out) + 3 * dst, ctx->pnm.p + 3 * k * n, sizeof(uint16_t) * 3 * (size_t)n,
                            cudaMemcpyDeviceToHost, ctx->stream));
@@ -2902,6 +2868,187 @@ int b2pt_denoise_views_temporal(b2pt_ctx* ctx, int nViews, const float* views, i
                            ctx->stream));
     }
   }
+  return B2PT_OK;
+}
+
+// temporal_sweep over the caller's host arrays: per chunk, K host-to-device copies of each input into the staging.
+int b2pt_denoise_views_temporal(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
+                                const int* checkpoints, const float* color, const float* moment2, const float* albedo,
+                                const float* normalDepth, const float* motion, const b2pt_temporal_params* temporal,
+                                const b2pt_denoise_params* denoise, uint32_t flags, void* out, float* historyOut)
+{
+  static const char* const fn = "b2pt_denoise_views_temporal";
+  if (int rc = bind(ctx))
+    return rc;
+  if (nViews < 0)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: negative view count", fn);
+  if (int rc = check_checkpoints(fn, nCheckpoints, checkpoints))
+    return rc;
+  if (!color || !albedo || !normalDepth || !out)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: color, albedo, normalDepth and out must not be NULL", fn);
+  if (W <= 0 || H <= 0)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: W and H must be positive", fn);
+  b2pt_denoise_params P;
+  if (denoise)
+    P = *denoise;
+  else
+    b2pt_denoise_defaults(&P);
+  if (int rc = check_denoise_params(fn, P))
+    return rc;
+  if (flags & ~B2PT_FLAG_VIEWS_PNM16)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: flags may only hold VIEWS_PNM16", fn);
+  const int K = nCheckpoints;
+  const int64_t N = (int64_t)W * H, KN = N * K;
+  if (KN > ((int64_t)1 << 30))
+    return fail(B2PT_ERR_BAD_VALUE, "%s: one view's %d slices exceed 2^30 float4", fn, K);
+  if (int rc = check_view_list(fn, nViews, views))
+    return rc;
+  if (nViews > 0 && !motion)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: NULL motion", fn);
+  b2pt_temporal_params T;
+  if (temporal)
+    T = *temporal;
+  else
+    b2pt_temporal_defaults(&T);
+  if (int rc = check_temporal_params(fn, T))
+    return rc;
+  std::vector<B2Camera> cams;
+  if (int rc = make_view_cameras(nViews, views, W, H, cams))
+    return rc;
+  if (nViews == 0)
+    return B2PT_OK;
+  const float* const in[5] = { color, moment2, albedo, normalDepth, motion };
+  auto upload = [&](int64_t v0, int, int64_t n) -> int {
+    float4* const stage[5] = { ctx->dnX[0].p, ctx->dnX[1].p, ctx->dnGuideA.p, ctx->dnGuideNZ.p, ctx->tmMotion.p };
+    for (int b = 0; b < 5; ++b)
+      for (int k = 0; in[b] && k < K; ++k)
+        CU(cudaMemcpyAsync(stage[b] + k * n, in[b] + 4 * (size_t)((k * (int64_t)nViews + v0) * N),
+                           sizeof(float4) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    return B2PT_OK;
+  };
+  if (int rc = temporal_sweep(ctx, cams, W, H, K, checkpoints, moment2 != nullptr, T, P,
+                              (flags & B2PT_FLAG_VIEWS_PNM16) != 0, out, historyOut, upload))
+    return rc;
+  CU(cudaStreamSynchronize(ctx->stream));
+  return B2PT_OK;
+}
+
+// A sweep rendered and temporally denoised in one call (DESIGN.md 8k): b2pt_render_views_checkpoints,
+// b2pt_render_views_features, b2pt_render_views_motion towards the previous view and b2pt_denoise_views_temporal, with
+// the sweep's state kept on the device.  The render keeps its snapshots (ckptSnap, viewColor) and sums of squares
+// (ckptMoment), slices nViews*W*H apart; per chunk of temporal_sweep, k_view_guides_motion writes the guide and motion
+// sums straight into the staging and K device-to-device copies per buffer stage the colour sums and their squares.
+// Only the requested outputs cross to the host, and the stream is synchronised once.
+int b2pt_render_views_temporal_denoised(b2pt_ctx* ctx, int nViews, const float* views, int W, int H, int nCheckpoints,
+                                        const int* checkpoints, int maxDepth, const b2pt_temporal_params* temporal,
+                                        const b2pt_denoise_params* denoise, uint32_t flags, void* out,
+                                        float* historyOut, float* colorOut, float* moment2Out, float* albedoOut,
+                                        float* normalDepthOut, float* motionOut)
+{
+  static const char* const fn = "b2pt_render_views_temporal_denoised";
+  if (int rc = bind(ctx))
+    return rc;
+  if (int rc = check_view_list(fn, nViews, views))
+    return rc;
+  if (int rc = check_checkpoints(fn, nCheckpoints, checkpoints))
+    return rc;
+  if (checkpoints[nCheckpoints - 1] > (1 << 24))
+    return fail(B2PT_ERR_BAD_VALUE, "%s: more than 2^24 samples (the hit count must stay an exact float)", fn);
+  if (maxDepth < 1 || maxDepth > 4096)
+    return fail(B2PT_ERR_BAD_VALUE, "maxDepth must be in [1,4096]");
+  if (flags & (B2PT_FLAG_REFERENCE_STREAM | B2PT_FLAG_VIEWS_NORMALIZE))
+    return fail(B2PT_ERR_BAD_VALUE, "%s: REFERENCE_STREAM and VIEWS_NORMALIZE cannot be combined with it", fn);
+  if (nViews > 0 && !out)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: NULL out", fn);
+  if (W <= 0 || H <= 0)
+    return fail(B2PT_ERR_BAD_VALUE, "%s: W and H must be positive", fn);
+  b2pt_denoise_params P;
+  if (denoise)
+    P = *denoise;
+  else
+    b2pt_denoise_defaults(&P);
+  if (int rc = check_denoise_params(fn, P))
+    return rc;
+  b2pt_temporal_params T;
+  if (temporal)
+    T = *temporal;
+  else
+    b2pt_temporal_defaults(&T);
+  if (int rc = check_temporal_params(fn, T))
+    return rc;
+  const int K = nCheckpoints;
+  const int64_t N = (int64_t)W * H, NV = N * nViews;
+  if (N * K > ((int64_t)1 << 30) || NV > ((int64_t)1 << 30) / (2 * K))
+    return fail(B2PT_ERR_BAD_VALUE, "%s: more than 2^30 float4 of render state (2K nViews W H); split the view list",
+                fn);
+  std::vector<B2Camera> cams;
+  if (int rc = make_view_cameras(nViews, views, W, H, cams))
+    return rc;
+  if (nViews == 0)
+    return B2PT_OK;
+  if (!ctx->haveScene)
+    return fail(B2PT_ERR_STATE, "%s before b2pt_set_scene", fn);
+
+  b2pt::CheckpointArgs ck{};
+  ck.n = K;
+  std::copy(checkpoints, checkpoints + K, ck.count);
+  const std::vector<B2Lens> lenses = make_view_lenses(ctx, views, cams);
+  const uint32_t renderFlags = flags & ~(uint32_t)B2PT_FLAG_VIEWS_PNM16;
+  if (int rc = render_view_sweep(ctx, cams, lenses, ck.count, K, maxDepth, renderFlags, &ck, nullptr, nullptr, true))
+    return rc;
+  // slice k of the colour sums: the snapshots, the last one the image itself
+  auto colorSlice = [&](int k) { return k + 1 < K ? ctx->ckptSnap.p + NV * k : ctx->viewColor.p; };
+  if (colorOut)
+  {
+    if (K > 1)
+      CU(cudaMemcpyAsync(colorOut, ctx->ckptSnap.p, sizeof(float4) * (size_t)(NV * (K - 1)), cudaMemcpyDeviceToHost,
+                         ctx->stream));
+    CU(cudaMemcpyAsync(colorOut + 4 * (size_t)(NV * (K - 1)), ctx->viewColor.p, sizeof(float4) * (size_t)NV,
+                       cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  if (moment2Out)
+    CU(cudaMemcpyAsync(moment2Out, ctx->ckptMoment.p, sizeof(float4) * (size_t)(NV * K), cudaMemcpyDeviceToHost,
+                       ctx->stream));
+
+  // the guides and motion trace the structure the render used (same build flags); every view towards the one before
+  // it in sweep order, the first towards itself
+  std::vector<B2Camera> prevCams(cams.size());
+  for (size_t v = 0; v < cams.size(); ++v)
+    prevCams[v] = cams[v > 0 ? v - 1 : 0];
+  CU(ctx->dViews.reserve(2 * (size_t)nViews));
+  CU(cudaMemcpyAsync(ctx->dViews.p, cams.data(), sizeof(B2Camera) * (size_t)nViews, cudaMemcpyHostToDevice,
+                     ctx->stream));
+  CU(cudaMemcpyAsync(ctx->dViews.p + nViews, prevCams.data(), sizeof(B2Camera) * (size_t)nViews,
+                     cudaMemcpyHostToDevice, ctx->stream));
+  if (int rc = upload_lenses(ctx, lenses))
+    return rc;
+  b2pt::FeatureCheckpoints fk{};
+  fk.n = K;
+  std::copy(checkpoints, checkpoints + K, fk.count);
+  float* const guideOut[3] = { albedoOut, normalDepthOut, motionOut };
+  auto fromDevice = [&](int64_t v0, int nv, int64_t n) -> int {
+    float4* const guide[3] = { ctx->dnGuideA.p, ctx->dnGuideNZ.p, ctx->tmMotion.p };
+    CU(b2pt::launch_view_guides_motion(ctx->useBvh ? nullptr : &ctx->small, ctx->useBvh ? &ctx->bvh : nullptr,
+                                       ctx->dViews.p + v0, ctx->dViews.p + nViews + v0, nv, (int)N, ctx->seedOffset,
+                                       fk, guide[0], guide[1], guide[2], ctx->stream,
+                                       lenses.empty() ? nullptr : ctx->dLens.p + v0));
+    for (int k = 0; k < K; ++k)
+    {
+      const size_t src = (size_t)(NV * k + v0 * N);
+      CU(cudaMemcpyAsync(ctx->dnX[0].p + k * n, colorSlice(k) + v0 * N, sizeof(float4) * (size_t)n,
+                         cudaMemcpyDeviceToDevice, ctx->stream));
+      CU(cudaMemcpyAsync(ctx->dnX[1].p + k * n, ctx->ckptMoment.p + src, sizeof(float4) * (size_t)n,
+                         cudaMemcpyDeviceToDevice, ctx->stream));
+      for (int b = 0; b < 3; ++b) // before the prep turns the guide sums into guides
+        if (guideOut[b])
+          CU(cudaMemcpyAsync(guideOut[b] + 4 * src, guide[b] + k * n, sizeof(float4) * (size_t)n,
+                             cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    return B2PT_OK;
+  };
+  if (int rc = temporal_sweep(ctx, cams, W, H, K, checkpoints, true, T, P, (flags & B2PT_FLAG_VIEWS_PNM16) != 0, out,
+                              historyOut, fromDevice))
+    return rc;
   CU(cudaStreamSynchronize(ctx->stream));
   return B2PT_OK;
 }

@@ -29,6 +29,7 @@
 //                                 the primary-ray kernels with every camera ray through a thin lens (b2pt_set_lens).
 //   k_view_motion<Scene,LENS>     per (view, pixel): motion vectors and disocclusion of its primary hits towards a
 //                                 previous camera (a projection and one visibility trace per hit), at chosen counts.
+//   k_view_guides_motion<Scene,LENS>  k_view_features' and k_view_motion's sums from one trace of each primary ray.
 //   k_temporal                    per (slice, pixel) of one view: temporal accumulation of a sweep, the previous
 //                                 view's unfiltered result reprojected along the motion sums (one launch per view).
 //   k_create_rays, k_intersect, k_normalize, k_pnm16, k_fill_seeds, k_sum_peers: stage-level API kernels.
@@ -2173,6 +2174,88 @@ __global__ void __launch_bounds__(256)
   }
 }
 
+// k_view_features and k_view_motion in one pass (b2pt_render_views_temporal_denoised): every sample's primary ray is
+// traced once, and its hit feeds add_feature_sample's albedo / normal-depth sums and k_view_motion's (motion.x,
+// motion.y, visible, valid) sums.  Each sum is the same float32 operations in the same sample order as in those
+// kernels, so the three outputs hold their bits; they are stored at every checkpoint as k_view_features stores its.
+template <class SceneT, bool LENS>
+__global__ void __launch_bounds__(256)
+  k_view_guides_motion(const __grid_constant__ SceneT scene, const B2Camera* __restrict__ cams,
+                       const B2Camera* __restrict__ prevCams, int64_t n, uint32_t nPixels, uint32_t divMagic,
+                       uint32_t divShift, uint32_t seedOffset, const __grid_constant__ FeatureCheckpoints ck,
+                       float4* albedoOut, float4* normalDepthOut, float4* motionOut, const B2Lens* __restrict__ lenses)
+{
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n)
+    return;
+  const uint32_t view = fastdiv((uint32_t)idx, divMagic, divShift);
+  const int p = (int)((uint32_t)idx - view * nPixels);
+  const B2Camera cam = cams[view], prev = prevCams[view];
+  B2Lens lens;
+  if constexpr (LENS)
+    lens = lenses[view];
+  const f3 pos = ld3(cam.pos), prevPos = ld3(prev.pos);
+  const float W = (float)cam.W, H = (float)cam.H;
+  float4 alb = make_float4(0.f, 0.f, 0.f, 0.f), nd = alb, mot = alb;
+  const int last = ck.count[ck.n - 1];
+  int k = 0, next = ck.count[0];
+  for (int s = 0; s < last; ++s)
+  {
+    uint32_t rng = (uint32_t)p + seedOffset + (uint32_t)s * B2PT_GOLDEN;
+    f3 o = pos, d = raygen(cam, p, rng);
+    if constexpr (LENS)
+      lens_ray(cam, lens, d, rng, o, d);
+    Hit hit;
+    f3 a = mk3(0.f, 0.f, 0.f), nrm = a;
+    float h = 0.f, t = 0.f;
+    if (trace(scene, o, d, 0.001f, FLT_MAX, hit))
+    {
+      a = hit.kind == 2 ? mk3(1.f, 1.f, 1.f)
+        : hit.kind == 1 ? mk3(fminf(fmaxf(hit.alb.x, 0.f), 1.f), fminf(fmaxf(hit.alb.y, 0.f), 1.f),
+                              fminf(fmaxf(hit.alb.z, 0.f), 1.f))
+                        : hit.alb;
+      nrm = hit.n;
+      h = 1.f;
+      t = hit.t;
+      const f3 X = o + d * hit.t;
+      float x, y, xp, yp;
+      const float w = project(cam, X, x, y);
+      const float wp = project(prev, X, xp, yp);
+      if (w > 0.f && wp > 0.f)
+      {
+        float visible = 0.f;
+        if (xp >= 0.f && xp < W && yp >= 0.f && yp < H)
+        {
+          f3 e = X - prevPos;
+          if (e.x == 0.f)
+            e.x += 0.0000001f;
+          if (e.y == 0.f)
+            e.y += 0.0000001f;
+          if (e.z == 0.f)
+            e.z += 0.0000001f;
+          const float L = sqrtf(dot3(e, e));
+          e = mk3(e.x / L, e.y / L, e.z / L);
+          Hit occ;
+          if (!trace(scene, prevPos, e, 0.001f, FLT_MAX, occ) || occ.t >= L * 0.999755859375f)
+            visible = 1.f;
+        }
+        mot.x += xp - x, mot.y += yp - y, mot.z += visible, mot.w += 1.f;
+      }
+    }
+    alb.x += a.x, alb.y += a.y, alb.z += a.z, alb.w += h;
+    nd.x += nrm.x, nd.y += nrm.y, nd.z += nrm.z, nd.w += t;
+    if (s + 1 == next)
+    {
+      const int64_t e = (int64_t)k * n + idx;
+      albedoOut[e] = alb;
+      normalDepthOut[e] = nd;
+      motionOut[e] = mot;
+      ++k;
+      next = k < ck.n ? ck.count[k] : 0;
+    }
+  }
+}
+
 // pathtracing/Camera.cxx:894-953: fills + RayGen + origin broadcast, fused.
 __global__ void __launch_bounds__(256)
   k_create_rays(const __grid_constant__ B2Camera cam, uint32_t* seeds, float* dx, float* dy, float* dz, float* ox,
@@ -2924,6 +3007,33 @@ cudaError_t launch_view_motion(const B2SmallScene* small, const B2BvhScene* bvh,
     else
       k_view_motion<SceneT, false><<<grid, 256, 0, stream>>>(S, cams, prevCams, n, (uint32_t)nPixels, magic, shift,
                                                              seedOffset, ck, motion, nullptr);
+  });
+  return cudaGetLastError();
+}
+
+cudaError_t launch_view_guides_motion(const B2SmallScene* small, const B2BvhScene* bvh, const B2Camera* cams,
+                                      const B2Camera* prevCams, int nViews, int nPixels, uint32_t seedOffset,
+                                      const FeatureCheckpoints& ck, float4* albedo, float4* normalDepth,
+                                      float4* motion, cudaStream_t stream, const B2Lens* lenses)
+{
+  const int64_t n = (int64_t)nViews * nPixels;
+  if (n <= 0)
+    return cudaSuccess;
+  if (n > 0xffffffffLL || ck.n < 1 || ck.n > kMaxCheckpoints)
+    return cudaErrorInvalidValue;
+  uint32_t magic, shift;
+  make_fastdiv((uint32_t)nPixels, magic, shift);
+  const unsigned grid = (unsigned)((n + 255) / 256);
+  with_trace_scene(small, bvh, [&](const auto& S) {
+    using SceneT = std::decay_t<decltype(S)>;
+    if (lenses)
+      k_view_guides_motion<SceneT, true><<<grid, 256, 0, stream>>>(S, cams, prevCams, n, (uint32_t)nPixels, magic,
+                                                                   shift, seedOffset, ck, albedo, normalDepth, motion,
+                                                                   lenses);
+    else
+      k_view_guides_motion<SceneT, false><<<grid, 256, 0, stream>>>(S, cams, prevCams, n, (uint32_t)nPixels, magic,
+                                                                    shift, seedOffset, ck, albedo, normalDepth,
+                                                                    motion, nullptr);
   });
   return cudaGetLastError();
 }

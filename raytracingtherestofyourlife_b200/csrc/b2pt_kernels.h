@@ -137,6 +137,12 @@ cudaError_t launch_view_motion(const B2SmallScene* small, const B2BvhScene* bvh,
                                const B2Camera* prevCams, int nViews, int nPixels, uint32_t seedOffset,
                                const FeatureCheckpoints& ck, float4* motion, cudaStream_t stream,
                                const B2Lens* lenses = nullptr);
+// launch_view_features and launch_view_motion in one pass (k_view_guides_motion): each sample's primary ray traced
+// once, the three outputs (all required) hold the bits the two launches store.
+cudaError_t launch_view_guides_motion(const B2SmallScene* small, const B2BvhScene* bvh, const B2Camera* cams,
+                                      const B2Camera* prevCams, int nViews, int nPixels, uint32_t seedOffset,
+                                      const FeatureCheckpoints& ck, float4* albedo, float4* normalDepth,
+                                      float4* motion, cudaStream_t stream, const B2Lens* lenses = nullptr);
 // Spatial denoiser of b2pt_denoise_views over one chunk of nImages = K * nViews images of W x H pixels, stored
 // [k][view][pixel] (image z = k * nViews + v; its checkpoint count is count[z / nViews]).
 // launch_denoise_prep: in place, x (color sums in, (m, V0) out), moment (sums of squares, may be null; read only),

@@ -544,25 +544,22 @@ void MapperPathTracer::RenderCellsViewsTemporalPnm(const vtkm::cont::DynamicCell
     temporalPnm.clear();
     return;
   }
-  std::vector<float> color, moment2, albedo, normalDepth, motion;
-  const size_t n = static_cast<size_t>(Internals->Canvas->GetWidth()) * Internals->Canvas->GetHeight();
-  const size_t n4 = checkpoints.size() * cameras.size() * n * 4;
-  color.assign(n4, 0.f);
-  moment2.assign(n4, 0.f);
-  RenderViewsImpl(cellset, coords, cameras, 0, color.data(), &checkpoints, moment2.data());
-  RenderCellsViewsFeatures(cellset, coords, cameras, checkpoints, albedo, normalDepth);
-  // every view towards the one before it in sweep order (the first towards itself; its motion is not read)
-  std::vector<vtkm::rendering::Camera> prevCameras(cameras.begin(), cameras.end() - 1);
-  prevCameras.insert(prevCameras.begin(), cameras.front());
-  RenderCellsViewsMotion(cellset, coords, cameras, prevCameras, checkpoints, motion);
-  const std::vector<float> views = packViews(cameras);
-  b2pt_ctx* ctx = b2pt_facade::Context();
-  const int V = static_cast<int>(cameras.size()), K = static_cast<int>(checkpoints.size());
+  // one call: the render, its guides, the motion of every view towards the one before it in sweep order, and the
+  // temporal denoiser, with nothing but the result copied to the host
+  const std::vector<float> views = PrepareSweep(cellset, coords, cameras);
   const int nx = static_cast<int>(Internals->Canvas->GetWidth()), ny = static_cast<int>(Internals->Canvas->GetHeight());
-  temporalPnm.assign(n4 / 4 * 3, 0);
-  b2pt_facade::Check(b2pt_denoise_views_temporal(ctx, V, views.data(), nx, ny, K, checkpoints.data(), color.data(),
-                                                 moment2.data(), albedo.data(), normalDepth.data(), motion.data(),
-                                                 nullptr, nullptr, B2PT_FLAG_VIEWS_PNM16, temporalPnm.data(), nullptr));
+  temporalPnm.assign(checkpoints.size() * cameras.size() * static_cast<size_t>(nx) * ny * 3, 0);
+  b2pt_ctx* ctx = b2pt_facade::Context();
+  b2pt_facade::Check(b2pt_seed(ctx, 0)); // the streams RenderCellsViews* render with
+  b2pt_facade::Check(b2pt_set_lens(ctx, LensAperture, LensFocus));
+  b2pt_facade::Check(b2pt_render_views_temporal_denoised(
+    ctx, static_cast<int>(cameras.size()), views.data(), nx, ny, static_cast<int>(checkpoints.size()),
+    checkpoints.data(), depthcount, nullptr, nullptr, RenderFlags | B2PT_FLAG_VIEWS_PNM16, temporalPnm.data(), nullptr,
+    nullptr, nullptr, nullptr, nullptr, nullptr));
+  b2pt_stats st;
+  b2pt_facade::Check(b2pt_get_stats(ctx, &st));
+  LastRenderMs = st.renderMs;
+  LastSegments = st.segments;
 }
 
 void MapperPathTracer::RenderCellsViewsAdaptivePnm(const vtkm::cont::DynamicCellSet& cellset,
