@@ -4,9 +4,10 @@ Bar: the image and counts are b2pt_render_views_adaptive's bits under every view
 guides at every pixel are b2pt_render_views_features' slice at the pixel's own count, on the small scene and the three
 BVH trace paths; with levels = 0 the output is the float32 prep at each pixel's own count bit for bit, and its PNM
 integers are the adaptive image's; at tau = 0 and tau = +inf (one count everywhere) it is b2pt_denoise_views of the
-uniform sweep bit for bit; at a general tau one level and the default levels agree with the float64 restatement; the
-result does not depend on the chunking and two calls agree; it lowers the error of the adaptive image; bad inputs fail
-before anything runs; the driver's -adaptive-denoise files are the binding's."""
+uniform sweep bit for bit; at a general tau one level, the default levels and ten levels agree with the float64
+restatement, on the sweep's canvas, a 1 x 37 and a 13 x 5 one; the result does not depend on the chunking and two
+calls agree; it lowers the error of the adaptive image; bad inputs fail before anything runs; the driver's
+-adaptive-denoise files are the binding's."""
 import ctypes
 import os
 import subprocess
@@ -154,23 +155,25 @@ def test_one_count_everywhere_is_the_uniform_filter(ctx, b2pt, tau, k):
         assert np.array_equal(den.view(np.uint8), want[0].view(np.uint8)), flags
 
 
-# the tolerances of test_gpu_denoise: one level, then the default five
-@pytest.mark.parametrize("levels, tol", [(1, 1e-4), (5, 1e-3)])
+# the tolerances of test_gpu_denoise: one level, then the default five and all ten; on the sweep's canvas, one column
+# and a canvas narrower and shorter than k_atrous' 16 x 16 tile
+@pytest.mark.parametrize("levels, tol", [(1, 1e-4), (5, 1e-3), (10, 1e-3)])
 def test_general_tau_against_restatement(ctx, b2pt, cornell_tau, levels, tol):
     views = tilted_views(6)
     p = aparams(b2pt, cornell_tau)
-    S, Q, counts, _ = ctx.render_views_adaptive(views, W, H, ROUNDS, DEPTH, p)
-    _, _, den, A, ND = ctx.render_views_adaptive_denoised(views, W, H, ROUNDS, DEPTH, p, dparams(b2pt, levels),
-                                                          features=True)
-    nv = views.shape[0]
-    img = lambda a: a.astype(np.float64).reshape((nv, H, W) + a.shape[2:])
-    x, V, ga, gn, z = (img(a) for a in per_pixel_prep(S, Q, A, ND, counts))
-    d = R.DEFAULTS
-    for lev in range(levels):
-        x, V = R.atrous_level(x, V, ga, gn, z, H, W, 1 << lev, True, d["sigma_lum"], d["sigma_albedo"],
-                              d["sigma_normal"], d["sigma_depth"])
-    e = rel_err(den[None, ..., :3], x.reshape(1, nv, H * W, 3))
-    assert e < tol, (levels, e)
+    for w, h in ((W, H), (1, 37), (13, 5)):
+        S, Q, counts, _ = ctx.render_views_adaptive(views, w, h, ROUNDS, DEPTH, p)
+        _, _, den, A, ND = ctx.render_views_adaptive_denoised(views, w, h, ROUNDS, DEPTH, p, dparams(b2pt, levels),
+                                                              features=True)
+        nv = views.shape[0]
+        img = lambda a: a.astype(np.float64).reshape((nv, h, w) + a.shape[2:])
+        x, V, ga, gn, z = (img(a) for a in per_pixel_prep(S, Q, A, ND, counts))
+        d = R.DEFAULTS
+        for lev in range(levels):
+            x, V = R.atrous_level(x, V, ga, gn, z, h, w, 1 << lev, True, d["sigma_lum"], d["sigma_albedo"],
+                                  d["sigma_normal"], d["sigma_depth"])
+        e = rel_err(den[None, ..., :3], x.reshape(1, nv, h * w, 3))
+        assert e < tol, (w, h, levels, e)
 
 
 def test_chunking_and_determinism(ctx, b2pt, cornell_tau):

@@ -3,7 +3,9 @@
 Bar: with levels = 0 the output is the mean bit for bit, and its PNM integers are those of
 b2pt_render_views_checkpoints(PNM16); one level and the default levels agree with the float64 restatement
 (tests/denoise_ref.py) within a stated tolerance, on synthetic inputs with hard edges, misses and NaNs and on rendered
-sweeps, with and without sums of squares; every image is filtered on its own, whatever the chunking, and two calls give
+sweeps, with and without sums of squares; on synthetic canvases from 1 x 1, one column and one row up to one pixel past
+the 16 x 16 tile, levels 0 is the restatement's prep and PNM integers bit for bit and 1, 2, 5 and 10 levels agree with
+it, also with every sigma = +inf; every image is filtered on its own, whatever the chunking, and two calls give
 the same bits; the filter lowers the error against a 4096-spp target, and its guides are what keeps edges; bad inputs
 fail before anything runs; the driver's -denoise files are the binding's pipeline."""
 import ctypes
@@ -17,7 +19,7 @@ import pytest
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import denoise_ref as R  # noqa: E402
-from test_gpu_features import driver_view_names, hemisphere_positions, view_row  # noqa: E402
+from test_gpu_features import driver_view_names, hemisphere_positions, same_bits, view_row  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -82,13 +84,16 @@ def pnm_of(mean):
 
 
 def synthetic(K, V, h, w, seed=0):
-    """Noisy sums with hard edges: albedo blocks, a missed region, a depth step, a normal crease and NaN pixels."""
+    """Noisy sums with hard edges: albedo blocks, a missed corner a quarter of the canvas across, a depth step and a
+    normal crease; misses and NaN sums are scattered over the (view, pixel) pairs, so every canvas down to 1 x 1 has
+    hits, misses and NaNs."""
     rng = np.random.default_rng(seed)
     ck = np.array([3, 8][:K], np.int32)
     N = h * w
     j, i = np.divmod(np.arange(N), w)
     region = (i >= w // 3).astype(int) + (j >= h // 2).astype(int)
     base = np.array([[0.2, 0.3, 0.4], [0.9, 0.6, 0.1], [0.05, 0.05, 0.5]])[region]
+    miss = ((i < w // 4) & (j < h // 4))[None] | (np.arange(V * N).reshape(V, N) % 7 == 2)
     S = np.zeros((K, V, N, 4), np.float32)
     Q = np.zeros_like(S)
     A = np.zeros_like(S)
@@ -97,15 +102,14 @@ def synthetic(K, V, h, w, seed=0):
         samples = base[None, None, :, None, :] * rng.exponential(1.0, (1, V, N, c, 3))
         S[k, ..., :3] = samples.sum(3)
         Q[k, ..., :3] = (samples ** 2).sum(3)
-        miss = (i < 4) & (j < 4)
         hits = np.where(miss, 0, c)
-        A[k, ..., :3] = (np.array([[0.1, 0.1, 0.1], [0.7, 0.7, 0.2], [0.3, 0.3, 0.9]])[region] * hits[:, None])
+        A[k, ..., :3] = (np.array([[0.1, 0.1, 0.1], [0.7, 0.7, 0.2], [0.3, 0.3, 0.9]])[region] * hits[..., None])
         A[k, ..., 3] = hits
         nrm = np.where((i < w // 2)[:, None], [0.0, 0.0, -1.0], [0.7071, 0.0, -0.7071])
-        ND[k, ..., :3] = nrm * hits[:, None]
+        ND[k, ..., :3] = nrm * hits[..., None]
         ND[k, ..., 3] = np.where(i < 2 * w // 3, 2.0, 3.5) * hits
-    S[:, :, ::37, 1] = np.nan
-    Q[:, :, ::53, 2] = np.nan
+    S.reshape(K, V * N, 4)[:, ::37, 1] = np.nan
+    Q.reshape(K, V * N, 4)[:, ::53, 2] = np.nan
     return ck, S, Q, A, ND
 
 
@@ -140,21 +144,35 @@ def test_levels_zero_is_the_mean(ctx, b2pt, sweep):
 # difference is the rounding of the edge-stop terms, exp and the 25-tap sums.  Several levels feed each level's fp32
 # output into the next one's edge-stops, so the bound is looser; measured values are in DESIGN.md 8e.
 TOL_ONE, TOL_ALL = 1e-4, 1e-3
+# (W, H): one pixel, one column, one row, smaller than k_atrous' 16 x 16 tile, exactly one tile, one pixel past it in
+# either direction, and wider than level 6's step (32) so that level's taps land
+CANVASES = ((27, 20), (1, 1), (1, 23), (23, 1), (2, 3), (15, 17), (16, 16), (17, 16), (33, 5))
 
 
 @pytest.mark.parametrize("moments", [True, False])
 def test_synthetic_against_restatement(ctx, b2pt, moments):
-    ck, S, Q, A, ND = synthetic(2, 3, 20, 27)
-    Q = Q if moments else None
-    for levels, tol in ((1, TOL_ONE), (5, TOL_ALL)):
-        out = ctx.denoise_views(S, Q, A, ND, 27, 20, ck, params(b2pt, levels=levels))
-        x, V = R.denoise(S, Q, A, ND, 27, 20, ck, levels=levels)
-        e = rel_err(out[..., :3], x)
-        assert e < tol, (levels, e)
-        if moments:
-            assert rel_err(out[..., 3:], V[..., None]) < 10 * tol, levels
-        else:
-            assert (out[..., 3] == 0).all()
+    """On every canvas of CANVASES: levels 0 is the prep and its PNM integers bit for bit; levels 1, 2, 5 and 10
+    (steps up to 512, far wider than the image) agree with the restatement, at the default sigmas and with every sigma
+    = +inf."""
+    for w, h in CANVASES:
+        ck, S, Q, A, ND = synthetic(2, 3, h, w)
+        Q = Q if moments else None
+        m, V0, *_ = R.prep(S, Q, A, ND, ck)
+        out = ctx.denoise_views(S, Q, A, ND, w, h, ck, params(b2pt, levels=0))
+        assert same_bits(out[..., :3], m) and same_bits(out[..., 3], V0), (w, h)
+        pnm = ctx.denoise_views(S, Q, A, ND, w, h, ck, params(b2pt, levels=0), b2pt.FLAG_VIEWS_PNM16)
+        assert np.array_equal(pnm, pnm_of(m)), (w, h)
+        for sigma in (None, INF):
+            for levels, tol in ((1, TOL_ONE), (2, TOL_ALL), (5, TOL_ALL), (10, TOL_ALL)):
+                p = params(b2pt, levels, sigma, sigma, sigma, sigma)
+                out = ctx.denoise_views(S, Q, A, ND, w, h, ck, p)
+                x, V = R.denoise(S, Q, A, ND, w, h, ck, levels, sigma, sigma, sigma, sigma)
+                e = rel_err(out[..., :3], x)
+                assert e < tol, (w, h, sigma, levels, e)
+                if moments:
+                    assert rel_err(out[..., 3:], V[..., None]) < 10 * tol, (w, h, sigma, levels)
+                else:
+                    assert (out[..., 3] == 0).all()
 
 
 @pytest.mark.parametrize("moments", [True, False])

@@ -1,9 +1,11 @@
 """Temporal accumulation of a view sweep (b2pt_denoise_views_temporal, DESIGN.md 8j) on the GPU: alpha = 1 is
 b2pt_denoise_views bit for bit; levels = 0 is the float32 restatement (tests/temporal_ref.py) bit for bit on a ring of
-the driver's hemisphere and on synthetic inputs with NaN, off-canvas and exact-integer motion and hard guide edges;
-the default levels agree with denoise_ref applied to the restated history; a view chain that crosses a chunk boundary
-is still the restatement; disoccluded pixels take no history; the accumulation lowers the error against a 4096-spp
-target; bad calls fail before anything runs; the driver's -temporal files are the binding's pipeline."""
+the driver's hemisphere and on synthetic inputs with NaN, off-canvas and exact-integer motion, motion onto and just
+past the canvas' first and last columns and rows, and hard guide edges, on canvases from 1 x 1, one column and one row
+up to one pixel past the 16 x 16 tile; the default levels agree with denoise_ref applied to the restated history, and
+so do ten levels on the synthetic canvases; a view chain that crosses a chunk boundary is still the restatement;
+disoccluded pixels take no history; the accumulation lowers the error against a 4096-spp target; bad calls fail before
+anything runs; the driver's -temporal files are the binding's pipeline."""
 import ctypes
 import os
 import subprocess
@@ -15,7 +17,7 @@ import pytest
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import denoise_ref as R  # noqa: E402
 import temporal_ref as T  # noqa: E402
-from test_gpu_denoise import TOL_ALL, rel_err, rel_mse, synthetic  # noqa: E402
+from test_gpu_denoise import CANVASES, TOL_ALL, rel_err, rel_mse, synthetic  # noqa: E402
 from test_gpu_features import driver_view_names, hemisphere_positions, same_bits, view_row  # noqa: E402
 from test_gpu_motion import FRONT, right_of  # noqa: E402
 
@@ -105,19 +107,29 @@ def test_ring_levels_zero_is_the_restatement(b2pt, ring, moments):
 
 def synthetic_motion(K, V, h, w, ck, seed=0):
     """Motion sums with fractional, exact-integer, off-canvas and NaN motion, NaN sums, no valid sample and partial
-    visibility."""
+    visibility, and motion onto the canvas' edges: exactly onto the last column or row (zero fraction, so the second
+    column or row of taps is off the canvas), a little left of or above it (floorf gives -1, so the first is), and a
+    little right of or below it (the second is)."""
     rng = np.random.default_rng(seed)
     N = h * w
+    j, i = np.divmod(np.arange(N), w)
     M = np.zeros((K, V, N, 4), np.float32)
     for k, c in enumerate(ck):
         cf = np.float32(c)
         mx = rng.uniform(-1.5, 1.5, (V, N)).astype(np.float32)
         my = rng.uniform(-1.5, 1.5, (V, N)).astype(np.float32)
-        kind = rng.integers(0, 8, (V, N))
+        kind = rng.integers(0, 14, (V, N))
         mx = np.where(kind == 1, np.round(mx), mx)  # exact integers
         my = np.where(kind == 1, np.round(my), my)
         mx = np.where(kind == 2, np.float32(3 * w), mx)  # off the canvas
         my = np.where(kind == 3, np.float32(-1e30), my)
+        # every one exact in float32, and so are its sums and i + Sx / Sval
+        mx = np.where(kind == 8, (w - 1 - i).astype(np.float32), mx)
+        my = np.where(kind == 9, (h - 1 - j).astype(np.float32), my)
+        mx = np.where(kind == 10, (-0.125 - i).astype(np.float32), mx)
+        my = np.where(kind == 11, (-0.125 - j).astype(np.float32), my)
+        mx = np.where(kind == 12, (w - 1 - i + 0.375).astype(np.float32), mx)
+        my = np.where(kind == 13, (h - 1 - j + 0.375).astype(np.float32), my)
         M[k, ..., 0] = mx * cf
         M[k, ..., 1] = my * cf
         M[k, ..., 3] = cf
@@ -130,20 +142,29 @@ def synthetic_motion(K, V, h, w, ck, seed=0):
 
 @pytest.mark.parametrize("moments", [True, False])
 def test_synthetic_levels_zero_is_the_restatement(b2pt, moments):
-    ck, S, Q, A, ND = synthetic(2, 5, 20, 27)
-    Q = Q if moments else None
-    h, w = 20, 27
-    views = np.stack([view_row(FRONT, fov=40.0)] * 5)
-    M = synthetic_motion(2, 5, h, w, ck)
+    """On every canvas of test_gpu_denoise.CANVASES (at least 240 pixels of views in all): levels 0 is the restatement
+    bit for bit, and ten levels agree with it within TOL_ALL."""
+    names = dict(alpha="alpha", minVisible="min_visible", normalTol="normal_tol", albedoTol="albedo_tol",
+                 depthTol="depth_tol")
     with b2pt.Context(0) as c:
-        for tp in (dict(), dict(alpha=0.05, minVisible=0.0), dict(normalTol=INF, albedoTol=INF, depthTol=INF)):
-            out, n = c.denoise_views_temporal(S, Q, A, ND, M, views, w, h, ck, tparams(b2pt, **tp), dparams(b2pt, 0),
-                                              history=True)
-            names = dict(alpha="alpha", minVisible="min_visible", normalTol="normal_tol", albedoTol="albedo_tol",
-                         depthTol="depth_tol")
-            x, V, hn = T.temporal(S, Q, A, ND, M, views, w, h, ck, **{names[k]: v for k, v in tp.items()})
-            assert same_bits(out[..., :3], x) and same_bits(out[..., 3], V) and same_bits(n, hn), tp
-            assert (n[:, 1:] > 1).mean() > 0.1 and (n[:, 1:] == 1).mean() > 0.1, tp
+        for w, h in CANVASES:
+            nv = max(5, 240 // (w * h))
+            ck, S, Q, A, ND = synthetic(2, nv, h, w)
+            Q = Q if moments else None
+            views = np.stack([view_row(FRONT, fov=40.0)] * nv)
+            M = synthetic_motion(2, nv, h, w, ck)
+            for tp in (dict(), dict(alpha=0.05, minVisible=0.0), dict(normalTol=INF, albedoTol=INF, depthTol=INF)):
+                out, n = c.denoise_views_temporal(S, Q, A, ND, M, views, w, h, ck, tparams(b2pt, **tp),
+                                                  dparams(b2pt, 0), history=True)
+                rp = {names[k]: v for k, v in tp.items()}
+                x, V, hn = T.temporal(S, Q, A, ND, M, views, w, h, ck, **rp)
+                assert same_bits(out[..., :3], x) and same_bits(out[..., 3], V) and same_bits(n, hn), (w, h, tp)
+                assert (n[:, 1:] > 1).mean() > 0.1 and (n[:, 1:] == 1).mean() > 0.1, (w, h, tp)
+                out = c.denoise_views_temporal(S, Q, A, ND, M, views, w, h, ck, tparams(b2pt, **tp), dparams(b2pt, 10))
+                x, V = T.filtered(S, Q, A, ND, M, views, w, h, ck, rp, levels=10)
+                assert rel_err(out[..., :3], x) < TOL_ALL, (w, h, tp)
+                if moments:
+                    assert rel_err(out[..., 3:], V[..., None]) < 10 * TOL_ALL, (w, h, tp)
 
 
 def test_default_levels_against_the_restatement(b2pt, ring):
